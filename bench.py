@@ -4,6 +4,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --steps K --warmup W    # the reference's CPU torch path
+    python bench.py --steps K --dump-outputs bench_outputs   # + the last timed step's outputs as <dir>/<name>.npy
 
 One JSON line on stdout (rank 0).  A "step" is one pass of the hot path over one batch of
 synthetic sim state.  The headline keys (`value`, `e2e`, `roofline`) are measured on BASELINE.json
@@ -61,6 +62,8 @@ BYTES_PER_ENV_STEP_T = lambda T: 1248 + 54 + (T + 2) * 1248 + (358 + 576 * T) * 
 METRIC = "env_steps_per_sec"
 UNIT = "env-steps/s"
 SEED = 1234
+DUMP_BYTES = 64 * 10**6  # --dump-outputs writes at most this much, .npy headers included
+NPY_HEADER = 1024  # bound on one .npy header of these arrays (numpy writes 128 B)
 
 
 def workload_name(n, workload="config2", clips=0):
@@ -368,15 +371,19 @@ class Ring:
         self.prog0_all = [e.progress_buf.clone() for e in self.envs] if self.config4 else None
         torch.cuda.synchronize()
 
+    def rewind(self):
+        """Every clock back to where the ring started it."""
+        if self.config4:
+            for e, p0 in zip(self.envs, self.prog0_all):
+                e.progress_buf.copy_(p0)
+        else:
+            self.first.progress_buf.copy_(self.progress0)
+
     def run_steps(self, k):
         R = self.R
         for i in range(k):
-            if self.config4:
-                if i >= R and i % R == 0:  # every lap: each slot's clock back to its start
-                    for e, p0 in zip(self.envs, self.prog0_all):
-                        e.progress_buf.copy_(p0)
-            elif i % R == 0:
-                self.first.progress_buf.copy_(self.progress0)  # re-seed the clock at every lap of the ring
+            if i % R == 0 and (i >= R or not self.config4):  # re-seed the clocks at every lap (config4: from the 2nd)
+                self.rewind()
             self.envs[i % R].post_physics_step(True)
 
     def free(self):
@@ -453,6 +460,36 @@ def measure_steps(ctx, ring, K, reps, label):
         out["frac_dram"] = traffic / (us * 1e-6) / 1e9 / ctx.peak
     del graph
     return out
+
+
+def dump_outputs(ring, K, out_dir):
+    """--dump-outputs: what the last of the K timed steps hands its caller — ``obs``, ``reward``, ``reward_raw``,
+    ``reset`` and ``terminate`` (HumanoidPHC.step's obs_buf, rew_buf, reward_raw, reset_buf, extras["terminate"]) — as
+    float32 ``<name>.npy`` files, so that two builds can be compared output for output.  The K steps are run once more
+    from the ring's starting clocks first: config4's clocks move on from one graph replay to the next, so what the
+    timing leaves behind would depend on how many replays it took.  (So with config4 the measurements after this one
+    start from the ring's starting clocks, not from where the timed replays left them: the frames they gather differ,
+    the work per step does not.)  Above DUMP_BYTES in all, a fixed seeded sample of env rows is written, and
+    ``env_index.npy`` (float64) names them."""
+    import numpy as np
+
+    ring.rewind()
+    ring.run_steps(K)
+    env = ring.envs[(K - 1) % ring.R]
+    outs = {"obs": env.obs_buf, "reward": env.rew_buf, "reward_raw": env.reward_raw, "reset": env.reset_buf,
+            "terminate": env._terminate_out}  # fmt: skip
+    outs = {k: v.float().cpu() for k, v in outs.items()}
+    row_bytes = sum(v[0].numel() for v in outs.values()) * 4
+    if ring.N * row_bytes + len(outs) * NPY_HEADER > DUMP_BYTES:
+        keep = (DUMP_BYTES - (len(outs) + 1) * NPY_HEADER) // (row_bytes + 8)
+        rows = torch.randperm(ring.N, generator=torch.Generator().manual_seed(SEED))[:keep].sort().values
+        outs = {k: v[rows] for k, v in outs.items()}
+        outs["env_index"] = rows.double()
+    os.makedirs(out_dir, exist_ok=True)
+    paths = [os.path.join(out_dir, k + ".npy") for k in outs]
+    for path, v in zip(paths, outs.values()):
+        np.save(path, v.numpy())
+    assert sum(os.path.getsize(p) for p in paths) <= DUMP_BYTES, "--dump-outputs exceeded its size bound"
 
 
 def make_running_norms(ctx, obs_dim):
@@ -693,6 +730,8 @@ def run_gpu(args):
     main = measure_steps(ctx, ring, K, reps, "step_kernel" if args.workload == "config2" else args.workload)
     ms_per_step = main["us_per_step"] * 1e-3
     frac_term = float(ring.envs[(K - 1) % ring.R]._terminate_buf.float().mean().item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(ring, K, args.dump_outputs)
     long_run = None
     if K < 256 and not args.no_long_run:  # the same measurement over a longer timed region (512 steps per replay)
         lr = measure_steps(ctx, ring, 512, args.repeats, "step_kernel")
@@ -939,7 +978,14 @@ def main():
     ap.add_argument("--no-torch-cuda-baseline", action="store_true")
     ap.add_argument("--no-extra-configs", action="store_true", help="skip BASELINE configs 3 / 4 / 5 (the `configs` key)")
     ap.add_argument("--no-long-run", action="store_true", help="skip the 512-step re-measurement when --steps is small")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the headline's last timed step (obs, reward, reward_raw, reset, terminate; rank 0) as "
+                         "DIR/<name>.npy, at most 64 MB (64e6 bytes)")  # fmt: skip
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs; it does not apply to --impl reference")
     if args.impl == "reference":
         run_reference(args)
     else:
