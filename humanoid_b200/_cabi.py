@@ -16,7 +16,7 @@ import torch
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libphc_b200.so")
 
-ABI_VERSION = 4
+ABI_VERSION = 5
 NUM_BODIES = 24
 SELF_OBS_DIM = 358
 TASK_OBS_DIM = 576
@@ -253,6 +253,8 @@ EPISODE_SUM_COLS = 12
 PEER_MAX_WORLD = 16
 PEER_HANDLE_BYTES = 64
 PEER_TIMEOUT = -7
+PHC_ERR_BUSY = -8
+HOST_SLOTS = 2
 
 
 class PhcBuildArgs(C.Structure):
@@ -319,6 +321,8 @@ SIGNATURES = {
     ),  # fmt: skip
     "phc_host_step": (C.c_int, [C.c_void_p, C.POINTER(PhcHostStepArgs), C.c_int64]),
     "phc_host_step_destroy": (None, [C.c_void_p]),
+    "phc_host_step_submit": (C.c_int, [C.c_void_p, C.c_int32, C.POINTER(PhcHostStepArgs), C.c_int64]),
+    "phc_host_step_wait": (C.c_int, [C.c_void_p, C.c_int32]),
     "phc_host_step_path": (C.c_int, [C.c_void_p]),
     "phc_host_step_chunks": (C.c_int, [C.c_void_p]),
     "phc_host_step_tuning_calls": (C.c_int, [C.c_void_p]),

@@ -15,8 +15,13 @@
 // device->host copy of a third overlap (PCIe is full duplex; the B200 has copy engines per
 // direction).  The five small clock arrays and the five small outputs of a chunk travel as ONE
 // transfer each through pinned staging buffers owned by the context (a DMA descriptor costs a
-// few microseconds regardless of size; 22 of them per chunk were half of the step time).  The
-// call returns when every output is in the caller's host memory.
+// few microseconds regardless of size; 22 of them per chunk were half of the step time).
+//
+// Slots.  A context owns PHC_HOST_SLOTS independent pipelines, each with its own device buffers, pinned staging and
+// three streams.  phc_host_step_submit enqueues one step on a slot and returns; phc_host_step_wait waits for the
+// slot's events and, on the staged path, unpacks the scalar outputs.  With two slots the inbound copy of one batch
+// rides under the outbound traffic of the other (the slots' streams do not queue behind each other), and the caller's
+// thread is free between submit and wait.  phc_host_step is submit + wait on slot 0.
 #include <chrono>
 #include <cstdint>
 #include <cstdio>
@@ -30,6 +35,9 @@
 
 // phc_kernels.cu: phc_step_fused that also writes the advanced progress to a second address
 int step_fused_mirrored(const PhcLib* lib, const PhcStepArgs* args, int64_t n, phc_stream_t stream, int16_t* progress_mirror);
+namespace phc {
+int record_cuda_error(int cuda_error);  // phc_kernels.cu; returns PHC_ERR_CUDA
+}
 
 namespace {
 
@@ -39,8 +47,55 @@ constexpr int kStateFloats = PHC_NUM_BODIES * 13;
 constexpr size_t kClockBytes = 8 + 12 + 4 + 4 + 2;
 // packed scalars out, per env: rew f32 | raw 4 f32 | progress i16 | reset u8 | term u8
 constexpr size_t kOutBytes = 4 + 16 + 2 + 1 + 1;
+constexpr int kMaxChunks = 1024;
 
 inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
+
+// sub-array offsets inside a chunk's packed regions (each 16-B aligned)
+struct Layout {
+  size_t ids, goff, start, soff, prog, clock_bytes;
+  size_t rew, raw, oprog, reset, term, out_bytes;
+};
+Layout layout(int64_t m) {
+  Layout L;
+  size_t o = 0;
+  L.ids = o, o = align_up(o + (size_t)m * 8, 16);
+  L.goff = o, o = align_up(o + (size_t)m * 12, 16);
+  L.start = o, o = align_up(o + (size_t)m * 4, 16);
+  L.soff = o, o = align_up(o + (size_t)m * 4, 16);
+  L.prog = o, o = align_up(o + (size_t)m * 2, 16);
+  L.clock_bytes = o;
+  o = 0;
+  L.rew = o, o = align_up(o + (size_t)m * 4, 16);
+  L.raw = o, o = align_up(o + (size_t)m * 16, 16);
+  L.oprog = o, o = align_up(o + (size_t)m * 2, 16);
+  L.reset = o, o = align_up(o + (size_t)m, 16);
+  L.term = o, o = align_up(o + (size_t)m, 16);
+  L.out_bytes = o;
+  return L;
+}
+
+// One pipeline: what a step in flight uses, and what phc_host_step_wait needs to finish it.
+struct Slot {
+  bool ready = false;  // buffers, streams and events allocated
+  float* d_state = nullptr;
+  float* d_obs = nullptr;
+  unsigned char* d_clock = nullptr;  // packed clock, device
+  unsigned char* d_out = nullptr;    // packed scalar outputs, device
+  unsigned char* h_clock = nullptr;  // pinned staging
+  unsigned char* h_out = nullptr;    // pinned staging
+  cudaStream_t streams[kStreams] = {};
+  cudaEvent_t done[kStreams] = {};  // recorded on each stream at the end of an enqueue
+  // direct path: verdict cached per set of caller pointers
+  const void* seen[11] = {};
+  int seen_direct = -1;
+  // the step in flight
+  bool busy = false;
+  int path = 0;  // 1 direct, 2 staged
+  PhcHostStepArgs args{};
+  int nchunks = 0;
+  int64_t bounds[kMaxChunks + 2] = {};  // staged path: chunk boundaries, for the unpack in wait
+};
 
 }  // namespace
 
@@ -55,18 +110,9 @@ struct PhcHostStep {
   int32_t use_mean = 0, early = 1;
   float dt = 0.f;
   PhcRewardSpec rwd{};
-  float* d_state = nullptr;
-  float* d_obs = nullptr;
-  unsigned char* d_clock = nullptr;  // packed clock, device
-  unsigned char* d_out = nullptr;    // packed scalar outputs, device
-  unsigned char* h_clock = nullptr;  // pinned staging
-  unsigned char* h_out = nullptr;    // pinned staging
   size_t pack_capacity = 0;
-  cudaStream_t streams[kStreams] = {};
-  int last_cuda = 0;
-  // direct path: verdict cached per set of caller pointers
-  const void* seen[11] = {};
-  int seen_direct = -1;
+  Slot slots[PHC_HOST_SLOTS];
+  int last_slot = 0;  // the slot of the last submit: phc_host_step_path / _chunks report its verdict
   // which output path pinned callers take: 0 = auto (time both over the first calls, keep the faster), 1 = direct
   // (kernels post into the mapped host buffers), 2 = staged (copy-engine D2H).  PHC_HOST_PATH=auto|direct|staged.
   int mode = 0;
@@ -82,37 +128,364 @@ struct PhcHostStep {
 constexpr int kTuneWarm = 2, kTuneReps = 4;
 
 // After the first enqueue an early return must not leave kernels writing into the caller's (mapped) buffers or
-// into the staging buffers the next call reuses: every error path drains the three streams first.
-static int host_fail(PhcHostStep* c, int rc, cudaError_t e);
-#define HOST_CUDA(ctx, call)                                        \
-  do {                                                              \
-    cudaError_t e__ = (call);                                       \
-    if (e__ != cudaSuccess) return host_fail((ctx), PHC_ERR_CUDA, e__); \
+// into the staging buffers the next call reuses: every error path drains the slot's three streams first.
+static int host_fail(Slot& s, int rc, cudaError_t e) {
+  for (auto& st : s.streams)
+    if (st) (void)cudaStreamSynchronize(st);
+  (void)cudaGetLastError();
+  return e != cudaSuccess ? phc::record_cuda_error((int)e) : rc;
+}
+#define HOST_CUDA(slot, call)                                        \
+  do {                                                               \
+    cudaError_t e__ = (call);                                        \
+    if (e__ != cudaSuccess) return host_fail((slot), PHC_ERR_CUDA, e__); \
   } while (0)
 
-static int host_fail(PhcHostStep* c, int rc, cudaError_t e) {
-  if (c) {
-    if (e != cudaSuccess) c->last_cuda = e;
-    for (auto& s : c->streams)
-      if (s) (void)cudaStreamSynchronize(s);
-    (void)cudaGetLastError();
+static cudaError_t slot_alloc(const PhcHostStep* c, Slot& s) {
+  const size_t n = (size_t)c->max_envs;
+  cudaError_t e = cudaSuccess;
+  auto dmalloc = [&](void** p, size_t bytes) {
+    if (e == cudaSuccess) e = cudaMalloc(p, bytes);
+  };
+  dmalloc((void**)&s.d_state, n * kStateFloats * sizeof(float));
+  dmalloc((void**)&s.d_obs, n * c->obs_dim * sizeof(float));
+  dmalloc((void**)&s.d_clock, c->pack_capacity);
+  dmalloc((void**)&s.d_out, c->pack_capacity);
+  if (e == cudaSuccess) e = cudaMallocHost((void**)&s.h_clock, c->pack_capacity);
+  if (e == cudaSuccess) e = cudaMallocHost((void**)&s.h_out, c->pack_capacity);
+  for (int i = 0; i < kStreams && e == cudaSuccess; ++i) {
+    e = cudaStreamCreateWithFlags(&s.streams[i], cudaStreamNonBlocking);
+    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&s.done[i], cudaEventDisableTiming);
   }
-  return rc;
+  s.ready = e == cudaSuccess;
+  return e;
+}
+
+static void slot_free(Slot& s) {
+  for (auto& st : s.streams)
+    if (st) (void)cudaStreamSynchronize(st);
+  cudaFree(s.d_state);
+  cudaFree(s.d_obs);
+  cudaFree(s.d_clock);
+  cudaFree(s.d_out);
+  if (s.h_clock) cudaFreeHost(s.h_clock);
+  if (s.h_out) cudaFreeHost(s.h_out);
+  for (int i = 0; i < kStreams; ++i) {
+    if (s.done[i]) cudaEventDestroy(s.done[i]);
+    if (s.streams[i]) cudaStreamDestroy(s.streams[i]);
+  }
+  s = Slot{};
+}
+
+// Everything phc_host_step validates, before anything is enqueued; fills the slot's direct-path verdict.
+static int check_args(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, int64_t n) {
+  if (n < 0 || n > c->max_envs) return PHC_ERR_SHAPE;
+  if (!a->state || !a->progress_buf || !a->motion_start_times || !a->motion_start_times_offset ||
+      !a->global_offset || !a->sampled_motion_ids || !a->obs_buf || !a->rew_buf || !a->reward_raw || !a->reset_buf ||
+      !a->terminate_buf)
+    return PHC_ERR_NULL;
+  // ---- can the direct path be used: every buffer is pinned / managed host memory mapped at its own address ----------
+  const void* ptrs[11] = {a->state, a->progress_buf, a->motion_start_times, a->motion_start_times_offset,
+                          a->global_offset, a->sampled_motion_ids, a->obs_buf, a->rew_buf, a->reward_raw,
+                          a->reset_buf, a->terminate_buf};
+  if (s.seen_direct < 0 || memcmp(ptrs, s.seen, sizeof(ptrs)) != 0) {
+    int direct = 1;
+    for (int i = 0; i < 11 && direct; ++i) {
+      cudaPointerAttributes at{};
+      if (cudaPointerGetAttributes(&at, ptrs[i]) != cudaSuccess) {
+        (void)cudaGetLastError();
+        direct = 0;
+      } else if (at.type == cudaMemoryTypeDevice) {
+        return PHC_ERR_UNSUPPORTED;  // this entry point takes HOST buffers (the clock arrays are memcpy'd by the CPU)
+      } else if ((at.type != cudaMemoryTypeHost && at.type != cudaMemoryTypeManaged) || at.devicePointer != ptrs[i]) {
+        direct = 0;  // pageable, or mapped at a different device address
+      }
+    }
+    memcpy(s.seen, ptrs, sizeof(ptrs));
+    s.seen_direct = direct;
+  }
+  return PHC_OK;
+}
+
+static int direct_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, int64_t n, const int chunks) {
+  // Hybrid: everything INBOUND rides the host->device copy engine in a few chunks — the sim
+  // rows directly from the caller's buffer, the five small clock arrays packed into one
+  // transfer (SM-issued reads of system memory are 32-B PCIe round trips: 6 per block, ~70 us
+  // per 4096-env step when the kernel read the clock in place) — while each chunk's kernel
+  // WRITES obs rows, rewards and flags straight into the mapped host buffers.  The copy
+  // engine pulling chunk c+1 and the kernel pushing chunk c's rows use opposite directions of
+  // the link.  The advanced progress is written to the caller's buffer by the kernel as well.
+  // equal chunks here: measured, a small first chunk does not help this path (the step is
+  // bound by the kernels' posted writes, ~300 us per 4096 envs, plus the first copy)
+  const int C = chunks < 1 ? 1 : chunks;
+  int64_t per = (n + C - 1) / C;
+  per = (per + 7) / 8 * 8;
+  size_t coff = 0;
+  int ci = 0;
+  static const bool trace_on = getenv("PHC_HOST_TRACE") != nullptr;
+  static int trace_calls = 0;
+  const bool trace = trace_on && ++trace_calls == 20;
+  cudaEvent_t ev0 = nullptr, evh[64], evk[64];
+  double host_us[64];
+  const auto th0 = std::chrono::steady_clock::now();
+  if (trace) {
+    cudaEventCreate(&ev0);
+    cudaEventRecord(ev0, s.streams[0]);
+  }
+  for (int64_t lo = 0; lo < n; lo += per, ++ci) {
+    const int64_t m = (n - lo) < per ? (n - lo) : per;
+    const Layout L = layout(m);
+    if (coff + L.clock_bytes > c->pack_capacity) return host_fail(s, PHC_ERR_SHAPE, cudaSuccess);
+    cudaStream_t st_ = s.streams[ci % kStreams];
+    float* st = s.d_state + lo * kStateFloats;
+    unsigned char* hc = s.h_clock + coff;
+    unsigned char* dc = s.d_clock + coff;
+    memcpy(hc + L.ids, a->sampled_motion_ids + lo, (size_t)m * 8);
+    memcpy(hc + L.goff, a->global_offset + lo * 3, (size_t)m * 12);
+    memcpy(hc + L.start, a->motion_start_times + lo, (size_t)m * 4);
+    memcpy(hc + L.soff, a->motion_start_times_offset + lo, (size_t)m * 4);
+    memcpy(hc + L.prog, a->progress_buf + lo, (size_t)m * 2);
+    HOST_CUDA(s, cudaMemcpyAsync(dc, hc, L.clock_bytes, cudaMemcpyHostToDevice, st_));
+    HOST_CUDA(s, cudaMemcpyAsync(st, a->state + lo * kStateFloats, (size_t)m * kStateFloats * sizeof(float),
+                                 cudaMemcpyHostToDevice, st_));
+    PhcStepArgs k{};
+    if (trace && ci < 64) {
+      cudaEventCreate(&evh[ci]);
+      cudaEventRecord(evh[ci], st_);
+    }
+    k.body.pos = PhcView{st, kStateFloats, 13};
+    k.body.rot = PhcView{st + 3, kStateFloats, 13};
+    k.body.vel = PhcView{st + 7, kStateFloats, 13};
+    k.body.ang_vel = PhcView{st + 10, kStateFloats, 13};
+    k.body.num_bodies = PHC_NUM_BODIES;
+    k.progress_buf = (int16_t*)(dc + L.prog);
+    k.motion_start_times = (const float*)(dc + L.start);
+    k.motion_start_times_offset = (const float*)(dc + L.soff);
+    k.global_offset = (const float*)(dc + L.goff);
+    k.sampled_motion_ids = (const int64_t*)(dc + L.ids);
+    k.termination_distances = c->term_dist;
+    k.reset_body_mask = c->reset_mask;
+    k.use_mean = c->use_mean;
+    k.enable_early_termination = c->early;
+    k.advance_progress = 1;
+    k.time_steps = c->T;
+    k.dt = c->dt;
+    k.rwd = c->rwd;
+    k.obs_buf = a->obs_buf + lo * c->obs_dim;
+    k.obs_stride = c->obs_dim;
+    k.rew_buf = a->rew_buf + lo;
+    k.reward_raw = a->reward_raw + lo * 4;
+    k.reward_raw_stride = 4;
+    k.reset_buf = a->reset_buf + lo;
+    k.terminate_buf = a->terminate_buf + lo;
+    k.flags = PHC_STEP_MAPPED_HOST_IO;
+    k.obs_moments = nullptr;
+    // the advanced progress goes straight into the caller's buffer too (no device->host copy at the tail)
+    int rc = step_fused_mirrored(c->lib, &k, m, st_, a->progress_buf + lo);
+    if (rc) return host_fail(s, rc, cudaSuccess);
+    if (trace && ci < 64) {
+      cudaEventCreate(&evk[ci]);
+      cudaEventRecord(evk[ci], st_);
+      host_us[ci] = std::chrono::duration<double>(std::chrono::steady_clock::now() - th0).count() * 1e6;
+    }
+    coff += L.clock_bytes;
+  }
+  if (trace) {
+    for (auto st_ : s.streams) HOST_CUDA(s, cudaStreamSynchronize(st_));
+    const double tot = std::chrono::duration<double>(std::chrono::steady_clock::now() - th0).count() * 1e6;
+    fprintf(stderr, "[phc_host trace] %d chunks of %lld envs, host total %.1f us\n", ci, (long long)per, tot);
+    for (int i = 0; i < ci && i < 64; ++i) {
+      float a_ms = 0, b_ms = 0;
+      cudaEventElapsedTime(&a_ms, ev0, evh[i]);
+      cudaEventElapsedTime(&b_ms, ev0, evk[i]);
+      fprintf(stderr, "  chunk %d: submitted at %.1f us (host), H2D done %.1f us, kernel done %.1f us\n", i, host_us[i],
+              a_ms * 1e3, b_ms * 1e3);
+    }
+  }
+  return PHC_OK;
+}
+
+static int staged_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, int64_t n, const int chunks) {
+  const cudaMemcpyKind H2D = cudaMemcpyHostToDevice, D2H = cudaMemcpyDeviceToHost;
+  // Chunk sizes double (n/2^(C-1), n/2^(C-1), n/2^(C-2), .., n/2): the device->host direction
+  // carries 3x the bytes and is the bottleneck, so the first chunk is small to start it early
+  // while the later, larger chunks keep the per-transfer overhead low.  Boundaries fall on
+  // multiples of 8 envs so every chunk's obs rows start 16-B aligned.
+  {
+    const int C = chunks < 1 ? 1 : chunks;
+    int64_t lo = 0;
+    s.nchunks = 0;
+    s.bounds[0] = 0;
+    for (int i = 0; i < C && lo < n; ++i) {
+      const int shift = (i == 0) ? C - 1 : C - i;
+      int64_t sz = shift < 62 ? (n >> shift) : 0;
+      sz = (sz + 7) / 8 * 8;
+      if (sz < 8) sz = 8;
+      int64_t hi = (i == C - 1) ? n : (lo + sz < n ? lo + sz : n);
+      s.bounds[++s.nchunks] = hi;
+      lo = hi;
+    }
+    s.bounds[s.nchunks] = n;
+  }
+  const int nchunks = s.nchunks;
+  const int64_t* bounds = s.bounds;
+
+  size_t coff = 0, ooff = 0;
+  static const bool strace_on = getenv("PHC_HOST_TRACE") != nullptr;
+  static int strace_calls = 0;
+  const bool strace = strace_on && ++strace_calls == 20;
+  cudaEvent_t sev0 = nullptr, sevh[16], sevk[16], sevd[16];
+  if (strace) {
+    cudaEventCreate(&sev0);
+    cudaEventRecord(sev0, s.streams[0]);
+  }
+  for (int ci = 0; ci < nchunks; ++ci) {
+    const int64_t lo = bounds[ci], m = bounds[ci + 1] - bounds[ci];
+    if (m <= 0) continue;
+    const Layout L = layout(m);
+    if (coff + L.clock_bytes > c->pack_capacity || ooff + L.out_bytes > c->pack_capacity)
+      return host_fail(s, PHC_ERR_SHAPE, cudaSuccess);
+    cudaStream_t st_ = s.streams[ci % kStreams];
+    // pack the chunk's clock on the host (tens of KB), then ONE transfer
+    unsigned char* hc = s.h_clock + coff;
+    memcpy(hc + L.ids, a->sampled_motion_ids + lo, (size_t)m * 8);
+    memcpy(hc + L.goff, a->global_offset + lo * 3, (size_t)m * 12);
+    memcpy(hc + L.start, a->motion_start_times + lo, (size_t)m * 4);
+    memcpy(hc + L.soff, a->motion_start_times_offset + lo, (size_t)m * 4);
+    memcpy(hc + L.prog, a->progress_buf + lo, (size_t)m * 2);
+    unsigned char* dc = s.d_clock + coff;
+    unsigned char* dout = s.d_out + ooff;
+    HOST_CUDA(s, cudaMemcpyAsync(s.d_state + lo * kStateFloats, a->state + lo * kStateFloats,
+                                 (size_t)m * kStateFloats * sizeof(float), H2D, st_));
+    HOST_CUDA(s, cudaMemcpyAsync(dc, hc, L.clock_bytes, H2D, st_));
+
+    PhcStepArgs k{};
+    float* st = s.d_state + lo * kStateFloats;
+    k.body.pos = PhcView{st, kStateFloats, 13};
+    k.body.rot = PhcView{st + 3, kStateFloats, 13};
+    k.body.vel = PhcView{st + 7, kStateFloats, 13};
+    k.body.ang_vel = PhcView{st + 10, kStateFloats, 13};
+    k.body.num_bodies = PHC_NUM_BODIES;
+    k.progress_buf = (int16_t*)(dc + L.prog);
+    k.motion_start_times = (const float*)(dc + L.start);
+    k.motion_start_times_offset = (const float*)(dc + L.soff);
+    k.global_offset = (const float*)(dc + L.goff);
+    k.sampled_motion_ids = (const int64_t*)(dc + L.ids);
+    k.termination_distances = c->term_dist;
+    k.reset_body_mask = c->reset_mask;
+    k.use_mean = c->use_mean;
+    k.enable_early_termination = c->early;
+    k.advance_progress = 1;
+    k.time_steps = c->T;
+    k.dt = c->dt;
+    k.rwd = c->rwd;
+    k.obs_buf = s.d_obs + lo * c->obs_dim;
+    k.obs_stride = c->obs_dim;
+    k.rew_buf = (float*)(dout + L.rew);
+    k.reward_raw = (float*)(dout + L.raw);
+    k.reward_raw_stride = 4;
+    k.reset_buf = dout + L.reset;
+    k.terminate_buf = dout + L.term;
+    k.obs_moments = nullptr;
+    if (strace && ci < 16) {
+      cudaEventCreate(&sevh[ci]);
+      cudaEventRecord(sevh[ci], st_);
+    }
+    int rc = phc_step_fused(c->lib, &k, m, st_);
+    if (rc) return host_fail(s, rc, cudaSuccess);
+    if (strace && ci < 16) {
+      cudaEventCreate(&sevk[ci]);
+      cudaEventRecord(sevk[ci], st_);
+    }
+    // the advanced progress rides back with the scalar outputs
+    HOST_CUDA(s, cudaMemcpyAsync(dout + L.oprog, dc + L.prog, (size_t)m * 2, cudaMemcpyDeviceToDevice, st_));
+    HOST_CUDA(s, cudaMemcpyAsync(a->obs_buf + lo * c->obs_dim, s.d_obs + lo * c->obs_dim,
+                                 (size_t)m * c->obs_dim * sizeof(float), D2H, st_));
+    HOST_CUDA(s, cudaMemcpyAsync(s.h_out + ooff, dout, L.out_bytes, D2H, st_));
+    if (strace && ci < 16) {
+      cudaEventCreate(&sevd[ci]);
+      cudaEventRecord(sevd[ci], st_);
+    }
+    coff += L.clock_bytes;
+    ooff += L.out_bytes;
+  }
+  if (strace) {
+    for (auto st_ : s.streams) HOST_CUDA(s, cudaStreamSynchronize(st_));
+    fprintf(stderr, "[phc_host trace] staged, %d chunks\n", nchunks);
+    for (int i = 0; i < nchunks && i < 16; ++i) {
+      float a_ms = 0, b_ms = 0, d_ms = 0;
+      cudaEventElapsedTime(&a_ms, sev0, sevh[i]);
+      cudaEventElapsedTime(&b_ms, sev0, sevk[i]);
+      cudaEventElapsedTime(&d_ms, sev0, sevd[i]);
+      fprintf(stderr, "  chunk %d (%lld envs): H2D done %.1f us, kernel done %.1f us, D2H done %.1f us\n", i,
+              (long long)(bounds[i + 1] - bounds[i]), a_ms * 1e3, b_ms * 1e3, d_ms * 1e3);
+    }
+  }
+  return PHC_OK;
+}
+
+// Enqueues one step on a slot (arguments already checked) and marks it in flight.
+static int slot_enqueue(PhcHostStep* c, int slot, const PhcHostStepArgs* a, int64_t n, const PhcHostStep::Cand& k) {
+  Slot& s = c->slots[slot];
+  const int rc = k.path == 1 ? direct_enqueue(c, s, a, n, k.chunks) : staged_enqueue(c, s, a, n, k.chunks);
+  if (rc) return rc;
+  for (int i = 0; i < kStreams; ++i) HOST_CUDA(s, cudaEventRecord(s.done[i], s.streams[i]));
+  s.args = *a;
+  s.path = k.path;
+  s.busy = true;
+  c->last_slot = slot;
+  return PHC_OK;
+}
+
+// Waits for a slot's step; on the staged path unpacks the scalar outputs into the caller's buffers.
+static int slot_finish(Slot& s) {
+  if (!s.busy) return PHC_OK;
+  s.busy = false;
+  cudaError_t err = cudaSuccess;
+  for (auto& ev : s.done) {
+    const cudaError_t e = cudaEventSynchronize(ev);
+    if (err == cudaSuccess) err = e;
+  }
+  if (err != cudaSuccess) return host_fail(s, PHC_ERR_CUDA, err);
+  if (s.path != 2) return PHC_OK;
+  const PhcHostStepArgs* a = &s.args;
+  size_t ooff = 0;
+  for (int ci = 0; ci < s.nchunks; ++ci) {
+    const int64_t lo = s.bounds[ci], m = s.bounds[ci + 1] - s.bounds[ci];
+    if (m <= 0) continue;
+    const Layout L = layout(m);
+    const unsigned char* ho = s.h_out + ooff;
+    memcpy(a->rew_buf + lo, ho + L.rew, (size_t)m * 4);
+    memcpy(a->reward_raw + lo * 4, ho + L.raw, (size_t)m * 16);
+    memcpy(a->progress_buf + lo, ho + L.oprog, (size_t)m * 2);
+    memcpy(a->reset_buf + lo, ho + L.reset, (size_t)m);
+    memcpy(a->terminate_buf + lo, ho + L.term, (size_t)m);
+    ooff += L.out_bytes;
+  }
+  return PHC_OK;
+}
+
+// The schedule of a step that is not timed by the tuner: pageable callers take the copy-engine path; pinned callers
+// the settled schedule, or the first candidate while tuning has not finished.
+static PhcHostStep::Cand untimed_schedule(const PhcHostStep* c, const Slot& s) {
+  if (s.seen_direct != 1) return {2, c->chunks > 0 ? c->chunks : 3, 0.0, 0};
+  return c->cand[c->chosen >= 0 ? c->chosen : 0];
+}
+
+static int run_sync(PhcHostStep* c, const PhcHostStepArgs* a, int64_t n, const PhcHostStep::Cand& k) {
+  const int rc = slot_enqueue(c, 0, a, n, k);
+  return rc ? rc : slot_finish(c->slots[0]);
 }
 
 extern "C" {
 
 void phc_host_step_destroy(PhcHostStep* c) {
   if (!c) return;
-  cudaFree(c->d_state);
-  cudaFree(c->d_obs);
-  cudaFree(c->d_clock);
-  cudaFree(c->d_out);
+  for (auto& s : c->slots) {
+    (void)slot_finish(s);  // a pending DMA or posting kernel must not land in freed memory
+    slot_free(s);
+  }
   cudaFree(c->term_dist);
-  if (c->h_clock) cudaFreeHost(c->h_clock);
-  if (c->h_out) cudaFreeHost(c->h_out);
-  for (auto& s : c->streams)
-    if (s) cudaStreamDestroy(s);
   delete c;
 }
 
@@ -120,7 +493,7 @@ int phc_host_step_create(const PhcLib* lib, int64_t max_envs, int32_t time_steps
                          const float* termination_distances_host, uint32_t reset_body_mask, int32_t use_mean,
                          int32_t enable_early_termination, float dt, const PhcRewardSpec* rwd, PhcHostStep** out) {
   if (!lib || !termination_distances_host || !rwd || !out) return PHC_ERR_NULL;
-  if (max_envs <= 0 || time_steps < 1 || time_steps > PHC_MAX_TIME_STEPS || num_chunks < 0 || num_chunks > 1024)
+  if (max_envs <= 0 || time_steps < 1 || time_steps > PHC_MAX_TIME_STEPS || num_chunks < 0 || num_chunks > kMaxChunks)
     return PHC_ERR_SHAPE;
   PhcHostStep* c = new (std::nothrow) PhcHostStep;
   if (!c) return PHC_ERR_ALLOC;
@@ -155,21 +528,11 @@ int phc_host_step_create(const PhcLib* lib, int64_t max_envs, int32_t time_steps
     }
     if (c->ncand == 1) c->chosen = 0;
   }
-  cudaError_t e = cudaSuccess;
-  auto dmalloc = [&](void** p, size_t bytes) {
-    if (e == cudaSuccess) e = cudaMalloc(p, bytes);
-  };
-  dmalloc((void**)&c->d_state, n * kStateFloats * sizeof(float));
-  dmalloc((void**)&c->d_obs, n * c->obs_dim * sizeof(float));
-  dmalloc((void**)&c->d_clock, c->pack_capacity);
-  dmalloc((void**)&c->d_out, c->pack_capacity);
-  dmalloc((void**)&c->term_dist, PHC_NUM_BODIES * sizeof(float));
-  if (e == cudaSuccess) e = cudaMallocHost((void**)&c->h_clock, c->pack_capacity);
-  if (e == cudaSuccess) e = cudaMallocHost((void**)&c->h_out, c->pack_capacity);
+  // slot 0 (the synchronous call's) is allocated here, slot 1 at its first submit
+  cudaError_t e = cudaMalloc((void**)&c->term_dist, PHC_NUM_BODIES * sizeof(float));
   if (e == cudaSuccess)
     e = cudaMemcpy(c->term_dist, termination_distances_host, PHC_NUM_BODIES * sizeof(float), cudaMemcpyHostToDevice);
-  for (int i = 0; i < kStreams && e == cudaSuccess; ++i)
-    e = cudaStreamCreateWithFlags(&c->streams[i], cudaStreamNonBlocking);
+  if (e == cudaSuccess) e = slot_alloc(c, c->slots[0]);
   if (e != cudaSuccess) {
     phc_host_step_destroy(c);
     return e == cudaErrorMemoryAllocation ? PHC_ERR_ALLOC : PHC_ERR_CUDA;
@@ -188,292 +551,15 @@ int64_t phc_host_step_d2h_bytes(const PhcHostStep* c, int64_t n) {
 
 int phc_host_step(PhcHostStep* c, const PhcHostStepArgs* a, int64_t n) {
   if (!c || !a) return PHC_ERR_NULL;
+  if (c->slots[0].busy) return PHC_ERR_BUSY;
   if (n == 0) return PHC_OK;
-  if (n < 0 || n > c->max_envs) return PHC_ERR_SHAPE;
-  if (!a->state || !a->progress_buf || !a->motion_start_times || !a->motion_start_times_offset ||
-      !a->global_offset || !a->sampled_motion_ids || !a->obs_buf || !a->rew_buf || !a->reward_raw || !a->reset_buf ||
-      !a->terminate_buf)
-    return PHC_ERR_NULL;
-  // Chunk sizes double (n/2^(C-1), n/2^(C-1), n/2^(C-2), .., n/2): the device->host direction
-  // carries 3x the bytes and is the bottleneck, so the first chunk is small to start it early
-  // while the later, larger chunks keep the per-transfer overhead low.  Boundaries fall on
-  // multiples of 8 envs so every chunk's obs rows start 16-B aligned.
-  int64_t bounds[1026];
-  int nchunks = 0;
-  auto make_bounds = [&](const int C) {
-    nchunks = 0;
-    int64_t lo = 0;
-    bounds[0] = 0;
-    for (int i = 0; i < C && lo < n; ++i) {
-      const int shift = (i == 0) ? C - 1 : C - i;
-      int64_t sz = shift < 62 ? (n >> shift) : 0;
-      sz = (sz + 7) / 8 * 8;
-      if (sz < 8) sz = 8;
-      int64_t hi = (i == C - 1) ? n : (lo + sz < n ? lo + sz : n);
-      bounds[++nchunks] = hi;
-      lo = hi;
-    }
-    bounds[nchunks] = n;
-  };
-  // sub-array offsets inside a chunk's packed regions (each 16-B aligned)
-  struct Layout {
-    size_t ids, goff, start, soff, prog, clock_bytes;
-    size_t rew, raw, oprog, reset, term, out_bytes;
-  };
-  auto layout = [](int64_t m) {
-    Layout L;
-    size_t o = 0;
-    L.ids = o, o = align_up(o + (size_t)m * 8, 16);
-    L.goff = o, o = align_up(o + (size_t)m * 12, 16);
-    L.start = o, o = align_up(o + (size_t)m * 4, 16);
-    L.soff = o, o = align_up(o + (size_t)m * 4, 16);
-    L.prog = o, o = align_up(o + (size_t)m * 2, 16);
-    L.clock_bytes = o;
-    o = 0;
-    L.rew = o, o = align_up(o + (size_t)m * 4, 16);
-    L.raw = o, o = align_up(o + (size_t)m * 16, 16);
-    L.oprog = o, o = align_up(o + (size_t)m * 2, 16);
-    L.reset = o, o = align_up(o + (size_t)m, 16);
-    L.term = o, o = align_up(o + (size_t)m, 16);
-    L.out_bytes = o;
-    return L;
-  };
-
-  {  // ---- can the direct path be used: every buffer is pinned / managed host memory mapped at its own address ----------------------
-    const void* ptrs[11] = {a->state, a->progress_buf, a->motion_start_times, a->motion_start_times_offset,
-                            a->global_offset, a->sampled_motion_ids, a->obs_buf, a->rew_buf, a->reward_raw,
-                            a->reset_buf, a->terminate_buf};
-    if (c->seen_direct < 0 || memcmp(ptrs, c->seen, sizeof(ptrs)) != 0) {
-      int direct = 1;
-      for (int i = 0; i < 11 && direct; ++i) {
-        cudaPointerAttributes at{};
-        if (cudaPointerGetAttributes(&at, ptrs[i]) != cudaSuccess) {
-          (void)cudaGetLastError();
-          direct = 0;
-        } else if (at.type == cudaMemoryTypeDevice) {
-          return PHC_ERR_UNSUPPORTED;  // this entry point takes HOST buffers (the clock arrays are memcpy'd by the CPU)
-        } else if ((at.type != cudaMemoryTypeHost && at.type != cudaMemoryTypeManaged) || at.devicePointer != ptrs[i]) {
-          direct = 0;  // pageable, or mapped at a different device address
-        }
-      }
-      memcpy(c->seen, ptrs, sizeof(ptrs));
-      c->seen_direct = direct;
-    }
-  }
-  auto direct_path = [&](const int chunks) -> int {
-      // Hybrid: everything INBOUND rides the host->device copy engine in a few chunks — the sim
-      // rows directly from the caller's buffer, the five small clock arrays packed into one
-      // transfer (SM-issued reads of system memory are 32-B PCIe round trips: 6 per block, ~70 us
-      // per 4096-env step when the kernel read the clock in place) — while each chunk's kernel
-      // WRITES obs rows, rewards and flags straight into the mapped host buffers.  The copy
-      // engine pulling chunk c+1 and the kernel pushing chunk c's rows use opposite directions of
-      // the link.  The advanced progress is written to the caller's buffer by the kernel as well.
-      // equal chunks here: measured, a small first chunk does not help this path (the step is
-      // bound by the kernels' posted writes, ~300 us per 4096 envs, plus the first copy)
-      const int C = chunks < 1 ? 1 : chunks;
-      int64_t per = (n + C - 1) / C;
-      per = (per + 7) / 8 * 8;
-      size_t coff = 0;
-      int ci = 0;
-      static const bool trace_on = getenv("PHC_HOST_TRACE") != nullptr;
-      static int trace_calls = 0;
-      const bool trace = trace_on && ++trace_calls == 20;
-      cudaEvent_t ev0 = nullptr, evh[64], evk[64];
-      double host_us[64];
-      const auto th0 = std::chrono::steady_clock::now();
-      if (trace) {
-        cudaEventCreate(&ev0);
-        cudaEventRecord(ev0, c->streams[0]);
-      }
-      for (int64_t lo = 0; lo < n; lo += per, ++ci) {
-        const int64_t m = (n - lo) < per ? (n - lo) : per;
-        const Layout L = layout(m);
-        if (coff + L.clock_bytes > c->pack_capacity) return host_fail(c, PHC_ERR_SHAPE, cudaSuccess);
-        cudaStream_t s = c->streams[ci % kStreams];
-        float* st = c->d_state + lo * kStateFloats;
-        unsigned char* hc = c->h_clock + coff;
-        unsigned char* dc = c->d_clock + coff;
-        memcpy(hc + L.ids, a->sampled_motion_ids + lo, (size_t)m * 8);
-        memcpy(hc + L.goff, a->global_offset + lo * 3, (size_t)m * 12);
-        memcpy(hc + L.start, a->motion_start_times + lo, (size_t)m * 4);
-        memcpy(hc + L.soff, a->motion_start_times_offset + lo, (size_t)m * 4);
-        memcpy(hc + L.prog, a->progress_buf + lo, (size_t)m * 2);
-        HOST_CUDA(c, cudaMemcpyAsync(dc, hc, L.clock_bytes, cudaMemcpyHostToDevice, s));
-        HOST_CUDA(c, cudaMemcpyAsync(st, a->state + lo * kStateFloats, (size_t)m * kStateFloats * sizeof(float),
-                                     cudaMemcpyHostToDevice, s));
-        PhcStepArgs k{};
-        if (trace && ci < 64) {
-          cudaEventCreate(&evh[ci]);
-          cudaEventRecord(evh[ci], s);
-        }
-        k.body.pos = PhcView{st, kStateFloats, 13};
-        k.body.rot = PhcView{st + 3, kStateFloats, 13};
-        k.body.vel = PhcView{st + 7, kStateFloats, 13};
-        k.body.ang_vel = PhcView{st + 10, kStateFloats, 13};
-        k.body.num_bodies = PHC_NUM_BODIES;
-        k.progress_buf = (int16_t*)(dc + L.prog);
-        k.motion_start_times = (const float*)(dc + L.start);
-        k.motion_start_times_offset = (const float*)(dc + L.soff);
-        k.global_offset = (const float*)(dc + L.goff);
-        k.sampled_motion_ids = (const int64_t*)(dc + L.ids);
-        k.termination_distances = c->term_dist;
-        k.reset_body_mask = c->reset_mask;
-        k.use_mean = c->use_mean;
-        k.enable_early_termination = c->early;
-        k.advance_progress = 1;
-        k.time_steps = c->T;
-        k.dt = c->dt;
-        k.rwd = c->rwd;
-        k.obs_buf = a->obs_buf + lo * c->obs_dim;
-        k.obs_stride = c->obs_dim;
-        k.rew_buf = a->rew_buf + lo;
-        k.reward_raw = a->reward_raw + lo * 4;
-        k.reward_raw_stride = 4;
-        k.reset_buf = a->reset_buf + lo;
-        k.terminate_buf = a->terminate_buf + lo;
-        k.flags = PHC_STEP_MAPPED_HOST_IO;
-        k.obs_moments = nullptr;
-        // the advanced progress goes straight into the caller's buffer too (no device->host copy at the tail)
-        int rc = step_fused_mirrored(c->lib, &k, m, s, a->progress_buf + lo);
-        if (rc) return host_fail(c, rc, cudaSuccess);
-        if (trace && ci < 64) {
-          cudaEventCreate(&evk[ci]);
-          cudaEventRecord(evk[ci], s);
-          host_us[ci] = std::chrono::duration<double>(std::chrono::steady_clock::now() - th0).count() * 1e6;
-        }
-        coff += L.clock_bytes;
-      }
-      for (int i = 0; i < kStreams; ++i) HOST_CUDA(c, cudaStreamSynchronize(c->streams[i]));
-      if (trace) {
-        const double tot = std::chrono::duration<double>(std::chrono::steady_clock::now() - th0).count() * 1e6;
-        fprintf(stderr, "[phc_host trace] %d chunks of %lld envs, host total %.1f us\n", ci, (long long)per, tot);
-        for (int i = 0; i < ci && i < 64; ++i) {
-          float a_ms = 0, b_ms = 0;
-          cudaEventElapsedTime(&a_ms, ev0, evh[i]);
-          cudaEventElapsedTime(&b_ms, ev0, evk[i]);
-          fprintf(stderr, "  chunk %d: submitted at %.1f us (host), H2D done %.1f us, kernel done %.1f us\n", i, host_us[i],
-                  a_ms * 1e3, b_ms * 1e3);
-        }
-      }
-      return PHC_OK;
-  };
-  auto staged_path = [&](const int chunks) -> int {
-  const cudaMemcpyKind H2D = cudaMemcpyHostToDevice, D2H = cudaMemcpyDeviceToHost;
-  make_bounds(chunks < 1 ? 1 : chunks);
-
-  size_t coff = 0, ooff = 0;
-  static const bool strace_on = getenv("PHC_HOST_TRACE") != nullptr;
-  static int strace_calls = 0;
-  const bool strace = strace_on && ++strace_calls == 20;
-  cudaEvent_t sev0 = nullptr, sevh[16], sevk[16], sevd[16];
-  if (strace) {
-    cudaEventCreate(&sev0);
-    cudaEventRecord(sev0, c->streams[0]);
-  }
-  for (int ci = 0; ci < nchunks; ++ci) {
-    const int64_t lo = bounds[ci], m = bounds[ci + 1] - bounds[ci];
-    if (m <= 0) continue;
-    const Layout L = layout(m);
-    if (coff + L.clock_bytes > c->pack_capacity || ooff + L.out_bytes > c->pack_capacity)
-      return host_fail(c, PHC_ERR_SHAPE, cudaSuccess);
-    cudaStream_t s = c->streams[ci % kStreams];
-    // pack the chunk's clock on the host (tens of KB), then ONE transfer
-    unsigned char* hc = c->h_clock + coff;
-    memcpy(hc + L.ids, a->sampled_motion_ids + lo, (size_t)m * 8);
-    memcpy(hc + L.goff, a->global_offset + lo * 3, (size_t)m * 12);
-    memcpy(hc + L.start, a->motion_start_times + lo, (size_t)m * 4);
-    memcpy(hc + L.soff, a->motion_start_times_offset + lo, (size_t)m * 4);
-    memcpy(hc + L.prog, a->progress_buf + lo, (size_t)m * 2);
-    unsigned char* dc = c->d_clock + coff;
-    unsigned char* dout = c->d_out + ooff;
-    HOST_CUDA(c, cudaMemcpyAsync(c->d_state + lo * kStateFloats, a->state + lo * kStateFloats,
-                                 (size_t)m * kStateFloats * sizeof(float), H2D, s));
-    HOST_CUDA(c, cudaMemcpyAsync(dc, hc, L.clock_bytes, H2D, s));
-
-    PhcStepArgs k{};
-    float* st = c->d_state + lo * kStateFloats;
-    k.body.pos = PhcView{st, kStateFloats, 13};
-    k.body.rot = PhcView{st + 3, kStateFloats, 13};
-    k.body.vel = PhcView{st + 7, kStateFloats, 13};
-    k.body.ang_vel = PhcView{st + 10, kStateFloats, 13};
-    k.body.num_bodies = PHC_NUM_BODIES;
-    k.progress_buf = (int16_t*)(dc + L.prog);
-    k.motion_start_times = (const float*)(dc + L.start);
-    k.motion_start_times_offset = (const float*)(dc + L.soff);
-    k.global_offset = (const float*)(dc + L.goff);
-    k.sampled_motion_ids = (const int64_t*)(dc + L.ids);
-    k.termination_distances = c->term_dist;
-    k.reset_body_mask = c->reset_mask;
-    k.use_mean = c->use_mean;
-    k.enable_early_termination = c->early;
-    k.advance_progress = 1;
-    k.time_steps = c->T;
-    k.dt = c->dt;
-    k.rwd = c->rwd;
-    k.obs_buf = c->d_obs + lo * c->obs_dim;
-    k.obs_stride = c->obs_dim;
-    k.rew_buf = (float*)(dout + L.rew);
-    k.reward_raw = (float*)(dout + L.raw);
-    k.reward_raw_stride = 4;
-    k.reset_buf = dout + L.reset;
-    k.terminate_buf = dout + L.term;
-    k.obs_moments = nullptr;
-    if (strace && ci < 16) {
-      cudaEventCreate(&sevh[ci]);
-      cudaEventRecord(sevh[ci], s);
-    }
-    int rc = phc_step_fused(c->lib, &k, m, s);
-    if (rc) return host_fail(c, rc, cudaSuccess);
-    if (strace && ci < 16) {
-      cudaEventCreate(&sevk[ci]);
-      cudaEventRecord(sevk[ci], s);
-    }
-    // the advanced progress rides back with the scalar outputs
-    HOST_CUDA(c, cudaMemcpyAsync(dout + L.oprog, dc + L.prog, (size_t)m * 2, cudaMemcpyDeviceToDevice, s));
-    HOST_CUDA(c, cudaMemcpyAsync(a->obs_buf + lo * c->obs_dim, c->d_obs + lo * c->obs_dim,
-                                 (size_t)m * c->obs_dim * sizeof(float), D2H, s));
-    HOST_CUDA(c, cudaMemcpyAsync(c->h_out + ooff, dout, L.out_bytes, D2H, s));
-    if (strace && ci < 16) {
-      cudaEventCreate(&sevd[ci]);
-      cudaEventRecord(sevd[ci], s);
-    }
-    coff += L.clock_bytes;
-    ooff += L.out_bytes;
-  }
-  for (int i = 0; i < kStreams; ++i) HOST_CUDA(c, cudaStreamSynchronize(c->streams[i]));
-  if (strace) {
-    fprintf(stderr, "[phc_host trace] staged, %d chunks\n", nchunks);
-    for (int i = 0; i < nchunks && i < 16; ++i) {
-      float a_ms = 0, b_ms = 0, d_ms = 0;
-      cudaEventElapsedTime(&a_ms, sev0, sevh[i]);
-      cudaEventElapsedTime(&b_ms, sev0, sevk[i]);
-      cudaEventElapsedTime(&d_ms, sev0, sevd[i]);
-      fprintf(stderr, "  chunk %d (%lld envs): H2D done %.1f us, kernel done %.1f us, D2H done %.1f us\n", i,
-              (long long)(bounds[i + 1] - bounds[i]), a_ms * 1e3, b_ms * 1e3, d_ms * 1e3);
-    }
-  }
-  // unpack the scalar outputs
-  ooff = 0;
-  for (int ci = 0; ci < nchunks; ++ci) {
-    const int64_t lo = bounds[ci], m = bounds[ci + 1] - bounds[ci];
-    if (m <= 0) continue;
-    const Layout L = layout(m);
-    const unsigned char* ho = c->h_out + ooff;
-    memcpy(a->rew_buf + lo, ho + L.rew, (size_t)m * 4);
-    memcpy(a->reward_raw + lo * 4, ho + L.raw, (size_t)m * 16);
-    memcpy(a->progress_buf + lo, ho + L.oprog, (size_t)m * 2);
-    memcpy(a->reset_buf + lo, ho + L.reset, (size_t)m);
-    memcpy(a->terminate_buf + lo, ho + L.term, (size_t)m);
-    ooff += L.out_bytes;
-  }
-  return PHC_OK;
-  };
+  int rc = check_args(c, c->slots[0], a, n);
+  if (rc) return rc;
 
   // ---- which schedule ------------------------------------------------------------------------
-  const int fallback_chunks = c->chunks > 0 ? c->chunks : 3;
-  if (c->seen_direct != 1) return staged_path(fallback_chunks);  // pageable caller: copy-engine path only
-  auto run = [&](const PhcHostStep::Cand& k) { return k.path == 1 ? direct_path(k.chunks) : staged_path(k.chunks); };
-  if (c->chosen >= 0) return run(c->cand[c->chosen]);
+  // Only calls made while no slot is in flight are timed: a step of the other slot would share the link.
+  if (c->slots[0].seen_direct != 1 || c->chosen >= 0 || c->slots[1].busy)
+    return run_sync(c, a, n, untimed_schedule(c, c->slots[0]));
   // Tuning: calls 0-1 warm up, then the candidates take turns (kTuneReps timed calls each) and the fastest mean
   // stays.  What decides is the machine, under whatever load the other GPUs of the box put on the host at that moment:
   // one GPU posts its obs rows into host memory faster than a copy engine drains a staging buffer, eight GPUs posting
@@ -483,7 +569,7 @@ int phc_host_step(PhcHostStep* c, const PhcHostStepArgs* a, int64_t n) {
   const int k = c->calls++;
   const int which = k < kTuneWarm ? k % c->ncand : (k - kTuneWarm) % c->ncand;
   const auto t0 = std::chrono::steady_clock::now();
-  const int rc = run(c->cand[which]);
+  rc = run_sync(c, a, n, c->cand[which]);
   const double dt = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
   if (rc == PHC_OK && k >= kTuneWarm) {
     // the first timed call of a candidate warms its own launch configuration: not counted.  A candidate's figure is
@@ -510,15 +596,40 @@ int phc_host_step(PhcHostStep* c, const PhcHostStepArgs* a, int64_t n) {
   return rc;
 }
 
+int phc_host_step_submit(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, int64_t n) {
+  if (!c || !a) return PHC_ERR_NULL;
+  if (slot < 0 || slot >= PHC_HOST_SLOTS) return PHC_ERR_SHAPE;
+  Slot& s = c->slots[slot];
+  if (s.busy) return PHC_ERR_BUSY;
+  if (n == 0) return PHC_OK;
+  const int rc = check_args(c, s, a, n);
+  if (rc) return rc;
+  if (!s.ready) {
+    const cudaError_t e = slot_alloc(c, s);
+    if (e != cudaSuccess) {
+      slot_free(s);
+      (void)cudaGetLastError();
+      return e == cudaErrorMemoryAllocation ? PHC_ERR_ALLOC : phc::record_cuda_error((int)e);
+    }
+  }
+  return slot_enqueue(c, slot, a, n, untimed_schedule(c, s));
+}
+
+int phc_host_step_wait(PhcHostStep* c, int32_t slot) {
+  if (!c) return PHC_ERR_NULL;
+  if (slot < 0 || slot >= PHC_HOST_SLOTS) return PHC_ERR_SHAPE;
+  return slot_finish(c->slots[slot]);
+}
+
 int phc_host_step_path(const PhcHostStep* c) {
   if (!c) return 0;
-  if (c->seen_direct == 0) return 2;
+  if (c->slots[c->last_slot].seen_direct == 0) return 2;
   return c->chosen >= 0 ? c->cand[c->chosen].path : 0;
 }
 
 int phc_host_step_chunks(const PhcHostStep* c) {
   if (!c) return 0;
-  if (c->seen_direct == 0) return c->chunks > 0 ? c->chunks : 3;
+  if (c->slots[c->last_slot].seen_direct == 0) return c->chunks > 0 ? c->chunks : 3;
   return c->chosen >= 0 ? c->cand[c->chosen].chunks : 0;
 }
 

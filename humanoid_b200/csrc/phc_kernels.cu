@@ -3572,6 +3572,7 @@ const char* phc_strerror(int code) {
     case PHC_ERR_CUDA: return "CUDA runtime error";
     case PHC_ERR_ALLOC: return "allocation failed";
     case PHC_PEER_TIMEOUT: return "a peer rank did not publish its partials in time";
+    case PHC_ERR_BUSY: return "the host-step slot already has a step in flight";
     default: return "unknown error";
   }
 }

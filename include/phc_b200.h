@@ -13,8 +13,8 @@
  *   - nothing is allocated, retained or freed on behalf of the caller except the opaque
  *     handles (PhcLib borrows the motion tensors; the caller keeps them alive);
  *   - all functions return 0 on success and a negative PHC_ERR_* code otherwise, never
- *     throw, never synchronise (except the *_host_* pipeline, which returns when the host
- *     buffers are filled) and launch on the stream passed last, so they can be captured
+ *     throw, never synchronise (except phc_host_step and phc_host_step_wait, which return when
+ *     the host buffers are filled) and launch on the stream passed last, so they can be captured
  *     in a CUDA graph;
  *   - views of rigid-body state carry element strides so that the reference's stride-13
  *     AoS views (envs/humanoid_phc.py:542-549) and contiguous tensors both work; the last
@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define PHC_ABI_VERSION 4 /* 4: PhcResetArgs grew (initial_*, default_mask: StateInit.Default / Hybrid); 3: PhcStepArgs grew (rew_out, reset_out, terminate_out, auto_reset, ref_dof_pos, obs_flags), PhcResetArgs grew (obs_norm*, obs_moments*),
+#define PHC_ABI_VERSION 5 /* 5: phc_host_step_submit / phc_host_step_wait, PHC_ERR_BUSY; 4: PhcResetArgs grew (initial_*, default_mask: StateInit.Default / Hybrid); 3: PhcStepArgs grew (rew_out, reset_out, terminate_out, auto_reset, ref_dof_pos, obs_flags), PhcResetArgs grew (obs_norm*, obs_moments*),
                               phc_action_to_pd_targets takes the action clip; 2: obs_moments_buckets, ep_*, phc_motion_build / phc_peer_reduce_* / phc_episode_fold */
 #define PHC_NUM_BODIES 24      /* SMPL humanoid, body_sets.py:11-36 */
 #define PHC_SELF_OBS_DIM 358   /* envs/humanoid_phc.py:461 */
@@ -52,7 +52,8 @@ enum {
   PHC_ERR_UNSUPPORTED = -4, /* valid in the reference, not implemented here */
   PHC_ERR_CUDA = -5,        /* CUDA runtime error (phc_last_cuda_error() has the code) */
   PHC_ERR_ALLOC = -6,
-  PHC_PEER_TIMEOUT = -7     /* a peer rank did not publish its partials within the timeout */
+  PHC_PEER_TIMEOUT = -7,    /* a peer rank did not publish its partials within the timeout */
+  PHC_ERR_BUSY = -8         /* the host-step slot already has a step in flight */
 };
 
 PHC_API const char* phc_strerror(int code);
@@ -465,10 +466,38 @@ PHC_API int phc_host_step_create(const PhcLib* lib, int64_t max_envs, int32_t ti
                          int32_t use_mean, int32_t enable_early_termination, float dt,
                          const PhcRewardSpec* rwd, PhcHostStep** out);
 PHC_API int phc_host_step(PhcHostStep* ctx, const PhcHostStepArgs* args, int64_t n);
+/* Destroy waits for every slot in flight (as phc_host_step_wait would) before it frees anything. */
 PHC_API void phc_host_step_destroy(PhcHostStep* ctx);
+
+/* Asynchronous form: submit a step on one of PHC_HOST_SLOTS slots, collect it later.  Each slot is a pipeline of its
+ * own (device buffers, pinned staging, three streams), so two batches can be in flight at once: the inbound copy of
+ * one rides under the outbound traffic of the other, and the caller's thread is free between submit and wait (the
+ * send / recv of a double-buffered env loop).
+ *
+ *   submit   Checks everything phc_host_step checks (NULL pointers, 0 <= n <= max_envs, device pointers ->
+ *            PHC_ERR_UNSUPPORTED) and 0 <= slot < PHC_HOST_SLOTS (PHC_ERR_SHAPE), all before anything is enqueued.
+ *            Packs the clock into the slot's pinned staging, enqueues the slot's chunks and returns without waiting.
+ *            The first submit on slot 1 allocates that slot's buffers and may block on the allocation.
+ *   buffers  From submit until wait returns, all 11 buffers of args belong to the library: on the direct path the
+ *            kernels write obs, rewards, flags and progress into them asynchronously, and the copy engine reads state.
+ *   wait     Blocks until the slot's outputs are in the caller's buffers (on the staged path it also unpacks the
+ *            scalar outputs).  Returns PHC_OK, or the step's deferred error (PHC_ERR_CUDA + phc_last_cuda_error()).
+ *            Waiting on an idle slot returns PHC_OK at once.
+ *   busy     A submit to a slot with a step in flight returns PHC_ERR_BUSY, enqueues nothing and leaves the step in
+ *            flight untouched.  phc_host_step is submit + wait on slot 0: it returns PHC_ERR_BUSY while slot 0 is in
+ *            flight and runs normally while only slot 1 is.
+ *   tuning   Only phc_host_step calls made while no slot is in flight count toward the (path, chunks) tuner.  A
+ *            submit uses the settled schedule; before tuning has finished it uses the first candidate (direct, three
+ *            chunks, unless num_chunks / PHC_HOST_PATH narrow it); pageable callers always take the staged path.
+ *   errors   An error inside submit after the first enqueue drains that slot's streams before returning; the other
+ *            slot is not touched.  After any error the slot is idle.
+ *   threads  One host thread drives a context.  Contexts over one PhcLib may be driven from different threads. */
+#define PHC_HOST_SLOTS 2
+PHC_API int phc_host_step_submit(PhcHostStep* ctx, int32_t slot, const PhcHostStepArgs* args, int64_t n);
+PHC_API int phc_host_step_wait(PhcHostStep* ctx, int32_t slot);
 /* The schedule pinned callers are on.  phc_host_step_path: 1 = direct (each chunk's kernel posts obs rows / rewards /
  * flags into the mapped host buffers), 2 = staged (device buffers + copy-engine D2H; always the case for pageable
- * callers), 0 = not decided yet.  phc_host_step_chunks: the chunk count in use (0 = not decided yet).  With
+ * callers; the buffers of the last submit decide), 0 = not decided yet.  phc_host_step_chunks: the chunk count in use (0 = not decided yet).  With
  * num_chunks = 0 at create the context tunes (path, chunk count) over its first phc_host_step_tuning_calls() calls —
  * every candidate timed four times, interleaved, under whatever load the other GPUs of the box put on the host at
  * that moment — and keeps the fastest (three chunks on the direct path unless another schedule is 2 % faster); num_chunks > 0 fixes the chunk count and PHC_HOST_PATH=direct|staged the path. */
