@@ -17,7 +17,7 @@ from .common import (  # noqa: F401
     compute_imitation_reward,
 )
 from .env import HumanoidPHC, build_pd_action_offset_scale  # noqa: F401
-from .host_step import HostStep, HostStepBuffers  # noqa: F401
+from .host_step import HostResetBuffers, HostStep, HostStepBuffers  # noqa: F401
 from .motion_lib import MotionLib  # noqa: F401
 from .puffer_env import PHCPufferEnv  # noqa: F401
 from .running_norm import RunningNorm  # noqa: F401
@@ -37,4 +37,5 @@ __all__ = [
     "build_pd_action_offset_scale",
     "HostStep",
     "HostStepBuffers",
+    "HostResetBuffers",
 ]

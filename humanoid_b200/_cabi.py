@@ -16,7 +16,7 @@ import torch
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libphc_b200.so")
 
-ABI_VERSION = 5
+ABI_VERSION = 6
 NUM_BODIES = 24
 SELF_OBS_DIM = 358
 TASK_OBS_DIM = 576
@@ -248,6 +248,22 @@ class PhcHostStepArgs(C.Structure):
     ]  # fmt: skip
 
 
+class PhcHostResetArgs(C.Structure):
+    _fields_ = [
+        ("phase", C.c_void_p),
+        ("env_mask", C.c_void_p),
+        ("state_init", C.c_int32),
+        ("flag_test", C.c_int32),
+        ("state_out", C.c_void_p),
+        ("root_states", C.c_void_p),
+        ("dof_pos", C.c_void_p),
+        ("dof_vel", C.c_void_p),
+        ("motion_start_times_out", C.c_void_p),
+        ("motion_start_times_offset_out", C.c_void_p),
+        ("global_offset_out", C.c_void_p),
+    ]
+
+
 BUILD_FILTER_RADIUS = 8
 EPISODE_SUM_COLS = 12
 PEER_MAX_WORLD = 16
@@ -323,6 +339,14 @@ SIGNATURES = {
     "phc_host_step_destroy": (None, [C.c_void_p]),
     "phc_host_step_submit": (C.c_int, [C.c_void_p, C.c_int32, C.POINTER(PhcHostStepArgs), C.c_int64]),
     "phc_host_step_wait": (C.c_int, [C.c_void_p, C.c_int32]),
+    "phc_host_step_submit_reset": (
+        C.c_int,
+        [C.c_void_p, C.c_int32, C.POINTER(PhcHostStepArgs), C.POINTER(PhcHostResetArgs), C.c_int64],
+    ),
+    "phc_host_reset_submit": (
+        C.c_int,
+        [C.c_void_p, C.c_int32, C.POINTER(PhcHostStepArgs), C.POINTER(PhcHostResetArgs), C.c_int64],
+    ),
     "phc_host_step_path": (C.c_int, [C.c_void_p]),
     "phc_host_step_chunks": (C.c_int, [C.c_void_p]),
     "phc_host_step_tuning_calls": (C.c_int, [C.c_void_p]),

@@ -22,6 +22,13 @@
 // slot's events and, on the staged path, unpacks the scalar outputs.  With two slots the inbound copy of one batch
 // rides under the outbound traffic of the other (the slots' streams do not queue behind each other), and the caller's
 // thread is free between submit and wait.  phc_host_step is submit + wait on slot 0.
+//
+// Resets.  phc_host_step_submit_reset runs each chunk's step with PhcStepArgs.auto_reset over the chunk's own device
+// copies (sim state, packed clock, per-slot root / dof scratch); phc_host_reset_submit runs phc_reset_envs over them.
+// The uniform numbers and the env mask ride in the chunk's packed clock transfer.  The new state of a re-posed env
+// (~1.9 KB) is not in any buffer the plain step sends back, and only a few percent of the envs are re-posed per step:
+// one small kernel per chunk (host_export_kernel) writes the rows of those envs alone into the caller's buffers when
+// they are pinned, else into the slot's pinned staging, from which wait copies the rows of the flagged envs.
 #include <chrono>
 #include <cstdint>
 #include <cstdio>
@@ -35,6 +42,7 @@
 
 // phc_kernels.cu: phc_step_fused that also writes the advanced progress to a second address
 int step_fused_mirrored(const PhcLib* lib, const PhcStepArgs* args, int64_t n, phc_stream_t stream, int16_t* progress_mirror);
+bool lib_has_dof_state(const PhcLib* lib);  // phc_kernels.cu
 namespace phc {
 int record_cuda_error(int cuda_error);  // phc_kernels.cu; returns PHC_ERR_CUDA
 }
@@ -53,10 +61,11 @@ inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
 // sub-array offsets inside a chunk's packed regions (each 16-B aligned)
 struct Layout {
-  size_t ids, goff, start, soff, prog, clock_bytes;
+  size_t ids, goff, start, soff, prog, phase, mask, clock_bytes;
   size_t rew, raw, oprog, reset, term, out_bytes;
 };
-Layout layout(int64_t m) {
+// with_reset: the clock also carries phase f32 | env_mask u8 per env
+Layout layout(int64_t m, bool with_reset = false) {
   Layout L;
   size_t o = 0;
   L.ids = o, o = align_up(o + (size_t)m * 8, 16);
@@ -64,6 +73,11 @@ Layout layout(int64_t m) {
   L.start = o, o = align_up(o + (size_t)m * 4, 16);
   L.soff = o, o = align_up(o + (size_t)m * 4, 16);
   L.prog = o, o = align_up(o + (size_t)m * 2, 16);
+  L.phase = L.mask = o;
+  if (with_reset) {
+    L.phase = o, o = align_up(o + (size_t)m * 4, 16);
+    L.mask = o, o = align_up(o + (size_t)m, 16);
+  }
   L.clock_bytes = o;
   o = 0;
   L.rew = o, o = align_up(o + (size_t)m * 4, 16);
@@ -73,6 +87,65 @@ Layout layout(int64_t m) {
   L.term = o, o = align_up(o + (size_t)m, 16);
   L.out_bytes = o;
   return L;
+}
+
+enum Op { kStep, kStepReset, kReset };  // phc_host_step(_submit) / phc_host_step_submit_reset / phc_host_reset_submit
+
+// The per-env host arrays a reset writes (rows of re-posed envs only): the caller's buffers, or the slot's staging.
+struct Rows {
+  float *state, *root, *dofp, *dofv, *start, *soff, *goff, *obs;
+  int16_t* prog;
+  uint8_t *rst, *term;
+};
+Rows rows_at(const Rows& R, int64_t lo, int64_t obs_dim) {
+  auto at = [](auto* p, int64_t off) { return p ? p + off : p; };
+  return {at(R.state, lo * kStateFloats), at(R.root, lo * 13), at(R.dofp, lo * 69), at(R.dofv, lo * 69),
+          at(R.start, lo), at(R.soff, lo), at(R.goff, lo * 3), at(R.obs, lo * obs_dim), at(R.prog, lo),
+          at(R.rst, lo), at(R.term, lo)};
+}
+
+// The export of one chunk: every array is chunk-local; `out` points into mapped host memory.
+struct ExportParams {
+  const uint8_t* flag;       // device [m]: env i is exported when set (the step's reset_out, or the reset's env mask)
+  const uint8_t* step_term;  // device [m] or NULL: with it, flag / step_term / prog of EVERY env go to out.rst / .term / .prog
+  const float *state, *root, *dofp, *dofv, *start, *soff, *goff, *obs;  // device; obs may be NULL
+  const int16_t* prog;
+  Rows out;                  // out.obs / .prog / .rst / .term may be NULL (not exported)
+  int zero_flags;            // the host reset: rst / term of exported envs -> 0
+  int64_t obs_dim, m;
+};
+
+__device__ __forceinline__ void warp_copy(float* dst, const float* src, int count, int lane) {
+  for (int j = lane; j < count; j += 32) dst[j] = src[j];
+}
+
+// One warp per env; an env that is not flagged costs one byte read.  A warp's stores are consecutive words, so the
+// rows leave as full 128-B posted writes.
+constexpr int kExportEnvs = 8;
+__global__ void __launch_bounds__(kExportEnvs * 32) host_export_kernel(const ExportParams p) {
+  const int lane = threadIdx.x & 31;
+  if (p.step_term && threadIdx.x < kExportEnvs) {  // the block's flags and progress as one write each
+    const int64_t e = (int64_t)blockIdx.x * kExportEnvs + threadIdx.x;
+    if (e < p.m) {
+      p.out.rst[e] = p.flag[e];
+      p.out.term[e] = p.step_term[e];
+      p.out.prog[e] = p.prog[e];
+    }
+  }
+  const int64_t i = (int64_t)blockIdx.x * kExportEnvs + (threadIdx.x >> 5);
+  if (i >= p.m || !p.flag[i]) return;
+  warp_copy(p.out.state + i * kStateFloats, p.state + i * kStateFloats, kStateFloats, lane);
+  warp_copy(p.out.root + i * 13, p.root + i * 13, 13, lane);
+  warp_copy(p.out.dofp + i * 69, p.dofp + i * 69, 69, lane);
+  warp_copy(p.out.dofv + i * 69, p.dofv + i * 69, 69, lane);
+  warp_copy(p.out.goff + i * 3, p.goff + i * 3, 3, lane);
+  if (p.out.obs) warp_copy(p.out.obs + i * p.obs_dim, p.obs + i * p.obs_dim, (int)p.obs_dim, lane);
+  if (lane == 0) {
+    p.out.start[i] = p.start[i];
+    p.out.soff[i] = p.soff[i];
+    if (p.out.prog && !p.step_term) p.out.prog[i] = p.prog[i];
+    if (p.zero_flags) p.out.rst[i] = p.out.term[i] = 0;
+  }
 }
 
 // One pipeline: what a step in flight uses, and what phc_host_step_wait needs to finish it.
@@ -89,10 +162,23 @@ struct Slot {
   // direct path: verdict cached per set of caller pointers
   const void* seen[11] = {};
   int seen_direct = -1;
+  // resets, allocated at the first submit that needs them: device root / dof rows of re-posed envs and the flags the
+  // reset clears (the caller gets the step's own flags), [max_envs] each; pinned staging of the reset outputs
+  unsigned char* d_reset = nullptr;
+  float *d_root = nullptr, *d_dofp = nullptr, *d_dofv = nullptr;
+  uint8_t *d_kreset = nullptr, *d_kterm = nullptr;
+  unsigned char* h_rows = nullptr;
+  Rows stage{};
+  const void* rseen[9] = {};  // verdict of the reset pointers: the outputs are all pinned and mapped at their address
+  int rseen_direct = -1;
   // the step in flight
   bool busy = false;
   int path = 0;  // 1 direct, 2 staged
+  int op = kStep;
+  bool rows_staged = false;  // the reset rows go through `stage`, wait copies those of the flagged envs
+  int64_t n = 0;
   PhcHostStepArgs args{};
+  PhcHostResetArgs rargs{};
   int nchunks = 0;
   int64_t bounds[kMaxChunks + 2] = {};  // staged path: chunk boundaries, for the unpack in wait
 };
@@ -168,8 +254,10 @@ static void slot_free(Slot& s) {
   cudaFree(s.d_obs);
   cudaFree(s.d_clock);
   cudaFree(s.d_out);
+  cudaFree(s.d_reset);
   if (s.h_clock) cudaFreeHost(s.h_clock);
   if (s.h_out) cudaFreeHost(s.h_out);
+  if (s.h_rows) cudaFreeHost(s.h_rows);
   for (int i = 0; i < kStreams; ++i) {
     if (s.done[i]) cudaEventDestroy(s.done[i]);
     if (s.streams[i]) cudaStreamDestroy(s.streams[i]);
@@ -207,7 +295,146 @@ static int check_args(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, int64_t
   return PHC_OK;
 }
 
-static int direct_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, int64_t n, const int chunks) {
+// Everything the two reset submits validate on top of check_args; fills the slot's verdict for the reset outputs.
+static int check_reset(const PhcHostStep* c, Slot& s, const PhcHostResetArgs* r, int op) {
+  if (!r->state_out || !r->root_states || !r->dof_pos || !r->dof_vel || !r->motion_start_times_out ||
+      !r->motion_start_times_offset_out || !r->global_offset_out || (op == kReset && !r->env_mask))
+    return PHC_ERR_NULL;
+  // StateInit.Default / Hybrid need the per-env initial_* buffers on the device: not on this path
+  if (r->state_init != PHC_STATE_INIT_START && r->state_init != PHC_STATE_INIT_RANDOM) return PHC_ERR_UNSUPPORTED;
+  if (r->state_init == PHC_STATE_INIT_RANDOM && !r->phase) return PHC_ERR_NULL;
+  if (!lib_has_dof_state(c->lib)) return PHC_ERR_UNSUPPORTED;
+  // outputs first (their verdict), then the two inputs the CPU packs (only refused when on the device)
+  const void* ptrs[9] = {r->state_out, r->root_states, r->dof_pos, r->dof_vel, r->motion_start_times_out,
+                         r->motion_start_times_offset_out, r->global_offset_out, r->phase, r->env_mask};
+  if (s.rseen_direct < 0 || memcmp(ptrs, s.rseen, sizeof(ptrs)) != 0) {
+    int direct = 1;
+    for (int i = 0; i < 9; ++i) {
+      if (!ptrs[i]) continue;
+      cudaPointerAttributes at{};
+      if (cudaPointerGetAttributes(&at, ptrs[i]) != cudaSuccess) {
+        (void)cudaGetLastError();
+        if (i < 7) direct = 0;
+      } else if (at.type == cudaMemoryTypeDevice) {
+        return PHC_ERR_UNSUPPORTED;
+      } else if (i < 7 && ((at.type != cudaMemoryTypeHost && at.type != cudaMemoryTypeManaged) || at.devicePointer != ptrs[i])) {
+        direct = 0;
+      }
+    }
+    memcpy(s.rseen, ptrs, sizeof(ptrs));
+    s.rseen_direct = direct;
+  }
+  return PHC_OK;
+}
+
+// The reset scratch of a slot; the pinned staging only when the rows of this submit go through it.
+static cudaError_t reset_alloc(const PhcHostStep* c, Slot& s, bool staging) {
+  const size_t n = (size_t)c->max_envs;
+  cudaError_t e = cudaSuccess;
+  if (!s.d_reset) {
+    e = cudaMalloc((void**)&s.d_reset, n * (13 + 69 + 69) * sizeof(float) + 2 * n);
+    if (e != cudaSuccess) return e;
+    s.d_root = (float*)s.d_reset;
+    s.d_dofp = s.d_root + n * 13;
+    s.d_dofv = s.d_dofp + n * 69;
+    s.d_kreset = (uint8_t*)(s.d_dofv + n * 69);
+    s.d_kterm = s.d_kreset + n;
+  }
+  if (staging && !s.h_rows) {
+    const size_t floats[8] = {n * kStateFloats, n * 13, n * 69, n * 69, n, n, n * 3, n * (size_t)c->obs_dim};
+    size_t off[8], o = 0;
+    for (int i = 0; i < 8; ++i) off[i] = o, o = align_up(o + floats[i] * sizeof(float), 16);
+    const size_t prog = o, rst = align_up(prog + n * 2, 16), term = rst + n;
+    e = cudaMallocHost((void**)&s.h_rows, term + n);
+    if (e != cudaSuccess) return e;
+    float* f[8];
+    for (int i = 0; i < 8; ++i) f[i] = (float*)(s.h_rows + off[i]);
+    s.stage = Rows{f[0], f[1], f[2], f[3], f[4], f[5], f[6], f[7], (int16_t*)(s.h_rows + prog), s.h_rows + rst,
+                   s.h_rows + term};
+  }
+  return e;
+}
+
+// The caller's buffers as export targets
+static Rows caller_rows(const PhcHostStepArgs* a, const PhcHostResetArgs* r) {
+  return {r->state_out, r->root_states, r->dof_pos, r->dof_vel, r->motion_start_times_out,
+          r->motion_start_times_offset_out, r->global_offset_out, a->obs_buf, a->progress_buf, a->reset_buf,
+          a->terminate_buf};
+}
+
+static PhcBodyState chunk_body(float* st) {
+  return PhcBodyState{PhcView{st, kStateFloats, 13}, PhcView{st + 3, kStateFloats, 13}, PhcView{st + 7, kStateFloats, 13},
+                      PhcView{st + 10, kStateFloats, 13}, PHC_NUM_BODIES};
+}
+
+// Packs a chunk's clock (and, with a reset, its uniform numbers and env mask) into pinned staging.
+static void pack_clock(unsigned char* hc, const Layout& L, const PhcHostStepArgs* a, const PhcHostResetArgs* r,
+                       int64_t lo, int64_t m) {
+  memcpy(hc + L.ids, a->sampled_motion_ids + lo, (size_t)m * 8);
+  memcpy(hc + L.goff, a->global_offset + lo * 3, (size_t)m * 12);
+  memcpy(hc + L.start, a->motion_start_times + lo, (size_t)m * 4);
+  memcpy(hc + L.soff, a->motion_start_times_offset + lo, (size_t)m * 4);
+  memcpy(hc + L.prog, a->progress_buf + lo, (size_t)m * 2);
+  if (r && r->phase) memcpy(hc + L.phase, r->phase + lo, (size_t)m * 4);
+  if (r && r->env_mask) memcpy(hc + L.mask, r->env_mask + lo, (size_t)m);
+}
+
+// The reset over a chunk's device copies.  A step's auto_reset must name the step's own body / clock / flag / obs
+// pointers (phc_step_fused checks it), so both are derived from the same chunk offsets.
+static PhcResetArgs chunk_reset_args(const PhcHostStep* c, const Slot& s, const PhcHostResetArgs* r, float* st,
+                                     unsigned char* dc, const Layout& L, int64_t lo, float* obs) {
+  PhcResetArgs ra{};
+  ra.body = chunk_body(st);
+  ra.humanoid_root_states = s.d_root + lo * 13;
+  ra.root_stride = 13;
+  ra.dof_pos = s.d_dofp + lo * 69;
+  ra.dof_vel = s.d_dofv + lo * 69;
+  ra.dof_stride = 69;
+  ra.dof_elem_stride = 1;
+  ra.progress_buf = (int16_t*)(dc + L.prog);
+  ra.reset_buf = s.d_kreset + lo;
+  ra.terminate_buf = s.d_kterm + lo;
+  ra.motion_start_times = (float*)(dc + L.start);
+  ra.motion_start_times_offset = (float*)(dc + L.soff);
+  ra.global_offset = (float*)(dc + L.goff);
+  ra.sampled_motion_ids = (const int64_t*)(dc + L.ids);
+  ra.env_mask = dc + L.mask;
+  ra.phase = r->phase ? (const float*)(dc + L.phase) : nullptr;
+  ra.state_init = r->state_init;
+  ra.flag_test = r->flag_test;
+  ra.time_steps = c->T;
+  ra.dt = c->dt;
+  ra.obs_buf = obs;
+  ra.obs_stride = c->obs_dim;
+  return ra;
+}
+
+// The export of the reset rows of one chunk whose device copies `ra` names.
+static cudaError_t export_rows(const PhcHostStep* c, const PhcResetArgs& ra, const uint8_t* flag,
+                               const uint8_t* step_term, const float* obs, const Rows& out, int zero_flags, int64_t m,
+                               cudaStream_t st) {
+  ExportParams p{};
+  p.flag = flag;
+  p.step_term = step_term;
+  p.state = ra.body.pos.ptr;
+  p.root = ra.humanoid_root_states;
+  p.dofp = ra.dof_pos;
+  p.dofv = ra.dof_vel;
+  p.start = ra.motion_start_times;
+  p.soff = ra.motion_start_times_offset;
+  p.goff = ra.global_offset;
+  p.obs = obs;
+  p.prog = ra.progress_buf;
+  p.out = out;
+  p.zero_flags = zero_flags;
+  p.obs_dim = c->obs_dim;
+  p.m = m;
+  host_export_kernel<<<(unsigned)((m + kExportEnvs - 1) / kExportEnvs), kExportEnvs * 32, 0, st>>>(p);
+  return cudaGetLastError();
+}
+
+static int direct_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, const PhcHostResetArgs* r, int64_t n,
+                          const int chunks) {
   // Hybrid: everything INBOUND rides the host->device copy engine in a few chunks — the sim
   // rows directly from the caller's buffer, the five small clock arrays packed into one
   // transfer (SM-issued reads of system memory are 32-B PCIe round trips: 6 per block, ~70 us
@@ -220,8 +447,10 @@ static int direct_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, int
   const int C = chunks < 1 ? 1 : chunks;
   int64_t per = (n + C - 1) / C;
   per = (per + 7) / 8 * 8;
-  size_t coff = 0;
+  size_t coff = 0, ooff = 0;
   int ci = 0;
+  // with a reset the step's own flags go to device scratch (the export kernel posts them to the caller with the rows)
+  const Rows rows = r ? (s.rows_staged ? s.stage : caller_rows(a, r)) : Rows{};
   static const bool trace_on = getenv("PHC_HOST_TRACE") != nullptr;
   static int trace_calls = 0;
   const bool trace = trace_on && ++trace_calls == 20;
@@ -234,17 +463,15 @@ static int direct_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, int
   }
   for (int64_t lo = 0; lo < n; lo += per, ++ci) {
     const int64_t m = (n - lo) < per ? (n - lo) : per;
-    const Layout L = layout(m);
-    if (coff + L.clock_bytes > c->pack_capacity) return host_fail(s, PHC_ERR_SHAPE, cudaSuccess);
+    const Layout L = layout(m, r != nullptr);
+    if (coff + L.clock_bytes > c->pack_capacity || ooff + L.out_bytes > c->pack_capacity)
+      return host_fail(s, PHC_ERR_SHAPE, cudaSuccess);
     cudaStream_t st_ = s.streams[ci % kStreams];
     float* st = s.d_state + lo * kStateFloats;
     unsigned char* hc = s.h_clock + coff;
     unsigned char* dc = s.d_clock + coff;
-    memcpy(hc + L.ids, a->sampled_motion_ids + lo, (size_t)m * 8);
-    memcpy(hc + L.goff, a->global_offset + lo * 3, (size_t)m * 12);
-    memcpy(hc + L.start, a->motion_start_times + lo, (size_t)m * 4);
-    memcpy(hc + L.soff, a->motion_start_times_offset + lo, (size_t)m * 4);
-    memcpy(hc + L.prog, a->progress_buf + lo, (size_t)m * 2);
+    unsigned char* dout = s.d_out + ooff;
+    pack_clock(hc, L, a, r, lo, m);
     HOST_CUDA(s, cudaMemcpyAsync(dc, hc, L.clock_bytes, cudaMemcpyHostToDevice, st_));
     HOST_CUDA(s, cudaMemcpyAsync(st, a->state + lo * kStateFloats, (size_t)m * kStateFloats * sizeof(float),
                                  cudaMemcpyHostToDevice, st_));
@@ -253,11 +480,7 @@ static int direct_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, int
       cudaEventCreate(&evh[ci]);
       cudaEventRecord(evh[ci], st_);
     }
-    k.body.pos = PhcView{st, kStateFloats, 13};
-    k.body.rot = PhcView{st + 3, kStateFloats, 13};
-    k.body.vel = PhcView{st + 7, kStateFloats, 13};
-    k.body.ang_vel = PhcView{st + 10, kStateFloats, 13};
-    k.body.num_bodies = PHC_NUM_BODIES;
+    k.body = chunk_body(st);
     k.progress_buf = (int16_t*)(dc + L.prog);
     k.motion_start_times = (const float*)(dc + L.start);
     k.motion_start_times_offset = (const float*)(dc + L.soff);
@@ -280,9 +503,29 @@ static int direct_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, int
     k.terminate_buf = a->terminate_buf + lo;
     k.flags = PHC_STEP_MAPPED_HOST_IO;
     k.obs_moments = nullptr;
-    // the advanced progress goes straight into the caller's buffer too (no device->host copy at the tail)
-    int rc = step_fused_mirrored(c->lib, &k, m, st_, a->progress_buf + lo);
+    PhcResetArgs ra;
+    if (r) {
+      k.reset_buf = s.d_kreset + lo;
+      k.terminate_buf = s.d_kterm + lo;
+      k.reset_out = dout + L.reset;
+      k.terminate_out = dout + L.term;
+      ra = chunk_reset_args(c, s, r, st, dc, L, lo, k.obs_buf);
+      k.auto_reset = &ra;
+    }
+    // the advanced progress goes straight into the caller's buffer too (no device->host copy at the tail).  Not with a
+    // reset: where it runs as a second launch (T > 1 here, or the generic kernel) the mirror would keep the advanced
+    // progress of the re-posed envs, so the progress leaves with the flags, from the device clock after the reset.
+    int rc = step_fused_mirrored(c->lib, &k, m, st_, r ? nullptr : a->progress_buf + lo);
     if (rc) return host_fail(s, rc, cudaSuccess);
+    if (r) {
+      Rows out = rows_at(rows, lo, c->obs_dim);
+      out.obs = nullptr;
+      out.prog = a->progress_buf + lo;
+      out.rst = a->reset_buf + lo;
+      out.term = a->terminate_buf + lo;
+      HOST_CUDA(s, export_rows(c, ra, dout + L.reset, dout + L.term, nullptr, out, 0, m, st_));
+      ooff += L.out_bytes;
+    }
     if (trace && ci < 64) {
       cudaEventCreate(&evk[ci]);
       cudaEventRecord(evk[ci], st_);
@@ -305,7 +548,8 @@ static int direct_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, int
   return PHC_OK;
 }
 
-static int staged_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, int64_t n, const int chunks) {
+static int staged_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, const PhcHostResetArgs* r, int64_t n,
+                          const int chunks) {
   const cudaMemcpyKind H2D = cudaMemcpyHostToDevice, D2H = cudaMemcpyDeviceToHost;
   // Chunk sizes double (n/2^(C-1), n/2^(C-1), n/2^(C-2), .., n/2): the device->host direction
   // carries 3x the bytes and is the bottleneck, so the first chunk is small to start it early
@@ -331,6 +575,7 @@ static int staged_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, int
   const int64_t* bounds = s.bounds;
 
   size_t coff = 0, ooff = 0;
+  const Rows rows = r ? (s.rows_staged ? s.stage : caller_rows(a, r)) : Rows{};
   static const bool strace_on = getenv("PHC_HOST_TRACE") != nullptr;
   static int strace_calls = 0;
   const bool strace = strace_on && ++strace_calls == 20;
@@ -342,17 +587,13 @@ static int staged_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, int
   for (int ci = 0; ci < nchunks; ++ci) {
     const int64_t lo = bounds[ci], m = bounds[ci + 1] - bounds[ci];
     if (m <= 0) continue;
-    const Layout L = layout(m);
+    const Layout L = layout(m, r != nullptr);
     if (coff + L.clock_bytes > c->pack_capacity || ooff + L.out_bytes > c->pack_capacity)
       return host_fail(s, PHC_ERR_SHAPE, cudaSuccess);
     cudaStream_t st_ = s.streams[ci % kStreams];
     // pack the chunk's clock on the host (tens of KB), then ONE transfer
     unsigned char* hc = s.h_clock + coff;
-    memcpy(hc + L.ids, a->sampled_motion_ids + lo, (size_t)m * 8);
-    memcpy(hc + L.goff, a->global_offset + lo * 3, (size_t)m * 12);
-    memcpy(hc + L.start, a->motion_start_times + lo, (size_t)m * 4);
-    memcpy(hc + L.soff, a->motion_start_times_offset + lo, (size_t)m * 4);
-    memcpy(hc + L.prog, a->progress_buf + lo, (size_t)m * 2);
+    pack_clock(hc, L, a, r, lo, m);
     unsigned char* dc = s.d_clock + coff;
     unsigned char* dout = s.d_out + ooff;
     HOST_CUDA(s, cudaMemcpyAsync(s.d_state + lo * kStateFloats, a->state + lo * kStateFloats,
@@ -361,11 +602,7 @@ static int staged_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, int
 
     PhcStepArgs k{};
     float* st = s.d_state + lo * kStateFloats;
-    k.body.pos = PhcView{st, kStateFloats, 13};
-    k.body.rot = PhcView{st + 3, kStateFloats, 13};
-    k.body.vel = PhcView{st + 7, kStateFloats, 13};
-    k.body.ang_vel = PhcView{st + 10, kStateFloats, 13};
-    k.body.num_bodies = PHC_NUM_BODIES;
+    k.body = chunk_body(st);
     k.progress_buf = (int16_t*)(dc + L.prog);
     k.motion_start_times = (const float*)(dc + L.start);
     k.motion_start_times_offset = (const float*)(dc + L.soff);
@@ -387,12 +624,28 @@ static int staged_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, int
     k.reset_buf = dout + L.reset;
     k.terminate_buf = dout + L.term;
     k.obs_moments = nullptr;
+    PhcResetArgs ra;
+    if (r) {  // the step's own flags still leave in the packed scalars
+      k.reset_buf = s.d_kreset + lo;
+      k.terminate_buf = s.d_kterm + lo;
+      k.reset_out = dout + L.reset;
+      k.terminate_out = dout + L.term;
+      ra = chunk_reset_args(c, s, r, st, dc, L, lo, k.obs_buf);
+      k.auto_reset = &ra;
+    }
     if (strace && ci < 16) {
       cudaEventCreate(&sevh[ci]);
       cudaEventRecord(sevh[ci], st_);
     }
     int rc = phc_step_fused(c->lib, &k, m, st_);
     if (rc) return host_fail(s, rc, cudaSuccess);
+    if (r) {
+      Rows out = rows_at(rows, lo, c->obs_dim);
+      out.obs = nullptr;
+      out.prog = nullptr;
+      out.rst = out.term = nullptr;
+      HOST_CUDA(s, export_rows(c, ra, dout + L.reset, nullptr, nullptr, out, 0, m, st_));
+    }
     if (strace && ci < 16) {
       cudaEventCreate(&sevk[ci]);
       cudaEventRecord(sevk[ci], st_);
@@ -424,21 +677,81 @@ static int staged_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, int
   return PHC_OK;
 }
 
-// Enqueues one step on a slot (arguments already checked) and marks it in flight.
-static int slot_enqueue(PhcHostStep* c, int slot, const PhcHostStepArgs* a, int64_t n, const PhcHostStep::Cand& k) {
+// The host reset: H2D(packed clock + phase + mask) -> phc_reset_envs -> export of the masked envs' rows (obs included)
+// on equal chunks.  Nothing else is read or written: no sim state comes in, no whole obs chunk goes out.
+static int reset_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, const PhcHostResetArgs* r, int64_t n,
+                         const int chunks) {
+  const int C = chunks < 1 ? 1 : chunks;
+  int64_t per = (n + C - 1) / C;
+  per = (per + 7) / 8 * 8;
+  const Rows rows = s.rows_staged ? s.stage : caller_rows(a, r);
+  size_t coff = 0;
+  int ci = 0;
+  for (int64_t lo = 0; lo < n; lo += per, ++ci) {
+    const int64_t m = (n - lo) < per ? (n - lo) : per;
+    const Layout L = layout(m, true);
+    if (coff + L.clock_bytes > c->pack_capacity) return host_fail(s, PHC_ERR_SHAPE, cudaSuccess);
+    cudaStream_t st_ = s.streams[ci % kStreams];
+    unsigned char* hc = s.h_clock + coff;
+    unsigned char* dc = s.d_clock + coff;
+    pack_clock(hc, L, a, r, lo, m);
+    HOST_CUDA(s, cudaMemcpyAsync(dc, hc, L.clock_bytes, cudaMemcpyHostToDevice, st_));
+    float* obs = s.d_obs + lo * c->obs_dim;
+    const PhcResetArgs ra = chunk_reset_args(c, s, r, s.d_state + lo * kStateFloats, dc, L, lo, obs);
+    const int rc = phc_reset_envs(c->lib, &ra, m, st_);
+    if (rc) return host_fail(s, rc, cudaSuccess);
+    HOST_CUDA(s, export_rows(c, ra, dc + L.mask, nullptr, obs, rows_at(rows, lo, c->obs_dim), 1, m, st_));
+    coff += L.clock_bytes;
+  }
+  return PHC_OK;
+}
+
+// Enqueues one step (or reset) on a slot (arguments already checked) and marks it in flight.
+static int slot_enqueue(PhcHostStep* c, int slot, const PhcHostStepArgs* a, const PhcHostResetArgs* r, int op,
+                        int64_t n, const PhcHostStep::Cand& k) {
   Slot& s = c->slots[slot];
-  const int rc = k.path == 1 ? direct_enqueue(c, s, a, n, k.chunks) : staged_enqueue(c, s, a, n, k.chunks);
+  const int rc = op == kReset   ? reset_enqueue(c, s, a, r, n, k.chunks)
+                 : k.path == 1 ? direct_enqueue(c, s, a, r, n, k.chunks)
+                               : staged_enqueue(c, s, a, r, n, k.chunks);
   if (rc) return rc;
   for (int i = 0; i < kStreams; ++i) HOST_CUDA(s, cudaEventRecord(s.done[i], s.streams[i]));
   s.args = *a;
+  s.rargs = r ? *r : PhcHostResetArgs{};
+  s.op = op;
+  s.n = n;
   s.path = k.path;
   s.busy = true;
   c->last_slot = slot;
   return PHC_OK;
 }
 
-// Waits for a slot's step; on the staged path unpacks the scalar outputs into the caller's buffers.
-static int slot_finish(Slot& s) {
+// The reset rows of the flagged envs (the step's reset flags, or the reset's env mask), from the slot's staging into
+// the caller's buffers.
+static void unpack_rows(const PhcHostStep* c, const Slot& s) {
+  const Rows src = s.stage, dst = caller_rows(&s.args, &s.rargs);
+  const uint8_t* flag = s.op == kReset ? s.rargs.env_mask : s.args.reset_buf;
+  const size_t D = (size_t)c->obs_dim;
+  for (int64_t i = 0; i < s.n; ++i) {
+    if (!flag[i]) continue;
+    memcpy(dst.state + i * kStateFloats, src.state + i * kStateFloats, kStateFloats * sizeof(float));
+    memcpy(dst.root + i * 13, src.root + i * 13, 13 * sizeof(float));
+    memcpy(dst.dofp + i * 69, src.dofp + i * 69, 69 * sizeof(float));
+    memcpy(dst.dofv + i * 69, src.dofv + i * 69, 69 * sizeof(float));
+    memcpy(dst.goff + i * 3, src.goff + i * 3, 3 * sizeof(float));
+    dst.start[i] = src.start[i];
+    dst.soff[i] = src.soff[i];
+    if (s.op == kReset) {
+      memcpy(dst.obs + i * D, src.obs + i * D, D * sizeof(float));
+      dst.prog[i] = src.prog[i];
+      dst.rst[i] = src.rst[i];
+      dst.term[i] = src.term[i];
+    }
+  }
+}
+
+// Waits for a slot's step; on the staged path unpacks the scalar outputs into the caller's buffers, and the reset rows
+// that went through staging.
+static int slot_finish(const PhcHostStep* c, Slot& s) {
   if (!s.busy) return PHC_OK;
   s.busy = false;
   cudaError_t err = cudaSuccess;
@@ -447,21 +760,23 @@ static int slot_finish(Slot& s) {
     if (err == cudaSuccess) err = e;
   }
   if (err != cudaSuccess) return host_fail(s, PHC_ERR_CUDA, err);
-  if (s.path != 2) return PHC_OK;
-  const PhcHostStepArgs* a = &s.args;
-  size_t ooff = 0;
-  for (int ci = 0; ci < s.nchunks; ++ci) {
-    const int64_t lo = s.bounds[ci], m = s.bounds[ci + 1] - s.bounds[ci];
-    if (m <= 0) continue;
-    const Layout L = layout(m);
-    const unsigned char* ho = s.h_out + ooff;
-    memcpy(a->rew_buf + lo, ho + L.rew, (size_t)m * 4);
-    memcpy(a->reward_raw + lo * 4, ho + L.raw, (size_t)m * 16);
-    memcpy(a->progress_buf + lo, ho + L.oprog, (size_t)m * 2);
-    memcpy(a->reset_buf + lo, ho + L.reset, (size_t)m);
-    memcpy(a->terminate_buf + lo, ho + L.term, (size_t)m);
-    ooff += L.out_bytes;
+  if (s.path == 2 && s.op != kReset) {
+    const PhcHostStepArgs* a = &s.args;
+    size_t ooff = 0;
+    for (int ci = 0; ci < s.nchunks; ++ci) {
+      const int64_t lo = s.bounds[ci], m = s.bounds[ci + 1] - s.bounds[ci];
+      if (m <= 0) continue;
+      const Layout L = layout(m, s.op != kStep);
+      const unsigned char* ho = s.h_out + ooff;
+      memcpy(a->rew_buf + lo, ho + L.rew, (size_t)m * 4);
+      memcpy(a->reward_raw + lo * 4, ho + L.raw, (size_t)m * 16);
+      memcpy(a->progress_buf + lo, ho + L.oprog, (size_t)m * 2);
+      memcpy(a->reset_buf + lo, ho + L.reset, (size_t)m);
+      memcpy(a->terminate_buf + lo, ho + L.term, (size_t)m);
+      ooff += L.out_bytes;
+    }
   }
+  if (s.op != kStep && s.rows_staged) unpack_rows(c, s);
   return PHC_OK;
 }
 
@@ -473,8 +788,8 @@ static PhcHostStep::Cand untimed_schedule(const PhcHostStep* c, const Slot& s) {
 }
 
 static int run_sync(PhcHostStep* c, const PhcHostStepArgs* a, int64_t n, const PhcHostStep::Cand& k) {
-  const int rc = slot_enqueue(c, 0, a, n, k);
-  return rc ? rc : slot_finish(c->slots[0]);
+  const int rc = slot_enqueue(c, 0, a, nullptr, kStep, n, k);
+  return rc ? rc : slot_finish(c, c->slots[0]);
 }
 
 extern "C" {
@@ -482,7 +797,7 @@ extern "C" {
 void phc_host_step_destroy(PhcHostStep* c) {
   if (!c) return;
   for (auto& s : c->slots) {
-    (void)slot_finish(s);  // a pending DMA or posting kernel must not land in freed memory
+    (void)slot_finish(c, s);  // a pending DMA or posting kernel must not land in freed memory
     slot_free(s);
   }
   cudaFree(c->term_dist);
@@ -510,8 +825,8 @@ int phc_host_step_create(const PhcLib* lib, int64_t max_envs, int32_t time_steps
   if (const char* m = getenv("PHC_HOST_PATH")) c->mode = !strcmp(m, "direct") ? 1 : !strcmp(m, "staged") ? 2 : 0;
   if (getenv("PHC_HOST_STAGED")) c->mode = 2;
   const size_t n = (size_t)max_envs;
-  // every chunk's packed region is padded so each sub-array starts 16-B aligned
-  c->pack_capacity = n * 32 + (size_t)(num_chunks > 8 ? num_chunks : 8) * 6 * 64 + 4096;
+  // every chunk's packed region is padded so each sub-array starts 16-B aligned (35 B per env with a reset's clock)
+  c->pack_capacity = n * 40 + (size_t)(num_chunks > 8 ? num_chunks : 8) * 8 * 64 + 4096;
   {  // candidates: direct with 2 / 3 / 4 / 6 equal chunks, staged with 3 / 4 doubling chunks
     static const int direct_chunks[] = {3, 4, 2, 6}, staged_chunks[] = {3, 4};
     auto add = [&](int path, int chunks) {
@@ -596,29 +911,55 @@ int phc_host_step(PhcHostStep* c, const PhcHostStepArgs* a, int64_t n) {
   return rc;
 }
 
-int phc_host_step_submit(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, int64_t n) {
-  if (!c || !a) return PHC_ERR_NULL;
+}  // extern "C"
+
+// The three submits: every check before anything is enqueued, then the slot's buffers, then the enqueue.
+static int submit(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, const PhcHostResetArgs* r, int op, int64_t n) {
+  if (!c || !a || (op != kStep && !r)) return PHC_ERR_NULL;
   if (slot < 0 || slot >= PHC_HOST_SLOTS) return PHC_ERR_SHAPE;
   Slot& s = c->slots[slot];
   if (s.busy) return PHC_ERR_BUSY;
   if (n == 0) return PHC_OK;
-  const int rc = check_args(c, s, a, n);
+  int rc = check_args(c, s, a, n);
   if (rc) return rc;
+  if (op != kStep && (rc = check_reset(c, s, r, op))) return rc;
+  cudaError_t e = cudaSuccess;
   if (!s.ready) {
-    const cudaError_t e = slot_alloc(c, s);
-    if (e != cudaSuccess) {
-      slot_free(s);
-      (void)cudaGetLastError();
-      return e == cudaErrorMemoryAllocation ? PHC_ERR_ALLOC : phc::record_cuda_error((int)e);
-    }
+    e = slot_alloc(c, s);
+    if (e != cudaSuccess) slot_free(s);
   }
-  return slot_enqueue(c, slot, a, n, untimed_schedule(c, s));
+  if (op != kStep && e == cudaSuccess) {
+    // the host reset writes the step buffers' rows too (obs, progress, flags): straight only when they are pinned as well
+    s.rows_staged = !s.rseen_direct || (op == kReset && s.seen_direct != 1);
+    e = reset_alloc(c, s, s.rows_staged);
+  }
+  if (e != cudaSuccess) {
+    (void)cudaGetLastError();
+    return e == cudaErrorMemoryAllocation ? PHC_ERR_ALLOC : phc::record_cuda_error((int)e);
+  }
+  return slot_enqueue(c, slot, a, r, op, n, untimed_schedule(c, s));
+}
+
+extern "C" {
+
+int phc_host_step_submit(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, int64_t n) {
+  return submit(c, slot, a, nullptr, kStep, n);
+}
+
+int phc_host_step_submit_reset(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, const PhcHostResetArgs* r,
+                               int64_t n) {
+  return submit(c, slot, a, r, kStepReset, n);
+}
+
+int phc_host_reset_submit(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, const PhcHostResetArgs* r,
+                          int64_t n) {
+  return submit(c, slot, a, r, kReset, n);
 }
 
 int phc_host_step_wait(PhcHostStep* c, int32_t slot) {
   if (!c) return PHC_ERR_NULL;
   if (slot < 0 || slot >= PHC_HOST_SLOTS) return PHC_ERR_SHAPE;
-  return slot_finish(c->slots[slot]);
+  return slot_finish(c, c->slots[slot]);
 }
 
 int phc_host_step_path(const PhcHostStep* c) {

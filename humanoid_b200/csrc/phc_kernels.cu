@@ -4231,6 +4231,9 @@ int step_fused_mirrored(const PhcLib* lib, const PhcStepArgs* args, int64_t n, p
   return rc;
 }
 
+// the host reset path always writes dof_pos / dof_vel: it needs the library's local rotations and dof velocities
+bool lib_has_dof_state(const PhcLib* lib) { return lib && lib->d.lrs && lib->d.dvs; }
+
 extern "C" {
 
 int phc_step_fused(const PhcLib* lib, const PhcStepArgs* args, int64_t n, phc_stream_t stream) {

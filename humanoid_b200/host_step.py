@@ -6,6 +6,11 @@ asynchronous form over two slots: submit a batch, do other work (run the policy 
 From ``submit`` until ``wait`` the library writes into the batch's tensors, so the wrapper holds them until then:
 a caller that drops its own references cannot free a pinned buffer under a DMA or a posting kernel.
 
+With ``reset=HostResetBuffers`` a step also re-poses the envs it flags (``HumanoidPHC.step()`` with auto-reset), and
+``reset_submit`` / ``reset`` re-pose the envs of a mask (``HumanoidPHC.reset(env_ids, phase)``): a host env loop is
+``reset`` of every env once, then ``submit(slot, bufs, reset=...)`` / ``wait(slot)`` per batch; after each ``wait`` the
+caller's physics takes the root and dof state of the envs in ``bufs.reset_buf`` from the reset buffers.
+
 Pinned buffers (``HostStepBuffers.allocate(..., pinned=True)``) take the fast paths; pageable ones work through
 staging.  The CUDA device of the motion library must be current when the context is created and stepped; after
 ``MotionLib.repack()`` synchronise the device before the next host step (the steps run on the context's own streams).
@@ -90,6 +95,74 @@ class HostStepBuffers:
         return _cabi.PhcHostStepArgs(*[getattr(self, f.name).data_ptr() for f in fields(self)])
 
 
+_RESET_FIELDS = (  # name, dtype, trailing shape
+    ("phase", torch.float32, ()),
+    ("root_states", torch.float32, (13,)),
+    ("dof_pos", torch.float32, (69,)),
+    ("dof_vel", torch.float32, (69,)),
+)
+_STATE_INIT = {"start": _cabi.STATE_INIT_START, "random": _cabi.STATE_INIT_RANDOM,
+               "default": _cabi.STATE_INIT_DEFAULT, "hybrid": _cabi.STATE_INIT_HYBRID}  # fmt: skip
+
+
+@dataclass(eq=False)
+class HostResetBuffers:
+    """The CPU tensors a reset on the host path reads and writes besides a ``HostStepBuffers``.  Input: ``phase`` [n]
+    f32, the uniform [0, 1) numbers of ``sample_time_interval`` (state init "random"), and for ``reset_submit`` the
+    ``env_mask`` [n] (uint8 or bool, 1 = reset the env).  Outputs, written for the re-posed envs only:
+    ``root_states`` [n, 13] (pos 3 | rot 4 | vel 3 | ang vel 3) and ``dof_pos`` / ``dof_vel`` [n, 69] — what the
+    caller's physics sets for those envs.  The rigid-body rows and the new clock go into the ``HostStepBuffers``'
+    own ``state`` and clock tensors."""
+
+    phase: torch.Tensor
+    root_states: torch.Tensor
+    dof_pos: torch.Tensor
+    dof_vel: torch.Tensor
+    env_mask: Optional[torch.Tensor] = None
+
+    @classmethod
+    def allocate(cls, n: int, pinned: bool = True) -> "HostResetBuffers":
+        """Zeroed buffers for ``n`` envs (with a zeroed ``env_mask``); ``pinned`` page-locks them."""
+
+        def make(dtype, trailing):
+            t = torch.zeros((n, *trailing), dtype=dtype)
+            return t.pin_memory() if pinned else t
+
+        return cls(**{name: make(dtype, shape) for name, dtype, shape in _RESET_FIELDS}, env_mask=make(torch.uint8, ()))
+
+    @property
+    def n(self) -> int:
+        return int(self.phase.shape[0])
+
+    def validate(self, n: Optional[int] = None) -> int:
+        """Checks device (CPU), dtype, shape and contiguity of every tensor (``n`` rows: the batch's); returns ``n``."""
+        n = self.n if n is None else int(n)
+        fields_ = [(name, (dtype,), shape) for name, dtype, shape in _RESET_FIELDS]
+        if self.env_mask is not None:
+            fields_.append(("env_mask", (torch.uint8, torch.bool), ()))
+        for name, dtypes, shape in fields_:
+            t = getattr(self, name)
+            if not isinstance(t, torch.Tensor) or t.device.type != "cpu":
+                raise _cabi.PhcError(f"{name} must be a CPU tensor (the host step takes host buffers)")
+            if t.dtype not in dtypes:
+                raise _cabi.PhcError(f"{name} must be {' or '.join(map(str, dtypes))}, got {t.dtype}")
+            if tuple(t.shape) != (n, *shape):
+                raise ValueError(f"{name} has shape {tuple(t.shape)}, expected {(n, *shape)}")
+            if not t.is_contiguous():
+                raise _cabi.PhcError(f"{name} must be contiguous")
+        return n
+
+    def _args(self, bufs: HostStepBuffers, state_init: str, flag_test: bool) -> _cabi.PhcHostResetArgs:
+        """The reset's outputs alias ``bufs``' own state and clock tensors."""
+        if state_init not in _STATE_INIT:
+            raise ValueError(f"state_init must be one of {sorted(_STATE_INIT)}, got {state_init!r}")
+        return _cabi.PhcHostResetArgs(
+            self.phase.data_ptr(), _cabi.ptr(self.env_mask), _STATE_INIT[state_init], int(bool(flag_test)),
+            bufs.state.data_ptr(), self.root_states.data_ptr(), self.dof_pos.data_ptr(), self.dof_vel.data_ptr(),
+            bufs.motion_start_times.data_ptr(), bufs.motion_start_times_offset.data_ptr(), bufs.global_offset.data_ptr(),
+        )  # fmt: skip
+
+
 class HostStep:
     """A ``phc_host_step`` context on the current CUDA device for batches of up to ``max_envs`` envs.
 
@@ -112,6 +185,7 @@ class HostStep:
     ):
         self._ctx = None
         self._inflight: List[Optional[HostStepBuffers]] = [None] * _cabi.HOST_SLOTS
+        self._inflight_reset: List[Optional[HostResetBuffers]] = [None] * _cabi.HOST_SLOTS
         self.time_steps = int(time_steps)
         self._capi = _cabi.load()
         term = torch.as_tensor(termination_distances, dtype=torch.float32).cpu().expand(_cabi.NUM_BODIES)
@@ -133,20 +207,61 @@ class HostStep:
             raise _cabi.PhcError("HostStep is closed")
         return self._ctx
 
-    def step(self, bufs: HostStepBuffers) -> HostStepBuffers:
-        """One step of ``bufs``; returns when every output is in ``bufs`` (``progress_buf`` advanced in place)."""
+    def step(self, bufs: HostStepBuffers, reset: Optional[HostResetBuffers] = None, state_init: str = "random",
+             flag_test: bool = False) -> HostStepBuffers:  # fmt: skip
+        """One step of ``bufs``; returns when every output is in ``bufs`` (``progress_buf`` advanced in place).  With
+        ``reset`` the envs the step flags are re-posed as well (see ``submit``); this runs on slot 0."""
+        if reset is not None:
+            self.submit(0, bufs, reset, state_init, flag_test)
+            return self.wait(0)
         n = bufs.validate(self.time_steps)
         args = bufs._args()
         _cabi.check(self._capi.phc_host_step(self._live(), C.byref(args), n), "phc_host_step")
         return bufs
 
-    def submit(self, slot: int, bufs: HostStepBuffers) -> None:
-        """Enqueue one step of ``bufs`` on ``slot`` (0 or 1) and return.  ``bufs`` belongs to the library until
-        ``wait(slot)`` returns: do not read or write it before then."""
+    def submit(self, slot: int, bufs: HostStepBuffers, reset: Optional[HostResetBuffers] = None,
+               state_init: str = "random", flag_test: bool = False) -> None:  # fmt: skip
+        """Enqueue one step of ``bufs`` on ``slot`` (0 or 1) and return.  ``bufs`` (and ``reset``) belong to the library
+        until ``wait(slot)`` returns: do not read or write them before then.
+
+        With ``reset`` it is ``HumanoidPHC.step()`` with auto-reset: the envs the step flags are re-posed from the
+        motion library (``state_init`` "random": at ``reset.phase``; "start": at time 0; ``flag_test``: the eval
+        mode's time 0).  After ``wait``, ``obs_buf`` holds the final rows, ``reset_buf`` / ``terminate_buf`` the step's
+        own flags, ``progress_buf`` is 0 for re-posed envs, and for those envs only ``bufs.state``, the clock tensors
+        and ``reset.root_states`` / ``dof_pos`` / ``dof_vel`` hold the new state."""
         n = bufs.validate(self.time_steps)
         args = bufs._args()
-        _cabi.check(self._capi.phc_host_step_submit(self._live(), int(slot), C.byref(args), n), "phc_host_step_submit")
+        if reset is None:
+            _cabi.check(self._capi.phc_host_step_submit(self._live(), int(slot), C.byref(args), n), "phc_host_step_submit")
+        else:
+            reset.validate(n)
+            rargs = reset._args(bufs, state_init, flag_test)
+            _cabi.check(self._capi.phc_host_step_submit_reset(self._live(), int(slot), C.byref(args), C.byref(rargs), n),
+                        "phc_host_step_submit_reset")  # fmt: skip
         self._inflight[slot] = bufs
+        self._inflight_reset[slot] = reset
+
+    def reset_submit(self, slot: int, bufs: HostStepBuffers, reset: HostResetBuffers, state_init: str = "random",
+                     flag_test: bool = False) -> None:  # fmt: skip
+        """Enqueue ``HumanoidPHC.reset(env_ids, phase)`` for the envs of ``reset.env_mask`` on ``slot`` and return:
+        reads the clock and ids of ``bufs``; after ``wait``, for the masked envs only, ``obs_buf`` rows, ``state``,
+        the clock, ``progress_buf`` = 0, ``reset_buf`` = ``terminate_buf`` = 0 and ``reset``'s root / dof rows hold
+        the re-posed envs.  How a host loop gets its first observation."""
+        n = bufs.validate(self.time_steps)
+        reset.validate(n)
+        if reset.env_mask is None:
+            raise ValueError("reset_submit needs reset.env_mask")
+        args, rargs = bufs._args(), reset._args(bufs, state_init, flag_test)
+        _cabi.check(self._capi.phc_host_reset_submit(self._live(), int(slot), C.byref(args), C.byref(rargs), n),
+                    "phc_host_reset_submit")  # fmt: skip
+        self._inflight[slot] = bufs
+        self._inflight_reset[slot] = reset
+
+    def reset(self, bufs: HostStepBuffers, reset: HostResetBuffers, state_init: str = "random",
+              flag_test: bool = False) -> HostStepBuffers:  # fmt: skip
+        """``reset_submit`` on slot 0 + ``wait(0)``."""
+        self.reset_submit(0, bufs, reset, state_init, flag_test)
+        return self.wait(0)
 
     def wait(self, slot: int) -> Optional[HostStepBuffers]:
         """Block until ``slot``'s step has finished; returns its buffers (None if the slot was idle)."""
@@ -154,6 +269,7 @@ class HostStep:
         bufs = None
         if 0 <= slot < _cabi.HOST_SLOTS:  # the slot is idle after wait, also when it reports an error
             bufs, self._inflight[slot] = self._inflight[slot], None
+            self._inflight_reset[slot] = None
         _cabi.check(rc, "phc_host_step_wait")
         return bufs
 
@@ -172,6 +288,7 @@ class HostStep:
         if ctx is not None:
             self._capi.phc_host_step_destroy(ctx)  # finishes every slot in flight before freeing
         self._inflight = [None] * _cabi.HOST_SLOTS
+        self._inflight_reset = [None] * _cabi.HOST_SLOTS
 
     def __enter__(self) -> "HostStep":
         return self

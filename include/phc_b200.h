@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define PHC_ABI_VERSION 5 /* 5: phc_host_step_submit / phc_host_step_wait, PHC_ERR_BUSY; 4: PhcResetArgs grew (initial_*, default_mask: StateInit.Default / Hybrid); 3: PhcStepArgs grew (rew_out, reset_out, terminate_out, auto_reset, ref_dof_pos, obs_flags), PhcResetArgs grew (obs_norm*, obs_moments*),
+#define PHC_ABI_VERSION 6 /* 6: PhcHostResetArgs, phc_host_step_submit_reset / phc_host_reset_submit; 5: phc_host_step_submit / phc_host_step_wait, PHC_ERR_BUSY; 4: PhcResetArgs grew (initial_*, default_mask: StateInit.Default / Hybrid); 3: PhcStepArgs grew (rew_out, reset_out, terminate_out, auto_reset, ref_dof_pos, obs_flags), PhcResetArgs grew (obs_norm*, obs_moments*),
                               phc_action_to_pd_targets takes the action clip; 2: obs_moments_buckets, ep_*, phc_motion_build / phc_peer_reduce_* / phc_episode_fold */
 #define PHC_NUM_BODIES 24      /* SMPL humanoid, body_sets.py:11-36 */
 #define PHC_SELF_OBS_DIM 358   /* envs/humanoid_phc.py:461 */
@@ -482,7 +482,7 @@ PHC_API void phc_host_step_destroy(PhcHostStep* ctx);
  *            kernels write obs, rewards, flags and progress into them asynchronously, and the copy engine reads state.
  *   wait     Blocks until the slot's outputs are in the caller's buffers (on the staged path it also unpacks the
  *            scalar outputs).  Returns PHC_OK, or the step's deferred error (PHC_ERR_CUDA + phc_last_cuda_error()).
- *            Waiting on an idle slot returns PHC_OK at once.
+ *            Waiting on an idle slot returns PHC_OK at once.  It also collects the two submits with resets below.
  *   busy     A submit to a slot with a step in flight returns PHC_ERR_BUSY, enqueues nothing and leaves the step in
  *            flight untouched.  phc_host_step is submit + wait on slot 0: it returns PHC_ERR_BUSY while slot 0 is in
  *            flight and runs normally while only slot 1 is.
@@ -506,6 +506,53 @@ PHC_API int phc_host_step_chunks(const PhcHostStep* ctx);
 PHC_API int phc_host_step_tuning_calls(const PhcHostStep* ctx);
 PHC_API int64_t phc_host_step_h2d_bytes(const PhcHostStep* ctx, int64_t n);
 PHC_API int64_t phc_host_step_d2h_bytes(const PhcHostStep* ctx, int64_t n);
+
+/* Resets on the host-buffer path (ABI 6): what HumanoidPHC.step() with auto-reset and HumanoidPHC.reset(env_ids, phase)
+ * do (phc_step_fused with PhcStepArgs.auto_reset / phc_reset_envs, humanoid_phc.py:665-676), on host buffers.  The
+ * reset runs over the slot's device copies of the chunk; then one small kernel per chunk writes the rows of the re-posed
+ * envs (and nothing else) into the caller's buffers — straight into them when every output buffer below is pinned, else
+ * through the slot's pinned staging, unpacked by phc_host_step_wait.  A re-posed env's new state is about 1.9 KB, so
+ * only the reset envs' rows cross the link.  The clock arrays of PhcHostStepArgs are const: the new clock leaves through
+ * the *_out pointers, which may alias them (and state_out may alias args->state): the inputs are consumed before any
+ * output of the same rows is written.  Everything here is a HOST pointer.
+ *
+ *   phc_host_step_submit_reset  The step with auto-reset.  When phc_host_step_wait returns: obs_buf holds the final rows
+ *            (a re-posed env's row is recomputed from its new state), rew_buf / reward_raw the step's, reset_buf /
+ *            terminate_buf the STEP's flags (extras["reset"] / ["terminate"] of the device path: the envs whose
+ *            physics the caller must re-pose, and the dones), progress_buf advanced and 0 for re-posed envs; for the
+ *            re-posed envs only: the clock outs (new start time, offset 0, global offset 0) and state_out / root_states /
+ *            dof_pos / dof_vel (what _set_env_state writes, humanoid_phc.py:901-931).  Other rows of the reset outputs
+ *            are not written.  env_mask is ignored.
+ *   phc_host_reset_submit  HumanoidPHC.reset(env_ids, phase) for the envs whose env_mask byte is set: reads the clock,
+ *            sampled_motion_ids, phase and env_mask (not state, not obs_buf; progress is not advanced).  For the masked
+ *            envs only it writes obs rows, state_out / root_states / dof_pos / dof_vel rows, the clock outs,
+ *            progress_buf = 0 and reset_buf = terminate_buf = 0; rew_buf / reward_raw are not touched.  This is how a
+ *            host loop gets its first observation and resets envs it picks itself.
+ *   validation  Everything phc_host_step_submit checks, plus: NULL reset pointers (env_mask for phc_host_reset_submit,
+ *            phase for PHC_STATE_INIT_RANDOM) -> PHC_ERR_NULL; PHC_STATE_INIT_DEFAULT / HYBRID (they need per-env
+ *            initial_* buffers) or any other state_init, a device pointer, or a motion library without local rotations
+ *            / dof velocities -> PHC_ERR_UNSUPPORTED; a busy slot -> PHC_ERR_BUSY.  All before anything is enqueued;
+ *            after any error the slot is idle.
+ *   buffers / tuning / destroy  As for phc_host_step_submit: the reset buffers belong to the library until
+ *            phc_host_step_wait returns; these submits are not timed by the tuner and use the settled schedule;
+ *            destroy waits for them. */
+typedef struct PhcHostResetArgs {
+  const float* phase;                   /* host [n]: the uniform [0,1) numbers of sample_time_interval (RANDOM)  */
+  const uint8_t* env_mask;              /* host [n]: phc_host_reset_submit only, 1 = reset this env             */
+  int32_t state_init;                   /* PHC_STATE_INIT_START | PHC_STATE_INIT_RANDOM                          */
+  int32_t flag_test;                    /* motion_times[:] = 0         humanoid_phc.py:856                       */
+  float* state_out;                     /* host [n,24,13] rigid-body rows of re-posed envs (may alias args->state) */
+  float* root_states;                   /* host [n,13] humanoid_root_states rows    humanoid_phc.py:518          */
+  float* dof_pos;                       /* host [n,69] dense                        humanoid_phc.py:535          */
+  float* dof_vel;                       /* host [n,69] dense                        humanoid_phc.py:536          */
+  float* motion_start_times_out;        /* host [n]   (may alias args->motion_start_times)                       */
+  float* motion_start_times_offset_out; /* host [n]   (may alias args->motion_start_times_offset)                */
+  float* global_offset_out;             /* host [n,3] (may alias args->global_offset)                            */
+} PhcHostResetArgs;
+PHC_API int phc_host_step_submit_reset(PhcHostStep* ctx, int32_t slot, const PhcHostStepArgs* args,
+                                       const PhcHostResetArgs* reset, int64_t n);
+PHC_API int phc_host_reset_submit(PhcHostStep* ctx, int32_t slot, const PhcHostStepArgs* args,
+                                  const PhcHostResetArgs* reset, int64_t n);
 
 /* ------------------------------------------------------------------------------------
  * RunningNorm statistics                                   policies/running_norm.py:23-34
