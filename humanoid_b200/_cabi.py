@@ -264,6 +264,21 @@ class PhcHostResetArgs(C.Structure):
     ]
 
 
+class PhcHostDeviceOut(C.Structure):
+    _fields_ = [
+        ("obs", C.c_void_p),
+        ("obs_norm", C.c_void_p),
+        ("norm_mean", C.c_void_p),
+        ("norm_var", C.c_void_p),
+        ("norm_epsilon", C.c_float),
+        ("norm_clip", C.c_float),
+        ("flags", C.c_uint32),
+        ("obs_moments", C.c_void_p),
+        ("obs_moments_buckets", C.c_int32),
+        ("stream", C.c_void_p),
+    ]
+
+
 BUILD_FILTER_RADIUS = 8
 EPISODE_SUM_COLS = 12
 PEER_MAX_WORLD = 16
@@ -347,6 +362,16 @@ SIGNATURES = {
         C.c_int,
         [C.c_void_p, C.c_int32, C.POINTER(PhcHostStepArgs), C.POINTER(PhcHostResetArgs), C.c_int64],
     ),
+    "phc_host_step_submit_device": (
+        C.c_int,
+        [C.c_void_p, C.c_int32, C.POINTER(PhcHostStepArgs), C.POINTER(PhcHostResetArgs), C.POINTER(PhcHostDeviceOut),
+         C.c_int64],
+    ),  # fmt: skip
+    "phc_host_reset_submit_device": (
+        C.c_int,
+        [C.c_void_p, C.c_int32, C.POINTER(PhcHostStepArgs), C.POINTER(PhcHostResetArgs), C.POINTER(PhcHostDeviceOut),
+         C.c_int64],
+    ),  # fmt: skip
     "phc_host_step_path": (C.c_int, [C.c_void_p]),
     "phc_host_step_chunks": (C.c_int, [C.c_void_p]),
     "phc_host_step_tuning_calls": (C.c_int, [C.c_void_p]),

@@ -29,6 +29,11 @@
 // (~1.9 KB) is not in any buffer the plain step sends back, and only a few percent of the envs are re-posed per step:
 // one small kernel per chunk (host_export_kernel) writes the rows of those envs alone into the caller's buffers when
 // they are pinned, else into the slot's pinned staging, from which wait copies the rows of the flagged envs.
+//
+// Device outputs.  phc_host_step_submit_device / phc_host_reset_submit_device run the same pipelines with the obs rows
+// (and the normalised rows and RunningNorm moments) written by the kernels into the caller's device tensors: no obs
+// transfer at all, only the scalars and the reset rows return to the host.  Each chunk's stream waits for an event
+// recorded on the caller's stream before its kernel, so the policy's reads of the previous rows come first.
 #include <chrono>
 #include <cstdint>
 #include <cstdio>
@@ -159,6 +164,7 @@ struct Slot {
   unsigned char* h_out = nullptr;    // pinned staging
   cudaStream_t streams[kStreams] = {};
   cudaEvent_t done[kStreams] = {};  // recorded on each stream at the end of an enqueue
+  cudaEvent_t dev_ready = nullptr;  // device-output submits: recorded on the caller's stream, waited on before a kernel
   // direct path: verdict cached per set of caller pointers
   const void* seen[11] = {};
   int seen_direct = -1;
@@ -191,6 +197,7 @@ struct PhcHostStep {
   int32_t T = 1;
   int32_t chunks = 1;
   int64_t obs_dim = 0;
+  int device = 0;  // the device current at create: device outputs must live there
   float* term_dist = nullptr;
   uint32_t reset_mask = 0xFFFFFF;
   int32_t use_mean = 0, early = 1;
@@ -243,6 +250,7 @@ static cudaError_t slot_alloc(const PhcHostStep* c, Slot& s) {
     e = cudaStreamCreateWithFlags(&s.streams[i], cudaStreamNonBlocking);
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&s.done[i], cudaEventDisableTiming);
   }
+  if (e == cudaSuccess) e = cudaEventCreateWithFlags(&s.dev_ready, cudaEventDisableTiming);
   s.ready = e == cudaSuccess;
   return e;
 }
@@ -262,16 +270,19 @@ static void slot_free(Slot& s) {
     if (s.done[i]) cudaEventDestroy(s.done[i]);
     if (s.streams[i]) cudaStreamDestroy(s.streams[i]);
   }
+  if (s.dev_ready) cudaEventDestroy(s.dev_ready);
   s = Slot{};
 }
 
-// Everything phc_host_step validates, before anything is enqueued; fills the slot's direct-path verdict.
-static int check_args(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, int64_t n) {
+// Everything phc_host_step validates, before anything is enqueued; fills the slot's direct-path verdict.  With device
+// outputs (dev_out) obs_buf must be NULL: the rows go to the device tensors only.
+static int check_args(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, int64_t n, bool dev_out = false) {
   if (n < 0 || n > c->max_envs) return PHC_ERR_SHAPE;
   if (!a->state || !a->progress_buf || !a->motion_start_times || !a->motion_start_times_offset ||
-      !a->global_offset || !a->sampled_motion_ids || !a->obs_buf || !a->rew_buf || !a->reward_raw || !a->reset_buf ||
-      !a->terminate_buf)
+      !a->global_offset || !a->sampled_motion_ids || (!dev_out && !a->obs_buf) || !a->rew_buf || !a->reward_raw ||
+      !a->reset_buf || !a->terminate_buf)
     return PHC_ERR_NULL;
+  if (dev_out && a->obs_buf) return PHC_ERR_UNSUPPORTED;
   // ---- can the direct path be used: every buffer is pinned / managed host memory mapped at its own address ----------
   const void* ptrs[11] = {a->state, a->progress_buf, a->motion_start_times, a->motion_start_times_offset,
                           a->global_offset, a->sampled_motion_ids, a->obs_buf, a->rew_buf, a->reward_raw,
@@ -279,6 +290,7 @@ static int check_args(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, int64_t
   if (s.seen_direct < 0 || memcmp(ptrs, s.seen, sizeof(ptrs)) != 0) {
     int direct = 1;
     for (int i = 0; i < 11 && direct; ++i) {
+      if (!ptrs[i]) continue;  // obs_buf of a device-output submit
       cudaPointerAttributes at{};
       if (cudaPointerGetAttributes(&at, ptrs[i]) != cudaSuccess) {
         (void)cudaGetLastError();
@@ -325,6 +337,47 @@ static int check_reset(const PhcHostStep* c, Slot& s, const PhcHostResetArgs* r,
     s.rseen_direct = direct;
   }
   return PHC_OK;
+}
+
+// What the device-output submits validate on top of check_args (and check_reset).
+static int check_dev(const PhcHostStep* c, const PhcHostDeviceOut* d) {
+  if (d->obs_norm && (!d->norm_mean || !d->norm_var)) return PHC_ERR_NULL;
+  if (d->flags & ~PHC_STEP_OBS_NORM_BF16) return PHC_ERR_UNSUPPORTED;
+  const void* ptrs[5] = {d->obs, d->obs_norm, d->norm_mean, d->norm_var, d->obs_moments};
+  for (const void* p : ptrs) {
+    if (!p) continue;
+    cudaPointerAttributes at{};
+    if (cudaPointerGetAttributes(&at, p) != cudaSuccess) {
+      (void)cudaGetLastError();
+      return PHC_ERR_UNSUPPORTED;
+    }
+    if (at.type != cudaMemoryTypeDevice || at.device != c->device) return PHC_ERR_UNSUPPORTED;
+  }
+  if ((((uintptr_t)d->obs | (uintptr_t)d->obs_norm) & 15) != 0) return PHC_ERR_ALIGN;
+  if (d->obs_moments_buckets < 0 || d->obs_moments_buckets > 4096 || (d->obs_norm && !(d->norm_clip > 0.0f)))
+    return PHC_ERR_SHAPE;
+  return PHC_OK;
+}
+
+// The chunk's rows in the caller's device tensors.  Chunks start on multiples of 8 envs, so the fp32 and the bf16 rows
+// of every chunk start 16-B aligned.
+static float* dev_obs(const PhcHostStep* c, const PhcHostDeviceOut* d, int64_t lo) { return d->obs + lo * c->obs_dim; }
+static float* dev_obs_norm(const PhcHostStep* c, const PhcHostDeviceOut* d, int64_t lo) {
+  if (!d->obs_norm) return nullptr;
+  const int64_t bytes = (d->flags & PHC_STEP_OBS_NORM_BF16) ? 2 : 4;
+  return (float*)((char*)d->obs_norm + lo * c->obs_dim * bytes);
+}
+static void dev_step_outputs(const PhcHostStep* c, const PhcHostDeviceOut* d, int64_t lo, PhcStepArgs& k) {
+  k.obs_buf = dev_obs(c, d, lo);
+  k.obs_norm = dev_obs_norm(c, d, lo);
+  k.obs_norm_stride = c->obs_dim;
+  k.norm_mean = d->norm_mean;
+  k.norm_var = d->norm_var;
+  k.norm_epsilon = d->norm_epsilon;
+  k.norm_clip = d->norm_clip;
+  k.flags |= d->flags;
+  k.obs_moments = d->obs_moments;
+  k.obs_moments_buckets = d->obs_moments_buckets;
 }
 
 // The reset scratch of a slot; the pinned staging only when the rows of this submit go through it.
@@ -433,8 +486,8 @@ static cudaError_t export_rows(const PhcHostStep* c, const PhcResetArgs& ra, con
   return cudaGetLastError();
 }
 
-static int direct_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, const PhcHostResetArgs* r, int64_t n,
-                          const int chunks) {
+static int direct_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, const PhcHostResetArgs* r,
+                          const PhcHostDeviceOut* dev, int64_t n, const int chunks) {
   // Hybrid: everything INBOUND rides the host->device copy engine in a few chunks — the sim
   // rows directly from the caller's buffer, the five small clock arrays packed into one
   // transfer (SM-issued reads of system memory are 32-B PCIe round trips: 6 per block, ~70 us
@@ -503,6 +556,7 @@ static int direct_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, con
     k.terminate_buf = a->terminate_buf + lo;
     k.flags = PHC_STEP_MAPPED_HOST_IO;
     k.obs_moments = nullptr;
+    if (dev) dev_step_outputs(c, dev, lo, k);
     PhcResetArgs ra;
     if (r) {
       k.reset_buf = s.d_kreset + lo;
@@ -515,6 +569,7 @@ static int direct_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, con
     // the advanced progress goes straight into the caller's buffer too (no device->host copy at the tail).  Not with a
     // reset: where it runs as a second launch (T > 1 here, or the generic kernel) the mirror would keep the advanced
     // progress of the re-posed envs, so the progress leaves with the flags, from the device clock after the reset.
+    if (dev) HOST_CUDA(s, cudaStreamWaitEvent(st_, s.dev_ready, 0));
     int rc = step_fused_mirrored(c->lib, &k, m, st_, r ? nullptr : a->progress_buf + lo);
     if (rc) return host_fail(s, rc, cudaSuccess);
     if (r) {
@@ -548,8 +603,8 @@ static int direct_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, con
   return PHC_OK;
 }
 
-static int staged_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, const PhcHostResetArgs* r, int64_t n,
-                          const int chunks) {
+static int staged_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, const PhcHostResetArgs* r,
+                          const PhcHostDeviceOut* dev, int64_t n, const int chunks) {
   const cudaMemcpyKind H2D = cudaMemcpyHostToDevice, D2H = cudaMemcpyDeviceToHost;
   // Chunk sizes double (n/2^(C-1), n/2^(C-1), n/2^(C-2), .., n/2): the device->host direction
   // carries 3x the bytes and is the bottleneck, so the first chunk is small to start it early
@@ -624,6 +679,7 @@ static int staged_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, con
     k.reset_buf = dout + L.reset;
     k.terminate_buf = dout + L.term;
     k.obs_moments = nullptr;
+    if (dev) dev_step_outputs(c, dev, lo, k);
     PhcResetArgs ra;
     if (r) {  // the step's own flags still leave in the packed scalars
       k.reset_buf = s.d_kreset + lo;
@@ -637,6 +693,7 @@ static int staged_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, con
       cudaEventCreate(&sevh[ci]);
       cudaEventRecord(sevh[ci], st_);
     }
+    if (dev) HOST_CUDA(s, cudaStreamWaitEvent(st_, s.dev_ready, 0));
     int rc = phc_step_fused(c->lib, &k, m, st_);
     if (rc) return host_fail(s, rc, cudaSuccess);
     if (r) {
@@ -652,8 +709,9 @@ static int staged_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, con
     }
     // the advanced progress rides back with the scalar outputs
     HOST_CUDA(s, cudaMemcpyAsync(dout + L.oprog, dc + L.prog, (size_t)m * 2, cudaMemcpyDeviceToDevice, st_));
-    HOST_CUDA(s, cudaMemcpyAsync(a->obs_buf + lo * c->obs_dim, s.d_obs + lo * c->obs_dim,
-                                 (size_t)m * c->obs_dim * sizeof(float), D2H, st_));
+    if (!dev)
+      HOST_CUDA(s, cudaMemcpyAsync(a->obs_buf + lo * c->obs_dim, s.d_obs + lo * c->obs_dim,
+                                   (size_t)m * c->obs_dim * sizeof(float), D2H, st_));
     HOST_CUDA(s, cudaMemcpyAsync(s.h_out + ooff, dout, L.out_bytes, D2H, st_));
     if (strace && ci < 16) {
       cudaEventCreate(&sevd[ci]);
@@ -678,9 +736,11 @@ static int staged_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, con
 }
 
 // The host reset: H2D(packed clock + phase + mask) -> phc_reset_envs -> export of the masked envs' rows (obs included)
-// on equal chunks.  Nothing else is read or written: no sim state comes in, no whole obs chunk goes out.
-static int reset_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, const PhcHostResetArgs* r, int64_t n,
-                         const int chunks) {
+// on equal chunks.  Nothing else is read or written: no sim state comes in, no whole obs chunk goes out.  With device
+// outputs the reset writes the masked envs' obs and normalised rows straight into the caller's tensors and adds them
+// to the moments (rows no step has counted, as HumanoidPHC.reset() does); the export then carries no obs.
+static int reset_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, const PhcHostResetArgs* r,
+                         const PhcHostDeviceOut* dev, int64_t n, const int chunks) {
   const int C = chunks < 1 ? 1 : chunks;
   int64_t per = (n + C - 1) / C;
   per = (per + 7) / 8 * 8;
@@ -696,11 +756,26 @@ static int reset_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, cons
     unsigned char* dc = s.d_clock + coff;
     pack_clock(hc, L, a, r, lo, m);
     HOST_CUDA(s, cudaMemcpyAsync(dc, hc, L.clock_bytes, cudaMemcpyHostToDevice, st_));
-    float* obs = s.d_obs + lo * c->obs_dim;
-    const PhcResetArgs ra = chunk_reset_args(c, s, r, s.d_state + lo * kStateFloats, dc, L, lo, obs);
+    float* obs = dev ? dev_obs(c, dev, lo) : s.d_obs + lo * c->obs_dim;
+    PhcResetArgs ra = chunk_reset_args(c, s, r, s.d_state + lo * kStateFloats, dc, L, lo, obs);
+    Rows out = rows_at(rows, lo, c->obs_dim);
+    if (dev) {
+      ra.obs_norm = dev_obs_norm(c, dev, lo);
+      ra.obs_norm_stride = c->obs_dim;
+      ra.norm_mean = dev->norm_mean;
+      ra.norm_var = dev->norm_var;
+      ra.norm_epsilon = dev->norm_epsilon;
+      ra.norm_clip = dev->norm_clip;
+      ra.obs_norm_bf16 = (dev->flags & PHC_STEP_OBS_NORM_BF16) ? 1 : 0;
+      ra.obs_moments_mode = dev->obs_moments ? 1 : 0;
+      ra.obs_moments = dev->obs_moments;
+      ra.obs_moments_buckets = dev->obs_moments_buckets;
+      out.obs = nullptr;
+      HOST_CUDA(s, cudaStreamWaitEvent(st_, s.dev_ready, 0));
+    }
     const int rc = phc_reset_envs(c->lib, &ra, m, st_);
     if (rc) return host_fail(s, rc, cudaSuccess);
-    HOST_CUDA(s, export_rows(c, ra, dc + L.mask, nullptr, obs, rows_at(rows, lo, c->obs_dim), 1, m, st_));
+    HOST_CUDA(s, export_rows(c, ra, dc + L.mask, nullptr, dev ? nullptr : obs, out, 1, m, st_));
     coff += L.clock_bytes;
   }
   return PHC_OK;
@@ -708,11 +783,12 @@ static int reset_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, cons
 
 // Enqueues one step (or reset) on a slot (arguments already checked) and marks it in flight.
 static int slot_enqueue(PhcHostStep* c, int slot, const PhcHostStepArgs* a, const PhcHostResetArgs* r, int op,
-                        int64_t n, const PhcHostStep::Cand& k) {
+                        int64_t n, const PhcHostStep::Cand& k, const PhcHostDeviceOut* dev = nullptr) {
   Slot& s = c->slots[slot];
-  const int rc = op == kReset   ? reset_enqueue(c, s, a, r, n, k.chunks)
-                 : k.path == 1 ? direct_enqueue(c, s, a, r, n, k.chunks)
-                               : staged_enqueue(c, s, a, r, n, k.chunks);
+  if (dev) HOST_CUDA(s, cudaEventRecord(s.dev_ready, dev->stream));
+  const int rc = op == kReset   ? reset_enqueue(c, s, a, r, dev, n, k.chunks)
+                 : k.path == 1 ? direct_enqueue(c, s, a, r, dev, n, k.chunks)
+                               : staged_enqueue(c, s, a, r, dev, n, k.chunks);
   if (rc) return rc;
   for (int i = 0; i < kStreams; ++i) HOST_CUDA(s, cudaEventRecord(s.done[i], s.streams[i]));
   s.args = *a;
@@ -741,7 +817,7 @@ static void unpack_rows(const PhcHostStep* c, const Slot& s) {
     dst.start[i] = src.start[i];
     dst.soff[i] = src.soff[i];
     if (s.op == kReset) {
-      memcpy(dst.obs + i * D, src.obs + i * D, D * sizeof(float));
+      if (dst.obs) memcpy(dst.obs + i * D, src.obs + i * D, D * sizeof(float));  // no host obs with device outputs
       dst.prog[i] = src.prog[i];
       dst.rst[i] = src.rst[i];
       dst.term[i] = src.term[i];
@@ -822,6 +898,7 @@ int phc_host_step_create(const PhcLib* lib, int64_t max_envs, int32_t time_steps
   c->early = enable_early_termination;
   c->dt = dt;
   c->rwd = *rwd;
+  (void)cudaGetDevice(&c->device);
   if (const char* m = getenv("PHC_HOST_PATH")) c->mode = !strcmp(m, "direct") ? 1 : !strcmp(m, "staged") ? 2 : 0;
   if (getenv("PHC_HOST_STAGED")) c->mode = 2;
   const size_t n = (size_t)max_envs;
@@ -913,16 +990,19 @@ int phc_host_step(PhcHostStep* c, const PhcHostStepArgs* a, int64_t n) {
 
 }  // extern "C"
 
-// The three submits: every check before anything is enqueued, then the slot's buffers, then the enqueue.
-static int submit(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, const PhcHostResetArgs* r, int op, int64_t n) {
-  if (!c || !a || (op != kStep && !r)) return PHC_ERR_NULL;
+// The submits: every check before anything is enqueued, then the slot's buffers, then the enqueue.  dev_out: one of
+// the device-output submits (dev must then name the device tensors).
+static int submit(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, const PhcHostResetArgs* r, int op, int64_t n,
+                  bool dev_out = false, const PhcHostDeviceOut* dev = nullptr) {
+  if (!c || !a || (op != kStep && !r) || (dev_out && (!dev || !dev->obs))) return PHC_ERR_NULL;
   if (slot < 0 || slot >= PHC_HOST_SLOTS) return PHC_ERR_SHAPE;
   Slot& s = c->slots[slot];
   if (s.busy) return PHC_ERR_BUSY;
   if (n == 0) return PHC_OK;
-  int rc = check_args(c, s, a, n);
+  int rc = check_args(c, s, a, n, dev_out);
   if (rc) return rc;
   if (op != kStep && (rc = check_reset(c, s, r, op))) return rc;
+  if (dev_out && (rc = check_dev(c, dev))) return rc;
   cudaError_t e = cudaSuccess;
   if (!s.ready) {
     e = slot_alloc(c, s);
@@ -937,7 +1017,7 @@ static int submit(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, const 
     (void)cudaGetLastError();
     return e == cudaErrorMemoryAllocation ? PHC_ERR_ALLOC : phc::record_cuda_error((int)e);
   }
-  return slot_enqueue(c, slot, a, r, op, n, untimed_schedule(c, s));
+  return slot_enqueue(c, slot, a, r, op, n, untimed_schedule(c, s), dev_out ? dev : nullptr);
 }
 
 extern "C" {
@@ -954,6 +1034,16 @@ int phc_host_step_submit_reset(PhcHostStep* c, int32_t slot, const PhcHostStepAr
 int phc_host_reset_submit(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, const PhcHostResetArgs* r,
                           int64_t n) {
   return submit(c, slot, a, r, kReset, n);
+}
+
+int phc_host_step_submit_device(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, const PhcHostResetArgs* r,
+                                const PhcHostDeviceOut* dev, int64_t n) {
+  return submit(c, slot, a, r, r ? kStepReset : kStep, n, true, dev);
+}
+
+int phc_host_reset_submit_device(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, const PhcHostResetArgs* r,
+                                 const PhcHostDeviceOut* dev, int64_t n) {
+  return submit(c, slot, a, r, kReset, n, true, dev);
 }
 
 int phc_host_step_wait(PhcHostStep* c, int32_t slot) {

@@ -11,6 +11,11 @@ With ``reset=HostResetBuffers`` a step also re-poses the envs it flags (``Humano
 ``reset`` of every env once, then ``submit(slot, bufs, reset=...)`` / ``wait(slot)`` per batch; after each ``wait`` the
 caller's physics takes the root and dof state of the envs in ``bufs.reset_buf`` from the reset buffers.
 
+With ``device_out=HostDeviceOutputs`` the observation rows (and optionally their normalised copy and the RunningNorm
+moments) are written into CUDA tensors instead of ``bufs.obs_buf``: the caller whose physics runs on the CPU and whose
+policy runs on the GPU gets the rows where the policy reads them, and only rewards, flags, progress and the reset rows
+cross back to the host.
+
 Pinned buffers (``HostStepBuffers.allocate(..., pinned=True)``) take the fast paths; pageable ones work through
 staging.  The CUDA device of the motion library must be current when the context is created and stepped; after
 ``MotionLib.repack()`` synchronise the device before the next host step (the steps run on the context's own streams).
@@ -20,7 +25,7 @@ from __future__ import annotations
 
 import ctypes as C
 from dataclasses import dataclass, fields
-from typing import List, Optional, Sequence, Union
+from typing import Any, List, Optional, Sequence, Union
 
 import torch
 
@@ -47,7 +52,8 @@ class HostStepBuffers:
     """The 11 CPU tensors of one batch of ``n`` envs, in the order of ``PhcHostStepArgs``.  Inputs: ``state``
     [n, 24, 13], the clock (``progress_buf`` int16, advanced in place, ``motion_start_times``,
     ``motion_start_times_offset``, ``global_offset`` [n, 3], ``sampled_motion_ids`` int64).  Outputs: ``obs_buf``
-    [n, 358 + 576 T], ``rew_buf``, ``reward_raw`` [n, 4], ``reset_buf`` / ``terminate_buf`` uint8."""
+    [n, 358 + 576 T] (None when the rows go to a ``HostDeviceOutputs``), ``rew_buf``, ``reward_raw`` [n, 4],
+    ``reset_buf`` / ``terminate_buf`` uint8."""
 
     state: torch.Tensor
     progress_buf: torch.Tensor
@@ -55,31 +61,38 @@ class HostStepBuffers:
     motion_start_times_offset: torch.Tensor
     global_offset: torch.Tensor
     sampled_motion_ids: torch.Tensor
-    obs_buf: torch.Tensor
+    obs_buf: Optional[torch.Tensor]
     rew_buf: torch.Tensor
     reward_raw: torch.Tensor
     reset_buf: torch.Tensor
     terminate_buf: torch.Tensor
 
     @classmethod
-    def allocate(cls, n: int, time_steps: int = 1, pinned: bool = True) -> "HostStepBuffers":
-        """Zeroed buffers for ``n`` envs; ``pinned`` page-locks them (needs the CUDA driver)."""
+    def allocate(cls, n: int, time_steps: int = 1, pinned: bool = True, host_obs: bool = True) -> "HostStepBuffers":
+        """Zeroed buffers for ``n`` envs; ``pinned`` page-locks them (needs the CUDA driver).  ``host_obs=False``
+        leaves ``obs_buf`` None, for steps whose rows go to a ``HostDeviceOutputs``."""
 
         def make(dtype, trailing):
             t = torch.zeros((n, *trailing), dtype=dtype)
             return t.pin_memory() if pinned else t
 
-        return cls(**{name: make(dtype, shape(time_steps)) for name, dtype, shape in _FIELDS})
+        return cls(**{name: make(dtype, shape(time_steps)) if host_obs or name != "obs_buf" else None
+                      for name, dtype, shape in _FIELDS})  # fmt: skip
 
     @property
     def n(self) -> int:
         return int(self.state.shape[0])
 
-    def validate(self, time_steps: int = 1) -> int:
-        """Checks device (CPU), dtype, shape and contiguity of every tensor; returns ``n``."""
+    def validate(self, time_steps: int = 1, device_out: bool = False) -> int:
+        """Checks device (CPU), dtype, shape and contiguity of every tensor; returns ``n``.  ``obs_buf`` must be None
+        when the rows go to device outputs (``device_out``), and a tensor otherwise."""
         n = self.n
+        if device_out and self.obs_buf is not None:
+            raise _cabi.PhcError("obs_buf must be None when the rows go to device outputs")
         for name, dtype, shape in _FIELDS:
             t = getattr(self, name)
+            if device_out and name == "obs_buf":
+                continue
             if not isinstance(t, torch.Tensor) or t.device.type != "cpu":
                 raise _cabi.PhcError(f"{name} must be a CPU tensor (the host step takes host buffers)")
             if t.dtype != dtype:
@@ -92,7 +105,7 @@ class HostStepBuffers:
         return n
 
     def _args(self) -> _cabi.PhcHostStepArgs:
-        return _cabi.PhcHostStepArgs(*[getattr(self, f.name).data_ptr() for f in fields(self)])
+        return _cabi.PhcHostStepArgs(*[_cabi.ptr(getattr(self, f.name)) for f in fields(self)])
 
 
 _RESET_FIELDS = (  # name, dtype, trailing shape
@@ -163,6 +176,108 @@ class HostResetBuffers:
         )  # fmt: skip
 
 
+@dataclass(eq=False)
+class HostDeviceOutputs:
+    """The CUDA tensors a host step writes its rows into instead of ``HostStepBuffers.obs_buf``
+    (``phc_host_step_submit_device`` / ``phc_host_reset_submit_device``).
+
+    ``obs`` [n, 358 + 576 T] fp32: the rows ``HumanoidPHC.obs_buf`` would hold.  ``obs_norm`` (optional, fp32 or bf16,
+    the same shape): ``clamp((obs - running_mean) / sqrt(running_var + epsilon), -clip, clip)`` of ``normalizer`` (a
+    ``RunningNorm``, the object ``HumanoidPHC.set_obs_normalizer`` takes; its buffers are read when the kernels run).
+    ``obs_moments`` (optional, fp64 [B, 2 (358 + 576 T)]): per-column sums and sums of squares of every row written
+    (+=), spread over B buckets; ``take_obs_moments`` folds them, as ``HumanoidPHC.take_obs_moments`` does.  ``rows``
+    counts the rows the moments hold."""
+
+    obs: torch.Tensor
+    obs_norm: Optional[torch.Tensor] = None
+    normalizer: Optional[Any] = None
+    obs_moments: Optional[torch.Tensor] = None
+    rows: int = 0
+
+    @classmethod
+    def allocate(cls, n: int, time_steps: int = 1, device=None, norm_dtype: Optional[torch.dtype] = None,
+                 normalizer=None, moments: bool = False) -> "HostDeviceOutputs":  # fmt: skip
+        """Zeroed tensors for ``n`` envs on ``device`` (default: the current CUDA device); ``norm_dtype`` (float32 or
+        bfloat16) adds ``obs_norm`` for ``normalizer``; ``moments`` adds 32 buckets of moments."""
+        from .env import OBS_MOMENT_BUCKETS
+
+        device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+        D = _cabi.SELF_OBS_DIM + _cabi.TASK_OBS_DIM * int(time_steps)
+        if norm_dtype is not None and normalizer is None:
+            raise ValueError("obs_norm needs the normalizer whose running_mean / running_var it uses")
+        return cls(
+            obs=torch.zeros((n, D), dtype=torch.float32, device=device),
+            obs_norm=None if norm_dtype is None else torch.zeros((n, D), dtype=norm_dtype, device=device),
+            normalizer=normalizer,
+            obs_moments=torch.zeros((OBS_MOMENT_BUCKETS, 2 * D), dtype=torch.float64, device=device) if moments else None,
+        )  # fmt: skip
+
+    def validate(self, n: int, time_steps: int = 1) -> None:
+        """Checks dtype, shape and contiguity of every tensor, that all live on one CUDA device, and that ``obs_norm``
+        comes with its normaliser."""
+        D = _cabi.SELF_OBS_DIM + _cabi.TASK_OBS_DIM * int(time_steps)
+        checks = [("obs", self.obs, (torch.float32,), (n, D))]
+        if self.obs_norm is not None:
+            rn = self.normalizer
+            if rn is None:
+                raise _cabi.PhcError("obs_norm needs the normalizer whose running_mean / running_var it uses")
+            checks.append(("obs_norm", self.obs_norm, (torch.float32, torch.bfloat16), (n, D)))
+            for name in ("running_mean", "running_var"):  # [D] or RunningNorm's [1, D]
+                checks.append((f"normalizer.{name}", getattr(rn, name, None), (torch.float32,), (D,)))
+            if not float(rn.clip) > 0.0:
+                raise ValueError(f"normalizer.clip must be > 0, got {rn.clip}")
+        if self.obs_moments is not None:
+            m = self.obs_moments
+            B = int(m.shape[0]) if isinstance(m, torch.Tensor) and m.dim() == 2 else -1
+            if not 1 <= B <= 4096:
+                raise ValueError(f"obs_moments must be [B, {2 * D}] with 1 <= B <= 4096")
+            checks.append(("obs_moments", m, (torch.float64,), (B, 2 * D)))
+        dev = self.obs.device if isinstance(self.obs, torch.Tensor) else None
+        for name, t, dtypes, shape in checks:
+            if not isinstance(t, torch.Tensor):
+                raise _cabi.PhcError(f"{name} must be a CUDA tensor")
+            if t.dtype not in dtypes:
+                raise _cabi.PhcError(f"{name} must be {' or '.join(map(str, dtypes))}, got {t.dtype}")
+            got = (t.numel(),) if name.startswith("normalizer") else tuple(t.shape)
+            if got != shape:
+                raise ValueError(f"{name} has shape {tuple(t.shape)}, expected {shape}")
+            if not t.is_contiguous():
+                raise _cabi.PhcError(f"{name} must be contiguous")
+        for name, t, _, _ in checks:
+            if t.device.type != "cuda" or t.device != dev:
+                raise _cabi.PhcError(f"{name} must be a CUDA tensor on the device of obs (got {t.device})")
+
+    def take_obs_moments(self, sums: Optional[torch.Tensor] = None):
+        """Fold the buckets into ``sums`` (+=, allocated when omitted), zero them, and return ``(sums, rows)`` — what
+        ``RunningNorm.update_from_moments`` takes.  Call it after ``wait``: the fold runs on the current stream."""
+        b = self.obs_moments
+        if b is None:
+            raise _cabi.PhcError("these device outputs have no obs_moments")
+        if sums is None:
+            sums = torch.zeros(b.shape[1], dtype=torch.float64, device=b.device)
+        _cabi.check(
+            _cabi.load().phc_obs_moments_fold(b.data_ptr(), b.shape[0], b.shape[1], sums.data_ptr(), _cabi.stream_ptr(b.device)),
+            "phc_obs_moments_fold",
+        )  # fmt: skip
+        rows, self.rows = self.rows, 0
+        return sums, rows
+
+    def _args(self) -> _cabi.PhcHostDeviceOut:
+        a = _cabi.PhcHostDeviceOut()
+        a.obs = self.obs.data_ptr()
+        if self.obs_norm is not None:
+            rn = self.normalizer
+            a.obs_norm = self.obs_norm.data_ptr()
+            a.norm_mean, a.norm_var = rn.running_mean.data_ptr(), rn.running_var.data_ptr()
+            a.norm_epsilon, a.norm_clip = float(rn.epsilon), float(rn.clip)
+            a.flags = _cabi.STEP_OBS_NORM_BF16 if self.obs_norm.dtype == torch.bfloat16 else 0
+        if self.obs_moments is not None:
+            a.obs_moments = self.obs_moments.data_ptr()
+            a.obs_moments_buckets = self.obs_moments.shape[0]
+        a.stream = _cabi.stream_ptr(self.obs.device)
+        return a
+
+
 class HostStep:
     """A ``phc_host_step`` context on the current CUDA device for batches of up to ``max_envs`` envs.
 
@@ -186,6 +301,7 @@ class HostStep:
         self._ctx = None
         self._inflight: List[Optional[HostStepBuffers]] = [None] * _cabi.HOST_SLOTS
         self._inflight_reset: List[Optional[HostResetBuffers]] = [None] * _cabi.HOST_SLOTS
+        self._inflight_dev: List[Optional[HostDeviceOutputs]] = [None] * _cabi.HOST_SLOTS
         self.time_steps = int(time_steps)
         self._capi = _cabi.load()
         term = torch.as_tensor(termination_distances, dtype=torch.float32).cpu().expand(_cabi.NUM_BODIES)
@@ -208,11 +324,12 @@ class HostStep:
         return self._ctx
 
     def step(self, bufs: HostStepBuffers, reset: Optional[HostResetBuffers] = None, state_init: str = "random",
-             flag_test: bool = False) -> HostStepBuffers:  # fmt: skip
-        """One step of ``bufs``; returns when every output is in ``bufs`` (``progress_buf`` advanced in place).  With
-        ``reset`` the envs the step flags are re-posed as well (see ``submit``); this runs on slot 0."""
-        if reset is not None:
-            self.submit(0, bufs, reset, state_init, flag_test)
+             flag_test: bool = False, device_out: Optional[HostDeviceOutputs] = None) -> HostStepBuffers:  # fmt: skip
+        """One step of ``bufs``; returns when every output is in ``bufs`` (``progress_buf`` advanced in place) and in
+        ``device_out``.  With ``reset`` the envs the step flags are re-posed as well (see ``submit``); with ``reset`` or
+        ``device_out`` this runs on slot 0."""
+        if reset is not None or device_out is not None:
+            self.submit(0, bufs, reset, state_init, flag_test, device_out=device_out)
             return self.wait(0)
         n = bufs.validate(self.time_steps)
         args = bufs._args()
@@ -220,7 +337,8 @@ class HostStep:
         return bufs
 
     def submit(self, slot: int, bufs: HostStepBuffers, reset: Optional[HostResetBuffers] = None,
-               state_init: str = "random", flag_test: bool = False) -> None:  # fmt: skip
+               state_init: str = "random", flag_test: bool = False,
+               device_out: Optional[HostDeviceOutputs] = None) -> None:  # fmt: skip
         """Enqueue one step of ``bufs`` on ``slot`` (0 or 1) and return.  ``bufs`` (and ``reset``) belong to the library
         until ``wait(slot)`` returns: do not read or write them before then.
 
@@ -228,39 +346,68 @@ class HostStep:
         motion library (``state_init`` "random": at ``reset.phase``; "start": at time 0; ``flag_test``: the eval
         mode's time 0).  After ``wait``, ``obs_buf`` holds the final rows, ``reset_buf`` / ``terminate_buf`` the step's
         own flags, ``progress_buf`` is 0 for re-posed envs, and for those envs only ``bufs.state``, the clock tensors
-        and ``reset.root_states`` / ``dof_pos`` / ``dof_vel`` hold the new state."""
-        n = bufs.validate(self.time_steps)
+        and ``reset.root_states`` / ``dof_pos`` / ``dof_vel`` hold the new state.
+
+        With ``device_out`` (``bufs.obs_buf`` None) the rows go to ``device_out.obs`` (and ``obs_norm`` /
+        ``obs_moments``) instead; the kernels writing them wait for the work enqueued so far on the current CUDA
+        stream, so the policy may still be reading the previous rows.  The tensors belong to the library until
+        ``wait(slot)`` returns."""
+        n = bufs.validate(self.time_steps, device_out=device_out is not None)
         args = bufs._args()
-        if reset is None:
+        if device_out is not None:
+            device_out.validate(n, self.time_steps)
+            rargs = None
+            if reset is not None:
+                reset.validate(n)
+                rargs = C.byref(reset._args(bufs, state_init, flag_test))
+            dargs = device_out._args()
+            _cabi.check(self._capi.phc_host_step_submit_device(self._live(), int(slot), C.byref(args), rargs,
+                                                               C.byref(dargs), n), "phc_host_step_submit_device")  # fmt: skip
+            if device_out.obs_moments is not None:
+                device_out.rows += n  # an auto-reset replaces counted rows and adds none
+        elif reset is None:
             _cabi.check(self._capi.phc_host_step_submit(self._live(), int(slot), C.byref(args), n), "phc_host_step_submit")
         else:
             reset.validate(n)
             rargs = reset._args(bufs, state_init, flag_test)
             _cabi.check(self._capi.phc_host_step_submit_reset(self._live(), int(slot), C.byref(args), C.byref(rargs), n),
                         "phc_host_step_submit_reset")  # fmt: skip
+        self._hold(slot, bufs, reset, device_out)
+
+    def _hold(self, slot, bufs, reset, device_out):
+        """Keep a batch's tensors alive until its ``wait``."""
         self._inflight[slot] = bufs
         self._inflight_reset[slot] = reset
+        self._inflight_dev[slot] = device_out
 
     def reset_submit(self, slot: int, bufs: HostStepBuffers, reset: HostResetBuffers, state_init: str = "random",
-                     flag_test: bool = False) -> None:  # fmt: skip
+                     flag_test: bool = False, device_out: Optional[HostDeviceOutputs] = None) -> None:  # fmt: skip
         """Enqueue ``HumanoidPHC.reset(env_ids, phase)`` for the envs of ``reset.env_mask`` on ``slot`` and return:
         reads the clock and ids of ``bufs``; after ``wait``, for the masked envs only, ``obs_buf`` rows, ``state``,
         the clock, ``progress_buf`` = 0, ``reset_buf`` = ``terminate_buf`` = 0 and ``reset``'s root / dof rows hold
-        the re-posed envs.  How a host loop gets its first observation."""
-        n = bufs.validate(self.time_steps)
+        the re-posed envs.  How a host loop gets its first observation.  With ``device_out`` the masked envs' rows go
+        to ``device_out.obs`` / ``obs_norm`` and are added to ``obs_moments`` (rows no step has counted)."""
+        n = bufs.validate(self.time_steps, device_out=device_out is not None)
         reset.validate(n)
         if reset.env_mask is None:
             raise ValueError("reset_submit needs reset.env_mask")
         args, rargs = bufs._args(), reset._args(bufs, state_init, flag_test)
-        _cabi.check(self._capi.phc_host_reset_submit(self._live(), int(slot), C.byref(args), C.byref(rargs), n),
-                    "phc_host_reset_submit")  # fmt: skip
-        self._inflight[slot] = bufs
-        self._inflight_reset[slot] = reset
+        if device_out is None:
+            _cabi.check(self._capi.phc_host_reset_submit(self._live(), int(slot), C.byref(args), C.byref(rargs), n),
+                        "phc_host_reset_submit")  # fmt: skip
+        else:
+            device_out.validate(n, self.time_steps)
+            dargs = device_out._args()
+            _cabi.check(self._capi.phc_host_reset_submit_device(self._live(), int(slot), C.byref(args), C.byref(rargs),
+                                                                C.byref(dargs), n), "phc_host_reset_submit_device")  # fmt: skip
+            if device_out.obs_moments is not None:
+                device_out.rows += int(reset.env_mask.count_nonzero())
+        self._hold(slot, bufs, reset, device_out)
 
     def reset(self, bufs: HostStepBuffers, reset: HostResetBuffers, state_init: str = "random",
-              flag_test: bool = False) -> HostStepBuffers:  # fmt: skip
+              flag_test: bool = False, device_out: Optional[HostDeviceOutputs] = None) -> HostStepBuffers:  # fmt: skip
         """``reset_submit`` on slot 0 + ``wait(0)``."""
-        self.reset_submit(0, bufs, reset, state_init, flag_test)
+        self.reset_submit(0, bufs, reset, state_init, flag_test, device_out)
         return self.wait(0)
 
     def wait(self, slot: int) -> Optional[HostStepBuffers]:
@@ -268,8 +415,8 @@ class HostStep:
         rc = self._capi.phc_host_step_wait(self._live(), int(slot))
         bufs = None
         if 0 <= slot < _cabi.HOST_SLOTS:  # the slot is idle after wait, also when it reports an error
-            bufs, self._inflight[slot] = self._inflight[slot], None
-            self._inflight_reset[slot] = None
+            bufs = self._inflight[slot]
+            self._hold(slot, None, None, None)
         _cabi.check(rc, "phc_host_step_wait")
         return bufs
 
@@ -289,6 +436,7 @@ class HostStep:
             self._capi.phc_host_step_destroy(ctx)  # finishes every slot in flight before freeing
         self._inflight = [None] * _cabi.HOST_SLOTS
         self._inflight_reset = [None] * _cabi.HOST_SLOTS
+        self._inflight_dev = [None] * _cabi.HOST_SLOTS
 
     def __enter__(self) -> "HostStep":
         return self

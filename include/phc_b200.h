@@ -554,6 +554,54 @@ PHC_API int phc_host_step_submit_reset(PhcHostStep* ctx, int32_t slot, const Phc
 PHC_API int phc_host_reset_submit(PhcHostStep* ctx, int32_t slot, const PhcHostStepArgs* args,
                                   const PhcHostResetArgs* reset, int64_t n);
 
+/* Host in, device out: the two submits above with the observation rows written into caller-owned device tensors
+ * instead of host memory.  For a caller whose physics runs on the CPU and whose policy runs on the GPU, the rows are
+ * 99 % of what a host step sends back (3736 B per env at T = 1, against 24 B of rewards, flags and progress); here they
+ * never cross the link, and the fused normaliser (PhcStepArgs.obs_norm) and the RunningNorm moments epilogue
+ * (obs_moments) are available as on the device path.  Sim state and clock still come from host buffers, and rewards,
+ * reward_raw, flags, progress and the reset rows still go to host buffers, exactly as in phc_host_step_submit /
+ * phc_host_step_submit_reset / phc_host_reset_submit.
+ *
+ *   phc_host_step_submit_device   The step (reset == NULL) or the step with auto-reset (reset != NULL).  obs holds
+ *            the step's rows (with a reset: the final rows, a re-posed env's recomputed from its new state), obs_norm
+ *            their normalised copy, and obs_moments += the column sums and sums of squares of the rows written (with a
+ *            reset the final rows are the ones counted, as on the device path with auto-reset).
+ *   phc_host_reset_submit_device  The host reset of the masked envs: their obs rows and normalised rows are written,
+ *            and with obs_moments the new rows are ADDED (HumanoidPHC.reset(): rows no step has counted).  Rows of
+ *            other envs are not touched.
+ *   rows     args->obs_buf must be NULL (writing the rows to both places is not offered: PHC_ERR_UNSUPPORTED).  Every
+ *            other field of PhcHostStepArgs / PhcHostResetArgs keeps its meaning and must be a host pointer.
+ *   ordering A submit records an event on dev->stream, and each of the slot's streams waits for it before its first
+ *            write into a device output; the host-to-device copies of the sim state do not wait.  So the policy may
+ *            still be reading the previous rows of the same tensors, enqueued on dev->stream, when the next submit is
+ *            issued.  When phc_host_step_wait returns, the device outputs are complete (wait blocks on the slot's
+ *            events); work the caller enqueues afterwards on any stream sees them.  `dev` itself is read during the
+ *            submit only; the tensors it names belong to the library until wait returns.
+ *   validation  Everything the host submits check, plus, before anything is enqueued: dev or dev->obs NULL, obs_norm
+ *            without norm_mean / norm_var -> PHC_ERR_NULL; a device field that is not device memory on the context's
+ *            device, or a flag other than PHC_STEP_OBS_NORM_BF16 -> PHC_ERR_UNSUPPORTED; obs or obs_norm not 16-B
+ *            aligned -> PHC_ERR_ALIGN; obs_moments_buckets outside 0..4096, or norm_clip <= 0 with obs_norm ->
+ *            PHC_ERR_SHAPE; a busy slot -> PHC_ERR_BUSY.  After any error the slot is idle and the device outputs are
+ *            untouched.
+ *   schedule As the other submits: not timed by the tuner, the settled schedule (pageable callers: staged).  On the
+ *            staged path no obs transfer is made; on the direct path the scalars are posted into the pinned buffers. */
+typedef struct PhcHostDeviceOut {
+  float* obs;                /* device [n, 358+576*T] fp32, dense rows, 16-B aligned                                   */
+  float* obs_norm;           /* NULL, or device [n, 358+576*T] fp32 (bf16 with PHC_STEP_OBS_NORM_BF16), 16-B aligned   */
+  const float* norm_mean;    /* device [358+576*T] running_mean, required with obs_norm                                */
+  const float* norm_var;     /* device [358+576*T] running_var                                                         */
+  float norm_epsilon, norm_clip;
+  uint32_t flags;            /* 0 or PHC_STEP_OBS_NORM_BF16                                                            */
+  double* obs_moments;       /* NULL, or device [buckets][2*(358+576*T)] fp64 accumulators (+=), as PhcStepArgs        */
+  int32_t obs_moments_buckets;
+  phc_stream_t stream;       /* the caller's stream that reads / writes these tensors (the policy's)                   */
+} PhcHostDeviceOut;
+PHC_API int phc_host_step_submit_device(PhcHostStep* ctx, int32_t slot, const PhcHostStepArgs* args,
+                                        const PhcHostResetArgs* reset /* NULL: no auto-reset */,
+                                        const PhcHostDeviceOut* dev, int64_t n);
+PHC_API int phc_host_reset_submit_device(PhcHostStep* ctx, int32_t slot, const PhcHostStepArgs* args,
+                                         const PhcHostResetArgs* reset, const PhcHostDeviceOut* dev, int64_t n);
+
 /* ------------------------------------------------------------------------------------
  * RunningNorm statistics                                   policies/running_norm.py:23-34
  * phc_obs_moments accumulates (+=) per-column fp64 sum and sum of squares of x[rows,cols]
