@@ -10,6 +10,7 @@
 // Compiled with -fmad=false (see phc_math.cuh).
 #include <algorithm>
 #include <atomic>
+#include <cfloat>
 #include <cstdint>
 #include <cstdio>
 #include <cstdlib>
@@ -703,7 +704,11 @@ __global__ void pd_targets_kernel(const float* __restrict__ action, const float*
     pd = ref_dof_pos[i] + scale[d] * a;
     const float q = dof_pos[env * dp_stride + d * dp_estride];
     const float half_pi = 1.57079637050628662f;  // f32(np.pi / 2)
-    pd = fmaxf(fminf(pd, q + half_pi), q - half_pi);  // maximum(minimum(pd, upper), lower)
+    // maximum(minimum(pd, upper), lower); torch.minimum / maximum propagate a NaN of either operand, fminf / fmaxf
+    // would drop it
+    const float upper = q + half_pi, lower = q - half_pi;
+    pd = pd < upper || pd != pd ? pd : upper;
+    pd = pd > lower || pd != pd ? pd : lower;
   } else {
     pd = offset[d] + scale[d] * a;
   }
@@ -1110,14 +1115,27 @@ __device__ __forceinline__ void write_ref_dof_pos(const StepParams& p, int64_t e
 }
 
 // RunningNorm.forward of one value (policies/running_norm.py:15-20): clamp((x - mean) / sqrt(var + eps)).
-// `sd` = sqrt(var + eps) and `r` ~ 1/sd are per column; the quotient is within 1 ulp of IEEE division.
-__device__ __forceinline__ void norm_column(const StepParams& p, int64_t col, float& mean, float& sd, float& r) {
-  mean = p.norm_mean[col];
-  sd = sqrt_faithful(p.norm_var[col] + p.norm_eps);
+// torch.clamp keeps NaN; fminf / fmaxf would turn it into -clip, so the clamp is two compare-selects.
+__device__ __forceinline__ float norm_clamp(float y, float clip) { return y < -clip ? -clip : (y > clip ? clip : y); }
+// `sd` = sqrt(var + eps) and `r` ~ 1/sd are per column.  sqrt_faithful needs a normal finite argument (rsqrt.approx.ftz
+// flushes a subnormal one, 0 * rsqrt(0) is NaN); 0, subnormals, inf and NaN take IEEE sqrtf.
+__device__ __forceinline__ void norm_column(const float* means, const float* vars, float eps, int64_t col, float& mean,
+                                            float& sd, float& r) {
+  mean = means[col];
+  const float v = vars[col] + eps;
+  sd = v >= FLT_MIN && v <= FLT_MAX ? sqrt_faithful(v) : sqrtf(v);
   r = rcp_approx(sd);
 }
+__device__ __forceinline__ void norm_column(const StepParams& p, int64_t col, float& mean, float& sd, float& r) {
+  norm_column(p.norm_mean, p.norm_var, p.norm_eps, col, mean, sd, r);
+}
+// The quotient is within 1 ulp of IEEE division where q = a * r is finite and sd is normal, and the Newton step is then
+// finite.  Where the step gives NaN, q already is what IEEE division gives (x or the statistics are inf / NaN, or sd
+// is 0 or inf), so q is taken.
 __device__ __forceinline__ float norm_value(float x, float mean, float sd, float r, float clip) {
-  return fminf(fmaxf(div_faithful(x - mean, sd, r), -clip), clip);
+  const float a = x - mean;
+  const float y = div_faithful(a, sd, r);
+  return norm_clamp(y != y ? a * r : y, clip);
 }
 
 // per-body share of power = sum_dof |dof_force * dof_vel| (humanoid_phc.py:1298): body b >= 1 owns
@@ -1522,8 +1540,9 @@ __global__ void __launch_bounds__(K7_EPB* J24) reset_obs_kernel(const ResetParam
           atomicAdd(mom + W + c, x * x);
         }
         if (p.norm.out) {  // policies/running_norm.py:15-20, the step kernels' arithmetic
-          const float sd = sqrt_faithful(p.norm.var[c] + p.norm.eps);
-          const float y = fminf(fmaxf(div_faithful(v - p.norm.mean[c], sd, rcp_approx(sd)), -p.norm.clip), p.norm.clip);
+          float m, sd, r;
+          norm_column(p.norm.mean, p.norm.var, p.norm.eps, c, m, sd, r);
+          const float y = norm_value(v, m, sd, r, p.norm.clip);
           const int64_t at = env * p.norm.stride + c;
           if (p.norm.bf16) reinterpret_cast<__nv_bfloat16*>(p.norm.out)[at] = __float2bfloat16_rn(y);
           else p.norm.out[at] = y;
@@ -3354,7 +3373,7 @@ __global__ void running_norm_forward_kernel(const float* __restrict__ x, int64_t
       if (r + u < r1) {
         float y[VEC];
 #pragma unroll
-        for (int v = 0; v < VEC; ++v) y[v] = fminf(fmaxf((vals[u][v] - m[v]) / sd[v], -clip), clip);
+        for (int v = 0; v < VEC; ++v) y[v] = norm_clamp((vals[u][v] - m[v]) / sd[v], clip);
         float* q = out + (r + u) * out_stride + c;
         if (VEC == 2) *reinterpret_cast<float2*>(q) = make_float2(y[0], y[VEC - 1]);
         else *q = y[0];
