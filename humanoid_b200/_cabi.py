@@ -279,6 +279,16 @@ class PhcHostDeviceOut(C.Structure):
     ]
 
 
+class PhcHostEnvArgs(C.Structure):
+    _fields_ = [
+        ("dof_force", C.c_void_p),
+        ("dof_vel", C.c_void_p),
+        ("rew_power_coef", C.c_float),
+        ("mpjpe", C.c_void_p),
+        ("default_mask", C.c_void_p),
+    ]
+
+
 BUILD_FILTER_RADIUS = 8
 EPISODE_SUM_COLS = 12
 PEER_MAX_WORLD = 16
@@ -372,6 +382,20 @@ SIGNATURES = {
         [C.c_void_p, C.c_int32, C.POINTER(PhcHostStepArgs), C.POINTER(PhcHostResetArgs), C.POINTER(PhcHostDeviceOut),
          C.c_int64],
     ),  # fmt: skip
+    "phc_host_step_submit_env": (
+        C.c_int,
+        [C.c_void_p, C.c_int32, C.POINTER(PhcHostStepArgs), C.POINTER(PhcHostResetArgs), C.POINTER(PhcHostDeviceOut),
+         C.POINTER(PhcHostEnvArgs), C.c_int64],
+    ),  # fmt: skip
+    "phc_host_reset_submit_env": (
+        C.c_int,
+        [C.c_void_p, C.c_int32, C.POINTER(PhcHostStepArgs), C.POINTER(PhcHostResetArgs), C.POINTER(PhcHostDeviceOut),
+         C.POINTER(PhcHostEnvArgs), C.c_int64],
+    ),  # fmt: skip
+    "phc_host_step_set_initial_state": (
+        C.c_int,
+        [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64],
+    ),
     "phc_host_step_path": (C.c_int, [C.c_void_p]),
     "phc_host_step_chunks": (C.c_int, [C.c_void_p]),
     "phc_host_step_tuning_calls": (C.c_int, [C.c_void_p]),

@@ -34,6 +34,13 @@
 // (and the normalised rows and RunningNorm moments) written by the kernels into the caller's device tensors: no obs
 // transfer at all, only the scalars and the reset rows return to the host.  Each chunk's stream waits for an event
 // recorded on the caller's stream before its kernel, so the policy's reads of the previous rows come first.
+//
+// Env options.  phc_host_step_submit_env / phc_host_reset_submit_env run the same pipelines with the power reward (each
+// chunk's dof force and dof velocity rows are copied by the copy engine straight from the caller's buffers into the
+// slot's device scratch: two transfers per chunk, no CPU copy), mpjpe (posted by the kernel on the direct path, in the
+// packed scalars on the staged path) and StateInit.Default / Hybrid (the initial rows are uploaded once per slot by
+// phc_host_step_set_initial_state; the hybrid mask rides in the packed clock).  Every other submit is one of these
+// with no options.
 #include <chrono>
 #include <cstdint>
 #include <cstdio>
@@ -59,18 +66,26 @@ constexpr int kStateFloats = PHC_NUM_BODIES * 13;
 // packed clock, per env: ids i64 | goff 3 f32 | start f32 | soff f32 | progress i16  (SoA per chunk)
 constexpr size_t kClockBytes = 8 + 12 + 4 + 4 + 2;
 // packed scalars out, per env: rew f32 | raw 4 f32 | progress i16 | reset u8 | term u8
+// (with the env options: raw 5 f32 with the power reward, mpjpe f32, and default_mask u8 in the clock)
 constexpr size_t kOutBytes = 4 + 16 + 2 + 1 + 1;
+constexpr int kDof = 69;
 constexpr int kMaxChunks = 1024;
 
 inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
 // sub-array offsets inside a chunk's packed regions (each 16-B aligned)
 struct Layout {
-  size_t ids, goff, start, soff, prog, phase, mask, clock_bytes;
-  size_t rew, raw, oprog, reset, term, out_bytes;
+  size_t ids, goff, start, soff, prog, phase, mask, dmask, clock_bytes;
+  size_t rew, raw, mpjpe, oprog, reset, term, out_bytes;
+};
+// What the env options add to a chunk's packed regions: reward_raw columns (5 with the power reward), mpjpe f32 out,
+// the hybrid default_mask u8 in the clock.
+struct Extra {
+  int raw_cols = 4;
+  bool mpjpe = false, dmask = false;
 };
 // with_reset: the clock also carries phase f32 | env_mask u8 per env
-Layout layout(int64_t m, bool with_reset = false) {
+Layout layout(int64_t m, bool with_reset = false, const Extra& x = Extra{}) {
   Layout L;
   size_t o = 0;
   L.ids = o, o = align_up(o + (size_t)m * 8, 16);
@@ -78,15 +93,19 @@ Layout layout(int64_t m, bool with_reset = false) {
   L.start = o, o = align_up(o + (size_t)m * 4, 16);
   L.soff = o, o = align_up(o + (size_t)m * 4, 16);
   L.prog = o, o = align_up(o + (size_t)m * 2, 16);
-  L.phase = L.mask = o;
+  L.phase = L.mask = L.dmask = o;
   if (with_reset) {
     L.phase = o, o = align_up(o + (size_t)m * 4, 16);
     L.mask = o, o = align_up(o + (size_t)m, 16);
+    L.dmask = o;
+    if (x.dmask) o = align_up(o + (size_t)m, 16);
   }
   L.clock_bytes = o;
   o = 0;
   L.rew = o, o = align_up(o + (size_t)m * 4, 16);
-  L.raw = o, o = align_up(o + (size_t)m * 16, 16);
+  L.raw = o, o = align_up(o + (size_t)m * 4 * x.raw_cols, 16);
+  L.mpjpe = o;
+  if (x.mpjpe) o = align_up(o + (size_t)m * 4, 16);
   L.oprog = o, o = align_up(o + (size_t)m * 2, 16);
   L.reset = o, o = align_up(o + (size_t)m, 16);
   L.term = o, o = align_up(o + (size_t)m, 16);
@@ -165,8 +184,8 @@ struct Slot {
   cudaStream_t streams[kStreams] = {};
   cudaEvent_t done[kStreams] = {};  // recorded on each stream at the end of an enqueue
   cudaEvent_t dev_ready = nullptr;  // device-output submits: recorded on the caller's stream, waited on before a kernel
-  // direct path: verdict cached per set of caller pointers
-  const void* seen[11] = {};
+  // direct path: verdict cached per set of caller pointers (the 11 of PhcHostStepArgs and PhcHostEnvArgs.mpjpe)
+  const void* seen[12] = {};
   int seen_direct = -1;
   // resets, allocated at the first submit that needs them: device root / dof rows of re-posed envs and the flags the
   // reset clears (the caller gets the step's own flags), [max_envs] each; pinned staging of the reset outputs
@@ -177,6 +196,12 @@ struct Slot {
   Rows stage{};
   const void* rseen[9] = {};  // verdict of the reset pointers: the outputs are all pinned and mapped at their address
   int rseen_direct = -1;
+  // env options, allocated at first use: the chunk's dof force and dof velocity rows ([max_envs, 2, 69]: per chunk
+  // m force rows, then m velocity rows), and the initial root / dof rows of StateInit.Default / Hybrid
+  float* d_dof = nullptr;
+  float* d_init = nullptr;  // [max_envs] x (13 root | 69 dof pos | 69 dof vel), init_rows of them set
+  int64_t init_rows = -1;   // -1: no initial state
+  const void* eseen[3] = {};  // the env inputs last found to be host memory
   // the step in flight
   bool busy = false;
   int path = 0;  // 1 direct, 2 staged
@@ -185,6 +210,8 @@ struct Slot {
   int64_t n = 0;
   PhcHostStepArgs args{};
   PhcHostResetArgs rargs{};
+  PhcHostEnvArgs env{};
+  Extra extra{};
   int nchunks = 0;
   int64_t bounds[kMaxChunks + 2] = {};  // staged path: chunk boundaries, for the unpack in wait
 };
@@ -263,6 +290,8 @@ static void slot_free(Slot& s) {
   cudaFree(s.d_clock);
   cudaFree(s.d_out);
   cudaFree(s.d_reset);
+  cudaFree(s.d_dof);
+  cudaFree(s.d_init);
   if (s.h_clock) cudaFreeHost(s.h_clock);
   if (s.h_out) cudaFreeHost(s.h_out);
   if (s.h_rows) cudaFreeHost(s.h_rows);
@@ -276,7 +305,8 @@ static void slot_free(Slot& s) {
 
 // Everything phc_host_step validates, before anything is enqueued; fills the slot's direct-path verdict.  With device
 // outputs (dev_out) obs_buf must be NULL: the rows go to the device tensors only.
-static int check_args(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, int64_t n, bool dev_out = false) {
+static int check_args(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, int64_t n, bool dev_out = false,
+                      const float* mpjpe = nullptr) {
   if (n < 0 || n > c->max_envs) return PHC_ERR_SHAPE;
   if (!a->state || !a->progress_buf || !a->motion_start_times || !a->motion_start_times_offset ||
       !a->global_offset || !a->sampled_motion_ids || (!dev_out && !a->obs_buf) || !a->rew_buf || !a->reward_raw ||
@@ -284,13 +314,13 @@ static int check_args(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, int64_t
     return PHC_ERR_NULL;
   if (dev_out && a->obs_buf) return PHC_ERR_UNSUPPORTED;
   // ---- can the direct path be used: every buffer is pinned / managed host memory mapped at its own address ----------
-  const void* ptrs[11] = {a->state, a->progress_buf, a->motion_start_times, a->motion_start_times_offset,
+  const void* ptrs[12] = {a->state, a->progress_buf, a->motion_start_times, a->motion_start_times_offset,
                           a->global_offset, a->sampled_motion_ids, a->obs_buf, a->rew_buf, a->reward_raw,
-                          a->reset_buf, a->terminate_buf};
+                          a->reset_buf, a->terminate_buf, mpjpe};
   if (s.seen_direct < 0 || memcmp(ptrs, s.seen, sizeof(ptrs)) != 0) {
     int direct = 1;
-    for (int i = 0; i < 11 && direct; ++i) {
-      if (!ptrs[i]) continue;  // obs_buf of a device-output submit
+    for (int i = 0; i < 12 && direct; ++i) {
+      if (!ptrs[i]) continue;  // obs_buf of a device-output submit, mpjpe when not asked for
       cudaPointerAttributes at{};
       if (cudaPointerGetAttributes(&at, ptrs[i]) != cudaSuccess) {
         (void)cudaGetLastError();
@@ -308,13 +338,21 @@ static int check_args(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, int64_t
 }
 
 // Everything the two reset submits validate on top of check_args; fills the slot's verdict for the reset outputs.
-static int check_reset(const PhcHostStep* c, Slot& s, const PhcHostResetArgs* r, int op) {
+// env: the env options of an _env submit, NULL for the submits without them (which refuse StateInit.Default / Hybrid).
+static int check_reset(const PhcHostStep* c, Slot& s, const PhcHostResetArgs* r, int op, const PhcHostEnvArgs* env,
+                       int64_t n) {
   if (!r->state_out || !r->root_states || !r->dof_pos || !r->dof_vel || !r->motion_start_times_out ||
       !r->motion_start_times_offset_out || !r->global_offset_out || (op == kReset && !r->env_mask))
     return PHC_ERR_NULL;
-  // StateInit.Default / Hybrid need the per-env initial_* buffers on the device: not on this path
-  if (r->state_init != PHC_STATE_INIT_START && r->state_init != PHC_STATE_INIT_RANDOM) return PHC_ERR_UNSUPPORTED;
-  if (r->state_init == PHC_STATE_INIT_RANDOM && !r->phase) return PHC_ERR_NULL;
+  if (r->state_init < PHC_STATE_INIT_START || r->state_init > (env ? PHC_STATE_INIT_HYBRID : PHC_STATE_INIT_RANDOM))
+    return PHC_ERR_UNSUPPORTED;
+  if ((r->state_init == PHC_STATE_INIT_RANDOM || r->state_init == PHC_STATE_INIT_HYBRID) && !r->phase)
+    return PHC_ERR_NULL;
+  // StateInit.Default / Hybrid: the slot's initial rows (phc_host_step_set_initial_state) stand for envs 0..n-1
+  if (r->state_init >= PHC_STATE_INIT_DEFAULT) {
+    if (s.init_rows < 0 || (r->state_init == PHC_STATE_INIT_HYBRID && !env->default_mask)) return PHC_ERR_NULL;
+    if (n > s.init_rows) return PHC_ERR_SHAPE;
+  }
   if (!lib_has_dof_state(c->lib)) return PHC_ERR_UNSUPPORTED;
   // outputs first (their verdict), then the two inputs the CPU packs (only refused when on the device)
   const void* ptrs[9] = {r->state_out, r->root_states, r->dof_pos, r->dof_vel, r->motion_start_times_out,
@@ -357,6 +395,47 @@ static int check_dev(const PhcHostStep* c, const PhcHostDeviceOut* d) {
   if (d->obs_moments_buckets < 0 || d->obs_moments_buckets > 4096 || (d->obs_norm && !(d->norm_clip > 0.0f)))
     return PHC_ERR_SHAPE;
   return PHC_OK;
+}
+
+// What the env-option submits validate on top of check_args (which takes mpjpe into the direct-path verdict): the power
+// inputs come in pairs, and every env field is host memory.  The verdict is cached per set of pointers.
+static int check_env(Slot& s, const PhcHostEnvArgs* e) {
+  if (!e->dof_force != !e->dof_vel) return PHC_ERR_NULL;
+  const void* ptrs[3] = {e->dof_force, e->dof_vel, e->default_mask};
+  if (memcmp(ptrs, s.eseen, sizeof(ptrs)) == 0) return PHC_OK;
+  for (const void* p : ptrs) {
+    if (!p) continue;
+    cudaPointerAttributes at{};
+    if (cudaPointerGetAttributes(&at, p) != cudaSuccess) {
+      (void)cudaGetLastError();  // pageable
+    } else if (at.type == cudaMemoryTypeDevice) {
+      return PHC_ERR_UNSUPPORTED;
+    }
+  }
+  memcpy(s.eseen, ptrs, sizeof(ptrs));
+  return PHC_OK;
+}
+
+// The power-reward inputs of one chunk: its dof force and dof velocity rows, copied by the copy engine from the caller's
+// buffers into the slot's scratch, and the step's power fields pointing there.  Two transfers rather than one through
+// staging: packing would first copy 552 B per env on the caller's thread (33 us per 4096-env batch-step on a B200 host,
+// profiles/r6_host_env_options.md).  Nothing without a dof force.
+static cudaError_t power_inputs(const Slot& s, int64_t lo, int64_t m, cudaStream_t st, PhcStepArgs& k) {
+  const PhcHostEnvArgs& e = s.env;
+  if (!e.dof_force) return cudaSuccess;
+  float* df = s.d_dof + lo * 2 * kDof;
+  float* dv = df + m * kDof;
+  const size_t bytes = (size_t)m * kDof * sizeof(float);
+  cudaError_t err = cudaMemcpyAsync(df, e.dof_force + lo * kDof, bytes, cudaMemcpyHostToDevice, st);
+  if (err == cudaSuccess) err = cudaMemcpyAsync(dv, e.dof_vel + lo * kDof, bytes, cudaMemcpyHostToDevice, st);
+  k.dof_force = df;
+  k.dof_force_stride = kDof;
+  k.dof_vel = dv;
+  k.dof_vel_stride = kDof;
+  k.dof_vel_elem_stride = 1;
+  k.rew_power_coef = e.rew_power_coef;
+  k.power_col = 4;
+  return err;
 }
 
 // The chunk's rows in the caller's device tensors.  Chunks start on multiples of 8 envs, so the fp32 and the bf16 rows
@@ -408,6 +487,12 @@ static cudaError_t reset_alloc(const PhcHostStep* c, Slot& s, bool staging) {
   return e;
 }
 
+// The env-option scratch of a slot: the dof rows when this submit has the power reward.
+static cudaError_t env_alloc(const PhcHostStep* c, Slot& s) {
+  if (!s.env.dof_force || s.d_dof) return cudaSuccess;
+  return cudaMalloc((void**)&s.d_dof, (size_t)c->max_envs * 2 * kDof * sizeof(float));
+}
+
 // The caller's buffers as export targets
 static Rows caller_rows(const PhcHostStepArgs* a, const PhcHostResetArgs* r) {
   return {r->state_out, r->root_states, r->dof_pos, r->dof_vel, r->motion_start_times_out,
@@ -422,7 +507,7 @@ static PhcBodyState chunk_body(float* st) {
 
 // Packs a chunk's clock (and, with a reset, its uniform numbers and env mask) into pinned staging.
 static void pack_clock(unsigned char* hc, const Layout& L, const PhcHostStepArgs* a, const PhcHostResetArgs* r,
-                       int64_t lo, int64_t m) {
+                       const PhcHostEnvArgs& env, int64_t lo, int64_t m) {
   memcpy(hc + L.ids, a->sampled_motion_ids + lo, (size_t)m * 8);
   memcpy(hc + L.goff, a->global_offset + lo * 3, (size_t)m * 12);
   memcpy(hc + L.start, a->motion_start_times + lo, (size_t)m * 4);
@@ -430,6 +515,7 @@ static void pack_clock(unsigned char* hc, const Layout& L, const PhcHostStepArgs
   memcpy(hc + L.prog, a->progress_buf + lo, (size_t)m * 2);
   if (r && r->phase) memcpy(hc + L.phase, r->phase + lo, (size_t)m * 4);
   if (r && r->env_mask) memcpy(hc + L.mask, r->env_mask + lo, (size_t)m);
+  if (r && r->state_init == PHC_STATE_INIT_HYBRID) memcpy(hc + L.dmask, env.default_mask + lo, (size_t)m);
 }
 
 // The reset over a chunk's device copies.  A step's auto_reset must name the step's own body / clock / flag / obs
@@ -455,6 +541,15 @@ static PhcResetArgs chunk_reset_args(const PhcHostStep* c, const Slot& s, const 
   ra.phase = r->phase ? (const float*)(dc + L.phase) : nullptr;
   ra.state_init = r->state_init;
   ra.flag_test = r->flag_test;
+  if (r->state_init >= PHC_STATE_INIT_DEFAULT) {  // the slot's initial rows of the chunk's envs
+    const int64_t N = c->max_envs;
+    ra.initial_root_states = s.d_init + lo * 13;
+    ra.initial_root_stride = 13;
+    ra.initial_dof_pos = s.d_init + N * 13 + lo * kDof;
+    ra.initial_dof_vel = s.d_init + N * (13 + kDof) + lo * kDof;
+    ra.initial_dof_stride = kDof;
+    if (r->state_init == PHC_STATE_INIT_HYBRID) ra.default_mask = dc + L.dmask;
+  }
   ra.time_steps = c->T;
   ra.dt = c->dt;
   ra.obs_buf = obs;
@@ -516,7 +611,7 @@ static int direct_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, con
   }
   for (int64_t lo = 0; lo < n; lo += per, ++ci) {
     const int64_t m = (n - lo) < per ? (n - lo) : per;
-    const Layout L = layout(m, r != nullptr);
+    const Layout L = layout(m, r != nullptr, s.extra);
     if (coff + L.clock_bytes > c->pack_capacity || ooff + L.out_bytes > c->pack_capacity)
       return host_fail(s, PHC_ERR_SHAPE, cudaSuccess);
     cudaStream_t st_ = s.streams[ci % kStreams];
@@ -524,7 +619,7 @@ static int direct_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, con
     unsigned char* hc = s.h_clock + coff;
     unsigned char* dc = s.d_clock + coff;
     unsigned char* dout = s.d_out + ooff;
-    pack_clock(hc, L, a, r, lo, m);
+    pack_clock(hc, L, a, r, s.env, lo, m);
     HOST_CUDA(s, cudaMemcpyAsync(dc, hc, L.clock_bytes, cudaMemcpyHostToDevice, st_));
     HOST_CUDA(s, cudaMemcpyAsync(st, a->state + lo * kStateFloats, (size_t)m * kStateFloats * sizeof(float),
                                  cudaMemcpyHostToDevice, st_));
@@ -550,12 +645,14 @@ static int direct_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, con
     k.obs_buf = a->obs_buf + lo * c->obs_dim;
     k.obs_stride = c->obs_dim;
     k.rew_buf = a->rew_buf + lo;
-    k.reward_raw = a->reward_raw + lo * 4;
-    k.reward_raw_stride = 4;
+    k.reward_raw = a->reward_raw + lo * s.extra.raw_cols;
+    k.reward_raw_stride = s.extra.raw_cols;
     k.reset_buf = a->reset_buf + lo;
     k.terminate_buf = a->terminate_buf + lo;
     k.flags = PHC_STEP_MAPPED_HOST_IO;
     k.obs_moments = nullptr;
+    k.mpjpe = s.env.mpjpe ? s.env.mpjpe + lo : nullptr;
+    HOST_CUDA(s, power_inputs(s, lo, m, st_, k));
     if (dev) dev_step_outputs(c, dev, lo, k);
     PhcResetArgs ra;
     if (r) {
@@ -642,13 +739,13 @@ static int staged_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, con
   for (int ci = 0; ci < nchunks; ++ci) {
     const int64_t lo = bounds[ci], m = bounds[ci + 1] - bounds[ci];
     if (m <= 0) continue;
-    const Layout L = layout(m, r != nullptr);
+    const Layout L = layout(m, r != nullptr, s.extra);
     if (coff + L.clock_bytes > c->pack_capacity || ooff + L.out_bytes > c->pack_capacity)
       return host_fail(s, PHC_ERR_SHAPE, cudaSuccess);
     cudaStream_t st_ = s.streams[ci % kStreams];
     // pack the chunk's clock on the host (tens of KB), then ONE transfer
     unsigned char* hc = s.h_clock + coff;
-    pack_clock(hc, L, a, r, lo, m);
+    pack_clock(hc, L, a, r, s.env, lo, m);
     unsigned char* dc = s.d_clock + coff;
     unsigned char* dout = s.d_out + ooff;
     HOST_CUDA(s, cudaMemcpyAsync(s.d_state + lo * kStateFloats, a->state + lo * kStateFloats,
@@ -675,10 +772,12 @@ static int staged_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, con
     k.obs_stride = c->obs_dim;
     k.rew_buf = (float*)(dout + L.rew);
     k.reward_raw = (float*)(dout + L.raw);
-    k.reward_raw_stride = 4;
+    k.reward_raw_stride = s.extra.raw_cols;
     k.reset_buf = dout + L.reset;
     k.terminate_buf = dout + L.term;
     k.obs_moments = nullptr;
+    k.mpjpe = s.extra.mpjpe ? (float*)(dout + L.mpjpe) : nullptr;
+    HOST_CUDA(s, power_inputs(s, lo, m, st_, k));
     if (dev) dev_step_outputs(c, dev, lo, k);
     PhcResetArgs ra;
     if (r) {  // the step's own flags still leave in the packed scalars
@@ -749,13 +848,18 @@ static int reset_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, cons
   int ci = 0;
   for (int64_t lo = 0; lo < n; lo += per, ++ci) {
     const int64_t m = (n - lo) < per ? (n - lo) : per;
-    const Layout L = layout(m, true);
+    const Layout L = layout(m, true, s.extra);
     if (coff + L.clock_bytes > c->pack_capacity) return host_fail(s, PHC_ERR_SHAPE, cudaSuccess);
     cudaStream_t st_ = s.streams[ci % kStreams];
     unsigned char* hc = s.h_clock + coff;
     unsigned char* dc = s.d_clock + coff;
-    pack_clock(hc, L, a, r, lo, m);
+    pack_clock(hc, L, a, r, s.env, lo, m);
     HOST_CUDA(s, cudaMemcpyAsync(dc, hc, L.clock_bytes, cudaMemcpyHostToDevice, st_));
+    // a default-path env keeps its rigid-body rows, and its observation is computed from them: the chunk's sim state
+    // comes in (read before the export writes state_out, which may alias it)
+    if (r->state_init >= PHC_STATE_INIT_DEFAULT)
+      HOST_CUDA(s, cudaMemcpyAsync(s.d_state + lo * kStateFloats, a->state + lo * kStateFloats,
+                                   (size_t)m * kStateFloats * sizeof(float), cudaMemcpyHostToDevice, st_));
     float* obs = dev ? dev_obs(c, dev, lo) : s.d_obs + lo * c->obs_dim;
     PhcResetArgs ra = chunk_reset_args(c, s, r, s.d_state + lo * kStateFloats, dc, L, lo, obs);
     Rows out = rows_at(rows, lo, c->obs_dim);
@@ -786,6 +890,7 @@ static int slot_enqueue(PhcHostStep* c, int slot, const PhcHostStepArgs* a, cons
                         int64_t n, const PhcHostStep::Cand& k, const PhcHostDeviceOut* dev = nullptr) {
   Slot& s = c->slots[slot];
   if (dev) HOST_CUDA(s, cudaEventRecord(s.dev_ready, dev->stream));
+  // s.env / s.extra were set by the submit (zero for phc_host_step)
   const int rc = op == kReset   ? reset_enqueue(c, s, a, r, dev, n, k.chunks)
                  : k.path == 1 ? direct_enqueue(c, s, a, r, dev, n, k.chunks)
                                : staged_enqueue(c, s, a, r, dev, n, k.chunks);
@@ -842,10 +947,12 @@ static int slot_finish(const PhcHostStep* c, Slot& s) {
     for (int ci = 0; ci < s.nchunks; ++ci) {
       const int64_t lo = s.bounds[ci], m = s.bounds[ci + 1] - s.bounds[ci];
       if (m <= 0) continue;
-      const Layout L = layout(m, s.op != kStep);
+      const Layout L = layout(m, s.op != kStep, s.extra);
       const unsigned char* ho = s.h_out + ooff;
+      const int W = s.extra.raw_cols;
       memcpy(a->rew_buf + lo, ho + L.rew, (size_t)m * 4);
-      memcpy(a->reward_raw + lo * 4, ho + L.raw, (size_t)m * 16);
+      memcpy(a->reward_raw + lo * W, ho + L.raw, (size_t)m * 4 * W);
+      if (s.extra.mpjpe) memcpy(s.env.mpjpe + lo, ho + L.mpjpe, (size_t)m * 4);
       memcpy(a->progress_buf + lo, ho + L.oprog, (size_t)m * 2);
       memcpy(a->reset_buf + lo, ho + L.reset, (size_t)m);
       memcpy(a->terminate_buf + lo, ho + L.term, (size_t)m);
@@ -864,8 +971,11 @@ static PhcHostStep::Cand untimed_schedule(const PhcHostStep* c, const Slot& s) {
 }
 
 static int run_sync(PhcHostStep* c, const PhcHostStepArgs* a, int64_t n, const PhcHostStep::Cand& k) {
+  Slot& s = c->slots[0];
+  s.env = PhcHostEnvArgs{};
+  s.extra = Extra{};
   const int rc = slot_enqueue(c, 0, a, nullptr, kStep, n, k);
-  return rc ? rc : slot_finish(c, c->slots[0]);
+  return rc ? rc : slot_finish(c, s);
 }
 
 extern "C" {
@@ -992,17 +1102,28 @@ int phc_host_step(PhcHostStep* c, const PhcHostStepArgs* a, int64_t n) {
 
 // The submits: every check before anything is enqueued, then the slot's buffers, then the enqueue.  dev_out: one of
 // the device-output submits (dev must then name the device tensors).
+// env_entry: one of the _env submits, whose env options (env, NULL for none) may be set; a host reset takes only their
+// default_mask.  The other submits have no options and refuse StateInit.Default / Hybrid, as they always did.
 static int submit(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, const PhcHostResetArgs* r, int op, int64_t n,
-                  bool dev_out = false, const PhcHostDeviceOut* dev = nullptr) {
+                  bool dev_out = false, const PhcHostDeviceOut* dev = nullptr, bool env_entry = false,
+                  const PhcHostEnvArgs* env = nullptr) {
   if (!c || !a || (op != kStep && !r) || (dev_out && (!dev || !dev->obs))) return PHC_ERR_NULL;
   if (slot < 0 || slot >= PHC_HOST_SLOTS) return PHC_ERR_SHAPE;
   Slot& s = c->slots[slot];
   if (s.busy) return PHC_ERR_BUSY;
   if (n == 0) return PHC_OK;
-  int rc = check_args(c, s, a, n, dev_out);
+  PhcHostEnvArgs ev{};
+  if (env && op == kReset) ev.default_mask = env->default_mask;
+  else if (env) ev = *env;
+  int rc = check_args(c, s, a, n, dev_out, ev.mpjpe);
   if (rc) return rc;
-  if (op != kStep && (rc = check_reset(c, s, r, op))) return rc;
+  if ((rc = check_env(s, &ev))) return rc;
+  if (op != kStep && (rc = check_reset(c, s, r, op, env_entry ? &ev : nullptr, n))) return rc;
   if (dev_out && (rc = check_dev(c, dev))) return rc;
+  s.env = ev;
+  s.extra.raw_cols = ev.dof_force ? 5 : 4;
+  s.extra.mpjpe = ev.mpjpe != nullptr;
+  s.extra.dmask = op != kStep && r->state_init == PHC_STATE_INIT_HYBRID;
   cudaError_t e = cudaSuccess;
   if (!s.ready) {
     e = slot_alloc(c, s);
@@ -1013,6 +1134,7 @@ static int submit(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, const 
     s.rows_staged = !s.rseen_direct || (op == kReset && s.seen_direct != 1);
     e = reset_alloc(c, s, s.rows_staged);
   }
+  if (e == cudaSuccess) e = env_alloc(c, s);
   if (e != cudaSuccess) {
     (void)cudaGetLastError();
     return e == cudaErrorMemoryAllocation ? PHC_ERR_ALLOC : phc::record_cuda_error((int)e);
@@ -1044,6 +1166,48 @@ int phc_host_step_submit_device(PhcHostStep* c, int32_t slot, const PhcHostStepA
 int phc_host_reset_submit_device(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, const PhcHostResetArgs* r,
                                  const PhcHostDeviceOut* dev, int64_t n) {
   return submit(c, slot, a, r, kReset, n, true, dev);
+}
+
+int phc_host_step_submit_env(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, const PhcHostResetArgs* r,
+                             const PhcHostDeviceOut* dev, const PhcHostEnvArgs* env, int64_t n) {
+  return submit(c, slot, a, r, r ? kStepReset : kStep, n, dev != nullptr, dev, true, env);
+}
+
+int phc_host_reset_submit_env(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, const PhcHostResetArgs* r,
+                              const PhcHostDeviceOut* dev, const PhcHostEnvArgs* env, int64_t n) {
+  return submit(c, slot, a, r, kReset, n, dev != nullptr, dev, true, env);
+}
+
+int phc_host_step_set_initial_state(PhcHostStep* c, int32_t slot, const float* root_states, const float* dof_pos,
+                                    const float* dof_vel, int64_t n) {
+  if (!c || !root_states || !dof_pos || !dof_vel) return PHC_ERR_NULL;
+  if (slot < 0 || slot >= PHC_HOST_SLOTS || n < 0 || n > c->max_envs) return PHC_ERR_SHAPE;
+  Slot& s = c->slots[slot];
+  if (s.busy) return PHC_ERR_BUSY;
+  const float* src[3] = {root_states, dof_pos, dof_vel};
+  for (const float* p : src) {
+    cudaPointerAttributes at{};
+    if (cudaPointerGetAttributes(&at, p) != cudaSuccess) (void)cudaGetLastError();
+    else if (at.type == cudaMemoryTypeDevice) return PHC_ERR_UNSUPPORTED;
+  }
+  const size_t N = (size_t)c->max_envs;
+  cudaError_t e = cudaSuccess;
+  if (!s.d_init) e = cudaMalloc((void**)&s.d_init, N * (13 + 2 * kDof) * sizeof(float));
+  if (e != cudaSuccess) {
+    (void)cudaGetLastError();
+    return e == cudaErrorMemoryAllocation ? PHC_ERR_ALLOC : phc::record_cuda_error((int)e);
+  }
+  s.init_rows = -1;  // not usable until all three copies have landed
+  float* dst[3] = {s.d_init, s.d_init + N * 13, s.d_init + N * (13 + kDof)};
+  const size_t row[3] = {13, kDof, kDof};
+  for (int i = 0; i < 3 && e == cudaSuccess; ++i)
+    e = cudaMemcpy(dst[i], src[i], (size_t)n * row[i] * sizeof(float), cudaMemcpyHostToDevice);
+  if (e != cudaSuccess) {
+    (void)cudaGetLastError();
+    return phc::record_cuda_error((int)e);
+  }
+  s.init_rows = n;
+  return PHC_OK;
 }
 
 int phc_host_step_wait(PhcHostStep* c, int32_t slot) {

@@ -16,6 +16,12 @@ moments) are written into CUDA tensors instead of ``bufs.obs_buf``: the caller w
 policy runs on the GPU gets the rows where the policy reads them, and only rewards, flags, progress and the reset rows
 cross back to the host.
 
+The reference's default configuration is available too (``phc_host_step_submit_env``): ``HostStep(...,
+use_power_reward=True)`` with ``HostStepBuffers.allocate(..., power=True)`` adds the power reward (the caller's dof force
+and velocity go in, ``reward_raw`` has five columns), ``allocate(..., mpjpe=True)`` the eval-mode mpjpe, and
+``set_initial_state`` per slot enables ``state_init="default"`` / ``"hybrid"`` (the hybrid mask in
+``HostResetBuffers.default_mask``).
+
 Pinned buffers (``HostStepBuffers.allocate(..., pinned=True)``) take the fast paths; pageable ones work through
 staging.  The CUDA device of the motion library must be current when the context is created and stepped; after
 ``MotionLib.repack()`` synchronise the device before the next host step (the steps run on the context's own streams).
@@ -24,7 +30,7 @@ staging.  The CUDA device of the motion library must be current when the context
 from __future__ import annotations
 
 import ctypes as C
-from dataclasses import dataclass, fields
+from dataclasses import dataclass
 from typing import Any, List, Optional, Sequence, Union
 
 import torch
@@ -45,6 +51,12 @@ _FIELDS = (  # name, dtype, trailing shape (T: the number of future steps of the
     ("reset_buf", torch.uint8, lambda T: ()),
     ("terminate_buf", torch.uint8, lambda T: ()),
 )
+_DOF = 69
+_OPTION_FIELDS = (  # the env options (PhcHostEnvArgs): name, trailing shape
+    ("dof_force", (_DOF,)),
+    ("dof_vel", (_DOF,)),
+    ("mpjpe", ()),
+)
 
 
 @dataclass(eq=False)
@@ -52,8 +64,11 @@ class HostStepBuffers:
     """The 11 CPU tensors of one batch of ``n`` envs, in the order of ``PhcHostStepArgs``.  Inputs: ``state``
     [n, 24, 13], the clock (``progress_buf`` int16, advanced in place, ``motion_start_times``,
     ``motion_start_times_offset``, ``global_offset`` [n, 3], ``sampled_motion_ids`` int64).  Outputs: ``obs_buf``
-    [n, 358 + 576 T] (None when the rows go to a ``HostDeviceOutputs``), ``rew_buf``, ``reward_raw`` [n, 4],
-    ``reset_buf`` / ``terminate_buf`` uint8."""
+    [n, 358 + 576 T] (None when the rows go to a ``HostDeviceOutputs``), ``rew_buf``, ``reward_raw`` [n, 4] ([n, 5]
+    with the power reward, its term in column 4), ``reset_buf`` / ``terminate_buf`` uint8.
+
+    Env options (attributes, not constructor arguments), None when off: ``dof_force`` / ``dof_vel`` [n, 69] f32 (inputs of the power reward: the physics'
+    dof force and the velocity half of its dof state), ``mpjpe`` [n] f32 (output, eval mode's ``extras["mpjpe"]``)."""
 
     state: torch.Tensor
     progress_buf: torch.Tensor
@@ -66,38 +81,61 @@ class HostStepBuffers:
     reward_raw: torch.Tensor
     reset_buf: torch.Tensor
     terminate_buf: torch.Tensor
+    # the env options are attributes, not constructor fields: set by allocate(power= / mpjpe=) or assigned
+    dof_force = None
+    dof_vel = None
+    mpjpe = None
 
     @classmethod
-    def allocate(cls, n: int, time_steps: int = 1, pinned: bool = True, host_obs: bool = True) -> "HostStepBuffers":
+    def allocate(cls, n: int, time_steps: int = 1, pinned: bool = True, host_obs: bool = True, power: bool = False,
+                 mpjpe: bool = False) -> "HostStepBuffers":  # fmt: skip
         """Zeroed buffers for ``n`` envs; ``pinned`` page-locks them (needs the CUDA driver).  ``host_obs=False``
-        leaves ``obs_buf`` None, for steps whose rows go to a ``HostDeviceOutputs``."""
+        leaves ``obs_buf`` None, for steps whose rows go to a ``HostDeviceOutputs``.  ``power`` adds ``dof_force`` /
+        ``dof_vel`` and makes ``reward_raw`` [n, 5]; ``mpjpe`` adds ``mpjpe``."""
 
         def make(dtype, trailing):
             t = torch.zeros((n, *trailing), dtype=dtype)
             return t.pin_memory() if pinned else t
 
-        return cls(**{name: make(dtype, shape(time_steps)) if host_obs or name != "obs_buf" else None
-                      for name, dtype, shape in _FIELDS})  # fmt: skip
+        b = cls(**{name: make(dtype, shape(time_steps)) if host_obs or name != "obs_buf" else None
+                   for name, dtype, shape in _FIELDS})  # fmt: skip
+        if power:
+            b.reward_raw = make(torch.float32, (5,))
+            b.dof_force, b.dof_vel = make(torch.float32, (_DOF,)), make(torch.float32, (_DOF,))
+        if mpjpe:
+            b.mpjpe = make(torch.float32, ())
+        return b
 
     @property
     def n(self) -> int:
         return int(self.state.shape[0])
 
-    def validate(self, time_steps: int = 1, device_out: bool = False) -> int:
+    def validate(self, time_steps: int = 1, device_out: bool = False, power: bool = False) -> int:
         """Checks device (CPU), dtype, shape and contiguity of every tensor; returns ``n``.  ``obs_buf`` must be None
-        when the rows go to device outputs (``device_out``), and a tensor otherwise."""
+        when the rows go to device outputs (``device_out``), and a tensor otherwise.  ``power``: the step has the power
+        reward, so ``dof_force`` / ``dof_vel`` are required and ``reward_raw`` is [n, 5]; without it they must be None."""
         n = self.n
         if device_out and self.obs_buf is not None:
             raise _cabi.PhcError("obs_buf must be None when the rows go to device outputs")
-        for name, dtype, shape in _FIELDS:
+        if not power and (self.dof_force is not None or self.dof_vel is not None):
+            raise _cabi.PhcError("dof_force / dof_vel are given but the step has no power reward (use_power_reward)")
+        checks = [(name, dtype, shape(time_steps)) for name, dtype, shape in _FIELDS]
+        if power:
+            checks[_NAMES.index("reward_raw")] = ("reward_raw", torch.float32, (5,))
+            checks += [("dof_force", torch.float32, (_DOF,)), ("dof_vel", torch.float32, (_DOF,))]
+        if self.mpjpe is not None:
+            checks.append(("mpjpe", torch.float32, ()))
+        for name, dtype, shape in checks:
             t = getattr(self, name)
             if device_out and name == "obs_buf":
                 continue
+            if power and t is None and name in ("dof_force", "dof_vel"):
+                raise _cabi.PhcError(f"the power reward needs {name} (HostStepBuffers.allocate(..., power=True))")
             if not isinstance(t, torch.Tensor) or t.device.type != "cpu":
                 raise _cabi.PhcError(f"{name} must be a CPU tensor (the host step takes host buffers)")
             if t.dtype != dtype:
                 raise _cabi.PhcError(f"{name} must be {dtype}, got {t.dtype}")
-            want = (n, *shape(time_steps))
+            want = (n, *shape)
             if tuple(t.shape) != want:
                 raise ValueError(f"{name} has shape {tuple(t.shape)}, expected {want}")
             if not t.is_contiguous():
@@ -105,7 +143,11 @@ class HostStepBuffers:
         return n
 
     def _args(self) -> _cabi.PhcHostStepArgs:
-        return _cabi.PhcHostStepArgs(*[_cabi.ptr(getattr(self, f.name)) for f in fields(self)])
+        """The 11 pointers of ``PhcHostStepArgs`` (the env options travel in ``PhcHostEnvArgs``)."""
+        return _cabi.PhcHostStepArgs(*[_cabi.ptr(getattr(self, name)) for name in _NAMES])
+
+
+_NAMES = [name for name, _, _ in _FIELDS]
 
 
 _RESET_FIELDS = (  # name, dtype, trailing shape
@@ -125,23 +167,27 @@ class HostResetBuffers:
     ``env_mask`` [n] (uint8 or bool, 1 = reset the env).  Outputs, written for the re-posed envs only:
     ``root_states`` [n, 13] (pos 3 | rot 4 | vel 3 | ang vel 3) and ``dof_pos`` / ``dof_vel`` [n, 69] — what the
     caller's physics sets for those envs.  The rigid-body rows and the new clock go into the ``HostStepBuffers``'
-    own ``state`` and clock tensors."""
+    own ``state`` and clock tensors.  ``default_mask`` [n] (uint8 or bool): state init "hybrid", 1 = the env takes the
+    default path (the reference draws it with ``torch.bernoulli``; the caller supplies it, like ``phase``)."""
 
     phase: torch.Tensor
     root_states: torch.Tensor
     dof_pos: torch.Tensor
     dof_vel: torch.Tensor
     env_mask: Optional[torch.Tensor] = None
+    default_mask: Optional[torch.Tensor] = None
 
     @classmethod
-    def allocate(cls, n: int, pinned: bool = True) -> "HostResetBuffers":
-        """Zeroed buffers for ``n`` envs (with a zeroed ``env_mask``); ``pinned`` page-locks them."""
+    def allocate(cls, n: int, pinned: bool = True, hybrid: bool = False) -> "HostResetBuffers":
+        """Zeroed buffers for ``n`` envs (with a zeroed ``env_mask``); ``pinned`` page-locks them; ``hybrid`` adds a
+        zeroed ``default_mask``."""
 
         def make(dtype, trailing):
             t = torch.zeros((n, *trailing), dtype=dtype)
             return t.pin_memory() if pinned else t
 
-        return cls(**{name: make(dtype, shape) for name, dtype, shape in _RESET_FIELDS}, env_mask=make(torch.uint8, ()))
+        return cls(**{name: make(dtype, shape) for name, dtype, shape in _RESET_FIELDS}, env_mask=make(torch.uint8, ()),
+                   default_mask=make(torch.uint8, ()) if hybrid else None)  # fmt: skip
 
     @property
     def n(self) -> int:
@@ -151,8 +197,9 @@ class HostResetBuffers:
         """Checks device (CPU), dtype, shape and contiguity of every tensor (``n`` rows: the batch's); returns ``n``."""
         n = self.n if n is None else int(n)
         fields_ = [(name, (dtype,), shape) for name, dtype, shape in _RESET_FIELDS]
-        if self.env_mask is not None:
-            fields_.append(("env_mask", (torch.uint8, torch.bool), ()))
+        for name in ("env_mask", "default_mask"):
+            if getattr(self, name) is not None:
+                fields_.append((name, (torch.uint8, torch.bool), ()))
         for name, dtypes, shape in fields_:
             t = getattr(self, name)
             if not isinstance(t, torch.Tensor) or t.device.type != "cpu":
@@ -283,7 +330,10 @@ class HostStep:
 
     ``num_chunks = 0`` lets the context tune its schedule (output path, chunk count) over its first synchronous
     ``step`` calls; ``path`` / ``chunks`` report the result (0 while undecided).  ``submit`` before that uses the
-    first candidate.  One thread drives a context."""
+    first candidate.  One thread drives a context.
+
+    ``use_power_reward`` adds ``-rew_power_coef * sum |dof_force * dof_vel|`` (0 while progress <= 3) to every step's
+    reward, as ``reward_raw[:, 4]``; every step then needs ``HostStepBuffers.allocate(..., power=True)``."""
 
     def __init__(
         self,
@@ -297,8 +347,13 @@ class HostStep:
         enable_early_termination: bool = True,
         dt: float = 2 * (1.0 / 60.0),
         rwd_specs: Optional[dict] = None,
+        use_power_reward: bool = False,  # config.py:50 (True in the reference)
+        rew_power_coef: float = 0.0005,  # config.py:112
     ):
         self._ctx = None
+        self.use_power_reward = bool(use_power_reward)
+        self.rew_power_coef = float(rew_power_coef)
+        self._initial_rows: List[Optional[int]] = [None] * _cabi.HOST_SLOTS
         self._inflight: List[Optional[HostStepBuffers]] = [None] * _cabi.HOST_SLOTS
         self._inflight_reset: List[Optional[HostResetBuffers]] = [None] * _cabi.HOST_SLOTS
         self._inflight_dev: List[Optional[HostDeviceOutputs]] = [None] * _cabi.HOST_SLOTS
@@ -328,7 +383,7 @@ class HostStep:
         """One step of ``bufs``; returns when every output is in ``bufs`` (``progress_buf`` advanced in place) and in
         ``device_out``.  With ``reset`` the envs the step flags are re-posed as well (see ``submit``); with ``reset`` or
         ``device_out`` this runs on slot 0."""
-        if reset is not None or device_out is not None:
+        if reset is not None or device_out is not None or self.use_power_reward or bufs.mpjpe is not None:
             self.submit(0, bufs, reset, state_init, flag_test, device_out=device_out)
             return self.wait(0)
         n = bufs.validate(self.time_steps)
@@ -351,10 +406,28 @@ class HostStep:
         With ``device_out`` (``bufs.obs_buf`` None) the rows go to ``device_out.obs`` (and ``obs_norm`` /
         ``obs_moments``) instead; the kernels writing them wait for the work enqueued so far on the current CUDA
         stream, so the policy may still be reading the previous rows.  The tensors belong to the library until
-        ``wait(slot)`` returns."""
-        n = bufs.validate(self.time_steps, device_out=device_out is not None)
+        ``wait(slot)`` returns.
+
+        With the power reward (``use_power_reward``) or ``bufs.mpjpe``, or ``state_init`` "default" / "hybrid" (after
+        ``set_initial_state(slot, ...)``; "hybrid" takes ``reset.default_mask`` and ``reset.phase``), this is
+        ``phc_host_step_submit_env``."""
+        n = bufs.validate(self.time_steps, device_out=device_out is not None, power=self.use_power_reward)
         args = bufs._args()
-        if device_out is not None:
+        env = self._env_args(slot, bufs, reset, state_init, n)
+        if env is not None:
+            rargs = None
+            if reset is not None:
+                reset.validate(n)
+                rargs = C.byref(reset._args(bufs, state_init, flag_test))
+            dargs = None
+            if device_out is not None:
+                device_out.validate(n, self.time_steps)
+                dargs = C.byref(device_out._args())
+            _cabi.check(self._capi.phc_host_step_submit_env(self._live(), int(slot), C.byref(args), rargs, dargs,
+                                                            C.byref(env), n), "phc_host_step_submit_env")  # fmt: skip
+            if device_out is not None and device_out.obs_moments is not None:
+                device_out.rows += n
+        elif device_out is not None:
             device_out.validate(n, self.time_steps)
             rargs = None
             if reset is not None:
@@ -374,6 +447,52 @@ class HostStep:
                         "phc_host_step_submit_reset")  # fmt: skip
         self._hold(slot, bufs, reset, device_out)
 
+    def _env_args(self, slot, bufs: HostStepBuffers, reset: Optional[HostResetBuffers], state_init: str,
+                  n: int, step: bool = True) -> Optional[_cabi.PhcHostEnvArgs]:  # fmt: skip
+        """The env options of one submit, or None when it has none (the submits without options then run)."""
+        power = step and self.use_power_reward
+        mpjpe = step and bufs.mpjpe is not None
+        init = reset is not None and state_init in ("default", "hybrid")
+        if not (power or mpjpe or init):
+            return None
+        e = _cabi.PhcHostEnvArgs()
+        if power:
+            e.dof_force, e.dof_vel = bufs.dof_force.data_ptr(), bufs.dof_vel.data_ptr()
+            e.rew_power_coef = self.rew_power_coef
+        if mpjpe:
+            e.mpjpe = bufs.mpjpe.data_ptr()
+        if init:
+            if not 0 <= slot < _cabi.HOST_SLOTS or self._initial_rows[slot] is None:
+                raise _cabi.PhcError(f"state_init {state_init!r} is not supported on slot {slot} before "
+                                     "set_initial_state(slot, ...) has given it the initial state")  # fmt: skip
+            if state_init == "hybrid":
+                if reset.default_mask is None:
+                    raise ValueError('state_init "hybrid" needs reset.default_mask (HostResetBuffers.allocate(..., hybrid=True))')
+                e.default_mask = reset.default_mask.data_ptr()
+        return e
+
+    def set_initial_state(self, slot: int, root_states: torch.Tensor, dof_pos: torch.Tensor,
+                          dof_vel: torch.Tensor) -> None:  # fmt: skip
+        """The reference's ``_initial_humanoid_root_states`` [n, 13] and ``_initial_dof_pos`` / ``_initial_dof_vel``
+        [n, 69] (f32 CPU tensors) of the envs submitted on ``slot``: row i is env i of every batch on that slot.  Copied
+        once, synchronously, to the device; the tensors may be freed afterwards.  Needed for state init "default" /
+        "hybrid"; the slot must be idle."""
+        n = None
+        for name, t, width in (("root_states", root_states, 13), ("dof_pos", dof_pos, _DOF), ("dof_vel", dof_vel, _DOF)):
+            if not isinstance(t, torch.Tensor) or t.device.type != "cpu":
+                raise _cabi.PhcError(f"{name} must be a CPU tensor (the host step takes host buffers)")
+            if t.dtype != torch.float32:
+                raise _cabi.PhcError(f"{name} must be torch.float32, got {t.dtype}")
+            n = int(t.shape[0]) if n is None and t.dim() == 2 else n
+            if t.dim() != 2 or tuple(t.shape) != (n, width):
+                raise ValueError(f"{name} has shape {tuple(t.shape)}, expected {(n, width)}")
+            if not t.is_contiguous():
+                raise _cabi.PhcError(f"{name} must be contiguous")
+        _cabi.check(self._capi.phc_host_step_set_initial_state(self._live(), int(slot), root_states.data_ptr(),
+                                                               dof_pos.data_ptr(), dof_vel.data_ptr(), n),
+                    "phc_host_step_set_initial_state")  # fmt: skip
+        self._initial_rows[slot] = n
+
     def _hold(self, slot, bufs, reset, device_out):
         """Keep a batch's tensors alive until its ``wait``."""
         self._inflight[slot] = bufs
@@ -386,13 +505,24 @@ class HostStep:
         reads the clock and ids of ``bufs``; after ``wait``, for the masked envs only, ``obs_buf`` rows, ``state``,
         the clock, ``progress_buf`` = 0, ``reset_buf`` = ``terminate_buf`` = 0 and ``reset``'s root / dof rows hold
         the re-posed envs.  How a host loop gets its first observation.  With ``device_out`` the masked envs' rows go
-        to ``device_out.obs`` / ``obs_norm`` and are added to ``obs_moments`` (rows no step has counted)."""
-        n = bufs.validate(self.time_steps, device_out=device_out is not None)
+        to ``device_out.obs`` / ``obs_norm`` and are added to ``obs_moments`` (rows no step has counted).  State init
+        "default" / "hybrid" as in ``submit`` (``phc_host_reset_submit_env``); the power inputs are not read."""
+        n = bufs.validate(self.time_steps, device_out=device_out is not None, power=self.use_power_reward)
         reset.validate(n)
         if reset.env_mask is None:
             raise ValueError("reset_submit needs reset.env_mask")
         args, rargs = bufs._args(), reset._args(bufs, state_init, flag_test)
-        if device_out is None:
+        env = self._env_args(slot, bufs, reset, state_init, n, step=False)
+        if env is not None:
+            dargs = None
+            if device_out is not None:
+                device_out.validate(n, self.time_steps)
+                dargs = C.byref(device_out._args())
+            _cabi.check(self._capi.phc_host_reset_submit_env(self._live(), int(slot), C.byref(args), C.byref(rargs),
+                                                             dargs, C.byref(env), n), "phc_host_reset_submit_env")  # fmt: skip
+            if device_out is not None and device_out.obs_moments is not None:
+                device_out.rows += int(reset.env_mask.count_nonzero())
+        elif device_out is None:
             _cabi.check(self._capi.phc_host_reset_submit(self._live(), int(slot), C.byref(args), C.byref(rargs), n),
                         "phc_host_reset_submit")  # fmt: skip
         else:

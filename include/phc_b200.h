@@ -530,7 +530,7 @@ PHC_API int64_t phc_host_step_d2h_bytes(const PhcHostStep* ctx, int64_t n);
  *            host loop gets its first observation and resets envs it picks itself.
  *   validation  Everything phc_host_step_submit checks, plus: NULL reset pointers (env_mask for phc_host_reset_submit,
  *            phase for PHC_STATE_INIT_RANDOM) -> PHC_ERR_NULL; PHC_STATE_INIT_DEFAULT / HYBRID (they need per-env
- *            initial_* buffers) or any other state_init, a device pointer, or a motion library without local rotations
+ *            initial_* buffers: phc_host_step_submit_env / phc_host_reset_submit_env below) or any other state_init, a device pointer, or a motion library without local rotations
  *            / dof velocities -> PHC_ERR_UNSUPPORTED; a busy slot -> PHC_ERR_BUSY.  All before anything is enqueued;
  *            after any error the slot is idle.
  *   buffers / tuning / destroy  As for phc_host_step_submit: the reset buffers belong to the library until
@@ -601,6 +601,59 @@ PHC_API int phc_host_step_submit_device(PhcHostStep* ctx, int32_t slot, const Ph
                                         const PhcHostDeviceOut* dev, int64_t n);
 PHC_API int phc_host_reset_submit_device(PhcHostStep* ctx, int32_t slot, const PhcHostStepArgs* args,
                                          const PhcHostResetArgs* reset, const PhcHostDeviceOut* dev, int64_t n);
+
+/* Env options on the host-buffer path: the power reward, eval-mode mpjpe and StateInit.Default / Hybrid, which the
+ * reference's default configuration uses (config.py:50, humanoid_phc.py:159-167, :678-745).  Added without a change to
+ * any existing struct or entry point, so PHC_ABI_VERSION stays 6; a caller finds these by their symbols.
+ *
+ *   phc_host_step_submit_env   phc_host_step_submit (reset == NULL, dev == NULL), _submit_reset (reset != NULL) or
+ *            _submit_device (dev != NULL) with the options of env (NULL: none).  Everything those submits do and check
+ *            still holds.
+ *   phc_host_reset_submit_env  phc_host_reset_submit (dev == NULL) or phc_host_reset_submit_device, likewise.  It
+ *            takes only env->default_mask: dof_force, dof_vel and mpjpe are ignored.
+ *   power    With dof_force set, args->reward_raw is [n, 5]: column 4 receives r = -rew_power_coef * sum_dof |dof_force *
+ *            dof_vel|, 0 while progress <= 3, and rew_buf includes it (reward_raw[:, -1] of the reference,
+ *            humanoid_phc.py:1297-1305); exactly PhcStepArgs.dof_force / power_col.  Each chunk's dof_force and dof_vel
+ *            rows are copied to the device by the copy engine, straight from these buffers (pin them for speed).
+ *   mpjpe    With mpjpe set, mpjpe[i] = mean over the 24 bodies of |rigid_body_pos - ref rg_pos| at the reward time
+ *            (PhcStepArgs.mpjpe), written like rew_buf: posted by the kernel on the direct path (mpjpe then joins the
+ *            buffers that decide it), unpacked by wait on the staged path.
+ *   state init  PHC_STATE_INIT_DEFAULT / HYBRID are accepted once phc_host_step_set_initial_state has given the slot its
+ *            initial rows: row i stands for env i of every batch submitted on that slot.  A default-path env keeps its
+ *            rigid-body rows and clock; its root / dof rows become the initial ones; its observation is that of the
+ *            unchanged state at the restarted progress.  HYBRID takes env->default_mask (1 = default path) and phase
+ *            (the envs that take reference-state init).  The re-posed rows leave as with the other reset modes.
+ *   validation  Before anything is enqueued, on top of the checks of the matching submit: dof_force without dof_vel
+ *            or the reverse, HYBRID without default_mask or phase, DEFAULT / HYBRID on a slot without initial rows ->
+ *            PHC_ERR_NULL; n larger than the slot's initial rows (DEFAULT / HYBRID) -> PHC_ERR_SHAPE; a device pointer
+ *            in env -> PHC_ERR_UNSUPPORTED.  After any error the slot is idle and nothing is written.
+ *   buffers / schedule  As the matching submit: env's buffers belong to the library until phc_host_step_wait returns;
+ *            not timed by the tuner; the settled schedule.  phc_host_step_h2d_bytes / _d2h_bytes describe the plain
+ *            step: the power reward adds 2 x 276 B per env inbound, mpjpe and the fifth reward column 4 B each outbound.
+ *
+ * phc_host_step_set_initial_state  Copies n initial rows (_initial_humanoid_root_states [n,13], _initial_dof_pos /
+ *            _initial_dof_vel [n,69], dense; humanoid_phc.py:521, 543-544) once, synchronously, into the slot's device
+ *            buffers (allocated at the first call, max_envs rows), replacing any earlier rows.  Host memory, pinned or
+ *            pageable: the reference sets them once at setup, so they do not travel with every submit.  NULL pointer ->
+ *            PHC_ERR_NULL; bad slot or n outside 0..max_envs -> PHC_ERR_SHAPE; a device pointer -> PHC_ERR_UNSUPPORTED;
+ *            the slot in flight -> PHC_ERR_BUSY. */
+typedef struct PhcHostEnvArgs {
+  const float* dof_force;    /* host [n,69] dense, or NULL: no power reward              humanoid_phc.py:506     */
+  const float* dof_vel;      /* host [n,69] dense, required with dof_force               humanoid_phc.py:536     */
+  float rew_power_coef;      /* config.py:112                                                                    */
+  float* mpjpe;              /* host [n] out, or NULL                                    humanoid_phc.py:159-167 */
+  const uint8_t* default_mask; /* host [n], PHC_STATE_INIT_HYBRID: 1 = default path      humanoid_phc.py:733-745 */
+} PhcHostEnvArgs;
+PHC_API int phc_host_step_submit_env(PhcHostStep* ctx, int32_t slot, const PhcHostStepArgs* args,
+                                     const PhcHostResetArgs* reset /* NULL: no auto-reset */,
+                                     const PhcHostDeviceOut* dev /* NULL: host obs */,
+                                     const PhcHostEnvArgs* env /* may be NULL */, int64_t n);
+PHC_API int phc_host_reset_submit_env(PhcHostStep* ctx, int32_t slot, const PhcHostStepArgs* args,
+                                      const PhcHostResetArgs* reset, const PhcHostDeviceOut* dev /* may be NULL */,
+                                      const PhcHostEnvArgs* env /* may be NULL */, int64_t n);
+PHC_API int phc_host_step_set_initial_state(PhcHostStep* ctx, int32_t slot, const float* root_states /* [n,13] */,
+                                            const float* dof_pos /* [n,69] */, const float* dof_vel /* [n,69] */,
+                                            int64_t n);
 
 /* ------------------------------------------------------------------------------------
  * RunningNorm statistics                                   policies/running_norm.py:23-34
