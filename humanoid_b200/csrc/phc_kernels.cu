@@ -1087,6 +1087,7 @@ struct StepParams {
   int power_col;
   int64_t n;
   int first_wave_blocks;      // blocks that can be resident at once (speculate before the dependency wait)
+  int spec4_blocks;           // blocks [0, spec4_blocks) speculate on progress + 3 too (the spare slots of one wave)
   int spec_fault;             // test hook: perturb the speculated clock (PHC_OPT_TEST_SPEC_FAULT)
   unsigned long long* trace;  // NULL, or [grid][8] globaltimer stamps (phc_set_trace_buffer)
   const uint8_t* env_mask;  // NULL, or [n]: only envs with a non-zero byte are processed (generic kernel)
@@ -1717,13 +1718,21 @@ __device__ __forceinline__ void reset_in_step(const StepParams& p, FastSmem<EPB>
 // EP: compiled with the wrapper's episode bookkeeping in the reduction warp (used when ep_returns is set)
 // RESET: compiled with the in-step reset of the flagged envs (used when reset_on is set)
 // DEF: the env's default self-obs flags (height column, local root, upright): constant columns, 934-float rows
-template <int EPB, int MINB, bool NORM = false, bool EP = false, bool RESET = false, bool DEF = true>
+// PLAIN: compiled without the per-step options — power reward, ref_dof_pos, mpjpe, eval mode (use_mean), RunningNorm
+// moments, rew_out, progress_mirror — and with goff set: the headline step issues their run-time branches in its
+// issue-bound phases, and the eval-mode selection arrays are most of its stack frame
+template <int EPB, int MINB, bool NORM = false, bool EP = false, bool RESET = false, bool DEF = true, bool PLAIN = false>
 __global__ void __launch_bounds__(EPB* J24, MINB) step_fast_kernel(const __grid_constant__ StepParams p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   FastSmem<EPB>& S = *reinterpret_cast<FastSmem<EPB>*>(smem_raw);
   constexpr int NT = EPB * J24;
   static_assert(4 * EPB <= 32, "reductions run on one warp");
   static_assert(!NORM || DEF, "the normaliser epilogue is laid out for the default 934-float rows");
+  static_assert(!PLAIN || (!NORM && !EP && !RESET && DEF), "the plain step carries none of the epilogues");
+  const bool use_mean = !PLAIN && p.use_mean;
+  const bool dof_force = !PLAIN && p.dof_force;
+  const bool ref_dof_pos = !PLAIN && p.ref_dof_pos;
+  const bool moments = !PLAIN && p.moments;
   const int tid = threadIdx.x;
   const int64_t env0 = (int64_t)blockIdx.x * EPB;
   const int nvalid = p.n <= env0 ? 0 : (int)((p.n - env0) < EPB ? (p.n - env0) : EPB);
@@ -1747,6 +1756,9 @@ __global__ void __launch_bounds__(EPB* J24, MINB) step_fast_kernel(const __grid_
   if (p.first_wave_blocks > 0) asm volatile("griddepcontrol.launch_dependents;\n" ::: "memory");
   // blocks beyond the first wave start after the dependency is long resolved: nothing to overlap
   const bool speculate = blockIdx.x < (unsigned)p.first_wave_blocks;
+  // only the blocks dispatched into the slots the previous step leaves free run this early enough to find progress not
+  // yet advanced; the others enter as the previous step's blocks exit, long after it was written
+  const bool spec4 = blockIdx.x < (unsigned)p.spec4_blocks;
   if (tid < 32) {
     static_assert(EPB == 4, "phase 0 maps 8 lanes to each of 4 envs");
     if (tid == 0) mbar_init(&S.bar, 1);
@@ -1784,14 +1796,16 @@ __global__ void __launch_bounds__(EPB* J24, MINB) step_fast_kernel(const __grid_
     }
     // Slots hold 4 frames.  Candidates 0..1 serve "progress unchanged since speculation" (the
     // usual case: the previous step wrote progress long before this block started), 1..2 serve
-    // "moved by one"; take all three when they fit, else the first two.
+    // "moved by one".  Blocks in spare slots (spec4) copy the frames of all three when they fit;
+    // the others copy those of the first two, and fetch the rest after validation if progress
+    // moved by one after all (slot = frame - s_lo either way).
     const int hi1 = __shfl_sync(0xffffffffu, c_f1, (tid & ~7) + 1);
     const int hi2 = __shfl_sync(0xffffffffu, c_f1, (tid & ~7) + 2);
     const int s_lo = c_f0;  // on the leader: candidate 0's first frame
     const bool all3 = hi2 - s_lo <= 3 && hi2 >= hi1;
-    const int s_hi = all3 ? hi2 : hi1;
+    const int s_hi = all3 && spec4 ? hi2 : hi1;
     const bool spec = speculate && lead && s_hi - s_lo <= 3 && s_hi >= s_lo;
-    if (spec) {  // frames of all three candidates -> slots 0..(hi-lo)
+    if (spec) {  // frames of the speculated candidates -> slots 0..(hi-lo)
       const uint32_t bytes = (uint32_t)(s_hi - s_lo + 1) * (uint32_t)(FRAME_FLOATS * 4);
       mbar_expect_tx(&S.bar, bytes);
       bulk_g2s(fr, p.L.packed + (st + s_lo) * FRAME_FLOATS, bytes, &S.bar);
@@ -1809,7 +1823,7 @@ __global__ void __launch_bounds__(EPB* J24, MINB) step_fast_kernel(const __grid_
     if (p.first_wave_blocks <= 0) asm volatile("griddepcontrol.launch_dependents;\n" ::: "memory");
     PHC_STAMP(2);
     // -- dependent data: one round of clock loads, the sim rows' copy issued under them
-    int prog_in = 0;
+    int prog_in = 0, dd = 0;
     bool ok = false;
     float start = 0.0f, soff = 0.0f, g0 = 0.0f, g1 = 0.0f, g2 = 0.0f;
     int64_t id = 0;
@@ -1818,7 +1832,7 @@ __global__ void __launch_bounds__(EPB* J24, MINB) step_fast_kernel(const __grid_
       id = __ldcg(p.ids + env);
       start = __ldcg(p.start + env);
       soff = __ldcg(p.start_off + env);
-      if (p.goff) {
+      if (PLAIN || p.goff) {
         g0 = __ldcg(p.goff + env * 3 + 0);
         g1 = __ldcg(p.goff + env * 3 + 1);
         g2 = __ldcg(p.goff + env * 3 + 2);
@@ -1828,7 +1842,7 @@ __global__ void __launch_bounds__(EPB* J24, MINB) step_fast_kernel(const __grid_
         mbar_expect_tx(&S.bar, bytes);
         bulk_g2s(S.sim + le * ROW13, p.body.pos.ptr + env * p.body.pos.stride_env, bytes, &S.bar);
       }
-      const int dd = prog_in - sprog;
+      dd = prog_in - sprog;
       ok = speculate && id == sid && __float_as_uint(start) == __float_as_uint(sstart) &&
            __float_as_uint(soff) == __float_as_uint(ssoff) && (dd == 0 || (dd == 1 && all3));
     }
@@ -1868,7 +1882,7 @@ __global__ void __launch_bounds__(EPB* J24, MINB) step_fast_kernel(const __grid_
       S.fallen[le] = 0;
       if (p.advance) {
         p.progress[env] = (int16_t)prog;
-        if (p.progress_mirror) p.progress_mirror[env] = (int16_t)prog;
+        if (!PLAIN && p.progress_mirror) p.progress_mirror[env] = (int16_t)prog;
       }
       S.goff[le][0] = g0;
       S.goff[le][1] = g1;
@@ -1876,12 +1890,17 @@ __global__ void __launch_bounds__(EPB* J24, MINB) step_fast_kernel(const __grid_
       if (RESET) {
         S.meta_len[le] = len, S.meta_mdt[le] = mdt, S.meta_nf[le] = nf, S.meta_st[le] = st;
       }
-      if (p.ref_dof_pos) S.row1[0][le] = st + b_f0, S.row1[1][le] = st + b_f1;
+      if (ref_dof_pos) S.row1[0][le] = st + b_f0, S.row1[1][le] = st + b_f1;
       if (ok && spec) {  // frames are already (arriving) in the slots
         S.slot[0][0][le] = a_f0 - s_lo;
         S.slot[0][1][le] = a_f1 - s_lo;
         S.slot[1][0][le] = b_f0 - s_lo;
         S.slot[1][1][le] = b_f1 - s_lo;
+        if (dd == 1 && s_hi < hi2) {  // moved by one in a block that speculated on two candidates: rows s_hi+1 .. hi2
+          const uint32_t bytes = (uint32_t)(hi2 - s_hi) * (uint32_t)(FRAME_FLOATS * 4);
+          mbar_expect_tx(&S.bar, bytes);
+          bulk_g2s(fr + (s_hi - s_lo + 1) * FRAME_FLOATS, p.L.packed + (st + s_hi + 1) * FRAME_FLOATS, bytes, &S.bar);
+        }
       } else {
         // frames of one clip are consecutive rows of the packed table: when the (up to four)
         // frames span <= 4 rows they arrive with ONE copy and slot = frame - first
@@ -1912,6 +1931,13 @@ __global__ void __launch_bounds__(EPB* J24, MINB) step_fast_kernel(const __grid_
       }
     }
     __syncwarp();
+    if (p.trace) {  // the block's phase-0 path, in warp 1's unused stamp 1 (profiles/trace_step.py)
+      const unsigned fetch = __ballot_sync(0xffffffffu, lead && ok && spec && dd == 1 && s_hi < hi2);
+      const unsigned fresh = __ballot_sync(0xffffffffu, lead && !spec);
+      if (tid == 0)
+        p.trace[((size_t)blockIdx.x * 3 + 1) * 8 + 1] =
+            16u | (spec4 ? 1u : 0u) | (fetch ? 2u : 0u) | (any_redo ? 4u : 0u) | (fresh ? 8u : 0u);
+    }
     if (tid == 0) {
       S.parity = any_redo ? 1 : 0;
       mbar_arrive(&S.bar);
@@ -1958,8 +1984,8 @@ __global__ void __launch_bounds__(EPB* J24, MINB) step_fast_kernel(const __grid_
       S.part[3][e][b] = sa;
       const float dist = norm3(pos - r0.pos);  // torch.norm(rigid_body_pos - ref_body_pos), common.py:343/348
       S.part[4][e][b] = dist;
-      if (!p.use_mean && (p.reset_mask >> b & 1u) && dist > p.term_dist[b]) S.fallen[e] = 1;  // any(), benign race
-      if (p.dof_force) S.part[5][e][b] = power_partial(p, env0 + e, b);
+      if (!use_mean && (p.reset_mask >> b & 1u) && dist > p.term_dist[b]) S.fallen[e] = 1;  // any(), benign race
+      if (dof_force) S.part[5][e][b] = power_partial(p, env0 + e, b);
     }
     r1 = blend_ref2(fr + S.slot[1][0][e] * FRAME_FLOATS, fr + S.slot[1][1][e] * FRAME_FLOATS, S.bl[1][e], S.goff[e], b);
   }
@@ -2035,7 +2061,7 @@ __global__ void __launch_bounds__(EPB* J24, MINB) step_fast_kernel(const __grid_
   } else {
     for (int i = tid; i < nvalid * RW; i += NT) p.obs[env0 * RW + i] = S.frames[i];
   }
-  if (p.moments) {
+  if (moments) {
     // RunningNorm partials: per-column fp64 sum / sum of squares of the block's staged rows, added to one of the
     // accumulator buckets: 1868 fp64 adds in L2 per block of four envs (1.9 M per 4096-env step: +3.8 us on a 6.7 us
     // step).  Two ways to cut that were built and measured in round 2 (profiles/r2_step_variants.md):
@@ -2095,7 +2121,7 @@ __global__ void __launch_bounds__(EPB* J24, MINB) step_fast_kernel(const __grid_
   }
   // res_action: dof_pos of the query at t + dt (humanoid_phc.py:1115-1120), off the critical path; a just-reset env
   // got its row from the reset above
-  if (p.ref_dof_pos && valid && !(RESET && my_rst))
+  if (ref_dof_pos && valid && !(RESET && my_rst))
     write_ref_dof_pos(p, env0 + e, b, S.row1[0][e], S.row1[1][e], S.bl[1][e]);
   // RunningNorm.forward, fp32 rows, full blocks: once the raw store has READ the stage, normalise it in place and
   // send it out with a second bulk store instead of 20 scattered 8-byte stores per thread
@@ -2177,18 +2203,18 @@ __global__ void __launch_bounds__(EPB* J24, MINB) step_fast_kernel(const __grid_
     int flags = 0;              // lanes k == 1: bit 0 = reset, bit 1 = terminated
     if (act && k == 0) {
       r = p.rwd.w_pos * t0 + p.rwd.w_rot * t1 + p.rwd.w_vel * t2 + p.rwd.w_ang_vel * t3;
-      if (p.dof_force) {
+      if (dof_force) {
         pr = power_reward(p, &S.part[5][le][0], S.prog[le]);
         r += pr;  // rew_buf[:] += power_reward (humanoid_phc.py:1304)
         p.raw[(env0 + le) * p.raw_stride + p.power_col] = pr;
       }
       p.rew[env0 + le] = r;
-      if (p.rew_out) p.rew_out[env0 + le] = r;
+      if (!PLAIN && p.rew_out) p.rew_out[env0 + le] = r;
     }
     if (act && k == 1) {
       bool fallen = false;
       if (p.early) {
-        if (p.use_mean) {  // eval mode: mean distance of the selected bodies vs the first one's threshold
+        if (use_mean) {  // eval mode: mean distance of the selected bodies vs the first one's threshold
           float sel[J24];
           int m = 0;
 #pragma unroll
@@ -2211,7 +2237,7 @@ __global__ void __launch_bounds__(EPB* J24, MINB) step_fast_kernel(const __grid_
       if (p.reset_out) p.reset_out[env0 + le] = rs ? 1 : 0;
       flags = (rs ? 1 : 0) | (fallen ? 2 : 0);
     }
-    if (act && k == 2 && p.mpjpe) p.mpjpe[env0 + le] = row_sum24(&S.part[4][le][0]) / 24.0f;  // humanoid_phc.py:167
+    if (!PLAIN && act && k == 2 && p.mpjpe) p.mpjpe[env0 + le] = row_sum24(&S.part[4][le][0]) / 24.0f;  // humanoid_phc.py:167
     if constexpr (EP) if (p.ep_returns) {
       // PHCPufferEnv.step's bookkeeping (clean_pufferl/env.py:121-159) for the block's envs, on the lanes that hold the
       // reward; the block's sums go to one of ep_buckets fp64 accumulators (atomics on one address serialise).  The sums
@@ -2281,7 +2307,7 @@ __global__ void __launch_bounds__(EPB* J24, MINB) step_fast_kernel(const __grid_
     }
   }
   if (bulk_ok && tid == NT - 1) bulk_wait_read();  // shared memory must outlive the store's reads
-  if (p.moments && p.moments_bulk && tid == 0) bulk_wait_read();  // ... and the reductions'
+  if (moments && p.moments_bulk && tid == 0) bulk_wait_read();  // ... and the reductions'
   PHC_STAMP(7);
 }
 
@@ -3987,6 +4013,7 @@ static int step_fill_params(const PhcLib* lib, const PhcStepArgs* a, int64_t n, 
       return PHC_ERR_SHAPE;
   }
   p.first_wave_blocks = 0;
+  p.spec4_blocks = 0;
   p.spec_fault = g_spec_fault;
   p.env_mask = nullptr;
   p.obs_only = 0;
@@ -4185,10 +4212,16 @@ int step_fused_mirrored(const PhcLib* lib, const PhcStepArgs* args, int64_t n, p
       p.first_wave_blocks = 0;
       --lib->unspeculated_steps;
     }
-    // instantiations <EPB, blocks/SM, NORM, EP, RESET, DEF>: the plain one carries none of the optional epilogues; the
-    // RESET ones are compiled with the bookkeeping too (both are switched at run time inside); one catch-all for
-    // non-default self-obs flags
-    static bool attr[7][64] = {};
+    // a grid smaller than one wave leaves first_wave_blocks - grid slots free: that many blocks enter before the
+    // previous step's blocks exit and speculate on a third candidate
+    const int64_t grid = (p.n + 3) / 4;
+    p.spec4_blocks = p.first_wave_blocks > grid ? (int)(p.first_wave_blocks - grid) : 0;
+    // instantiations <EPB, blocks/SM, NORM, EP, RESET, DEF, PLAIN>: <4, 8> carries none of the optional epilogues,
+    // the PLAIN one none of the per-step options either; the RESET ones are compiled with the bookkeeping too (both
+    // are switched at run time inside); one catch-all for non-default self-obs flags
+    const bool plain = !p.dof_force && !p.ref_dof_pos && !p.mpjpe && !p.use_mean && !p.moments && !p.rew_out &&
+                       !p.progress_mirror && p.goff;
+    static bool attr[8][64] = {};
     const bool pdl = g_pdl != 0;
     constexpr size_t SM = sizeof(FastSmem<4>);
     // the moments epilogue leaves as TMA bulk reductions when the accumulators are 16-B aligned
@@ -4207,6 +4240,8 @@ int step_fused_mirrored(const PhcLib* lib, const PhcStepArgs* args, int64_t n, p
       rc = launch_step(step_fast_kernel<4, 8, true, true>, SM, 4, pk, stream, &attr[3][dev], pdl);
     else if (p.ep_returns) rc = launch_step(step_fast_kernel<4, 8, false, true>, SM, 4, pk, stream, &attr[2][dev], pdl);
     else if (p.obs_norm) rc = launch_step(step_fast_kernel<4, 8, true>, SM, 4, pk, stream, &attr[1][dev], pdl);
+    else if (plain)
+      rc = launch_step(step_fast_kernel<4, 8, false, false, false, true, true>, SM, 4, pk, stream, &attr[7][dev], pdl);
     else rc = launch_step(step_fast_kernel<4, 8>, SM, 4, pk, stream, &attr[0][dev], pdl);
     if (rc != PHC_OK || !reset_after) return rc;
   } else {

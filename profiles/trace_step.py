@@ -84,3 +84,20 @@ for i in np.argsort(-exit_rel)[:10]:
 for name, arr in (("wait->issued", post), ("issued->landed", land), ("exit", exit_rel)):
     qs = np.percentile(arr, [50, 90, 99, 100])
     print(f"  {name:15s}: p50 {qs[0]:5.2f}  p90 {qs[1]:5.2f}  p99 {qs[2]:5.2f}  max {qs[3]:5.2f}")
+
+# phase-0 path of each block of the last kernel: warp 1's stamp 1 holds 16 | bit 0 below spec4_blocks | bit 1 extra-row
+# fetch | bit 2 redo | bit 3 fresh copies after the wait (nothing speculated), when the kernel records it
+code = T[-1][:, 1, 1].astype(np.int64)
+if (code & 16).all():
+    redo = (code & 4) != 0
+    fetch = ((code & 2) != 0) & ~redo
+    fresh = ((code & 8) != 0) & ~redo & ~fetch
+    hit = ~redo & ~fetch & ~fresh
+    spec4 = (code & 1) != 0
+    print(f"\nphase-0 paths of the last kernel's {len(code)} blocks ({int(spec4.sum())} below spec4_blocks): "
+          f"four-row hit {int((hit & spec4).sum())}, three-row hit {int((hit & ~spec4).sum())}, "
+          f"extra-row fetch {int(fetch.sum())}, redo {int(redo.sum())}, no speculation {int(fresh.sum())}")
+    for name, sel in (("four-row hit", hit & spec4), ("three-row hit", hit & ~spec4), ("extra-row fetch", fetch)):
+        if sel.any():
+            print(f"  {name:15s}: median entry {np.median(entry_rel[sel]):6.2f}  issued->landed {np.median(land[sel]):5.2f}"
+                  f"  exit {np.median(exit_rel[sel]):5.2f}")
