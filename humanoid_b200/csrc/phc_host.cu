@@ -1,46 +1,45 @@
-// Host-buffer entry point around phc_step_fused (the end-to-end call of include/phc_b200.h).
+// Host-buffer entry point around phc_step_fused (the end-to-end call of include/phc_b200.h): sim state, clock and
+// outputs live in the caller's host memory.
 //
-// Direct path (all caller buffers pinned, hence mapped into the device address space by UVA): the
-// sim state of each chunk is copied in by the host->device copy engine, and the chunk's fused
-// kernel writes obs rows, rewards and flags straight into the caller's host buffers with its
-// bulk stores (no device->host DMA descriptors, no device staging of outputs), so the two
-// directions of the link overlap.  Used whenever cudaPointerGetAttributes says every buffer is
-// pinned / managed host memory mapped at its own address (device pointers are rejected: PHC_ERR_UNSUPPORTED).
+// Chunks.  A step (or a host reset) cuts the env batch into chunks (partition); chunk c runs
+//     H2D(sim state) + H2D(packed clock)  ->  fused step  ->  outputs to the host
+// on stream c % 3, so the host->device copy of one chunk, the kernel of another and the outbound traffic of a third
+// overlap (PCIe is full duplex; the B200 has copy engines per direction).  The five small clock arrays of a chunk
+// travel as ONE transfer through pinned staging owned by the slot (a DMA descriptor costs a few microseconds regardless
+// of size; 22 of them per chunk were half of the step time).
 //
-// Staged path (any pageable buffer): chunked copy pipeline, below.
-//
-// The env batch is cut into chunks; chunk c runs
-//     H2D(sim state) + H2D(packed clock)  ->  fused step  ->  D2H(obs) + D2H(packed scalars)
-// on stream c % 3, so the host->device copy of one chunk, the kernel of another and the
-// device->host copy of a third overlap (PCIe is full duplex; the B200 has copy engines per
-// direction).  The five small clock arrays and the five small outputs of a chunk travel as ONE
-// transfer each through pinned staging buffers owned by the context (a DMA descriptor costs a
-// few microseconds regardless of size; 22 of them per chunk were half of the step time).
+// Output paths.  One step loop (step_enqueue) serves both:
+//   direct: every buffer is pinned / managed host memory mapped at its own address (classify; device pointers are
+//     refused with PHC_ERR_UNSUPPORTED).  The chunk's fused kernel writes obs rows, rewards and flags straight into the
+//     caller's buffers with its bulk stores (no device->host DMA descriptors, no device staging of outputs), so the
+//     copy engine pulling the next chunk and the kernel pushing this one use opposite directions of the link.
+//   staged: any pageable buffer.  The kernel writes into the slot's device obs rows and packed scalars, and the copy
+//     engine brings back the obs rows and, as ONE transfer, the five small outputs; wait unpacks them.
+// For pinned callers the schedule (path, chunk count) is tuned over the first synchronous calls (phc_host_step).
 //
 // Slots.  A context owns PHC_HOST_SLOTS independent pipelines, each with its own device buffers, pinned staging and
-// three streams.  phc_host_step_submit enqueues one step on a slot and returns; phc_host_step_wait waits for the
-// slot's events and, on the staged path, unpacks the scalar outputs.  With two slots the inbound copy of one batch
-// rides under the outbound traffic of the other (the slots' streams do not queue behind each other), and the caller's
-// thread is free between submit and wait.  phc_host_step is submit + wait on slot 0.
+// three streams.  A submit enqueues one step on a slot and returns; phc_host_step_wait waits for the slot's events and,
+// on the staged path, unpacks the scalar outputs.  With two slots the inbound copy of one batch rides under the
+// outbound traffic of the other (the slots' streams do not queue behind each other), and the caller's thread is free
+// between submit and wait.  phc_host_step is submit + wait on slot 0.
 //
-// Resets.  phc_host_step_submit_reset runs each chunk's step with PhcStepArgs.auto_reset over the chunk's own device
-// copies (sim state, packed clock, per-slot root / dof scratch); phc_host_reset_submit runs phc_reset_envs over them.
-// The uniform numbers and the env mask ride in the chunk's packed clock transfer.  The new state of a re-posed env
-// (~1.9 KB) is not in any buffer the plain step sends back, and only a few percent of the envs are re-posed per step:
-// one small kernel per chunk (host_export_kernel) writes the rows of those envs alone into the caller's buffers when
-// they are pinned, else into the slot's pinned staging, from which wait copies the rows of the flagged envs.
+// Resets.  A step with a PhcHostResetArgs runs each chunk's step with PhcStepArgs.auto_reset over the chunk's own device
+// copies (sim state, packed clock, per-slot root / dof scratch); the host reset (reset_enqueue) runs phc_reset_envs over
+// them.  The uniform numbers and the env mask ride in the chunk's packed clock transfer.  The new state of a re-posed
+// env (~1.9 KB) is not in any buffer the plain step sends back, and only a few percent of the envs are re-posed per
+// step: one small kernel per chunk (host_export_kernel) writes the rows of those envs alone into the caller's buffers
+// when they are pinned, else into the slot's pinned staging, from which wait copies the rows of the flagged envs.
 //
-// Device outputs.  phc_host_step_submit_device / phc_host_reset_submit_device run the same pipelines with the obs rows
-// (and the normalised rows and RunningNorm moments) written by the kernels into the caller's device tensors: no obs
-// transfer at all, only the scalars and the reset rows return to the host.  Each chunk's stream waits for an event
-// recorded on the caller's stream before its kernel, so the policy's reads of the previous rows come first.
+// Device outputs.  With a PhcHostDeviceOut the kernels write the obs rows (and the normalised rows and RunningNorm
+// moments) into the caller's device tensors: no obs transfer at all, only the scalars and the reset rows return to the
+// host.  Each chunk's stream waits for an event recorded on the caller's stream before its kernel, so the policy's
+// reads of the previous rows come first.
 //
-// Env options.  phc_host_step_submit_env / phc_host_reset_submit_env run the same pipelines with the power reward (each
-// chunk's dof force and dof velocity rows are copied by the copy engine straight from the caller's buffers into the
-// slot's device scratch: two transfers per chunk, no CPU copy), mpjpe (posted by the kernel on the direct path, in the
-// packed scalars on the staged path) and StateInit.Default / Hybrid (the initial rows are uploaded once per slot by
-// phc_host_step_set_initial_state; the hybrid mask rides in the packed clock).  Every other submit is one of these
-// with no options.
+// Env options (PhcHostEnvArgs).  The power reward (each chunk's dof force and dof velocity rows are copied by the copy
+// engine straight from the caller's buffers into the slot's device scratch: two transfers per chunk, no CPU copy),
+// mpjpe (posted by the kernel on the direct path, in the packed scalars on the staged path) and StateInit.Default /
+// Hybrid (the initial rows are uploaded once per slot by phc_host_step_set_initial_state; the hybrid mask rides in the
+// packed clock).  Every submit is submit() below: the _env submits pass their options, the others none.
 #include <chrono>
 #include <cstdint>
 #include <cstdio>
@@ -172,6 +171,37 @@ __global__ void __launch_bounds__(kExportEnvs * 32) host_export_kernel(const Exp
   }
 }
 
+// What a caller's pointer is.  A pointer the runtime does not know (cudaPointerGetAttributes fails; its sticky error
+// is cleared) counts as pageable.
+enum class Mem { kPageable, kMapped, kMappedElsewhere, kDevice };  // kMapped: host memory mapped at its own address
+struct PtrKind {
+  Mem mem;
+  int device;  // kDevice: the ordinal
+};
+PtrKind classify(const void* p) {
+  cudaPointerAttributes at{};
+  if (cudaPointerGetAttributes(&at, p) != cudaSuccess) {
+    (void)cudaGetLastError();
+    return {Mem::kPageable, -1};
+  }
+  if (at.type == cudaMemoryTypeDevice) return {Mem::kDevice, at.device};
+  if (at.type != cudaMemoryTypeHost && at.type != cudaMemoryTypeManaged) return {Mem::kPageable, -1};
+  return {at.devicePointer == p ? Mem::kMapped : Mem::kMappedElsewhere, -1};
+}
+
+// A verdict on a set of caller pointers, kept while the caller passes the same set again: a caller steps the same
+// buffers over and over, and classifying costs a driver call per pointer.
+template <int N>
+struct Seen {
+  const void* ptrs[N] = {};
+  int direct = -1;  // -1: nothing classified yet
+  bool hit(const void* const (&p)[N]) const { return direct >= 0 && memcmp(p, ptrs, sizeof(ptrs)) == 0; }
+  void keep(const void* const (&p)[N], int d) {
+    memcpy(ptrs, p, sizeof(ptrs));
+    direct = d;
+  }
+};
+
 // One pipeline: what a step in flight uses, and what phc_host_step_wait needs to finish it.
 struct Slot {
   bool ready = false;  // buffers, streams and events allocated
@@ -184,9 +214,8 @@ struct Slot {
   cudaStream_t streams[kStreams] = {};
   cudaEvent_t done[kStreams] = {};  // recorded on each stream at the end of an enqueue
   cudaEvent_t dev_ready = nullptr;  // device-output submits: recorded on the caller's stream, waited on before a kernel
-  // direct path: verdict cached per set of caller pointers (the 11 of PhcHostStepArgs and PhcHostEnvArgs.mpjpe)
-  const void* seen[12] = {};
-  int seen_direct = -1;
+  // can the direct path be used: the 11 pointers of PhcHostStepArgs and PhcHostEnvArgs.mpjpe
+  Seen<12> step_seen;
   // resets, allocated at the first submit that needs them: device root / dof rows of re-posed envs and the flags the
   // reset clears (the caller gets the step's own flags), [max_envs] each; pinned staging of the reset outputs
   unsigned char* d_reset = nullptr;
@@ -194,14 +223,13 @@ struct Slot {
   uint8_t *d_kreset = nullptr, *d_kterm = nullptr;
   unsigned char* h_rows = nullptr;
   Rows stage{};
-  const void* rseen[9] = {};  // verdict of the reset pointers: the outputs are all pinned and mapped at their address
-  int rseen_direct = -1;
+  Seen<9> reset_seen;  // the reset pointers: are its outputs all pinned and mapped at their address
   // env options, allocated at first use: the chunk's dof force and dof velocity rows ([max_envs, 2, 69]: per chunk
   // m force rows, then m velocity rows), and the initial root / dof rows of StateInit.Default / Hybrid
   float* d_dof = nullptr;
   float* d_init = nullptr;  // [max_envs] x (13 root | 69 dof pos | 69 dof vel), init_rows of them set
   int64_t init_rows = -1;   // -1: no initial state
-  const void* eseen[3] = {};  // the env inputs last found to be host memory
+  Seen<3> env_seen;         // the env inputs last found to be host memory
   // the step in flight
   bool busy = false;
   int path = 0;  // 1 direct, 2 staged
@@ -213,7 +241,7 @@ struct Slot {
   PhcHostEnvArgs env{};
   Extra extra{};
   int nchunks = 0;
-  int64_t bounds[kMaxChunks + 2] = {};  // staged path: chunk boundaries, for the unpack in wait
+  int64_t bounds[kMaxChunks + 2] = {};  // chunk c is envs [bounds[c], bounds[c + 1]) (partition)
 };
 
 }  // namespace
@@ -317,28 +345,22 @@ static int check_args(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, int64_t
   const void* ptrs[12] = {a->state, a->progress_buf, a->motion_start_times, a->motion_start_times_offset,
                           a->global_offset, a->sampled_motion_ids, a->obs_buf, a->rew_buf, a->reward_raw,
                           a->reset_buf, a->terminate_buf, mpjpe};
-  if (s.seen_direct < 0 || memcmp(ptrs, s.seen, sizeof(ptrs)) != 0) {
+  if (!s.step_seen.hit(ptrs)) {
     int direct = 1;
     for (int i = 0; i < 12 && direct; ++i) {
       if (!ptrs[i]) continue;  // obs_buf of a device-output submit, mpjpe when not asked for
-      cudaPointerAttributes at{};
-      if (cudaPointerGetAttributes(&at, ptrs[i]) != cudaSuccess) {
-        (void)cudaGetLastError();
-        direct = 0;
-      } else if (at.type == cudaMemoryTypeDevice) {
-        return PHC_ERR_UNSUPPORTED;  // this entry point takes HOST buffers (the clock arrays are memcpy'd by the CPU)
-      } else if ((at.type != cudaMemoryTypeHost && at.type != cudaMemoryTypeManaged) || at.devicePointer != ptrs[i]) {
-        direct = 0;  // pageable, or mapped at a different device address
-      }
+      const Mem m = classify(ptrs[i]).mem;
+      // this entry point takes HOST buffers (the clock arrays are memcpy'd by the CPU)
+      if (m == Mem::kDevice) return PHC_ERR_UNSUPPORTED;
+      direct = m == Mem::kMapped;
     }
-    memcpy(s.seen, ptrs, sizeof(ptrs));
-    s.seen_direct = direct;
+    s.step_seen.keep(ptrs, direct);
   }
   return PHC_OK;
 }
 
 // Everything the two reset submits validate on top of check_args; fills the slot's verdict for the reset outputs.
-// env: the env options of an _env submit, NULL for the submits without them (which refuse StateInit.Default / Hybrid).
+// env: the submit's env options, NULL when it refuses StateInit.Default / Hybrid.
 static int check_reset(const PhcHostStep* c, Slot& s, const PhcHostResetArgs* r, int op, const PhcHostEnvArgs* env,
                        int64_t n) {
   if (!r->state_out || !r->root_states || !r->dof_pos || !r->dof_vel || !r->motion_start_times_out ||
@@ -357,22 +379,15 @@ static int check_reset(const PhcHostStep* c, Slot& s, const PhcHostResetArgs* r,
   // outputs first (their verdict), then the two inputs the CPU packs (only refused when on the device)
   const void* ptrs[9] = {r->state_out, r->root_states, r->dof_pos, r->dof_vel, r->motion_start_times_out,
                          r->motion_start_times_offset_out, r->global_offset_out, r->phase, r->env_mask};
-  if (s.rseen_direct < 0 || memcmp(ptrs, s.rseen, sizeof(ptrs)) != 0) {
+  if (!s.reset_seen.hit(ptrs)) {
     int direct = 1;
     for (int i = 0; i < 9; ++i) {
       if (!ptrs[i]) continue;
-      cudaPointerAttributes at{};
-      if (cudaPointerGetAttributes(&at, ptrs[i]) != cudaSuccess) {
-        (void)cudaGetLastError();
-        if (i < 7) direct = 0;
-      } else if (at.type == cudaMemoryTypeDevice) {
-        return PHC_ERR_UNSUPPORTED;
-      } else if (i < 7 && ((at.type != cudaMemoryTypeHost && at.type != cudaMemoryTypeManaged) || at.devicePointer != ptrs[i])) {
-        direct = 0;
-      }
+      const Mem m = classify(ptrs[i]).mem;
+      if (m == Mem::kDevice) return PHC_ERR_UNSUPPORTED;
+      if (i < 7 && m != Mem::kMapped) direct = 0;
     }
-    memcpy(s.rseen, ptrs, sizeof(ptrs));
-    s.rseen_direct = direct;
+    s.reset_seen.keep(ptrs, direct);
   }
   return PHC_OK;
 }
@@ -384,12 +399,8 @@ static int check_dev(const PhcHostStep* c, const PhcHostDeviceOut* d) {
   const void* ptrs[5] = {d->obs, d->obs_norm, d->norm_mean, d->norm_var, d->obs_moments};
   for (const void* p : ptrs) {
     if (!p) continue;
-    cudaPointerAttributes at{};
-    if (cudaPointerGetAttributes(&at, p) != cudaSuccess) {
-      (void)cudaGetLastError();
-      return PHC_ERR_UNSUPPORTED;
-    }
-    if (at.type != cudaMemoryTypeDevice || at.device != c->device) return PHC_ERR_UNSUPPORTED;
+    const PtrKind k = classify(p);
+    if (k.mem != Mem::kDevice || k.device != c->device) return PHC_ERR_UNSUPPORTED;
   }
   if ((((uintptr_t)d->obs | (uintptr_t)d->obs_norm) & 15) != 0) return PHC_ERR_ALIGN;
   if (d->obs_moments_buckets < 0 || d->obs_moments_buckets > 4096 || (d->obs_norm && !(d->norm_clip > 0.0f)))
@@ -402,17 +413,10 @@ static int check_dev(const PhcHostStep* c, const PhcHostDeviceOut* d) {
 static int check_env(Slot& s, const PhcHostEnvArgs* e) {
   if (!e->dof_force != !e->dof_vel) return PHC_ERR_NULL;
   const void* ptrs[3] = {e->dof_force, e->dof_vel, e->default_mask};
-  if (memcmp(ptrs, s.eseen, sizeof(ptrs)) == 0) return PHC_OK;
-  for (const void* p : ptrs) {
-    if (!p) continue;
-    cudaPointerAttributes at{};
-    if (cudaPointerGetAttributes(&at, p) != cudaSuccess) {
-      (void)cudaGetLastError();  // pageable
-    } else if (at.type == cudaMemoryTypeDevice) {
-      return PHC_ERR_UNSUPPORTED;
-    }
-  }
-  memcpy(s.eseen, ptrs, sizeof(ptrs));
+  if (s.env_seen.hit(ptrs)) return PHC_OK;
+  for (const void* p : ptrs)
+    if (p && classify(p).mem == Mem::kDevice) return PHC_ERR_UNSUPPORTED;
+  s.env_seen.keep(ptrs, 0);
   return PHC_OK;
 }
 
@@ -581,285 +585,226 @@ static cudaError_t export_rows(const PhcHostStep* c, const PhcResetArgs& ra, con
   return cudaGetLastError();
 }
 
-static int direct_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, const PhcHostResetArgs* r,
-                          const PhcHostDeviceOut* dev, int64_t n, const int chunks) {
-  // Hybrid: everything INBOUND rides the host->device copy engine in a few chunks — the sim
-  // rows directly from the caller's buffer, the five small clock arrays packed into one
-  // transfer (SM-issued reads of system memory are 32-B PCIe round trips: 6 per block, ~70 us
-  // per 4096-env step when the kernel read the clock in place) — while each chunk's kernel
-  // WRITES obs rows, rewards and flags straight into the mapped host buffers.  The copy
-  // engine pulling chunk c+1 and the kernel pushing chunk c's rows use opposite directions of
-  // the link.  The advanced progress is written to the caller's buffer by the kernel as well.
-  // equal chunks here: measured, a small first chunk does not help this path (the step is
-  // bound by the kernels' posted writes, ~300 us per 4096 envs, plus the first copy)
+// Chunk boundaries into s.bounds[0..s.nchunks].  Every boundary but n is a multiple of 8 envs, so the obs rows (fp32
+// and bf16) of every chunk start 16-B aligned.
+//   equal (direct path, host reset): `chunks` chunks of one size.  Measured, a small first chunk does not help the
+//     direct path (the step is bound by the kernels' posted writes, ~300 us per 4096 envs, plus the first copy).
+//   doubling (staged path): n/2^(C-1), n/2^(C-1), n/2^(C-2), .., n/2.  The device->host direction carries 3x the bytes
+//     and is the bottleneck, so the first chunk is small to start it early while the later, larger chunks keep the
+//     per-transfer overhead low.
+static void partition(Slot& s, int64_t n, int chunks, bool doubling) {
   const int C = chunks < 1 ? 1 : chunks;
-  int64_t per = (n + C - 1) / C;
-  per = (per + 7) / 8 * 8;
-  size_t coff = 0, ooff = 0;
-  int ci = 0;
-  // with a reset the step's own flags go to device scratch (the export kernel posts them to the caller with the rows)
-  const Rows rows = r ? (s.rows_staged ? s.stage : caller_rows(a, r)) : Rows{};
-  static const bool trace_on = getenv("PHC_HOST_TRACE") != nullptr;
-  static int trace_calls = 0;
-  const bool trace = trace_on && ++trace_calls == 20;
-  cudaEvent_t ev0 = nullptr, evh[64], evk[64];
-  double host_us[64];
-  const auto th0 = std::chrono::steady_clock::now();
-  if (trace) {
-    cudaEventCreate(&ev0);
-    cudaEventRecord(ev0, s.streams[0]);
-  }
-  for (int64_t lo = 0; lo < n; lo += per, ++ci) {
-    const int64_t m = (n - lo) < per ? (n - lo) : per;
-    const Layout L = layout(m, r != nullptr, s.extra);
-    if (coff + L.clock_bytes > c->pack_capacity || ooff + L.out_bytes > c->pack_capacity)
-      return host_fail(s, PHC_ERR_SHAPE, cudaSuccess);
-    cudaStream_t st_ = s.streams[ci % kStreams];
-    float* st = s.d_state + lo * kStateFloats;
-    unsigned char* hc = s.h_clock + coff;
-    unsigned char* dc = s.d_clock + coff;
-    unsigned char* dout = s.d_out + ooff;
-    pack_clock(hc, L, a, r, s.env, lo, m);
-    HOST_CUDA(s, cudaMemcpyAsync(dc, hc, L.clock_bytes, cudaMemcpyHostToDevice, st_));
-    HOST_CUDA(s, cudaMemcpyAsync(st, a->state + lo * kStateFloats, (size_t)m * kStateFloats * sizeof(float),
-                                 cudaMemcpyHostToDevice, st_));
-    PhcStepArgs k{};
-    if (trace && ci < 64) {
-      cudaEventCreate(&evh[ci]);
-      cudaEventRecord(evh[ci], st_);
-    }
-    k.body = chunk_body(st);
-    k.progress_buf = (int16_t*)(dc + L.prog);
-    k.motion_start_times = (const float*)(dc + L.start);
-    k.motion_start_times_offset = (const float*)(dc + L.soff);
-    k.global_offset = (const float*)(dc + L.goff);
-    k.sampled_motion_ids = (const int64_t*)(dc + L.ids);
-    k.termination_distances = c->term_dist;
-    k.reset_body_mask = c->reset_mask;
-    k.use_mean = c->use_mean;
-    k.enable_early_termination = c->early;
-    k.advance_progress = 1;
-    k.time_steps = c->T;
-    k.dt = c->dt;
-    k.rwd = c->rwd;
-    k.obs_buf = a->obs_buf + lo * c->obs_dim;
-    k.obs_stride = c->obs_dim;
-    k.rew_buf = a->rew_buf + lo;
-    k.reward_raw = a->reward_raw + lo * s.extra.raw_cols;
-    k.reward_raw_stride = s.extra.raw_cols;
-    k.reset_buf = a->reset_buf + lo;
-    k.terminate_buf = a->terminate_buf + lo;
-    k.flags = PHC_STEP_MAPPED_HOST_IO;
-    k.obs_moments = nullptr;
-    k.mpjpe = s.env.mpjpe ? s.env.mpjpe + lo : nullptr;
-    HOST_CUDA(s, power_inputs(s, lo, m, st_, k));
-    if (dev) dev_step_outputs(c, dev, lo, k);
-    PhcResetArgs ra;
-    if (r) {
-      k.reset_buf = s.d_kreset + lo;
-      k.terminate_buf = s.d_kterm + lo;
-      k.reset_out = dout + L.reset;
-      k.terminate_out = dout + L.term;
-      ra = chunk_reset_args(c, s, r, st, dc, L, lo, k.obs_buf);
-      k.auto_reset = &ra;
-    }
-    // the advanced progress goes straight into the caller's buffer too (no device->host copy at the tail).  Not with a
-    // reset: where it runs as a second launch (T > 1 here, or the generic kernel) the mirror would keep the advanced
-    // progress of the re-posed envs, so the progress leaves with the flags, from the device clock after the reset.
-    if (dev) HOST_CUDA(s, cudaStreamWaitEvent(st_, s.dev_ready, 0));
-    int rc = step_fused_mirrored(c->lib, &k, m, st_, r ? nullptr : a->progress_buf + lo);
-    if (rc) return host_fail(s, rc, cudaSuccess);
-    if (r) {
-      Rows out = rows_at(rows, lo, c->obs_dim);
-      out.obs = nullptr;
-      out.prog = a->progress_buf + lo;
-      out.rst = a->reset_buf + lo;
-      out.term = a->terminate_buf + lo;
-      HOST_CUDA(s, export_rows(c, ra, dout + L.reset, dout + L.term, nullptr, out, 0, m, st_));
-      ooff += L.out_bytes;
-    }
-    if (trace && ci < 64) {
-      cudaEventCreate(&evk[ci]);
-      cudaEventRecord(evk[ci], st_);
-      host_us[ci] = std::chrono::duration<double>(std::chrono::steady_clock::now() - th0).count() * 1e6;
-    }
-    coff += L.clock_bytes;
-  }
-  if (trace) {
-    for (auto st_ : s.streams) HOST_CUDA(s, cudaStreamSynchronize(st_));
-    const double tot = std::chrono::duration<double>(std::chrono::steady_clock::now() - th0).count() * 1e6;
-    fprintf(stderr, "[phc_host trace] %d chunks of %lld envs, host total %.1f us\n", ci, (long long)per, tot);
-    for (int i = 0; i < ci && i < 64; ++i) {
-      float a_ms = 0, b_ms = 0;
-      cudaEventElapsedTime(&a_ms, ev0, evh[i]);
-      cudaEventElapsedTime(&b_ms, ev0, evk[i]);
-      fprintf(stderr, "  chunk %d: submitted at %.1f us (host), H2D done %.1f us, kernel done %.1f us\n", i, host_us[i],
-              a_ms * 1e3, b_ms * 1e3);
-    }
-  }
-  return PHC_OK;
-}
-
-static int staged_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, const PhcHostResetArgs* r,
-                          const PhcHostDeviceOut* dev, int64_t n, const int chunks) {
-  const cudaMemcpyKind H2D = cudaMemcpyHostToDevice, D2H = cudaMemcpyDeviceToHost;
-  // Chunk sizes double (n/2^(C-1), n/2^(C-1), n/2^(C-2), .., n/2): the device->host direction
-  // carries 3x the bytes and is the bottleneck, so the first chunk is small to start it early
-  // while the later, larger chunks keep the per-transfer overhead low.  Boundaries fall on
-  // multiples of 8 envs so every chunk's obs rows start 16-B aligned.
-  {
-    const int C = chunks < 1 ? 1 : chunks;
-    int64_t lo = 0;
-    s.nchunks = 0;
-    s.bounds[0] = 0;
-    for (int i = 0; i < C && lo < n; ++i) {
+  const int64_t per = ((n + C - 1) / C + 7) / 8 * 8;
+  int64_t lo = 0;
+  s.nchunks = 0;
+  s.bounds[0] = 0;
+  for (int i = 0; lo < n; ++i) {
+    int64_t hi = lo + per;
+    if (doubling) {
       const int shift = (i == 0) ? C - 1 : C - i;
       int64_t sz = shift < 62 ? (n >> shift) : 0;
       sz = (sz + 7) / 8 * 8;
-      if (sz < 8) sz = 8;
-      int64_t hi = (i == C - 1) ? n : (lo + sz < n ? lo + sz : n);
-      s.bounds[++s.nchunks] = hi;
-      lo = hi;
+      hi = (i == C - 1) ? n : lo + (sz < 8 ? 8 : sz);
     }
-    s.bounds[s.nchunks] = n;
+    lo = hi < n ? hi : n;
+    s.bounds[++s.nchunks] = lo;
   }
-  const int nchunks = s.nchunks;
-  const int64_t* bounds = s.bounds;
+}
 
-  size_t coff = 0, ooff = 0;
-  const Rows rows = r ? (s.rows_staged ? s.stage : caller_rows(a, r)) : Rows{};
-  static const bool strace_on = getenv("PHC_HOST_TRACE") != nullptr;
-  static int strace_calls = 0;
-  const bool strace = strace_on && ++strace_calls == 20;
-  cudaEvent_t sev0 = nullptr, sevh[16], sevk[16], sevd[16];
-  if (strace) {
-    cudaEventCreate(&sev0);
-    cudaEventRecord(sev0, s.streams[0]);
+// A chunk's inbound copies on `st`: its clock, packed into the slot's pinned staging and sent as one transfer, and with
+// `state` its sim state rows straight from the caller's buffer (first when `state_first`).
+static cudaError_t inbound(const Slot& s, const PhcHostStepArgs* a, const PhcHostResetArgs* r, const Layout& L,
+                           int64_t lo, int64_t m, size_t coff, bool state, bool state_first, cudaStream_t st) {
+  unsigned char* hc = s.h_clock + coff;
+  pack_clock(hc, L, a, r, s.env, lo, m);
+  auto state_h2d = [&] {
+    return cudaMemcpyAsync(s.d_state + lo * kStateFloats, a->state + lo * kStateFloats,
+                           (size_t)m * kStateFloats * sizeof(float), cudaMemcpyHostToDevice, st);
+  };
+  cudaError_t e = state && state_first ? state_h2d() : cudaSuccess;
+  if (e == cudaSuccess) e = cudaMemcpyAsync(s.d_clock + coff, hc, L.clock_bytes, cudaMemcpyHostToDevice, st);
+  if (e == cudaSuccess && state && !state_first) e = state_h2d();
+  return e;
+}
+
+// PHC_HOST_TRACE: the 20th step enqueued on each path records an event after every chunk's inbound copies, its kernels
+// and (staged) its outbound copies, and prints the timeline to stderr once the slot's streams have drained.
+struct Trace {
+  enum { kH2D, kKernel, kD2H };
+  static constexpr int kChunks = 64;  // chunks past these are not stamped
+  bool on = false;
+  std::chrono::steady_clock::time_point t0;
+  cudaEvent_t start = nullptr, ev[kChunks][3] = {};
+  double host_us[kChunks] = {};
+
+  Trace(bool staged, cudaStream_t st) {
+    static const bool enabled = getenv("PHC_HOST_TRACE") != nullptr;
+    static int calls[2] = {};
+    on = enabled && ++calls[staged] == 20;
+    if (!on) return;
+    t0 = std::chrono::steady_clock::now();
+    cudaEventCreate(&start);
+    cudaEventRecord(start, st);
   }
-  for (int ci = 0; ci < nchunks; ++ci) {
-    const int64_t lo = bounds[ci], m = bounds[ci + 1] - bounds[ci];
-    if (m <= 0) continue;
+  ~Trace() {
+    if (!on) return;
+    cudaEventDestroy(start);
+    for (auto& chunk : ev)
+      for (cudaEvent_t e : chunk)
+        if (e) cudaEventDestroy(e);
+  }
+  double us() const { return std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count() * 1e6; }
+  void stamp(int ci, int what, cudaStream_t st) {
+    if (!on || ci >= kChunks) return;
+    if (what == kKernel) host_us[ci] = us();
+    cudaEventCreate(&ev[ci][what]);
+    cudaEventRecord(ev[ci][what], st);
+  }
+  void print(const Slot& s, bool staged) const {
+    fprintf(stderr, "[phc_host trace] %s, %d chunks, host total %.1f us\n", staged ? "staged" : "direct", s.nchunks,
+            us());
+    for (int i = 0; i < s.nchunks && i < kChunks; ++i) {
+      float ms[3] = {};
+      for (int j = 0; j < (staged ? 3 : 2); ++j) cudaEventElapsedTime(&ms[j], start, ev[i][j]);
+      fprintf(stderr, "  chunk %d (%lld envs): submitted at %.1f us (host), H2D done %.1f us, kernel done %.1f us", i,
+              (long long)(s.bounds[i + 1] - s.bounds[i]), host_us[i], ms[0] * 1e3, ms[1] * 1e3);
+      if (staged) fprintf(stderr, ", D2H done %.1f us", ms[2] * 1e3);
+      fputc('\n', stderr);
+    }
+  }
+};
+
+// The fused step of one chunk: its device sim state and packed clock (dc) in; out, the caller's mapped host rows on the
+// direct path, the slot's device obs rows and packed scalars (dout) on the staged path, the caller's device tensors
+// with device outputs.  Enqueues the chunk's power inputs on `st`.  With a reset the step's own flags go to the slot's
+// scratch, the flags it reports to dout, and `ra` is the auto-reset over the same chunk.
+static cudaError_t chunk_step_args(const PhcHostStep* c, const Slot& s, const PhcHostStepArgs* a,
+                                   const PhcHostResetArgs* r, const PhcHostDeviceOut* dev, const Layout& L, int64_t lo,
+                                   int64_t m, unsigned char* dc, unsigned char* dout, bool staged, cudaStream_t st,
+                                   PhcStepArgs& k, PhcResetArgs& ra) {
+  const int64_t D = c->obs_dim;
+  const int W = s.extra.raw_cols;
+  float* state = s.d_state + lo * kStateFloats;
+  k = PhcStepArgs{};
+  k.body = chunk_body(state);
+  k.progress_buf = (int16_t*)(dc + L.prog);
+  k.motion_start_times = (const float*)(dc + L.start);
+  k.motion_start_times_offset = (const float*)(dc + L.soff);
+  k.global_offset = (const float*)(dc + L.goff);
+  k.sampled_motion_ids = (const int64_t*)(dc + L.ids);
+  k.termination_distances = c->term_dist;
+  k.reset_body_mask = c->reset_mask;
+  k.use_mean = c->use_mean;
+  k.enable_early_termination = c->early;
+  k.advance_progress = 1;
+  k.time_steps = c->T;
+  k.dt = c->dt;
+  k.rwd = c->rwd;
+  k.obs_stride = D;
+  k.reward_raw_stride = W;
+  if (staged) {
+    k.obs_buf = s.d_obs + lo * D;
+    k.rew_buf = (float*)(dout + L.rew);
+    k.reward_raw = (float*)(dout + L.raw);
+    k.reset_buf = dout + L.reset;
+    k.terminate_buf = dout + L.term;
+    if (s.env.mpjpe) k.mpjpe = (float*)(dout + L.mpjpe);
+  } else {
+    k.flags = PHC_STEP_MAPPED_HOST_IO;
+    if (a->obs_buf) k.obs_buf = a->obs_buf + lo * D;
+    k.rew_buf = a->rew_buf + lo;
+    k.reward_raw = a->reward_raw + lo * W;
+    k.reset_buf = a->reset_buf + lo;
+    k.terminate_buf = a->terminate_buf + lo;
+    if (s.env.mpjpe) k.mpjpe = s.env.mpjpe + lo;
+  }
+  const cudaError_t e = power_inputs(s, lo, m, st, k);
+  if (dev) dev_step_outputs(c, dev, lo, k);
+  if (r) {
+    k.reset_buf = s.d_kreset + lo;
+    k.terminate_buf = s.d_kterm + lo;
+    k.reset_out = dout + L.reset;
+    k.terminate_out = dout + L.term;
+    ra = chunk_reset_args(c, s, r, state, dc, L, lo, k.obs_buf);
+    k.auto_reset = &ra;
+  }
+  return e;
+}
+
+// One step over the chunks of s.bounds: inbound copies (the clock first on the direct path, the sim state first on the
+// staged path), the fused step, the export of the re-posed envs' rows, and on the staged path the outbound copies.
+static int step_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, const PhcHostResetArgs* r,
+                        const PhcHostDeviceOut* dev, bool staged) {
+  const int64_t D = c->obs_dim;
+  const Rows rows = r ? (s.rows_staged ? s.stage : caller_rows(a, r)) : Rows{};
+  Trace trace(staged, s.streams[0]);
+  size_t coff = 0, ooff = 0;
+  for (int ci = 0; ci < s.nchunks; ++ci) {
+    const int64_t lo = s.bounds[ci], m = s.bounds[ci + 1] - lo;
     const Layout L = layout(m, r != nullptr, s.extra);
     if (coff + L.clock_bytes > c->pack_capacity || ooff + L.out_bytes > c->pack_capacity)
       return host_fail(s, PHC_ERR_SHAPE, cudaSuccess);
-    cudaStream_t st_ = s.streams[ci % kStreams];
-    // pack the chunk's clock on the host (tens of KB), then ONE transfer
-    unsigned char* hc = s.h_clock + coff;
-    pack_clock(hc, L, a, r, s.env, lo, m);
+    cudaStream_t st = s.streams[ci % kStreams];
     unsigned char* dc = s.d_clock + coff;
     unsigned char* dout = s.d_out + ooff;
-    HOST_CUDA(s, cudaMemcpyAsync(s.d_state + lo * kStateFloats, a->state + lo * kStateFloats,
-                                 (size_t)m * kStateFloats * sizeof(float), H2D, st_));
-    HOST_CUDA(s, cudaMemcpyAsync(dc, hc, L.clock_bytes, H2D, st_));
-
-    PhcStepArgs k{};
-    float* st = s.d_state + lo * kStateFloats;
-    k.body = chunk_body(st);
-    k.progress_buf = (int16_t*)(dc + L.prog);
-    k.motion_start_times = (const float*)(dc + L.start);
-    k.motion_start_times_offset = (const float*)(dc + L.soff);
-    k.global_offset = (const float*)(dc + L.goff);
-    k.sampled_motion_ids = (const int64_t*)(dc + L.ids);
-    k.termination_distances = c->term_dist;
-    k.reset_body_mask = c->reset_mask;
-    k.use_mean = c->use_mean;
-    k.enable_early_termination = c->early;
-    k.advance_progress = 1;
-    k.time_steps = c->T;
-    k.dt = c->dt;
-    k.rwd = c->rwd;
-    k.obs_buf = s.d_obs + lo * c->obs_dim;
-    k.obs_stride = c->obs_dim;
-    k.rew_buf = (float*)(dout + L.rew);
-    k.reward_raw = (float*)(dout + L.raw);
-    k.reward_raw_stride = s.extra.raw_cols;
-    k.reset_buf = dout + L.reset;
-    k.terminate_buf = dout + L.term;
-    k.obs_moments = nullptr;
-    k.mpjpe = s.extra.mpjpe ? (float*)(dout + L.mpjpe) : nullptr;
-    HOST_CUDA(s, power_inputs(s, lo, m, st_, k));
-    if (dev) dev_step_outputs(c, dev, lo, k);
+    HOST_CUDA(s, inbound(s, a, r, L, lo, m, coff, true, staged, st));
+    PhcStepArgs k;
     PhcResetArgs ra;
-    if (r) {  // the step's own flags still leave in the packed scalars
-      k.reset_buf = s.d_kreset + lo;
-      k.terminate_buf = s.d_kterm + lo;
-      k.reset_out = dout + L.reset;
-      k.terminate_out = dout + L.term;
-      ra = chunk_reset_args(c, s, r, st, dc, L, lo, k.obs_buf);
-      k.auto_reset = &ra;
-    }
-    if (strace && ci < 16) {
-      cudaEventCreate(&sevh[ci]);
-      cudaEventRecord(sevh[ci], st_);
-    }
-    if (dev) HOST_CUDA(s, cudaStreamWaitEvent(st_, s.dev_ready, 0));
-    int rc = phc_step_fused(c->lib, &k, m, st_);
+    HOST_CUDA(s, chunk_step_args(c, s, a, r, dev, L, lo, m, dc, dout, staged, st, k, ra));
+    trace.stamp(ci, Trace::kH2D, st);
+    if (dev) HOST_CUDA(s, cudaStreamWaitEvent(st, s.dev_ready, 0));
+    // direct: the advanced progress goes straight into the caller's buffer too.  Not with a reset: where it runs as a
+    // second launch (T > 1, or the generic kernel) the mirror would keep the advanced progress of the re-posed envs, so
+    // the progress leaves with the flags, from the device clock after the reset.
+    int16_t* mirror = staged || r ? nullptr : a->progress_buf + lo;
+    const int rc = step_fused_mirrored(c->lib, &k, m, st, mirror);
     if (rc) return host_fail(s, rc, cudaSuccess);
-    if (r) {
-      Rows out = rows_at(rows, lo, c->obs_dim);
+    if (r) {  // direct: the export posts every env's flags and progress as well; staged: they leave in dout
+      Rows out = rows_at(rows, lo, D);
       out.obs = nullptr;
-      out.prog = nullptr;
-      out.rst = out.term = nullptr;
-      HOST_CUDA(s, export_rows(c, ra, dout + L.reset, nullptr, nullptr, out, 0, m, st_));
+      out.prog = staged ? nullptr : a->progress_buf + lo;
+      out.rst = staged ? nullptr : a->reset_buf + lo;
+      out.term = staged ? nullptr : a->terminate_buf + lo;
+      HOST_CUDA(s, export_rows(c, ra, dout + L.reset, staged ? nullptr : dout + L.term, nullptr, out, 0, m, st));
     }
-    if (strace && ci < 16) {
-      cudaEventCreate(&sevk[ci]);
-      cudaEventRecord(sevk[ci], st_);
-    }
-    // the advanced progress rides back with the scalar outputs
-    HOST_CUDA(s, cudaMemcpyAsync(dout + L.oprog, dc + L.prog, (size_t)m * 2, cudaMemcpyDeviceToDevice, st_));
-    if (!dev)
-      HOST_CUDA(s, cudaMemcpyAsync(a->obs_buf + lo * c->obs_dim, s.d_obs + lo * c->obs_dim,
-                                   (size_t)m * c->obs_dim * sizeof(float), D2H, st_));
-    HOST_CUDA(s, cudaMemcpyAsync(s.h_out + ooff, dout, L.out_bytes, D2H, st_));
-    if (strace && ci < 16) {
-      cudaEventCreate(&sevd[ci]);
-      cudaEventRecord(sevd[ci], st_);
+    trace.stamp(ci, Trace::kKernel, st);
+    if (staged) {  // the advanced progress rides back with the packed scalars
+      HOST_CUDA(s, cudaMemcpyAsync(dout + L.oprog, dc + L.prog, (size_t)m * 2, cudaMemcpyDeviceToDevice, st));
+      if (!dev)
+        HOST_CUDA(s, cudaMemcpyAsync(a->obs_buf + lo * D, s.d_obs + lo * D, (size_t)m * D * sizeof(float),
+                                     cudaMemcpyDeviceToHost, st));
+      HOST_CUDA(s, cudaMemcpyAsync(s.h_out + ooff, dout, L.out_bytes, cudaMemcpyDeviceToHost, st));
+      trace.stamp(ci, Trace::kD2H, st);
     }
     coff += L.clock_bytes;
     ooff += L.out_bytes;
   }
-  if (strace) {
-    for (auto st_ : s.streams) HOST_CUDA(s, cudaStreamSynchronize(st_));
-    fprintf(stderr, "[phc_host trace] staged, %d chunks\n", nchunks);
-    for (int i = 0; i < nchunks && i < 16; ++i) {
-      float a_ms = 0, b_ms = 0, d_ms = 0;
-      cudaEventElapsedTime(&a_ms, sev0, sevh[i]);
-      cudaEventElapsedTime(&b_ms, sev0, sevk[i]);
-      cudaEventElapsedTime(&d_ms, sev0, sevd[i]);
-      fprintf(stderr, "  chunk %d (%lld envs): H2D done %.1f us, kernel done %.1f us, D2H done %.1f us\n", i,
-              (long long)(bounds[i + 1] - bounds[i]), a_ms * 1e3, b_ms * 1e3, d_ms * 1e3);
-    }
+  if (trace.on) {
+    for (auto st : s.streams) HOST_CUDA(s, cudaStreamSynchronize(st));
+    trace.print(s, staged);
   }
   return PHC_OK;
 }
 
 // The host reset: H2D(packed clock + phase + mask) -> phc_reset_envs -> export of the masked envs' rows (obs included)
-// on equal chunks.  Nothing else is read or written: no sim state comes in, no whole obs chunk goes out.  With device
-// outputs the reset writes the masked envs' obs and normalised rows straight into the caller's tensors and adds them
-// to the moments (rows no step has counted, as HumanoidPHC.reset() does); the export then carries no obs.
+// over the chunks of s.bounds.  Nothing else is read or written: no sim state comes in (but for StateInit.Default /
+// Hybrid), no whole obs chunk goes out.  With device outputs the reset writes the masked envs' obs and normalised rows
+// straight into the caller's tensors and adds them to the moments (rows no step has counted, as HumanoidPHC.reset()
+// does); the export then carries no obs.
 static int reset_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, const PhcHostResetArgs* r,
-                         const PhcHostDeviceOut* dev, int64_t n, const int chunks) {
-  const int C = chunks < 1 ? 1 : chunks;
-  int64_t per = (n + C - 1) / C;
-  per = (per + 7) / 8 * 8;
+                         const PhcHostDeviceOut* dev) {
   const Rows rows = s.rows_staged ? s.stage : caller_rows(a, r);
+  // a default-path env keeps its rigid-body rows, and its observation is computed from them: the chunk's sim state
+  // comes in (read before the export writes state_out, which may alias it)
+  const bool state = r->state_init >= PHC_STATE_INIT_DEFAULT;
   size_t coff = 0;
-  int ci = 0;
-  for (int64_t lo = 0; lo < n; lo += per, ++ci) {
-    const int64_t m = (n - lo) < per ? (n - lo) : per;
+  for (int ci = 0; ci < s.nchunks; ++ci) {
+    const int64_t lo = s.bounds[ci], m = s.bounds[ci + 1] - lo;
     const Layout L = layout(m, true, s.extra);
     if (coff + L.clock_bytes > c->pack_capacity) return host_fail(s, PHC_ERR_SHAPE, cudaSuccess);
-    cudaStream_t st_ = s.streams[ci % kStreams];
-    unsigned char* hc = s.h_clock + coff;
+    cudaStream_t st = s.streams[ci % kStreams];
     unsigned char* dc = s.d_clock + coff;
-    pack_clock(hc, L, a, r, s.env, lo, m);
-    HOST_CUDA(s, cudaMemcpyAsync(dc, hc, L.clock_bytes, cudaMemcpyHostToDevice, st_));
-    // a default-path env keeps its rigid-body rows, and its observation is computed from them: the chunk's sim state
-    // comes in (read before the export writes state_out, which may alias it)
-    if (r->state_init >= PHC_STATE_INIT_DEFAULT)
-      HOST_CUDA(s, cudaMemcpyAsync(s.d_state + lo * kStateFloats, a->state + lo * kStateFloats,
-                                   (size_t)m * kStateFloats * sizeof(float), cudaMemcpyHostToDevice, st_));
+    HOST_CUDA(s, inbound(s, a, r, L, lo, m, coff, state, false, st));
     float* obs = dev ? dev_obs(c, dev, lo) : s.d_obs + lo * c->obs_dim;
     PhcResetArgs ra = chunk_reset_args(c, s, r, s.d_state + lo * kStateFloats, dc, L, lo, obs);
     Rows out = rows_at(rows, lo, c->obs_dim);
@@ -875,11 +820,11 @@ static int reset_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, cons
       ra.obs_moments = dev->obs_moments;
       ra.obs_moments_buckets = dev->obs_moments_buckets;
       out.obs = nullptr;
-      HOST_CUDA(s, cudaStreamWaitEvent(st_, s.dev_ready, 0));
+      HOST_CUDA(s, cudaStreamWaitEvent(st, s.dev_ready, 0));
     }
-    const int rc = phc_reset_envs(c->lib, &ra, m, st_);
+    const int rc = phc_reset_envs(c->lib, &ra, m, st);
     if (rc) return host_fail(s, rc, cudaSuccess);
-    HOST_CUDA(s, export_rows(c, ra, dc + L.mask, nullptr, dev ? nullptr : obs, out, 1, m, st_));
+    HOST_CUDA(s, export_rows(c, ra, dc + L.mask, nullptr, dev ? nullptr : obs, out, 1, m, st));
     coff += L.clock_bytes;
   }
   return PHC_OK;
@@ -891,9 +836,9 @@ static int slot_enqueue(PhcHostStep* c, int slot, const PhcHostStepArgs* a, cons
   Slot& s = c->slots[slot];
   if (dev) HOST_CUDA(s, cudaEventRecord(s.dev_ready, dev->stream));
   // s.env / s.extra were set by the submit (zero for phc_host_step)
-  const int rc = op == kReset   ? reset_enqueue(c, s, a, r, dev, n, k.chunks)
-                 : k.path == 1 ? direct_enqueue(c, s, a, r, dev, n, k.chunks)
-                               : staged_enqueue(c, s, a, r, dev, n, k.chunks);
+  const bool staged = op != kReset && k.path == 2;
+  partition(s, n, k.chunks, staged);
+  const int rc = op == kReset ? reset_enqueue(c, s, a, r, dev) : step_enqueue(c, s, a, r, dev, staged);
   if (rc) return rc;
   for (int i = 0; i < kStreams; ++i) HOST_CUDA(s, cudaEventRecord(s.done[i], s.streams[i]));
   s.args = *a;
@@ -945,8 +890,7 @@ static int slot_finish(const PhcHostStep* c, Slot& s) {
     const PhcHostStepArgs* a = &s.args;
     size_t ooff = 0;
     for (int ci = 0; ci < s.nchunks; ++ci) {
-      const int64_t lo = s.bounds[ci], m = s.bounds[ci + 1] - s.bounds[ci];
-      if (m <= 0) continue;
+      const int64_t lo = s.bounds[ci], m = s.bounds[ci + 1] - lo;
       const Layout L = layout(m, s.op != kStep, s.extra);
       const unsigned char* ho = s.h_out + ooff;
       const int W = s.extra.raw_cols;
@@ -966,7 +910,7 @@ static int slot_finish(const PhcHostStep* c, Slot& s) {
 // The schedule of a step that is not timed by the tuner: pageable callers take the copy-engine path; pinned callers
 // the settled schedule, or the first candidate while tuning has not finished.
 static PhcHostStep::Cand untimed_schedule(const PhcHostStep* c, const Slot& s) {
-  if (s.seen_direct != 1) return {2, c->chunks > 0 ? c->chunks : 3, 0.0, 0};
+  if (s.step_seen.direct != 1) return {2, c->chunks > 0 ? c->chunks : 3, 0.0, 0};
   return c->cand[c->chosen >= 0 ? c->chosen : 0];
 }
 
@@ -1010,7 +954,6 @@ int phc_host_step_create(const PhcLib* lib, int64_t max_envs, int32_t time_steps
   c->rwd = *rwd;
   (void)cudaGetDevice(&c->device);
   if (const char* m = getenv("PHC_HOST_PATH")) c->mode = !strcmp(m, "direct") ? 1 : !strcmp(m, "staged") ? 2 : 0;
-  if (getenv("PHC_HOST_STAGED")) c->mode = 2;
   const size_t n = (size_t)max_envs;
   // every chunk's packed region is padded so each sub-array starts 16-B aligned (35 B per env with a reset's clock)
   c->pack_capacity = n * 40 + (size_t)(num_chunks > 8 ? num_chunks : 8) * 8 * 64 + 4096;
@@ -1060,7 +1003,7 @@ int phc_host_step(PhcHostStep* c, const PhcHostStepArgs* a, int64_t n) {
 
   // ---- which schedule ------------------------------------------------------------------------
   // Only calls made while no slot is in flight are timed: a step of the other slot would share the link.
-  if (c->slots[0].seen_direct != 1 || c->chosen >= 0 || c->slots[1].busy)
+  if (c->slots[0].step_seen.direct != 1 || c->chosen >= 0 || c->slots[1].busy)
     return run_sync(c, a, n, untimed_schedule(c, c->slots[0]));
   // Tuning: calls 0-1 warm up, then the candidates take turns (kTuneReps timed calls each) and the fastest mean
   // stays.  What decides is the machine, under whatever load the other GPUs of the box put on the host at that moment:
@@ -1100,14 +1043,12 @@ int phc_host_step(PhcHostStep* c, const PhcHostStepArgs* a, int64_t n) {
 
 }  // extern "C"
 
-// The submits: every check before anything is enqueued, then the slot's buffers, then the enqueue.  dev_out: one of
-// the device-output submits (dev must then name the device tensors).
-// env_entry: one of the _env submits, whose env options (env, NULL for none) may be set; a host reset takes only their
-// default_mask.  The other submits have no options and refuse StateInit.Default / Hybrid, as they always did.
+// The submits: every check before anything is enqueued, then the slot's buffers, then the enqueue.  dev: the device
+// tensors the rows go to, or NULL for host obs.  env: the env options, or NULL for none; a host reset takes only their
+// default_mask.  init_modes: StateInit.Default / Hybrid may be asked for (the _env submits; the others refuse them).
 static int submit(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, const PhcHostResetArgs* r, int op, int64_t n,
-                  bool dev_out = false, const PhcHostDeviceOut* dev = nullptr, bool env_entry = false,
-                  const PhcHostEnvArgs* env = nullptr) {
-  if (!c || !a || (op != kStep && !r) || (dev_out && (!dev || !dev->obs))) return PHC_ERR_NULL;
+                  const PhcHostDeviceOut* dev, const PhcHostEnvArgs* env, bool init_modes) {
+  if (!c || !a || (op != kStep && !r) || (dev && !dev->obs)) return PHC_ERR_NULL;
   if (slot < 0 || slot >= PHC_HOST_SLOTS) return PHC_ERR_SHAPE;
   Slot& s = c->slots[slot];
   if (s.busy) return PHC_ERR_BUSY;
@@ -1115,11 +1056,11 @@ static int submit(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, const 
   PhcHostEnvArgs ev{};
   if (env && op == kReset) ev.default_mask = env->default_mask;
   else if (env) ev = *env;
-  int rc = check_args(c, s, a, n, dev_out, ev.mpjpe);
+  int rc = check_args(c, s, a, n, dev != nullptr, ev.mpjpe);
   if (rc) return rc;
   if ((rc = check_env(s, &ev))) return rc;
-  if (op != kStep && (rc = check_reset(c, s, r, op, env_entry ? &ev : nullptr, n))) return rc;
-  if (dev_out && (rc = check_dev(c, dev))) return rc;
+  if (op != kStep && (rc = check_reset(c, s, r, op, init_modes ? &ev : nullptr, n))) return rc;
+  if (dev && (rc = check_dev(c, dev))) return rc;
   s.env = ev;
   s.extra.raw_cols = ev.dof_force ? 5 : 4;
   s.extra.mpjpe = ev.mpjpe != nullptr;
@@ -1131,7 +1072,7 @@ static int submit(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, const 
   }
   if (op != kStep && e == cudaSuccess) {
     // the host reset writes the step buffers' rows too (obs, progress, flags): straight only when they are pinned as well
-    s.rows_staged = !s.rseen_direct || (op == kReset && s.seen_direct != 1);
+    s.rows_staged = !s.reset_seen.direct || (op == kReset && s.step_seen.direct != 1);
     e = reset_alloc(c, s, s.rows_staged);
   }
   if (e == cudaSuccess) e = env_alloc(c, s);
@@ -1139,43 +1080,45 @@ static int submit(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, const 
     (void)cudaGetLastError();
     return e == cudaErrorMemoryAllocation ? PHC_ERR_ALLOC : phc::record_cuda_error((int)e);
   }
-  return slot_enqueue(c, slot, a, r, op, n, untimed_schedule(c, s), dev_out ? dev : nullptr);
+  return slot_enqueue(c, slot, a, r, op, n, untimed_schedule(c, s), dev);
 }
 
 extern "C" {
 
 int phc_host_step_submit(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, int64_t n) {
-  return submit(c, slot, a, nullptr, kStep, n);
+  return submit(c, slot, a, nullptr, kStep, n, nullptr, nullptr, false);
 }
 
 int phc_host_step_submit_reset(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, const PhcHostResetArgs* r,
                                int64_t n) {
-  return submit(c, slot, a, r, kStepReset, n);
+  return submit(c, slot, a, r, kStepReset, n, nullptr, nullptr, false);
 }
 
 int phc_host_reset_submit(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, const PhcHostResetArgs* r,
                           int64_t n) {
-  return submit(c, slot, a, r, kReset, n);
+  return submit(c, slot, a, r, kReset, n, nullptr, nullptr, false);
 }
 
 int phc_host_step_submit_device(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, const PhcHostResetArgs* r,
                                 const PhcHostDeviceOut* dev, int64_t n) {
-  return submit(c, slot, a, r, r ? kStepReset : kStep, n, true, dev);
+  if (!dev) return PHC_ERR_NULL;
+  return submit(c, slot, a, r, r ? kStepReset : kStep, n, dev, nullptr, false);
 }
 
 int phc_host_reset_submit_device(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, const PhcHostResetArgs* r,
                                  const PhcHostDeviceOut* dev, int64_t n) {
-  return submit(c, slot, a, r, kReset, n, true, dev);
+  if (!dev) return PHC_ERR_NULL;
+  return submit(c, slot, a, r, kReset, n, dev, nullptr, false);
 }
 
 int phc_host_step_submit_env(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, const PhcHostResetArgs* r,
                              const PhcHostDeviceOut* dev, const PhcHostEnvArgs* env, int64_t n) {
-  return submit(c, slot, a, r, r ? kStepReset : kStep, n, dev != nullptr, dev, true, env);
+  return submit(c, slot, a, r, r ? kStepReset : kStep, n, dev, env, true);
 }
 
 int phc_host_reset_submit_env(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, const PhcHostResetArgs* r,
                               const PhcHostDeviceOut* dev, const PhcHostEnvArgs* env, int64_t n) {
-  return submit(c, slot, a, r, kReset, n, dev != nullptr, dev, true, env);
+  return submit(c, slot, a, r, kReset, n, dev, env, true);
 }
 
 int phc_host_step_set_initial_state(PhcHostStep* c, int32_t slot, const float* root_states, const float* dof_pos,
@@ -1185,11 +1128,8 @@ int phc_host_step_set_initial_state(PhcHostStep* c, int32_t slot, const float* r
   Slot& s = c->slots[slot];
   if (s.busy) return PHC_ERR_BUSY;
   const float* src[3] = {root_states, dof_pos, dof_vel};
-  for (const float* p : src) {
-    cudaPointerAttributes at{};
-    if (cudaPointerGetAttributes(&at, p) != cudaSuccess) (void)cudaGetLastError();
-    else if (at.type == cudaMemoryTypeDevice) return PHC_ERR_UNSUPPORTED;
-  }
+  for (const float* p : src)
+    if (classify(p).mem == Mem::kDevice) return PHC_ERR_UNSUPPORTED;
   const size_t N = (size_t)c->max_envs;
   cudaError_t e = cudaSuccess;
   if (!s.d_init) e = cudaMalloc((void**)&s.d_init, N * (13 + 2 * kDof) * sizeof(float));
@@ -1218,13 +1158,13 @@ int phc_host_step_wait(PhcHostStep* c, int32_t slot) {
 
 int phc_host_step_path(const PhcHostStep* c) {
   if (!c) return 0;
-  if (c->slots[c->last_slot].seen_direct == 0) return 2;
+  if (c->slots[c->last_slot].step_seen.direct == 0) return 2;
   return c->chosen >= 0 ? c->cand[c->chosen].path : 0;
 }
 
 int phc_host_step_chunks(const PhcHostStep* c) {
   if (!c) return 0;
-  if (c->slots[c->last_slot].seen_direct == 0) return c->chunks > 0 ? c->chunks : 3;
+  if (c->slots[c->last_slot].step_seen.direct == 0) return c->chunks > 0 ? c->chunks : 3;
   return c->chosen >= 0 ? c->cand[c->chosen].chunks : 0;
 }
 

@@ -225,8 +225,8 @@ class HostResetBuffers:
 
 @dataclass(eq=False)
 class HostDeviceOutputs:
-    """The CUDA tensors a host step writes its rows into instead of ``HostStepBuffers.obs_buf``
-    (``phc_host_step_submit_device`` / ``phc_host_reset_submit_device``).
+    """The CUDA tensors a host step writes its rows into instead of ``HostStepBuffers.obs_buf`` (``device_out`` of
+    ``HostStep.submit`` / ``reset_submit``).
 
     ``obs`` [n, 358 + 576 T] fp32: the rows ``HumanoidPHC.obs_buf`` would hold.  ``obs_norm`` (optional, fp32 or bf16,
     the same shape): ``clamp((obs - running_mean) / sqrt(running_var + epsilon), -clip, clip)`` of ``normalizer`` (a
@@ -408,48 +408,34 @@ class HostStep:
         stream, so the policy may still be reading the previous rows.  The tensors belong to the library until
         ``wait(slot)`` returns.
 
-        With the power reward (``use_power_reward``) or ``bufs.mpjpe``, or ``state_init`` "default" / "hybrid" (after
-        ``set_initial_state(slot, ...)``; "hybrid" takes ``reset.default_mask`` and ``reset.phase``), this is
-        ``phc_host_step_submit_env``."""
+        The env options are the power reward (``use_power_reward``), ``bufs.mpjpe`` and ``state_init`` "default" /
+        "hybrid" (after ``set_initial_state(slot, ...)``; "hybrid" takes ``reset.default_mask`` and ``reset.phase``).
+        This is ``phc_host_step_submit_env``, with no ``PhcHostEnvArgs`` (NULL) when no option is on."""
         n = bufs.validate(self.time_steps, device_out=device_out is not None, power=self.use_power_reward)
-        args = bufs._args()
         env = self._env_args(slot, bufs, reset, state_init, n)
-        if env is not None:
-            rargs = None
-            if reset is not None:
-                reset.validate(n)
-                rargs = C.byref(reset._args(bufs, state_init, flag_test))
-            dargs = None
-            if device_out is not None:
-                device_out.validate(n, self.time_steps)
-                dargs = C.byref(device_out._args())
-            _cabi.check(self._capi.phc_host_step_submit_env(self._live(), int(slot), C.byref(args), rargs, dargs,
-                                                            C.byref(env), n), "phc_host_step_submit_env")  # fmt: skip
-            if device_out is not None and device_out.obs_moments is not None:
-                device_out.rows += n
-        elif device_out is not None:
-            device_out.validate(n, self.time_steps)
-            rargs = None
-            if reset is not None:
-                reset.validate(n)
-                rargs = C.byref(reset._args(bufs, state_init, flag_test))
-            dargs = device_out._args()
-            _cabi.check(self._capi.phc_host_step_submit_device(self._live(), int(slot), C.byref(args), rargs,
-                                                               C.byref(dargs), n), "phc_host_step_submit_device")  # fmt: skip
-            if device_out.obs_moments is not None:
-                device_out.rows += n  # an auto-reset replaces counted rows and adds none
-        elif reset is None:
-            _cabi.check(self._capi.phc_host_step_submit(self._live(), int(slot), C.byref(args), n), "phc_host_step_submit")
-        else:
+        rargs = None
+        if reset is not None:
             reset.validate(n)
-            rargs = reset._args(bufs, state_init, flag_test)
-            _cabi.check(self._capi.phc_host_step_submit_reset(self._live(), int(slot), C.byref(args), C.byref(rargs), n),
-                        "phc_host_step_submit_reset")  # fmt: skip
+            rargs = C.byref(reset._args(bufs, state_init, flag_test))
+        # an auto-reset replaces counted rows and adds none
+        self._submit("phc_host_step_submit_env", slot, bufs, reset, rargs, device_out, env, n, lambda: n)
+
+    def _submit(self, name, slot, bufs, reset, rargs, device_out, env, n, new_rows):
+        """The C call of ``submit`` / ``reset_submit``; ``new_rows()``: the rows it adds to ``device_out``'s moments."""
+        dargs = None
+        if device_out is not None:
+            device_out.validate(n, self.time_steps)
+            dargs = C.byref(device_out._args())
+        fn = getattr(self._capi, name)
+        eargs = None if env is None else C.byref(env)
+        _cabi.check(fn(self._live(), int(slot), C.byref(bufs._args()), rargs, dargs, eargs, n), name)
+        if device_out is not None and device_out.obs_moments is not None:
+            device_out.rows += new_rows()
         self._hold(slot, bufs, reset, device_out)
 
     def _env_args(self, slot, bufs: HostStepBuffers, reset: Optional[HostResetBuffers], state_init: str,
                   n: int, step: bool = True) -> Optional[_cabi.PhcHostEnvArgs]:  # fmt: skip
-        """The env options of one submit, or None when it has none (the submits without options then run)."""
+        """The env options of one submit, or None when it has none (the _env submits then take NULL)."""
         power = step and self.use_power_reward
         mpjpe = step and bufs.mpjpe is not None
         init = reset is not None and state_init in ("default", "hybrid")
@@ -511,28 +497,10 @@ class HostStep:
         reset.validate(n)
         if reset.env_mask is None:
             raise ValueError("reset_submit needs reset.env_mask")
-        args, rargs = bufs._args(), reset._args(bufs, state_init, flag_test)
+        rargs = C.byref(reset._args(bufs, state_init, flag_test))
         env = self._env_args(slot, bufs, reset, state_init, n, step=False)
-        if env is not None:
-            dargs = None
-            if device_out is not None:
-                device_out.validate(n, self.time_steps)
-                dargs = C.byref(device_out._args())
-            _cabi.check(self._capi.phc_host_reset_submit_env(self._live(), int(slot), C.byref(args), C.byref(rargs),
-                                                             dargs, C.byref(env), n), "phc_host_reset_submit_env")  # fmt: skip
-            if device_out is not None and device_out.obs_moments is not None:
-                device_out.rows += int(reset.env_mask.count_nonzero())
-        elif device_out is None:
-            _cabi.check(self._capi.phc_host_reset_submit(self._live(), int(slot), C.byref(args), C.byref(rargs), n),
-                        "phc_host_reset_submit")  # fmt: skip
-        else:
-            device_out.validate(n, self.time_steps)
-            dargs = device_out._args()
-            _cabi.check(self._capi.phc_host_reset_submit_device(self._live(), int(slot), C.byref(args), C.byref(rargs),
-                                                                C.byref(dargs), n), "phc_host_reset_submit_device")  # fmt: skip
-            if device_out.obs_moments is not None:
-                device_out.rows += int(reset.env_mask.count_nonzero())
-        self._hold(slot, bufs, reset, device_out)
+        self._submit("phc_host_reset_submit_env", slot, bufs, reset, rargs, device_out, env, n,
+                     lambda: int(reset.env_mask.count_nonzero()))  # fmt: skip
 
     def reset(self, bufs: HostStepBuffers, reset: HostResetBuffers, state_init: str = "random",
               flag_test: bool = False, device_out: Optional[HostDeviceOutputs] = None) -> HostStepBuffers:  # fmt: skip

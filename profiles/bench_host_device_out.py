@@ -22,7 +22,8 @@ returns; also the host-obs step's D2H).  The last outputs of every loop are comp
 shapes.  Prints one JSON line.
 
     python profiles/bench_host_device_out.py [--rounds 200]
-    PHC_HOST_TRACE=1 python profiles/bench_host_device_out.py --trace   # per-chunk timeline of dev_obs async (stderr)
+    PHC_HOST_TRACE=1 python profiles/bench_host_device_out.py --trace   # per-chunk timeline of dev_obs async (stderr;
+                                                                        # direct unless PHC_HOST_PATH says otherwise)
 """
 
 from __future__ import annotations
@@ -172,7 +173,7 @@ def main():
                     failures.append(f"{kind} {mode} batch {name}")
 
     if args.trace:
-        os.environ["PHC_HOST_PATH"] = "direct"
+        os.environ.setdefault("PHC_HOST_PATH", "direct")
         with HostStep(lib, N, num_chunks=3) as hs:
             row = {}
             leg(hs._ctx, "dev_obs", row, ("async",))

@@ -164,7 +164,6 @@ def _set_path(monkeypatch, mode):
         monkeypatch.setenv("PHC_HOST_PATH", mode)
     else:
         monkeypatch.delenv("PHC_HOST_PATH", raising=False)
-    monkeypatch.delenv("PHC_HOST_STAGED", raising=False)
 
 
 def _steps(hs, case, slot, steps, what=""):

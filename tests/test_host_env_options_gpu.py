@@ -6,7 +6,8 @@
 2. Bit for bit against HumanoidPHC(use_power_reward=True) on seeded cases: direct, staged and pageable buffers, both
    slots, auto-reset with every state init, masked host resets, T = 3, the generic kernel, eval-mode mpjpe, and a NaN
    dof force.
-3. Error codes: every refusal leaves the slot idle and the outputs untouched."""
+3. Error codes: every refusal leaves the slot idle and the outputs untouched.
+4. The submits without options equal the _env submits with all-NULL options."""
 
 import ctypes as C
 
@@ -18,7 +19,7 @@ pytestmark = pytest.mark.gpu
 if torch.cuda.is_available():
     from conftest import assert_close, assert_equal_exact
     from humanoid_b200 import (HostDeviceOutputs, HostResetBuffers, HostStep, HostStepBuffers, HumanoidPHC, MotionLib,
-                               _cabi, synth)  # fmt: skip
+                               RunningNorm, _cabi, synth)  # fmt: skip
     from util_gpu import DEV, DOF_DERIVED_TOL, OBS_TOL, clock_from_golden, lib_from_golden
 
 OK, NULL, SHAPE, UNSUPPORTED, BUSY = 0, -1, -2, -4, -8
@@ -31,7 +32,6 @@ def _set_path(monkeypatch, mode):
         monkeypatch.setenv("PHC_HOST_PATH", mode)
     else:
         monkeypatch.delenv("PHC_HOST_PATH", raising=False)
-    monkeypatch.delenv("PHC_HOST_STAGED", raising=False)
 
 
 def _same(a, b):
@@ -571,3 +571,106 @@ def test_close_with_env_submits_in_flight(monkeypatch):
     hs.close()
     a.check_step(wa, "close, slot 0")
     b.check_step(wb, "close, slot 1")
+
+
+# ---------------------------------------------------------------------------------------
+# 4. the submits without options against the _env submits
+# ---------------------------------------------------------------------------------------
+def _plain_batch(data, mlib, n, seed, pinned, host_obs, rn):
+    """One seeded batch without env options, outputs poisoned: about 3 % of the envs are pushed 0.5 m from their
+    reference (the step flags them), the phase is fresh and the env mask holds 40 % of the envs."""
+    clock = synth.make_clock(data, n, seed=seed, ids="mod", aligned=True, max_progress=30)
+    ref = mlib.get_motion_state(clock.sampled_motion_ids, synth.reward_time(clock, extra_steps=1), clock.global_offset)
+    state = synth.make_sim_state(ref, seed=seed + 1).cpu()
+    state[torch.arange(n) % 29 == 0, :, 0] += 0.5
+    b = HostStepBuffers.allocate(n, pinned=pinned, host_obs=host_obs)
+    for name, v in (("state", state), ("progress_buf", clock.progress_buf), ("motion_start_times", clock.motion_start_times),
+                    ("motion_start_times_offset", clock.motion_start_times_offset),
+                    ("global_offset", clock.global_offset), ("sampled_motion_ids", clock.sampled_motion_ids)):  # fmt: skip
+        getattr(b, name).copy_(v.cpu())
+    b.rew_buf.fill_(float("nan"))
+    b.reward_raw.fill_(float("nan"))
+    b.reset_buf.fill_(7)
+    b.terminate_buf.fill_(7)
+    r = HostResetBuffers.allocate(n, pinned=pinned)
+    gen = torch.Generator().manual_seed(seed + 2)
+    r.phase.copy_(torch.rand(n, generator=gen))
+    r.env_mask.copy_(torch.rand(n, generator=gen) < 0.4)
+    d = None if host_obs else HostDeviceOutputs.allocate(n, 1, DEV, norm_dtype=torch.bfloat16, normalizer=rn, moments=True)
+    for t in (r.root_states, r.dof_pos, r.dof_vel) + ((b.obs_buf,) if host_obs else (d.obs, d.obs_norm)):
+        t.fill_(SENTINEL)
+    return b, r, d
+
+
+_STEP_FIELDS = ("state", "progress_buf", "motion_start_times", "motion_start_times_offset", "global_offset",
+                "sampled_motion_ids", "obs_buf", "rew_buf", "reward_raw", "reset_buf", "terminate_buf")  # fmt: skip
+_RESET_FIELDS = ("phase", "root_states", "dof_pos", "dof_vel", "env_mask")
+
+
+@pytest.mark.parametrize("out", ["host_obs", "device_out"])
+@pytest.mark.parametrize("mode", ["direct", "staged", "pageable"])
+def test_submits_without_options_equal_env_submits(mode, out, monkeypatch):
+    """Each submit without options, called through _cabi, against its _env submit with an all-NULL PhcHostEnvArgs on
+    a second copy of the same ragged batch (1003 envs; the step re-poses some envs and not others, the host reset masks
+    40 %): every output bit for bit, the fp64 moments (atomic sums, whose order varies) to the reordering bound."""
+    _set_path(monkeypatch, "staged" if mode == "staged" else "direct")
+    data, mlib = _motion_lib()
+    n, host_obs = 1003, out == "host_obs"
+    D = _cabi.SELF_OBS_DIM + _cabi.TASK_OBS_DIM
+    g = torch.Generator().manual_seed(133)
+    rn = RunningNorm(D, device=DEV)
+    rn.running_mean.copy_(torch.randn(1, D, generator=g).to(DEV) * 0.3)
+    rn.running_var.copy_(torch.rand(1, D, generator=g).to(DEV) * 2 + 0.05)
+    capi = _cabi.load()
+    env0 = _cabi.PhcHostEnvArgs()
+    # (entry point, with reset args)
+    if host_obs:
+        entries = [("phc_host_step_submit", False), ("phc_host_step_submit_reset", True), ("phc_host_reset_submit", True)]
+    else:
+        entries = [("phc_host_step_submit_device", False), ("phc_host_step_submit_device", True),
+                   ("phc_host_reset_submit_device", True)]  # fmt: skip
+    with HostStep(mlib, n, num_chunks=3) as hs:
+        for name, with_reset in entries:
+            host_reset = name.startswith("phc_host_reset")
+
+            def fixed(ctx, a, r, d):
+                fn = getattr(capi, name)
+                if r is None and d is None:
+                    return fn(ctx, 0, a, n)
+                return fn(ctx, 0, a, r, n) if d is None else fn(ctx, 0, a, r, d, n)
+
+            def with_env(ctx, a, r, d):
+                fn = capi.phc_host_reset_submit_env if host_reset else capi.phc_host_step_submit_env
+                return fn(ctx, 0, a, r, d, C.byref(env0), n)
+
+            got = []
+            for call in (fixed, with_env):
+                b, r, d = _plain_batch(data, mlib, n, 131, pinned=mode != "pageable", host_obs=host_obs, rn=rn)
+                a = b._args()
+                ra = r._args(b, "random", False)
+                da = None if d is None else d._args()
+                assert call(hs._ctx, C.byref(a), C.byref(ra) if with_reset else None,
+                            None if da is None else C.byref(da)) == OK, (name, call.__name__)  # fmt: skip
+                assert capi.phc_host_step_wait(hs._ctx, 0) == OK
+                torch.cuda.synchronize()
+                got.append((b, r, d))
+            (b0, r0, d0), (b1, r1, d1) = got
+            what = f"{name} {'with' if with_reset else 'without'} reset args"
+            if host_reset:
+                mask = r0.env_mask.bool()
+                assert 0 < int(mask.sum()) < n and int(b0.reset_buf[mask].max()) == 0, what
+            else:
+                assert bool(torch.isfinite(b0.rew_buf).all()), what
+                if with_reset:
+                    assert 0 < int(b0.reset_buf.sum()) < n, f"the step should flag some envs and spare others: {what}"
+            for field in _STEP_FIELDS:
+                x, y = getattr(b0, field), getattr(b1, field)
+                assert (x is None and y is None) or _same(x, y), f"{field}: {what}"
+            for field in _RESET_FIELDS:
+                assert _same(getattr(r0, field), getattr(r1, field)), f"{field}: {what}"
+            if d0 is not None:
+                assert _same(d0.obs, d1.obs) and _same(d0.obs_norm, d1.obs_norm), what
+                m0, m1 = d0.obs_moments, d1.obs_moments
+                assert bool(m0.abs().sum() > 0), what
+                assert bool(((m0 - m1).abs() <= 1e-12 * (m0.abs() + m1.abs()) + 1e-9).all()), f"obs_moments: {what}"
+        assert hs.path == (1 if mode == "direct" else 2)
