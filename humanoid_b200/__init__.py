@@ -17,7 +17,7 @@ from .common import (  # noqa: F401
     compute_imitation_reward,
 )
 from .env import HumanoidPHC, build_pd_action_offset_scale  # noqa: F401
-from .host_step import HostDeviceOutputs, HostResetBuffers, HostStep, HostStepBuffers  # noqa: F401
+from .host_step import HostDeviceOutputs, HostEpisodeBuffers, HostResetBuffers, HostStep, HostStepBuffers  # noqa: F401
 from .motion_lib import MotionLib  # noqa: F401
 from .puffer_env import PHCPufferEnv  # noqa: F401
 from .running_norm import RunningNorm  # noqa: F401
@@ -39,4 +39,5 @@ __all__ = [
     "HostStepBuffers",
     "HostResetBuffers",
     "HostDeviceOutputs",
+    "HostEpisodeBuffers",
 ]

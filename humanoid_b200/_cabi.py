@@ -289,6 +289,20 @@ class PhcHostEnvArgs(C.Structure):
     ]
 
 
+class PhcHostEpisodeOut(C.Structure):
+    _fields_ = [
+        ("terminals", C.c_void_p),
+        ("truncations", C.c_void_p),
+        ("masks", C.c_void_p),
+        ("episode_returns", C.c_void_p),
+        ("episode_lengths", C.c_void_p),
+        ("rewards", C.c_void_p),
+        ("sums", C.c_void_p),
+        ("buckets", C.c_int32),
+        ("stream", C.c_void_p),
+    ]
+
+
 BUILD_FILTER_RADIUS = 8
 EPISODE_SUM_COLS = 12
 PEER_MAX_WORLD = 16
@@ -391,6 +405,11 @@ SIGNATURES = {
         C.c_int,
         [C.c_void_p, C.c_int32, C.POINTER(PhcHostStepArgs), C.POINTER(PhcHostResetArgs), C.POINTER(PhcHostDeviceOut),
          C.POINTER(PhcHostEnvArgs), C.c_int64],
+    ),  # fmt: skip
+    "phc_host_step_submit_episode": (
+        C.c_int,
+        [C.c_void_p, C.c_int32, C.POINTER(PhcHostStepArgs), C.POINTER(PhcHostResetArgs), C.POINTER(PhcHostDeviceOut),
+         C.POINTER(PhcHostEnvArgs), C.POINTER(PhcHostEpisodeOut), C.c_int64],
     ),  # fmt: skip
     "phc_host_step_set_initial_state": (
         C.c_int,

@@ -40,6 +40,12 @@
 // mpjpe (posted by the kernel on the direct path, in the packed scalars on the staged path) and StateInit.Default /
 // Hybrid (the initial rows are uploaded once per slot by phc_host_step_set_initial_state; the hybrid mask rides in the
 // packed clock).  Every submit is submit() below: the _env submits pass their options, the others none.
+//
+// Episode bookkeeping (PhcHostEpisodeOut).  The step kernels' own PhcStepArgs.ep_* epilogue writes the flags, returns,
+// lengths and bucket sums of PHCPufferEnv.step into the caller's device tensors.  Each chunk's kernels take their
+// buckets by the block's index in the batch (step_fused_mirrored's env0), so the sums do not depend on the chunk count.
+// The T = 1 kernel has the rewards and flags in registers; the kernels that run the bookkeeping after the step (generic,
+// T > 1) read them from device copies (the packed scalars), never from the mapped host buffers.
 #include <chrono>
 #include <cstdint>
 #include <cstdio>
@@ -51,8 +57,10 @@
 
 #include "../../include/phc_b200.h"
 
-// phc_kernels.cu: phc_step_fused that also writes the advanced progress to a second address
-int step_fused_mirrored(const PhcLib* lib, const PhcStepArgs* args, int64_t n, phc_stream_t stream, int16_t* progress_mirror);
+// phc_kernels.cu: phc_step_fused for one chunk: a second address for the advanced progress, the chunk's first env (the
+// episode buckets), device scratch for the reward_raw rows the bookkeeping reads when the outputs are mapped
+int step_fused_mirrored(const PhcLib* lib, const PhcStepArgs* args, int64_t n, phc_stream_t stream,
+                        int16_t* progress_mirror, int64_t env0, float* ep_raw);
 bool lib_has_dof_state(const PhcLib* lib);  // phc_kernels.cu
 namespace phc {
 int record_cuda_error(int cuda_error);  // phc_kernels.cu; returns PHC_ERR_CUDA
@@ -214,6 +222,7 @@ struct Slot {
   cudaStream_t streams[kStreams] = {};
   cudaEvent_t done[kStreams] = {};  // recorded on each stream at the end of an enqueue
   cudaEvent_t dev_ready = nullptr;  // device-output submits: recorded on the caller's stream, waited on before a kernel
+  cudaEvent_t ep_ready = nullptr;   // episode submits: the same, on the learner's stream (PhcHostEpisodeOut.stream)
   // can the direct path be used: the 11 pointers of PhcHostStepArgs and PhcHostEnvArgs.mpjpe
   Seen<12> step_seen;
   // resets, allocated at the first submit that needs them: device root / dof rows of re-posed envs and the flags the
@@ -230,6 +239,7 @@ struct Slot {
   float* d_init = nullptr;  // [max_envs] x (13 root | 69 dof pos | 69 dof vel), init_rows of them set
   int64_t init_rows = -1;   // -1: no initial state
   Seen<3> env_seen;         // the env inputs last found to be host memory
+  Seen<7> ep_seen;          // the episode tensors last found to be device memory on the context's device
   // the step in flight
   bool busy = false;
   int path = 0;  // 1 direct, 2 staged
@@ -306,6 +316,7 @@ static cudaError_t slot_alloc(const PhcHostStep* c, Slot& s) {
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&s.done[i], cudaEventDisableTiming);
   }
   if (e == cudaSuccess) e = cudaEventCreateWithFlags(&s.dev_ready, cudaEventDisableTiming);
+  if (e == cudaSuccess) e = cudaEventCreateWithFlags(&s.ep_ready, cudaEventDisableTiming);
   s.ready = e == cudaSuccess;
   return e;
 }
@@ -328,6 +339,7 @@ static void slot_free(Slot& s) {
     if (s.streams[i]) cudaStreamDestroy(s.streams[i]);
   }
   if (s.dev_ready) cudaEventDestroy(s.dev_ready);
+  if (s.ep_ready) cudaEventDestroy(s.ep_ready);
   s = Slot{};
 }
 
@@ -417,6 +429,23 @@ static int check_env(Slot& s, const PhcHostEnvArgs* e) {
   for (const void* p : ptrs)
     if (p && classify(p).mem == Mem::kDevice) return PHC_ERR_UNSUPPORTED;
   s.env_seen.keep(ptrs, 0);
+  return PHC_OK;
+}
+
+// What the episode submit validates on top of the others (its NULL fields are checked before anything else).  The
+// verdict on the device pointers is cached per set of pointers.
+static int check_episode(const PhcHostStep* c, Slot& s, const PhcHostEpisodeOut* ep) {
+  const void* ptrs[7] = {ep->terminals, ep->truncations, ep->masks, ep->episode_returns, ep->episode_lengths,
+                         ep->sums, ep->rewards};
+  if (!s.ep_seen.hit(ptrs)) {
+    for (const void* p : ptrs) {
+      if (!p) continue;  // rewards
+      const PtrKind k = classify(p);
+      if (k.mem != Mem::kDevice || k.device != c->device) return PHC_ERR_UNSUPPORTED;
+    }
+    s.ep_seen.keep(ptrs, 1);
+  }
+  if (ep->buckets < 1 || ep->buckets > 4096) return PHC_ERR_SHAPE;
   return PHC_OK;
 }
 
@@ -677,11 +706,14 @@ struct Trace {
 // The fused step of one chunk: its device sim state and packed clock (dc) in; out, the caller's mapped host rows on the
 // direct path, the slot's device obs rows and packed scalars (dout) on the staged path, the caller's device tensors
 // with device outputs.  Enqueues the chunk's power inputs on `st`.  With a reset the step's own flags go to the slot's
-// scratch, the flags it reports to dout, and `ra` is the auto-reset over the same chunk.
+// scratch, the flags it reports to dout, and `ra` is the auto-reset over the same chunk.  With the episode bookkeeping
+// the chunk's rows of the caller's tensors; on the direct path the step also leaves device copies of its rewards and
+// flags in dout, and ep_raw is dout's reward_raw scratch (step_fused_mirrored).
 static cudaError_t chunk_step_args(const PhcHostStep* c, const Slot& s, const PhcHostStepArgs* a,
-                                   const PhcHostResetArgs* r, const PhcHostDeviceOut* dev, const Layout& L, int64_t lo,
-                                   int64_t m, unsigned char* dc, unsigned char* dout, bool staged, cudaStream_t st,
-                                   PhcStepArgs& k, PhcResetArgs& ra) {
+                                   const PhcHostResetArgs* r, const PhcHostDeviceOut* dev,
+                                   const PhcHostEpisodeOut* ep, const Layout& L, int64_t lo, int64_t m,
+                                   unsigned char* dc, unsigned char* dout, bool staged, cudaStream_t st,
+                                   PhcStepArgs& k, PhcResetArgs& ra, float*& ep_raw) {
   const int64_t D = c->obs_dim;
   const int W = s.extra.raw_cols;
   float* state = s.d_state + lo * kStateFloats;
@@ -728,13 +760,31 @@ static cudaError_t chunk_step_args(const PhcHostStep* c, const Slot& s, const Ph
     ra = chunk_reset_args(c, s, r, state, dc, L, lo, k.obs_buf);
     k.auto_reset = &ra;
   }
+  ep_raw = nullptr;
+  if (ep) {
+    k.ep_terminals = ep->terminals + lo;
+    k.ep_truncations = ep->truncations + lo;
+    k.ep_masks = ep->masks + lo;
+    k.ep_returns = ep->episode_returns + lo;
+    k.ep_lengths = ep->episode_lengths + lo;
+    k.ep_sums = ep->sums;
+    k.ep_buckets = ep->buckets;
+    k.ep_raw_cols = W;
+    if (ep->rewards) k.rew_out = ep->rewards + lo;
+    if (!staged) {
+      if (!k.rew_out) k.rew_out = (float*)(dout + L.rew);
+      k.reset_out = dout + L.reset;
+      k.terminate_out = dout + L.term;
+      ep_raw = (float*)(dout + L.raw);
+    }
+  }
   return e;
 }
 
 // One step over the chunks of s.bounds: inbound copies (the clock first on the direct path, the sim state first on the
 // staged path), the fused step, the export of the re-posed envs' rows, and on the staged path the outbound copies.
 static int step_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, const PhcHostResetArgs* r,
-                        const PhcHostDeviceOut* dev, bool staged) {
+                        const PhcHostDeviceOut* dev, const PhcHostEpisodeOut* ep, bool staged) {
   const int64_t D = c->obs_dim;
   const Rows rows = r ? (s.rows_staged ? s.stage : caller_rows(a, r)) : Rows{};
   Trace trace(staged, s.streams[0]);
@@ -750,14 +800,16 @@ static int step_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, const
     HOST_CUDA(s, inbound(s, a, r, L, lo, m, coff, true, staged, st));
     PhcStepArgs k;
     PhcResetArgs ra;
-    HOST_CUDA(s, chunk_step_args(c, s, a, r, dev, L, lo, m, dc, dout, staged, st, k, ra));
+    float* ep_raw;
+    HOST_CUDA(s, chunk_step_args(c, s, a, r, dev, ep, L, lo, m, dc, dout, staged, st, k, ra, ep_raw));
     trace.stamp(ci, Trace::kH2D, st);
     if (dev) HOST_CUDA(s, cudaStreamWaitEvent(st, s.dev_ready, 0));
+    if (ep) HOST_CUDA(s, cudaStreamWaitEvent(st, s.ep_ready, 0));
     // direct: the advanced progress goes straight into the caller's buffer too.  Not with a reset: where it runs as a
     // second launch (T > 1, or the generic kernel) the mirror would keep the advanced progress of the re-posed envs, so
     // the progress leaves with the flags, from the device clock after the reset.
     int16_t* mirror = staged || r ? nullptr : a->progress_buf + lo;
-    const int rc = step_fused_mirrored(c->lib, &k, m, st, mirror);
+    const int rc = step_fused_mirrored(c->lib, &k, m, st, mirror, lo, ep_raw);
     if (rc) return host_fail(s, rc, cudaSuccess);
     if (r) {  // direct: the export posts every env's flags and progress as well; staged: they leave in dout
       Rows out = rows_at(rows, lo, D);
@@ -832,13 +884,15 @@ static int reset_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, cons
 
 // Enqueues one step (or reset) on a slot (arguments already checked) and marks it in flight.
 static int slot_enqueue(PhcHostStep* c, int slot, const PhcHostStepArgs* a, const PhcHostResetArgs* r, int op,
-                        int64_t n, const PhcHostStep::Cand& k, const PhcHostDeviceOut* dev = nullptr) {
+                        int64_t n, const PhcHostStep::Cand& k, const PhcHostDeviceOut* dev = nullptr,
+                        const PhcHostEpisodeOut* ep = nullptr) {
   Slot& s = c->slots[slot];
   if (dev) HOST_CUDA(s, cudaEventRecord(s.dev_ready, dev->stream));
+  if (ep) HOST_CUDA(s, cudaEventRecord(s.ep_ready, ep->stream));
   // s.env / s.extra were set by the submit (zero for phc_host_step)
   const bool staged = op != kReset && k.path == 2;
   partition(s, n, k.chunks, staged);
-  const int rc = op == kReset ? reset_enqueue(c, s, a, r, dev) : step_enqueue(c, s, a, r, dev, staged);
+  const int rc = op == kReset ? reset_enqueue(c, s, a, r, dev) : step_enqueue(c, s, a, r, dev, ep, staged);
   if (rc) return rc;
   for (int i = 0; i < kStreams; ++i) HOST_CUDA(s, cudaEventRecord(s.done[i], s.streams[i]));
   s.args = *a;
@@ -1046,9 +1100,14 @@ int phc_host_step(PhcHostStep* c, const PhcHostStepArgs* a, int64_t n) {
 // The submits: every check before anything is enqueued, then the slot's buffers, then the enqueue.  dev: the device
 // tensors the rows go to, or NULL for host obs.  env: the env options, or NULL for none; a host reset takes only their
 // default_mask.  init_modes: StateInit.Default / Hybrid may be asked for (the _env submits; the others refuse them).
+// ep: the episode tensors of a step, or NULL.
 static int submit(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, const PhcHostResetArgs* r, int op, int64_t n,
-                  const PhcHostDeviceOut* dev, const PhcHostEnvArgs* env, bool init_modes) {
+                  const PhcHostDeviceOut* dev, const PhcHostEnvArgs* env, bool init_modes,
+                  const PhcHostEpisodeOut* ep = nullptr) {
   if (!c || !a || (op != kStep && !r) || (dev && !dev->obs)) return PHC_ERR_NULL;
+  if (ep && (!ep->terminals || !ep->truncations || !ep->masks || !ep->episode_returns || !ep->episode_lengths ||
+             !ep->sums))
+    return PHC_ERR_NULL;
   if (slot < 0 || slot >= PHC_HOST_SLOTS) return PHC_ERR_SHAPE;
   Slot& s = c->slots[slot];
   if (s.busy) return PHC_ERR_BUSY;
@@ -1061,6 +1120,7 @@ static int submit(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, const 
   if ((rc = check_env(s, &ev))) return rc;
   if (op != kStep && (rc = check_reset(c, s, r, op, init_modes ? &ev : nullptr, n))) return rc;
   if (dev && (rc = check_dev(c, dev))) return rc;
+  if (ep && (rc = check_episode(c, s, ep))) return rc;
   s.env = ev;
   s.extra.raw_cols = ev.dof_force ? 5 : 4;
   s.extra.mpjpe = ev.mpjpe != nullptr;
@@ -1080,7 +1140,7 @@ static int submit(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, const 
     (void)cudaGetLastError();
     return e == cudaErrorMemoryAllocation ? PHC_ERR_ALLOC : phc::record_cuda_error((int)e);
   }
-  return slot_enqueue(c, slot, a, r, op, n, untimed_schedule(c, s), dev);
+  return slot_enqueue(c, slot, a, r, op, n, untimed_schedule(c, s), dev, ep);
 }
 
 extern "C" {
@@ -1119,6 +1179,13 @@ int phc_host_step_submit_env(PhcHostStep* c, int32_t slot, const PhcHostStepArgs
 int phc_host_reset_submit_env(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, const PhcHostResetArgs* r,
                               const PhcHostDeviceOut* dev, const PhcHostEnvArgs* env, int64_t n) {
   return submit(c, slot, a, r, kReset, n, dev, env, true);
+}
+
+int phc_host_step_submit_episode(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, const PhcHostResetArgs* r,
+                                 const PhcHostDeviceOut* dev, const PhcHostEnvArgs* env, const PhcHostEpisodeOut* ep,
+                                 int64_t n) {
+  if (!ep) return PHC_ERR_NULL;
+  return submit(c, slot, a, r, r ? kStepReset : kStep, n, dev, env, true, ep);
 }
 
 int phc_host_step_set_initial_state(PhcHostStep* c, int32_t slot, const float* root_states, const float* dof_pos,

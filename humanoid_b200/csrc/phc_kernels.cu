@@ -1072,6 +1072,7 @@ struct StepParams {
   int32_t* ep_lengths;
   double* ep_sums;  // [ep_buckets][EP_SUM_COLS]: {episodes, sum of returns, sum of lengths, truncations, sum of reward_raw[:, c]}
   int ep_buckets, ep_raw_cols;
+  int ep_block0;    // the launch's first block in the batch (host chunks): block b adds into bucket (ep_block0 + b) % ep_buckets
   float* mpjpe;     // NULL, or [n]: mean over the 24 bodies of |body_pos - ref_body_pos| (extras["mpjpe"])
   float* obs_norm;  // NULL, or the normalised copy of the obs rows (RunningNorm.forward)
   int64_t obs_norm_stride;
@@ -2283,7 +2284,7 @@ __global__ void __launch_bounds__(EPB* J24, MINB) step_fast_kernel(const __grid_
         if (tid == i) mine = tot;
       }
       if (tid < 4 + p.ep_raw_cols && mine != 0.0f)
-        atomicAdd(p.ep_sums + (int64_t)(blockIdx.x % p.ep_buckets) * EP_SUM_COLS + tid, (double)mine);
+        atomicAdd(p.ep_sums + (int64_t)((p.ep_block0 + blockIdx.x) % p.ep_buckets) * EP_SUM_COLS + tid, (double)mine);
     }
   }
 
@@ -3497,8 +3498,9 @@ __global__ void __launch_bounds__(256) episode_update_kernel(EpisodeParams p) {
 }
 
 // The same bookkeeping for the step kernels that do not carry it (generic, T > 1): one thread per env after the step,
-// block sums into the bucket of the block.
-__global__ void __launch_bounds__(256) episode_bucket_kernel(StepParams p) {
+// block sums into the bucket of the block.  raw_post: NULL, or where the env's reward_raw row (dense, raw_stride
+// columns) is posted after it is read from p.raw (the host pipeline's mapped outputs: step_fused_mirrored).
+__global__ void __launch_bounds__(256) episode_bucket_kernel(StepParams p, float* raw_post) {
   const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   double v[EP_SUM_COLS];
 #pragma unroll
@@ -3523,6 +3525,8 @@ __global__ void __launch_bounds__(256) episode_bucket_kernel(StepParams p) {
 #pragma unroll
     for (int c = 0; c < EP_SUM_COLS - 4; ++c)
       if (c < p.ep_raw_cols) v[4 + c] = (double)p.raw[e * p.raw_stride + c];
+    if (raw_post)
+      for (int64_t c = 0; c < p.raw_stride; ++c) raw_post[e * p.raw_stride + c] = p.raw[e * p.raw_stride + c];
   }
   __shared__ double part[8][EP_SUM_COLS];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -3537,7 +3541,8 @@ __global__ void __launch_bounds__(256) episode_bucket_kernel(StepParams p) {
   if (threadIdx.x < 4 + p.ep_raw_cols) {
     double x = 0.0;
     for (int w = 0; w < 8; ++w) x += part[w][threadIdx.x];
-    if (x != 0.0) atomicAdd(p.ep_sums + (int64_t)(blockIdx.x % p.ep_buckets) * EP_SUM_COLS + threadIdx.x, x);
+    if (x != 0.0)
+      atomicAdd(p.ep_sums + (int64_t)((p.ep_block0 + blockIdx.x) % p.ep_buckets) * EP_SUM_COLS + threadIdx.x, x);
   }
 }
 
@@ -3982,6 +3987,7 @@ static int step_fill_params(const PhcLib* lib, const PhcStepArgs* a, int64_t n, 
   p.ep_sums = a->ep_sums;
   p.ep_buckets = a->ep_buckets;
   p.ep_raw_cols = a->ep_raw_cols;
+  p.ep_block0 = 0;
   if (a->ep_returns) {
     if (!a->ep_terminals || !a->ep_truncations || !a->ep_masks || !a->ep_lengths || !a->ep_sums) return PHC_ERR_NULL;
     if (a->ep_buckets < 1 || a->ep_buckets > 4096 || a->ep_raw_cols < 0 || a->ep_raw_cols > EP_SUM_COLS - 4) return PHC_ERR_SHAPE;
@@ -4135,13 +4141,25 @@ int phc_set_option(int key, int value) {
 
 }  // extern "C"
 
-// phc_step_fused plus a mirror for the advanced progress (the host pipeline points it at the caller's pinned buffer)
-int step_fused_mirrored(const PhcLib* lib, const PhcStepArgs* args, int64_t n, phc_stream_t stream, int16_t* progress_mirror) {
+// phc_step_fused for one chunk of the host pipeline (phc_host.cu).
+//   progress_mirror  NULL, or a second place (the caller's pinned buffer) that receives the advanced progress.
+//   env0             the chunk's first env in the batch.  The episode bookkeeping takes its buckets by the block's index
+//                    in the batch, so chunks do not pile onto the first rows: the T = 1 kernel's blocks (4 envs, chunks
+//                    start on multiples of 8) are the device path's blocks; episode_bucket_kernel's (256 envs) cannot be,
+//                    and start at the next row after the previous chunk's.
+//   ep_raw           NULL, or device scratch [n, reward_raw_stride] when the step's outputs are mapped host memory and
+//                    the episode bookkeeping is on: where the bookkeeping runs after the step it must not read those
+//                    back over the link, so the step leaves reward_raw here, the bookkeeping reads it and the step's
+//                    device copies rew_out / reset_out / terminate_out (which the caller sets), and posts the raw rows.
+int step_fused_mirrored(const PhcLib* lib, const PhcStepArgs* args, int64_t n, phc_stream_t stream,
+                        int16_t* progress_mirror, int64_t env0, float* ep_raw) {
   if (n == 0) return PHC_OK;
-  if (n < 0) return PHC_ERR_SHAPE;
+  if (n < 0 || env0 < 0) return PHC_ERR_SHAPE;
   StepParams p;
   int rc = step_fill_params(lib, args, n, p);
   if (rc) return rc;
+  if (!p.ep_returns) ep_raw = nullptr;
+  if (ep_raw && (!p.rew_out || !p.reset_out || !p.term_out)) return PHC_ERR_NULL;
   p.progress_mirror = progress_mirror;
   int dev = 0;
   PHC_CUDA(cudaGetDevice(&dev));
@@ -4232,6 +4250,7 @@ int step_fused_mirrored(const PhcLib* lib, const PhcStepArgs* args, int64_t n, p
     reset_after = p.reset_on && !in_kernel;
     StepParams pk = p;
     if (reset_after) pk.reset_on = 0;
+    pk.ep_block0 = (int)(env0 / 4);
     if (!def) rc = launch_step(step_fast_kernel<4, 8, false, true, true, false>, SM, 4, pk, stream, &attr[6][dev], pdl);
     else if (in_kernel) {
       if (p.obs_norm) rc = launch_step(step_fast_kernel<4, 8, true, true, true>, SM, 4, pk, stream, &attr[5][dev], pdl);
@@ -4245,6 +4264,8 @@ int step_fused_mirrored(const PhcLib* lib, const PhcStepArgs* args, int64_t n, p
     else rc = launch_step(step_fast_kernel<4, 8>, SM, 4, pk, stream, &attr[0][dev], pdl);
     if (rc != PHC_OK || !reset_after) return rc;
   } else {
+  float* raw_post = nullptr;  // the mapped reward_raw rows, posted by the bookkeeping (ep_raw)
+  if (ep_raw) raw_post = p.raw, p.raw = ep_raw;
   // T > 1 on the AoS tensor + packed table: the pipelined TMA kernel
   const bool multi = !g_force_generic && p.T > 1 && p.aos && p.L.packed && p.obs_vec2 && !p.obs_norm && def &&
                      !(args->flags & PHC_STEP_MAPPED_HOST_IO);
@@ -4264,7 +4285,10 @@ int step_fused_mirrored(const PhcLib* lib, const PhcStepArgs* args, int64_t n, p
     rc = launch_step(step_kernel<STEP_EPB>, sizeof(StepSmem<STEP_EPB>), STEP_EPB, p, stream, &attr_gen[dev], false);
   }
   if (rc == PHC_OK && p.ep_returns) {  // these kernels do not carry the episode bookkeeping: a second, small launch
-    episode_bucket_kernel<<<(unsigned)((p.n + 255) / 256), 256, 0, stream>>>(p);
+    StepParams q = p;
+    q.ep_block0 = (int)((env0 + 255) / 256);
+    if (raw_post) q.rew = p.rew_out, q.reset = p.reset_out, q.term = p.term_out;
+    episode_bucket_kernel<<<(unsigned)((p.n + 255) / 256), 256, 0, stream>>>(q, raw_post);
     rc = launch_status();
   }
   reset_after = p.reset_on != 0;  // ... nor the in-step reset
@@ -4291,7 +4315,7 @@ bool lib_has_dof_state(const PhcLib* lib) { return lib && lib->d.lrs && lib->d.d
 extern "C" {
 
 int phc_step_fused(const PhcLib* lib, const PhcStepArgs* args, int64_t n, phc_stream_t stream) {
-  return step_fused_mirrored(lib, args, n, stream, nullptr);
+  return step_fused_mirrored(lib, args, n, stream, nullptr, 0, nullptr);
 }
 
 // ---- RunningNorm ---------------------------------------------------------------------------

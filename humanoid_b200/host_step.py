@@ -22,6 +22,12 @@ and velocity go in, ``reward_raw`` has five columns), ``allocate(..., mpjpe=True
 ``set_initial_state`` per slot enables ``state_init="default"`` / ``"hybrid"`` (the hybrid mask in
 ``HostResetBuffers.default_mask``).
 
+With ``episode=HostEpisodeBuffers`` a step also does the per-step bookkeeping of the pufferlib wrapper
+(``PHCPufferEnv.step``, ``phc_host_step_submit_episode``): ``terminals`` / ``truncations`` / ``masks``, the running
+``episode_returns`` / ``episode_lengths``, the ``rewards`` copy and the sums ``mean_and_log`` reports are written into
+CUDA tensors, where the learner's experience buffer reads them, with no copy back to the device and no extra launch by
+the caller.  A loop over two batches on two slots logs both with ``HostEpisodeBuffers.log([ep0, ep1], log_interval)``.
+
 Pinned buffers (``HostStepBuffers.allocate(..., pinned=True)``) take the fast paths; pageable ones work through
 staging.  The CUDA device of the motion library must be current when the context is created and stepped; after
 ``MotionLib.repack()`` synchronise the device before the next host step (the steps run on the context's own streams).
@@ -37,6 +43,7 @@ import torch
 
 from . import _cabi
 from .env import DEFAULT_REWARD
+from .puffer_env import episode_info
 
 _FIELDS = (  # name, dtype, trailing shape (T: the number of future steps of the task obs)
     ("state", torch.float32, lambda T: (_cabi.NUM_BODIES, 13)),
@@ -325,6 +332,118 @@ class HostDeviceOutputs:
         return a
 
 
+@dataclass(eq=False)
+class HostEpisodeBuffers:
+    """The CUDA tensors of ``PHCPufferEnv``'s per-step bookkeeping for one batch of ``n`` envs (``episode`` of
+    ``HostStep.submit`` / ``step``).  Outputs: ``terminals``, ``truncations``, ``masks`` (bool [n]), ``rewards`` (f32
+    [n], the step's ``rew_buf``: the wrapper's ``rewards.clone()``; optional).  In / out: ``episode_returns`` f32 [n],
+    ``episode_lengths`` int32 [n].  ``sums`` f64 [B, EPISODE_SUM_COLS]: the running sums behind ``mean_and_log``, added
+    to every step and folded by ``log``.  ``raw_cols``: the logged reward terms, 4, or 5 with the power reward."""
+
+    terminals: torch.Tensor
+    truncations: torch.Tensor
+    masks: torch.Tensor
+    episode_returns: torch.Tensor
+    episode_lengths: torch.Tensor
+    sums: torch.Tensor
+    raw_cols: int = 4
+    rewards: Optional[torch.Tensor] = None
+
+    @classmethod
+    def allocate(cls, n: int, raw_cols: int, device=None, buckets: Optional[int] = None,
+                 rewards: bool = True) -> "HostEpisodeBuffers":  # fmt: skip
+        """Buffers for ``n`` envs on ``device`` (default: the current CUDA device) as ``PHCPufferEnv.reset`` leaves
+        them.  ``buckets`` rows of sums (default: one per block of the T = 1 step kernel, ``ceil(n / 4)``, within
+        32..4096 as ``PHCPufferEnv`` takes them); ``rewards`` adds the reward copy."""
+        device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+        B = max(32, min(4096, (n + 3) // 4)) if buckets is None else int(buckets)
+        return cls(
+            terminals=torch.zeros(n, dtype=torch.bool, device=device),
+            truncations=torch.zeros(n, dtype=torch.bool, device=device),
+            masks=torch.ones(n, dtype=torch.bool, device=device),
+            episode_returns=torch.zeros(n, dtype=torch.float32, device=device),
+            episode_lengths=torch.zeros(n, dtype=torch.int32, device=device),
+            sums=torch.zeros((B, _cabi.EPISODE_SUM_COLS), dtype=torch.float64, device=device),
+            raw_cols=int(raw_cols),
+            rewards=torch.zeros(n, dtype=torch.float32, device=device) if rewards else None,
+        )  # fmt: skip
+
+    @property
+    def n(self) -> int:
+        return int(self.terminals.shape[0])
+
+    def validate(self, n: int, raw_cols: int) -> None:
+        """Checks dtype, shape, contiguity and that every tensor lives on one CUDA device; ``raw_cols``: the reward
+        terms the step writes (4, or 5 with the power reward)."""
+        if self.raw_cols != raw_cols:
+            raise ValueError(f"these episode buffers log {self.raw_cols} reward terms, the step writes {raw_cols}")
+        s = self.sums
+        B = int(s.shape[0]) if isinstance(s, torch.Tensor) and s.dim() == 2 else -1
+        if not 1 <= B <= 4096:
+            raise ValueError(f"sums must be [B, {_cabi.EPISODE_SUM_COLS}] with 1 <= B <= 4096")
+        flag = (torch.bool, torch.uint8)
+        checks = [("terminals", flag, (n,)), ("truncations", flag, (n,)), ("masks", flag, (n,)),
+                  ("episode_returns", (torch.float32,), (n,)), ("episode_lengths", (torch.int32,), (n,)),
+                  ("sums", (torch.float64,), (B, _cabi.EPISODE_SUM_COLS))]  # fmt: skip
+        if self.rewards is not None:
+            checks.append(("rewards", (torch.float32,), (n,)))
+        dev = self.terminals.device if isinstance(self.terminals, torch.Tensor) else None
+        for name, dtypes, shape in checks:
+            t = getattr(self, name)
+            if not isinstance(t, torch.Tensor) or t.device.type != "cuda" or t.device != dev:
+                raise _cabi.PhcError(f"{name} must be a CUDA tensor on the device of terminals")
+            if t.dtype not in dtypes:
+                raise _cabi.PhcError(f"{name} must be {' or '.join(map(str, dtypes))}, got {t.dtype}")
+            if tuple(t.shape) != shape:
+                raise ValueError(f"{name} has shape {tuple(t.shape)}, expected {shape}")
+            if not t.is_contiguous():
+                raise _cabi.PhcError(f"{name} must be contiguous")
+
+    def reset(self) -> None:
+        """What ``PHCPufferEnv.reset`` clears (clean_pufferl/env.py:88-107): rewards, terminals, truncations, the sums;
+        masks set.  The running returns and lengths are kept, as there."""
+        if self.rewards is not None:
+            self.rewards.zero_()
+        self.terminals.zero_()
+        self.truncations.zero_()
+        self.masks.fill_(True)
+        self.sums.zero_()
+
+    def _args(self) -> _cabi.PhcHostEpisodeOut:
+        a = _cabi.PhcHostEpisodeOut()
+        a.terminals, a.truncations, a.masks = self.terminals.data_ptr(), self.truncations.data_ptr(), self.masks.data_ptr()
+        a.episode_returns, a.episode_lengths = self.episode_returns.data_ptr(), self.episode_lengths.data_ptr()
+        a.rewards = _cabi.ptr(self.rewards)
+        a.sums, a.buckets = self.sums.data_ptr(), self.sums.shape[0]
+        a.stream = _cabi.stream_ptr(self.terminals.device)
+        return a
+
+    @staticmethod
+    def log(batches: Sequence["HostEpisodeBuffers"], log_interval: int) -> List[dict]:
+        """``PHCPufferEnv.mean_and_log`` over every env of ``batches`` (the batches of one env loop, in env order),
+        after their steps have been waited for: folds the sums of all of them, zeroes them, and returns ``[info]``.
+        The reward-term means divide by the total env count, so two batches of n log what one batch of 2n envs
+        would; with one sums row per block the fold adds the same rows in the same order."""
+        batches = list(batches)
+        if not batches:
+            raise ValueError("log needs at least one batch")
+        raw_cols, dev = batches[0].raw_cols, batches[0].sums.device
+        if any(b.raw_cols != raw_cols or b.sums.device != dev for b in batches):
+            raise ValueError("the batches must log the same reward terms on one device")
+        sums = torch.cat([b.sums for b in batches])
+        stats = torch.zeros(4, dtype=torch.float64, device=dev)
+        raw = torch.zeros(raw_cols, dtype=torch.float32, device=dev)
+        n = sum(b.n for b in batches)
+        _cabi.check(
+            _cabi.load().phc_episode_fold(sums.data_ptr(), sums.shape[0], raw_cols, n, stats.data_ptr(), raw.data_ptr(),
+                                          _cabi.stream_ptr(dev)),
+            "phc_episode_fold",
+        )  # fmt: skip
+        for b in batches:
+            b.sums.zero_()
+        return [episode_info(stats, raw, log_interval)[0]]
+
+
 class HostStep:
     """A ``phc_host_step`` context on the current CUDA device for batches of up to ``max_envs`` envs.
 
@@ -357,6 +476,7 @@ class HostStep:
         self._inflight: List[Optional[HostStepBuffers]] = [None] * _cabi.HOST_SLOTS
         self._inflight_reset: List[Optional[HostResetBuffers]] = [None] * _cabi.HOST_SLOTS
         self._inflight_dev: List[Optional[HostDeviceOutputs]] = [None] * _cabi.HOST_SLOTS
+        self._inflight_ep: List[Optional[HostEpisodeBuffers]] = [None] * _cabi.HOST_SLOTS
         self.time_steps = int(time_steps)
         self._capi = _cabi.load()
         term = torch.as_tensor(termination_distances, dtype=torch.float32).cpu().expand(_cabi.NUM_BODIES)
@@ -379,12 +499,14 @@ class HostStep:
         return self._ctx
 
     def step(self, bufs: HostStepBuffers, reset: Optional[HostResetBuffers] = None, state_init: str = "random",
-             flag_test: bool = False, device_out: Optional[HostDeviceOutputs] = None) -> HostStepBuffers:  # fmt: skip
-        """One step of ``bufs``; returns when every output is in ``bufs`` (``progress_buf`` advanced in place) and in
-        ``device_out``.  With ``reset`` the envs the step flags are re-posed as well (see ``submit``); with ``reset`` or
-        ``device_out`` this runs on slot 0."""
-        if reset is not None or device_out is not None or self.use_power_reward or bufs.mpjpe is not None:
-            self.submit(0, bufs, reset, state_init, flag_test, device_out=device_out)
+             flag_test: bool = False, device_out: Optional[HostDeviceOutputs] = None,
+             episode: Optional[HostEpisodeBuffers] = None) -> HostStepBuffers:  # fmt: skip
+        """One step of ``bufs``; returns when every output is in ``bufs`` (``progress_buf`` advanced in place), in
+        ``device_out`` and in ``episode``.  With ``reset`` the envs the step flags are re-posed as well (see
+        ``submit``); with ``reset``, ``device_out`` or ``episode`` this runs on slot 0."""
+        if (reset is not None or device_out is not None or episode is not None or self.use_power_reward
+                or bufs.mpjpe is not None):  # fmt: skip
+            self.submit(0, bufs, reset, state_init, flag_test, device_out=device_out, episode=episode)
             return self.wait(0)
         n = bufs.validate(self.time_steps)
         args = bufs._args()
@@ -392,8 +514,8 @@ class HostStep:
         return bufs
 
     def submit(self, slot: int, bufs: HostStepBuffers, reset: Optional[HostResetBuffers] = None,
-               state_init: str = "random", flag_test: bool = False,
-               device_out: Optional[HostDeviceOutputs] = None) -> None:  # fmt: skip
+               state_init: str = "random", flag_test: bool = False, device_out: Optional[HostDeviceOutputs] = None,
+               episode: Optional[HostEpisodeBuffers] = None) -> None:  # fmt: skip
         """Enqueue one step of ``bufs`` on ``slot`` (0 or 1) and return.  ``bufs`` (and ``reset``) belong to the library
         until ``wait(slot)`` returns: do not read or write them before then.
 
@@ -410,28 +532,41 @@ class HostStep:
 
         The env options are the power reward (``use_power_reward``), ``bufs.mpjpe`` and ``state_init`` "default" /
         "hybrid" (after ``set_initial_state(slot, ...)``; "hybrid" takes ``reset.default_mask`` and ``reset.phase``).
-        This is ``phc_host_step_submit_env``, with no ``PhcHostEnvArgs`` (NULL) when no option is on."""
+        This is ``phc_host_step_submit_env``, with no ``PhcHostEnvArgs`` (NULL) when no option is on.
+
+        With ``episode`` the step also does ``PHCPufferEnv.step``'s bookkeeping into its CUDA tensors
+        (``phc_host_step_submit_episode``), from the step's own flags (with ``reset``: those before the reset); the
+        kernels writing them wait for the work enqueued so far on the current CUDA stream.  The tensors belong to the
+        library until ``wait(slot)`` returns; then they are complete."""
         n = bufs.validate(self.time_steps, device_out=device_out is not None, power=self.use_power_reward)
         env = self._env_args(slot, bufs, reset, state_init, n)
         rargs = None
         if reset is not None:
             reset.validate(n)
             rargs = C.byref(reset._args(bufs, state_init, flag_test))
+        name = "phc_host_step_submit_env"
+        if episode is not None:
+            episode.validate(n, 5 if self.use_power_reward else 4)
+            if device_out is not None and device_out.obs.device != episode.terminals.device:
+                raise _cabi.PhcError("episode and device_out must live on one CUDA device")
+            name = "phc_host_step_submit_episode"
         # an auto-reset replaces counted rows and adds none
-        self._submit("phc_host_step_submit_env", slot, bufs, reset, rargs, device_out, env, n, lambda: n)
+        self._submit(name, slot, bufs, reset, rargs, device_out, env, n, lambda: n, episode)
 
-    def _submit(self, name, slot, bufs, reset, rargs, device_out, env, n, new_rows):
-        """The C call of ``submit`` / ``reset_submit``; ``new_rows()``: the rows it adds to ``device_out``'s moments."""
+    def _submit(self, name, slot, bufs, reset, rargs, device_out, env, n, new_rows, episode=None):
+        """The C call of ``submit`` / ``reset_submit``; ``new_rows()``: the rows it adds to ``device_out``'s moments;
+        ``episode``: the bookkeeping tensors of ``phc_host_step_submit_episode``."""
         dargs = None
         if device_out is not None:
             device_out.validate(n, self.time_steps)
             dargs = C.byref(device_out._args())
         fn = getattr(self._capi, name)
         eargs = None if env is None else C.byref(env)
-        _cabi.check(fn(self._live(), int(slot), C.byref(bufs._args()), rargs, dargs, eargs, n), name)
+        args = (C.byref(bufs._args()), rargs, dargs, eargs) + (() if episode is None else (C.byref(episode._args()),))
+        _cabi.check(fn(self._live(), int(slot), *args, n), name)
         if device_out is not None and device_out.obs_moments is not None:
             device_out.rows += new_rows()
-        self._hold(slot, bufs, reset, device_out)
+        self._hold(slot, bufs, reset, device_out, episode)
 
     def _env_args(self, slot, bufs: HostStepBuffers, reset: Optional[HostResetBuffers], state_init: str,
                   n: int, step: bool = True) -> Optional[_cabi.PhcHostEnvArgs]:  # fmt: skip
@@ -479,11 +614,12 @@ class HostStep:
                     "phc_host_step_set_initial_state")  # fmt: skip
         self._initial_rows[slot] = n
 
-    def _hold(self, slot, bufs, reset, device_out):
+    def _hold(self, slot, bufs, reset, device_out, episode=None):
         """Keep a batch's tensors alive until its ``wait``."""
         self._inflight[slot] = bufs
         self._inflight_reset[slot] = reset
         self._inflight_dev[slot] = device_out
+        self._inflight_ep[slot] = episode
 
     def reset_submit(self, slot: int, bufs: HostStepBuffers, reset: HostResetBuffers, state_init: str = "random",
                      flag_test: bool = False, device_out: Optional[HostDeviceOutputs] = None) -> None:  # fmt: skip
@@ -535,6 +671,7 @@ class HostStep:
         self._inflight = [None] * _cabi.HOST_SLOTS
         self._inflight_reset = [None] * _cabi.HOST_SLOTS
         self._inflight_dev = [None] * _cabi.HOST_SLOTS
+        self._inflight_ep = [None] * _cabi.HOST_SLOTS
 
     def __enter__(self) -> "HostStep":
         return self

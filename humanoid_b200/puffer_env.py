@@ -148,18 +148,26 @@ class PHCPufferEnv:
     def mean_and_log(self):
         """:191-204 plus the reward terms of :164-176 — the one host read per ``log_interval`` steps."""
         self._fold()
-        stats = self._stats.tolist()
-        raw = (self.raw_rewards / self.log_interval).tolist()
+        info, done = episode_info(self._stats, self.raw_rewards, self.log_interval)
         self._stats.zero_()
         self.raw_rewards.zero_()
-        done = stats[0]
         self.episode_count += int(done)
-        nan = float("nan")  # np.mean([]) in the reference
-        info = {
-            "episode_return": stats[1] / done if done else nan,
-            "episode_length": stats[2] / done if done else nan,
-            "truncated_rate": stats[3] / done if done else nan,
-        }
-        for k, v in zip(("rew_body_pos", "rew_body_rot", "rew_lin_vel", "rew_ang_vel", "rew_power"), raw):
-            info[k] = v
         return [info]
+
+
+def episode_info(stats: torch.Tensor, raw_rewards: torch.Tensor, log_interval: int):
+    """The dict of ``mean_and_log`` (:191-204, the reward terms of :164-176) from the folded running sums: ``stats`` f64
+    [4] {episodes finished, sum of returns, sum of lengths, truncations} and ``raw_rewards`` f32 (the per-step means of
+    the reward terms, summed over ``log_interval`` steps).  Returns ``(info, episodes finished)``."""
+    stats = stats.tolist()
+    raw = (raw_rewards / log_interval).tolist()
+    done = stats[0]
+    nan = float("nan")  # np.mean([]) in the reference
+    info = {
+        "episode_return": stats[1] / done if done else nan,
+        "episode_length": stats[2] / done if done else nan,
+        "truncated_rate": stats[3] / done if done else nan,
+    }
+    for k, v in zip(("rew_body_pos", "rew_body_rot", "rew_lin_vel", "rew_ang_vel", "rew_power"), raw):
+        info[k] = v
+    return info, done

@@ -655,6 +655,45 @@ PHC_API int phc_host_step_set_initial_state(PhcHostStep* ctx, int32_t slot, cons
                                             const float* dof_pos /* [n,69] */, const float* dof_vel /* [n,69] */,
                                             int64_t n);
 
+/* Episode bookkeeping on the host-buffer path: PHCPufferEnv.step's per-step update (clean_pufferl/env.py:121-159) done
+ * by the host step itself into caller-owned device tensors, where the learner's experience buffer reads them.  Added
+ * without a change to any existing struct or entry point, so PHC_ABI_VERSION stays 6; a caller finds it by its symbol.
+ *
+ *   phc_host_step_submit_episode  phc_host_step_submit_env with the bookkeeping of PhcStepArgs.ep_* (phc_episode_update
+ *            documents the semantics) over the batch's n envs.  Everything phc_host_step_submit_env does, checks and
+ *            writes still holds: rew_buf, reward_raw, flags, progress and the reset rows go to the host buffers.
+ *   flags    The step's own reset / terminate flags: with auto-reset, those before the reset (what the caller gets in
+ *            reset_buf / terminate_buf).  The logged reward columns are all of reward_raw's: 4, or 5 with the power
+ *            reward.  rewards (optional) receives rew_buf, the wrapper's `rew = self.rewards.clone()`.
+ *   sums     Added to (+=) per step; block b of the batch adds into row b % buckets, whatever the chunk it runs in, so
+ *            phc_episode_fold(sums, buckets, raw_cols, n, ...) folds them as on the device path.  At T = 1 with
+ *            buckets >= ceil(n / 4) the rows are bit-identical to the device path's.  A caller stepping two batches
+ *            folds the rows of both with the total env count (HostEpisodeBuffers.log).
+ *   ordering A submit records an event on ep->stream; each of the slot's streams waits for it before its first write
+ *            into these tensors.  When phc_host_step_wait returns, they are complete; work enqueued afterwards on any
+ *            stream sees them.  The tensors belong to the library until then.
+ *   validation  Before anything is enqueued, on top of the checks of phc_host_step_submit_env: ep or any of its fields
+ *            but rewards NULL -> PHC_ERR_NULL; a field that is not device memory on the context's device ->
+ *            PHC_ERR_UNSUPPORTED; buckets outside 1..4096 -> PHC_ERR_SHAPE; a busy slot -> PHC_ERR_BUSY.  After any
+ *            error the slot is idle and nothing has been written.
+ *   resets   phc_host_reset_submit* neither take nor touch these tensors (the wrapper clears them in its reset()). */
+typedef struct PhcHostEpisodeOut {
+  uint8_t* terminals;        /* device [n] out                                                   */
+  uint8_t* truncations;      /* device [n] out                                                   */
+  uint8_t* masks;            /* device [n] out                                                   */
+  float* episode_returns;    /* device [n] in/out                                                */
+  int32_t* episode_lengths;  /* device [n] in/out                                                */
+  float* rewards;            /* device [n] out, or NULL: rew = rewards.clone()                   */
+  double* sums;              /* device [buckets][PHC_EPISODE_SUM_COLS], += ; zeroed by the caller once */
+  int32_t buckets;           /* 1 .. 4096                                                        */
+  phc_stream_t stream;       /* the learner's stream that reads these tensors                    */
+} PhcHostEpisodeOut;
+PHC_API int phc_host_step_submit_episode(PhcHostStep* ctx, int32_t slot, const PhcHostStepArgs* args,
+                                         const PhcHostResetArgs* reset /* may be NULL */,
+                                         const PhcHostDeviceOut* dev /* may be NULL */,
+                                         const PhcHostEnvArgs* env /* may be NULL */, const PhcHostEpisodeOut* ep,
+                                         int64_t n);
+
 /* ------------------------------------------------------------------------------------
  * RunningNorm statistics                                   policies/running_norm.py:23-34
  * phc_obs_moments accumulates (+=) per-column fp64 sum and sum of squares of x[rows,cols]
