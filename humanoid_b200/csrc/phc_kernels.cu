@@ -1024,6 +1024,48 @@ __device__ __forceinline__ void emit_task_obs(float* tk, int b, Heading hi, cons
   put6<DEF>(tk + 432 + b * 6, o.l_rot);
 }
 
+// emit_self_obs(row) and emit_task_obs(row + SW) of one body, bit for bit, with the vector work paired into fp32x2
+// instructions (phc_math.cuh): the seven heading rotations as (p_b - p_root, v_b) | (d_pos, l_pos) | (d_vel, d_ang)
+// and w_b alone, the two heading products and tan-norms of q_b and the reference rotation together.
+template <bool DEF>
+__device__ __forceinline__ void emit_obs_paired(float* row, int SW, const ObsFlags& of, int b, Vec3 root_pos, Heading hi,
+                                                const HeadingRot& hr, Vec3 pos, Quat rot, Vec3 vel, Vec3 ang,
+                                                const RefBody& r, float one) {
+  const int h = DEF ? 1 : of.hcol;
+  float* tk = row + SW;
+  const Vec3x2 pv = heading_rotate2(hr, pack3(pos - root_pos, vel));
+  const Vec3x2 dl = heading_rotate2(hr, sub3x2(pack3(r.pos, r.pos), pack3(pos, root_pos), one));
+  const Vec3x2 dva = heading_rotate2(hr, sub3x2(pack3(r.vel, r.ang), pack3(vel, ang), one));
+  if (b == 0) {
+    if (h) row[0] = root_pos.z;
+  } else {
+    st3(row + h + (b - 1) * 3, lane0(pv));
+  }
+  st3(row + h + 213 + b * 3, lane1(pv));
+  st3(row + h + 285 + b * 3, heading_rotate(hr, ang));
+  st3(tk + b * 3, lane0(dl));
+  st3(tk + 360 + b * 3, lane1(dl));
+  st3(tk + 216 + b * 3, lane0(dva));
+  st3(tk + 288 + b * 3, lane1(dva));
+  Quatx2 hq = heading_mul_left2(hi, pack4(rot, r.rot));
+  if (!DEF && b == 0 && !of.local_root) {  // as in emit_self_obs
+    const Quat s = heading_source(rot, of.upright);
+    hq.x.x = s.x, hq.y.x = s.y, hq.z.x = s.z, hq.w.x = s.w;
+  }
+  float2 t2[6];
+  quat_tan_norm2(hq, one, t2);
+  float t6[6];
+#pragma unroll
+  for (int k = 0; k < 6; ++k) t6[k] = t2[k].x;
+  put6<DEF>(row + h + 69 + b * 6, t6);
+#pragma unroll
+  for (int k = 0; k < 6; ++k) t6[k] = t2[k].y;
+  put6<DEF>(tk + 432 + b * 6, t6);
+  const Quat dg = quat_mul(r.rot, quat_conj(rot));  // task_obs_body's d_rot
+  quat_tan_norm(heading_mul_right(heading_mul_left(hi, dg), heading_conj(hi)), t6);
+  put6<DEF>(tk + 72 + b * 6, t6);
+}
+
 // ---------------------------------------------------------------------------------------
 // K6: the fused step.  One block = EPB envs x 24 bodies.
 //   phase 0  sim tile -> smem (cp.async 16 B when the four views are one 16-B aligned AoS-13
@@ -1054,6 +1096,7 @@ struct StepParams {
   uint32_t reset_mask;
   int use_mean, early, advance, T;
   float dt;
+  float one;  // 1.0f, the multiplier of the packed add (add2 in phc_math.cuh): a literal would let ptxas fuse it
   PhcRewardSpec rwd;
   float* obs;
   int64_t obs_stride;
@@ -1608,6 +1651,25 @@ __device__ __forceinline__ RefBody blend_ref3(const float* f0, const float* f1, 
   return r;
 }
 
+// blend_ref2 of two queries at once, in fp32x2 instructions: r0 equals blend_ref2(f00, f01, bl.x, goff, b) and r1
+// blend_ref2(f10, f11, bl.y, goff, b), bit for bit
+__device__ __forceinline__ void blend_ref_pair(const float* f00, const float* f01, const float* f10, const float* f11,
+                                               float2 bl, const float* goff, int b, float one, RefBody& r0, RefBody& r1) {
+  const float2 om = {1.0f - bl.x, 1.0f - bl.y};
+  Vec3x2 pos = lerp3x2(om, bl, pack3(ld3(f00 + b * 3), ld3(f10 + b * 3)), pack3(ld3(f01 + b * 3), ld3(f11 + b * 3)), one);
+  pos.x = add2(pos.x, bc2(goff[0]), one);
+  pos.y = add2(pos.y, bc2(goff[1]), one);
+  pos.z = add2(pos.z, bc2(goff[2]), one);
+  const Vec3x2 vel = lerp3x2(om, bl, pack3(ld3(f00 + 168 + b * 3), ld3(f10 + 168 + b * 3)),
+                             pack3(ld3(f01 + 168 + b * 3), ld3(f11 + 168 + b * 3)), one);
+  const Vec3x2 ang = lerp3x2(om, bl, pack3(ld3(f00 + 240 + b * 3), ld3(f10 + 240 + b * 3)),
+                             pack3(ld3(f01 + 240 + b * 3), ld3(f11 + 240 + b * 3)), one);
+  quat_slerp_pair(ld4v(f00 + 72 + b * 4), ld4v(f01 + 72 + b * 4), ld4v(f10 + 72 + b * 4), ld4v(f11 + 72 + b * 4), bl,
+                  r0.rot, r1.rot);
+  r0.pos = lane0(pos), r0.vel = lane0(vel), r0.ang = lane0(ang);
+  r1.pos = lane1(pos), r1.vel = lane1(vel), r1.ang = lane1(ang);
+}
+
 // The reset of the envs a step flags, inside the step (PhcStepArgs.auto_reset; clean_pufferl/env.py:133-135 ->
 // humanoid_phc.py:665-676).  Called by EVERY thread of a block that has a flagged env, once per flagged env, after
 // phase 2 (the frame buffer is the stage by now, the threads' own per-body state is dead).  A block with a flagged
@@ -1974,9 +2036,20 @@ __global__ void __launch_bounds__(EPB* J24, MINB) step_fast_kernel(const __grid_
     vel = {d[7], d[8], d[9]};
     ang = {d[10], d[11], d[12]};
     const float* fr = S.frames + e * (4 * FRAME_FLOATS);
+    // the reference bodies of both queries: r0 (t) feeds the reward and the distance, r1 (t + dt) the obs.  Paired
+    // into fp32x2 instructions, except in the RESET instantiations, which spill with the paired math at 80 registers.
+    RefBody r0;
+    const float* f00 = fr + S.slot[0][0][e] * FRAME_FLOATS;
+    const float* f01 = fr + S.slot[0][1][e] * FRAME_FLOATS;
+    const float* f10 = fr + S.slot[1][0][e] * FRAME_FLOATS;
+    const float* f11 = fr + S.slot[1][1][e] * FRAME_FLOATS;
+    if constexpr (RESET) {
+      r0 = blend_ref2(f00, f01, S.bl[0][e], S.goff[e], b);
+      r1 = blend_ref2(f10, f11, S.bl[1][e], S.goff[e], b);
+    } else {
+      blend_ref_pair(f00, f01, f10, f11, make_float2(S.bl[0][e], S.bl[1][e]), S.goff[e], b, p.one, r0, r1);
+    }
     {
-      const RefBody r0 = blend_ref2(fr + S.slot[0][0][e] * FRAME_FLOATS, fr + S.slot[0][1][e] * FRAME_FLOATS,
-                                    S.bl[0][e], S.goff[e], b);
       float sp, sr, sv, sa;
       reward_partials(pos, rot, vel, ang, r0, sp, sr, sv, sa);
       S.part[0][e][b] = sp;
@@ -1988,7 +2061,6 @@ __global__ void __launch_bounds__(EPB* J24, MINB) step_fast_kernel(const __grid_
       if (!use_mean && (p.reset_mask >> b & 1u) && dist > p.term_dist[b]) S.fallen[e] = 1;  // any(), benign race
       if (dof_force) S.part[5][e][b] = power_partial(p, env0 + e, b);
     }
-    r1 = blend_ref2(fr + S.slot[1][0][e] * FRAME_FLOATS, fr + S.slot[1][1][e] * FRAME_FLOATS, S.bl[1][e], S.goff[e], b);
   }
   PHC_STAMP(4);
   __syncthreads();  // #2: partials / heading visible; frame buffer dead -> becomes the obs stage
@@ -2036,8 +2108,12 @@ __global__ void __launch_bounds__(EPB* J24, MINB) step_fast_kernel(const __grid_
     const Heading hi = {S.hz[e], S.hw[e]};
     const HeadingRot hr = heading_rot(hi);
     float* row = S.frames + e * RW;
-    emit_self_obs<DEF>(row, p.of, b, root_pos, hi, hr, pos, rot, vel, ang);           // common.py:23-103
-    emit_task_obs<DEF>(row + SW, b, hi, hr, root_pos, pos, rot, vel, ang, r1);        // common.py:106-176
+    if constexpr (RESET) {
+      emit_self_obs<DEF>(row, p.of, b, root_pos, hi, hr, pos, rot, vel, ang);     // common.py:23-103
+      emit_task_obs<DEF>(row + SW, b, hi, hr, root_pos, pos, rot, vel, ang, r1);  // common.py:106-176
+    } else {
+      emit_obs_paired<DEF>(row, SW, p.of, b, root_pos, hi, hr, pos, rot, vel, ang, r1, p.one);  // common.py:23-176
+    }
   }
   if constexpr (RESET) {
     if (rst_mask) {  // the rows of the flagged envs, from their new state (one env at a time, the whole block on it)
@@ -3960,6 +4036,7 @@ static int step_fill_params(const PhcLib* lib, const PhcStepArgs* a, int64_t n, 
   p.advance = a->advance_progress;
   p.T = a->time_steps;
   p.dt = a->dt;
+  p.one = 1.0f;
   p.rwd = a->rwd;
   p.obs = a->obs_buf;
   p.obs_stride = a->obs_stride;

@@ -264,6 +264,120 @@ __device__ __forceinline__ float mean_sq3(Vec3 d) {
   return __fmaf_rn(d.z, d.z, __fmaf_rn(d.y, d.y, d.x * d.x)) * 0.333333343267440796f;
 }
 
+// ---- packed fp32x2 (sm_100: FFMA2 / FMUL2) -----------------------------------------------------------------------
+// Two independent evaluations of the same operation sequence in one instruction; each lane is rounded exactly as the
+// scalar instruction is, so lane k of every *x2 helper below equals the scalar helper it names, bit for bit.
+// ptxas fuses a packed multiply followed by a packed add into one FFMA2 even under -fmad=false (CUDA 12.9), which would
+// round a lerp once less than the reference.  So the packed add is an FMA by `one`, a 1.0f the compiler cannot see
+// (a kernel parameter): p * 1 is exact, so each lane is rn(p + q) for every input, ±0, subnormals, inf and NaN included,
+// and ptxas leaves the multiply that produced p alone.  Check new uses in SASS (profiles/sass_mix.py).
+struct Vec3x2 {
+  float2 x, y, z;
+};
+struct Quatx2 {
+  float2 x, y, z, w;
+};
+__device__ __forceinline__ float2 bc2(float a) { return make_float2(a, a); }
+__device__ __forceinline__ float2 neg2(float2 a) { return make_float2(-a.x, -a.y); }
+__device__ __forceinline__ float2 mul2(float2 a, float2 b) { return __fmul2_rn(a, b); }
+__device__ __forceinline__ float2 fma2(float2 a, float2 b, float2 c) { return __ffma2_rn(a, b, c); }
+__device__ __forceinline__ float2 add2(float2 a, float2 b, float one) { return __ffma2_rn(a, bc2(one), b); }
+// a - b as rn(b * -1 + a)
+__device__ __forceinline__ float2 sub2(float2 a, float2 b, float one) { return __ffma2_rn(b, bc2(-one), a); }
+
+__device__ __forceinline__ Vec3x2 pack3(Vec3 a, Vec3 b) { return {{a.x, b.x}, {a.y, b.y}, {a.z, b.z}}; }
+__device__ __forceinline__ Quatx2 pack4(Quat a, Quat b) { return {{a.x, b.x}, {a.y, b.y}, {a.z, b.z}, {a.w, b.w}}; }
+__device__ __forceinline__ Vec3 lane0(Vec3x2 v) { return {v.x.x, v.y.x, v.z.x}; }
+__device__ __forceinline__ Vec3 lane1(Vec3x2 v) { return {v.x.y, v.y.y, v.z.y}; }
+
+// lane k equals a - b (Vec3 operator-) bit for bit
+__device__ __forceinline__ Vec3x2 sub3x2(Vec3x2 a, Vec3x2 b, float one) {
+  return {sub2(a.x, b.x, one), sub2(a.y, b.y, one), sub2(a.z, b.z, one)};
+}
+// lane k equals lerp3 bit for bit
+__device__ __forceinline__ Vec3x2 lerp3x2(float2 om, float2 b, Vec3x2 x0, Vec3x2 x1, float one) {
+  return {add2(mul2(om, x0.x), mul2(b, x1.x), one), add2(mul2(om, x0.y), mul2(b, x1.y), one),
+          add2(mul2(om, x0.z), mul2(b, x1.z), one)};
+}
+// lane k equals sin_q1 bit for bit
+__device__ __forceinline__ float2 sin_q1x2(float2 x) {
+  const float2 u = mul2(x, x);
+  float2 q = fma2(u, bc2(2.6018724383902736e-06f), bc2(-0.00019807404896710068f));
+  q = fma2(q, u, bc2(0.008333024568855762f));
+  q = fma2(q, u, bc2(-0.16666656732559204f));
+  return fma2(mul2(x, u), q, x);
+}
+// lane k equals div_faithful bit for bit
+__device__ __forceinline__ float2 div_faithful2(float2 a, float2 b, float2 r) {
+  const float2 q = mul2(a, r);
+  return fma2(fma2(neg2(b), q, a), r, q);
+}
+// the per-lane part of quat_slerp: the sign fold, acos, the MUFU approximations and the select chain's inputs
+__device__ __forceinline__ void slerp_lane(float c, float& sg, float& ca, float& th, float& s, float& rs) {
+  sg = c < 0.0f ? -1.0f : 1.0f;
+  ca = fabsf(c);
+  th = acosf(ca);
+  s = sqrt_faithful(1.0f - ca * ca);
+  rs = rcp_approx(s);
+}
+__device__ __forceinline__ void slerp_select(float ca, float s, float sg, float& ra, float& rb) {
+  const bool avg = fabsf(s) < 0.001f;
+  ra = avg ? 0.5f : ra;
+  rb = avg ? 0.5f : rb;
+  const bool same = ca >= 1.0f;
+  ra = same ? 1.0f : ra;
+  rb = (same ? 0.0f : rb) * sg;
+}
+// (x, y) and (z, w) of a quaternion as they arrive from one 16-byte load: already register pairs
+__device__ __forceinline__ float2 qxy(Quat q) { return make_float2(q.x, q.y); }
+__device__ __forceinline__ float2 qzw(Quat q) { return make_float2(q.z, q.w); }
+// quat_slerp's c, ((x0x1 + y0y1) + z0z1) + w0w1, with the four products as two packed multiplies
+__device__ __forceinline__ float slerp_dot(Quat q0, Quat q1) {
+  const float2 xy = mul2(qxy(q0), qxy(q1)), zw = mul2(qzw(q0), qzw(q1));
+  return ((xy.x + xy.y) + zw.x) + zw.y;
+}
+// ra * q0 + rb * q1 componentwise, as quat_slerp's last line: __fmaf_rn(rb, q1.c, ra * q0.c)
+__device__ __forceinline__ Quat slerp_mix(Quat q0, Quat q1, float ra, float rb) {
+  const float2 xy = fma2(qxy(q1), bc2(rb), mul2(qxy(q0), bc2(ra)));
+  const float2 zw = fma2(qzw(q1), bc2(rb), mul2(qzw(q0), bc2(ra)));
+  return {xy.x, xy.y, zw.x, zw.y};
+}
+// Two slerps at once: out0 equals quat_slerp(a0, a1, t.x) and out1 quat_slerp(b0, b1, t.y), bit for bit.  The dot
+// products and the final mix pair the components of one quaternion; sin and the quotient pair the two slerps.
+__device__ __forceinline__ void quat_slerp_pair(Quat a0, Quat a1, Quat b0, Quat b1, float2 t, Quat& out0, Quat& out1) {
+  float2 sg, ca, th, s, rs;
+  slerp_lane(slerp_dot(a0, a1), sg.x, ca.x, th.x, s.x, rs.x);
+  slerp_lane(slerp_dot(b0, b1), sg.y, ca.y, th.y, s.y, rs.y);
+  const float2 om = {1.0f - t.x, 1.0f - t.y};
+  float2 ra = div_faithful2(sin_q1x2(mul2(om, th)), s, rs);
+  float2 rb = div_faithful2(sin_q1x2(mul2(t, th)), s, rs);
+  slerp_select(ca.x, s.x, sg.x, ra.x, rb.x);
+  slerp_select(ca.y, s.y, sg.y, ra.y, rb.y);
+  out0 = slerp_mix(a0, a1, ra.x, rb.x);
+  out1 = slerp_mix(b0, b1, ra.y, rb.y);
+}
+// lane k equals heading_mul_left(h, lane k of b) bit for bit (-(h.z * y) = (-h.z) * y exactly)
+__device__ __forceinline__ Quatx2 heading_mul_left2(Heading h, Quatx2 b) {
+  const float2 w = bc2(h.w), z = bc2(h.z), nz = bc2(-h.z);
+  return {fma2(b.x, w, mul2(b.y, nz)), fma2(b.y, w, mul2(b.x, z)), fma2(b.z, w, mul2(b.w, z)), fma2(b.w, w, mul2(b.z, nz))};
+}
+// lane k equals heading_rotate(c, lane k of v) bit for bit
+__device__ __forceinline__ Vec3x2 heading_rotate2(const HeadingRot& c, Vec3x2 v) {
+  return {fma2(v.x, bc2(c.a), mul2(v.y, bc2(-c.b))), fma2(v.y, bc2(c.a), mul2(v.x, bc2(c.b))), mul2(v.z, bc2(c.d))};
+}
+// lane k of out6[i] equals quat_tan_norm(lane k of q)[i] bit for bit
+__device__ __forceinline__ void quat_tan_norm2(Quatx2 q, float one, float2* out6) {
+  const float2 x2 = add2(q.x, q.x, one), y2 = add2(q.y, q.y, one), z2 = add2(q.z, q.z, one);
+  const float2 s = fma2(add2(q.w, q.w, one), q.w, bc2(-1.0f));
+  const float2 nw = neg2(q.w);
+  out6[0] = fma2(x2, q.x, s);
+  out6[1] = fma2(z2, q.w, mul2(y2, q.x));
+  out6[2] = fma2(z2, q.x, mul2(y2, nw));
+  out6[3] = fma2(y2, q.w, mul2(x2, q.z));
+  out6[4] = fma2(y2, q.z, mul2(x2, nw));
+  out6[5] = fma2(z2, q.z, s);
+}
+
 // ATen CPU sum over a contiguous row of n floats (aten/src/ATen/native/cpu/SumKernel.cpp, the AVX2 build that torch
 // dispatches to on AVX2 and AVX-512 hosts alike; checked against torch 2.11 for every n in 1..48, tests/test_oracle_c.py):
 //   n >= 8  vectorized_inner_sum: the n / 8 full vectors are added lane-wise in order (lane l = v[l] + v[l+8] + ..),
