@@ -17,7 +17,14 @@ from .common import (  # noqa: F401
     compute_imitation_reward,
 )
 from .env import HumanoidPHC, build_pd_action_offset_scale  # noqa: F401
-from .host_step import HostDeviceOutputs, HostEpisodeBuffers, HostResetBuffers, HostStep, HostStepBuffers  # noqa: F401
+from .host_step import (  # noqa: F401
+    HostAmpBuffers,
+    HostDeviceOutputs,
+    HostEpisodeBuffers,
+    HostResetBuffers,
+    HostStep,
+    HostStepBuffers,
+)
 from .motion_lib import MotionLib  # noqa: F401
 from .puffer_env import PHCPufferEnv  # noqa: F401
 from .running_norm import RunningNorm  # noqa: F401
@@ -40,4 +47,5 @@ __all__ = [
     "HostResetBuffers",
     "HostDeviceOutputs",
     "HostEpisodeBuffers",
+    "HostAmpBuffers",
 ]

@@ -303,6 +303,23 @@ class PhcHostEpisodeOut(C.Structure):
     ]
 
 
+class PhcHostAmp(C.Structure):
+    _fields_ = [
+        ("dof_pos", C.c_void_p),
+        ("dof_vel", C.c_void_p),
+        ("amp_obs", C.c_void_p),
+        ("amp_obs_demo", C.c_void_p),
+        ("num_steps", C.c_int32),
+        ("obs_per_step", C.c_int32),
+        ("key_body_ids", C.c_int32 * 8),
+        ("num_key_bodies", C.c_int32),
+        ("num_sel", C.c_int32),
+        ("dof_subset", C.c_void_p),
+        ("flags", C.c_uint32),
+        ("stream", C.c_void_p),
+    ]
+
+
 BUILD_FILTER_RADIUS = 8
 EPISODE_SUM_COLS = 12
 PEER_MAX_WORLD = 16
@@ -410,6 +427,16 @@ SIGNATURES = {
         C.c_int,
         [C.c_void_p, C.c_int32, C.POINTER(PhcHostStepArgs), C.POINTER(PhcHostResetArgs), C.POINTER(PhcHostDeviceOut),
          C.POINTER(PhcHostEnvArgs), C.POINTER(PhcHostEpisodeOut), C.c_int64],
+    ),  # fmt: skip
+    "phc_host_step_submit_amp": (
+        C.c_int,
+        [C.c_void_p, C.c_int32, C.POINTER(PhcHostStepArgs), C.POINTER(PhcHostResetArgs), C.POINTER(PhcHostDeviceOut),
+         C.POINTER(PhcHostEnvArgs), C.POINTER(PhcHostEpisodeOut), C.POINTER(PhcHostAmp), C.c_int64],
+    ),  # fmt: skip
+    "phc_host_reset_submit_amp": (
+        C.c_int,
+        [C.c_void_p, C.c_int32, C.POINTER(PhcHostStepArgs), C.POINTER(PhcHostResetArgs), C.POINTER(PhcHostDeviceOut),
+         C.POINTER(PhcHostEnvArgs), C.POINTER(PhcHostAmp), C.c_int64],
     ),  # fmt: skip
     "phc_host_step_set_initial_state": (
         C.c_int,

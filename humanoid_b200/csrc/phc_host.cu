@@ -46,6 +46,15 @@
 // buckets by the block's index in the batch (step_fused_mirrored's env0), so the sums do not depend on the chunk count.
 // The T = 1 kernel has the rewards and flags in registers; the kernels that run the bookkeeping after the step (generic,
 // T > 1) read them from device copies (the packed scalars), never from the mapped host buffers.
+//
+// AMP observations (PhcHostAmp).  phc_amp_step / phc_amp_init_ref, launched per chunk over the chunk's device copies
+// into the chunk's rows of the caller's tensors (they start at lo * S * P; chunks start on multiples of 8 envs, so the
+// roll's 16-B path stays aligned).  A step's chunk copies its dof rows into slot scratch with its other inbound rows
+// (measured on a B200, no slower than after the step); after the step kernel, the export and the staged D2H, so the
+// host-bound outputs do not wait behind them, the roll + slot 0 over every env,
+// and with auto-reset _init_amp_obs of the envs the step re-posed: masked by the step's own flags (reset_out in the
+// packed scalars; the kernel's reset_buf reads 0 after the in-step reset), their dof rows from the reset scratch, ids
+// and start times from the device clock the reset has rewritten.  A host reset runs _init_amp_obs of the masked envs.
 #include <chrono>
 #include <cstdint>
 #include <cstdio>
@@ -62,6 +71,7 @@
 int step_fused_mirrored(const PhcLib* lib, const PhcStepArgs* args, int64_t n, phc_stream_t stream,
                         int16_t* progress_mirror, int64_t env0, float* ep_raw);
 bool lib_has_dof_state(const PhcLib* lib);  // phc_kernels.cu
+extern "C" int amp_env_shape(const PhcAmpEnvArgs* a);  // phc_kernels.cu: phc_amp_step's shape rule
 namespace phc {
 int record_cuda_error(int cuda_error);  // phc_kernels.cu; returns PHC_ERR_CUDA
 }
@@ -223,6 +233,7 @@ struct Slot {
   cudaEvent_t done[kStreams] = {};  // recorded on each stream at the end of an enqueue
   cudaEvent_t dev_ready = nullptr;  // device-output submits: recorded on the caller's stream, waited on before a kernel
   cudaEvent_t ep_ready = nullptr;   // episode submits: the same, on the learner's stream (PhcHostEpisodeOut.stream)
+  cudaEvent_t amp_ready = nullptr;  // AMP submits: the same, on the discriminator's stream (PhcHostAmp.stream)
   // can the direct path be used: the 11 pointers of PhcHostStepArgs and PhcHostEnvArgs.mpjpe
   Seen<12> step_seen;
   // resets, allocated at the first submit that needs them: device root / dof rows of re-posed envs and the flags the
@@ -240,6 +251,10 @@ struct Slot {
   int64_t init_rows = -1;   // -1: no initial state
   Seen<3> env_seen;         // the env inputs last found to be host memory
   Seen<7> ep_seen;          // the episode tensors last found to be device memory on the context's device
+  // AMP, allocated at the first step that needs it: the chunk's dof position and velocity rows ([max_envs, 2, 69],
+  // laid out as d_dof)
+  float* d_amp = nullptr;
+  Seen<5> amp_seen;  // the AMP tensors last found on the context's device and the dof rows last found in host memory
   // the step in flight
   bool busy = false;
   int path = 0;  // 1 direct, 2 staged
@@ -317,6 +332,7 @@ static cudaError_t slot_alloc(const PhcHostStep* c, Slot& s) {
   }
   if (e == cudaSuccess) e = cudaEventCreateWithFlags(&s.dev_ready, cudaEventDisableTiming);
   if (e == cudaSuccess) e = cudaEventCreateWithFlags(&s.ep_ready, cudaEventDisableTiming);
+  if (e == cudaSuccess) e = cudaEventCreateWithFlags(&s.amp_ready, cudaEventDisableTiming);
   s.ready = e == cudaSuccess;
   return e;
 }
@@ -331,6 +347,7 @@ static void slot_free(Slot& s) {
   cudaFree(s.d_reset);
   cudaFree(s.d_dof);
   cudaFree(s.d_init);
+  cudaFree(s.d_amp);
   if (s.h_clock) cudaFreeHost(s.h_clock);
   if (s.h_out) cudaFreeHost(s.h_out);
   if (s.h_rows) cudaFreeHost(s.h_rows);
@@ -340,6 +357,7 @@ static void slot_free(Slot& s) {
   }
   if (s.dev_ready) cudaEventDestroy(s.dev_ready);
   if (s.ep_ready) cudaEventDestroy(s.ep_ready);
+  if (s.amp_ready) cudaEventDestroy(s.amp_ready);
   s = Slot{};
 }
 
@@ -446,6 +464,45 @@ static int check_episode(const PhcHostStep* c, Slot& s, const PhcHostEpisodeOut*
     s.ep_seen.keep(ptrs, 1);
   }
   if (ep->buckets < 1 || ep->buckets > 4096) return PHC_ERR_SHAPE;
+  return PHC_OK;
+}
+
+// The AMP fields of a submit as phc_amp_step takes them (chunk_amp_args fills the per-chunk pointers).
+static PhcAmpEnvArgs amp_env_args(const PhcHostAmp* a) {
+  PhcAmpEnvArgs x{};
+  x.body.num_bodies = PHC_NUM_BODIES;
+  x.dof_stride = kDof;
+  x.dof_elem_stride = 1;
+  for (int i = 0; i < 8; ++i) x.key_body_ids[i] = a->key_body_ids[i];
+  x.num_key_bodies = a->num_key_bodies;
+  x.num_sel = a->num_sel;
+  x.dof_subset = a->dof_subset;
+  x.flags = a->flags;
+  x.num_steps = a->num_steps;
+  x.obs_per_step = a->obs_per_step;
+  return x;
+}
+
+// What the AMP submits validate on top of the others.  step: the submit reads the dof rows (not a host reset); env:
+// its env options (the power reward's velocity rows); r: its reset args or NULL.  The verdict on the pointers is
+// cached per set of pointers.
+static int check_amp(const PhcHostStep* c, Slot& s, const PhcHostAmp* a, bool step, const PhcHostEnvArgs& env,
+                     const PhcHostResetArgs* r) {
+  if (!a->amp_obs || (step && (!a->dof_pos || (!a->dof_vel && !env.dof_vel)))) return PHC_ERR_NULL;
+  const PhcAmpEnvArgs x = amp_env_args(a);
+  if (const int rc = amp_env_shape(&x)) return rc;
+  if (step && a->dof_vel && env.dof_vel && a->dof_vel != env.dof_vel) return PHC_ERR_SHAPE;
+  const void* ptrs[5] = {a->amp_obs, a->amp_obs_demo, a->dof_subset, step ? a->dof_pos : nullptr,
+                         step ? a->dof_vel : nullptr};
+  if (!s.amp_seen.hit(ptrs)) {
+    for (int i = 0; i < 5; ++i) {
+      if (!ptrs[i]) continue;
+      const PtrKind k = classify(ptrs[i]);
+      if (i < 3 ? (k.mem != Mem::kDevice || k.device != c->device) : k.mem == Mem::kDevice) return PHC_ERR_UNSUPPORTED;
+    }
+    s.amp_seen.keep(ptrs, 1);
+  }
+  if (r && r->state_init >= PHC_STATE_INIT_DEFAULT) return PHC_ERR_UNSUPPORTED;
   return PHC_OK;
 }
 
@@ -612,6 +669,56 @@ static cudaError_t export_rows(const PhcHostStep* c, const PhcResetArgs& ra, con
   p.m = m;
   host_export_kernel<<<(unsigned)((m + kExportEnvs - 1) / kExportEnvs), kExportEnvs * 32, 0, st>>>(p);
   return cudaGetLastError();
+}
+
+// The AMP launch arguments of the chunk starting at env lo: its sim state rows, the given dof rows (dense, 69 per
+// env), its rows of the caller's tensors.
+static PhcAmpEnvArgs chunk_amp_args(const Slot& s, const PhcHostAmp* a, int64_t lo, const float* dofp,
+                                    const float* dofv) {
+  PhcAmpEnvArgs x = amp_env_args(a);
+  x.body = chunk_body(s.d_state + lo * kStateFloats);
+  x.dof_pos = dofp;
+  x.dof_vel = dofv;
+  const int64_t row = (int64_t)a->num_steps * a->obs_per_step;
+  x.amp_obs_buf = a->amp_obs + lo * row;
+  x.amp_obs_demo_buf = a->amp_obs_demo ? a->amp_obs_demo + lo * row : nullptr;
+  return x;
+}
+
+// _init_amp_obs of the chunk's envs whose `mask` byte is set, right after their reset: the new state in the chunk's
+// device rows, the new dof rows in the reset scratch, the ids and new start times in the device clock.
+static int amp_init_chunk(const PhcHostStep* c, Slot& s, const PhcHostAmp* a, const Layout& L, int64_t lo, int64_t m,
+                          const unsigned char* dc, const uint8_t* mask, cudaStream_t st) {
+  PhcAmpEnvArgs x = chunk_amp_args(s, a, lo, s.d_dofp + lo * kDof, s.d_dofv + lo * kDof);
+  x.env_mask = mask;
+  x.init_slot0 = 1;
+  return phc_amp_init_ref(c->lib, &x, (const int64_t*)(dc + L.ids), (const float*)(dc + L.start), c->dt, m, st);
+}
+
+// A step chunk's AMP inbound copies on `st`, with its other inbound rows: its dof position rows and, unless the power
+// reward already brings them (power_inputs), its dof velocity rows, straight from the caller's buffers into slot scratch.
+static cudaError_t amp_inbound(const Slot& s, const PhcHostAmp* a, int64_t lo, int64_t m, cudaStream_t st) {
+  float* dp = s.d_amp + lo * 2 * kDof;
+  float* dv = dp + m * kDof;
+  const size_t bytes = (size_t)m * kDof * sizeof(float);
+  cudaError_t e = cudaMemcpyAsync(dp, a->dof_pos + lo * kDof, bytes, cudaMemcpyHostToDevice, st);
+  if (e == cudaSuccess && !s.env.dof_vel) e = cudaMemcpyAsync(dv, a->dof_vel + lo * kDof, bytes, cudaMemcpyHostToDevice, st);
+  return e;
+}
+
+// The AMP launches of one step's chunk on `st`, enqueued after its host-bound traffic: the roll + slot 0 of every env
+// from the dof rows amp_inbound brought (the velocities from the power reward's copy when it has one), and with
+// auto-reset _init_amp_obs of the envs the step re-posed (its own flags, reset_out in dout).
+static int amp_step_chunk(const PhcHostStep* c, Slot& s, const PhcHostAmp* a, bool reset, const Layout& L, int64_t lo,
+                          int64_t m, const unsigned char* dc, const unsigned char* dout, cudaStream_t st) {
+  float* dp = s.d_amp + lo * 2 * kDof;
+  const float* vel = dp + m * kDof;
+  if (s.env.dof_vel) vel = s.d_dof + lo * 2 * kDof + m * kDof;  // power_inputs' copy
+  HOST_CUDA(s, cudaStreamWaitEvent(st, s.amp_ready, 0));
+  const PhcAmpEnvArgs x = chunk_amp_args(s, a, lo, dp, vel);
+  int rc = phc_amp_step(&x, m, 1, st);
+  if (rc == PHC_OK && reset) rc = amp_init_chunk(c, s, a, L, lo, m, dc, dout + L.reset, st);
+  return rc ? host_fail(s, rc, cudaSuccess) : PHC_OK;
 }
 
 // Chunk boundaries into s.bounds[0..s.nchunks].  Every boundary but n is a multiple of 8 envs, so the obs rows (fp32
@@ -782,9 +889,10 @@ static cudaError_t chunk_step_args(const PhcHostStep* c, const Slot& s, const Ph
 }
 
 // One step over the chunks of s.bounds: inbound copies (the clock first on the direct path, the sim state first on the
-// staged path), the fused step, the export of the re-posed envs' rows, and on the staged path the outbound copies.
+// staged path), the fused step, the export of the re-posed envs' rows, on the staged path the outbound copies, then the
+// AMP work.
 static int step_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, const PhcHostResetArgs* r,
-                        const PhcHostDeviceOut* dev, const PhcHostEpisodeOut* ep, bool staged) {
+                        const PhcHostDeviceOut* dev, const PhcHostEpisodeOut* ep, const PhcHostAmp* amp, bool staged) {
   const int64_t D = c->obs_dim;
   const Rows rows = r ? (s.rows_staged ? s.stage : caller_rows(a, r)) : Rows{};
   Trace trace(staged, s.streams[0]);
@@ -798,6 +906,7 @@ static int step_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, const
     unsigned char* dc = s.d_clock + coff;
     unsigned char* dout = s.d_out + ooff;
     HOST_CUDA(s, inbound(s, a, r, L, lo, m, coff, true, staged, st));
+    if (amp) HOST_CUDA(s, amp_inbound(s, amp, lo, m, st));
     PhcStepArgs k;
     PhcResetArgs ra;
     float* ep_raw;
@@ -828,6 +937,10 @@ static int step_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, const
       HOST_CUDA(s, cudaMemcpyAsync(s.h_out + ooff, dout, L.out_bytes, cudaMemcpyDeviceToHost, st));
       trace.stamp(ci, Trace::kD2H, st);
     }
+    if (amp) {
+      const int rc = amp_step_chunk(c, s, amp, r != nullptr, L, lo, m, dc, dout, st);
+      if (rc) return rc;
+    }
     coff += L.clock_bytes;
     ooff += L.out_bytes;
   }
@@ -842,9 +955,9 @@ static int step_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, const
 // over the chunks of s.bounds.  Nothing else is read or written: no sim state comes in (but for StateInit.Default /
 // Hybrid), no whole obs chunk goes out.  With device outputs the reset writes the masked envs' obs and normalised rows
 // straight into the caller's tensors and adds them to the moments (rows no step has counted, as HumanoidPHC.reset()
-// does); the export then carries no obs.
+// does); the export then carries no obs.  With AMP, _init_amp_obs of the masked envs follows on the chunk's stream.
 static int reset_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, const PhcHostResetArgs* r,
-                         const PhcHostDeviceOut* dev) {
+                         const PhcHostDeviceOut* dev, const PhcHostAmp* amp) {
   const Rows rows = s.rows_staged ? s.stage : caller_rows(a, r);
   // a default-path env keeps its rigid-body rows, and its observation is computed from them: the chunk's sim state
   // comes in (read before the export writes state_out, which may alias it)
@@ -877,6 +990,11 @@ static int reset_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, cons
     const int rc = phc_reset_envs(c->lib, &ra, m, st);
     if (rc) return host_fail(s, rc, cudaSuccess);
     HOST_CUDA(s, export_rows(c, ra, dc + L.mask, nullptr, dev ? nullptr : obs, out, 1, m, st));
+    if (amp) {
+      HOST_CUDA(s, cudaStreamWaitEvent(st, s.amp_ready, 0));
+      const int arc = amp_init_chunk(c, s, amp, L, lo, m, dc, dc + L.mask, st);
+      if (arc) return host_fail(s, arc, cudaSuccess);
+    }
     coff += L.clock_bytes;
   }
   return PHC_OK;
@@ -885,14 +1003,15 @@ static int reset_enqueue(PhcHostStep* c, Slot& s, const PhcHostStepArgs* a, cons
 // Enqueues one step (or reset) on a slot (arguments already checked) and marks it in flight.
 static int slot_enqueue(PhcHostStep* c, int slot, const PhcHostStepArgs* a, const PhcHostResetArgs* r, int op,
                         int64_t n, const PhcHostStep::Cand& k, const PhcHostDeviceOut* dev = nullptr,
-                        const PhcHostEpisodeOut* ep = nullptr) {
+                        const PhcHostEpisodeOut* ep = nullptr, const PhcHostAmp* amp = nullptr) {
   Slot& s = c->slots[slot];
   if (dev) HOST_CUDA(s, cudaEventRecord(s.dev_ready, dev->stream));
   if (ep) HOST_CUDA(s, cudaEventRecord(s.ep_ready, ep->stream));
+  if (amp) HOST_CUDA(s, cudaEventRecord(s.amp_ready, amp->stream));
   // s.env / s.extra were set by the submit (zero for phc_host_step)
   const bool staged = op != kReset && k.path == 2;
   partition(s, n, k.chunks, staged);
-  const int rc = op == kReset ? reset_enqueue(c, s, a, r, dev) : step_enqueue(c, s, a, r, dev, ep, staged);
+  const int rc = op == kReset ? reset_enqueue(c, s, a, r, dev, amp) : step_enqueue(c, s, a, r, dev, ep, amp, staged);
   if (rc) return rc;
   for (int i = 0; i < kStreams; ++i) HOST_CUDA(s, cudaEventRecord(s.done[i], s.streams[i]));
   s.args = *a;
@@ -1100,10 +1219,10 @@ int phc_host_step(PhcHostStep* c, const PhcHostStepArgs* a, int64_t n) {
 // The submits: every check before anything is enqueued, then the slot's buffers, then the enqueue.  dev: the device
 // tensors the rows go to, or NULL for host obs.  env: the env options, or NULL for none; a host reset takes only their
 // default_mask.  init_modes: StateInit.Default / Hybrid may be asked for (the _env submits; the others refuse them).
-// ep: the episode tensors of a step, or NULL.
+// ep: the episode tensors of a step, or NULL.  amp: the AMP tensors, or NULL.
 static int submit(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, const PhcHostResetArgs* r, int op, int64_t n,
                   const PhcHostDeviceOut* dev, const PhcHostEnvArgs* env, bool init_modes,
-                  const PhcHostEpisodeOut* ep = nullptr) {
+                  const PhcHostEpisodeOut* ep = nullptr, const PhcHostAmp* amp = nullptr) {
   if (!c || !a || (op != kStep && !r) || (dev && !dev->obs)) return PHC_ERR_NULL;
   if (ep && (!ep->terminals || !ep->truncations || !ep->masks || !ep->episode_returns || !ep->episode_lengths ||
              !ep->sums))
@@ -1121,6 +1240,7 @@ static int submit(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, const 
   if (op != kStep && (rc = check_reset(c, s, r, op, init_modes ? &ev : nullptr, n))) return rc;
   if (dev && (rc = check_dev(c, dev))) return rc;
   if (ep && (rc = check_episode(c, s, ep))) return rc;
+  if (amp && (rc = check_amp(c, s, amp, op != kReset, ev, r))) return rc;
   s.env = ev;
   s.extra.raw_cols = ev.dof_force ? 5 : 4;
   s.extra.mpjpe = ev.mpjpe != nullptr;
@@ -1136,11 +1256,13 @@ static int submit(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, const 
     e = reset_alloc(c, s, s.rows_staged);
   }
   if (e == cudaSuccess) e = env_alloc(c, s);
+  if (e == cudaSuccess && amp && op != kReset && !s.d_amp)
+    e = cudaMalloc((void**)&s.d_amp, (size_t)c->max_envs * 2 * kDof * sizeof(float));
   if (e != cudaSuccess) {
     (void)cudaGetLastError();
     return e == cudaErrorMemoryAllocation ? PHC_ERR_ALLOC : phc::record_cuda_error((int)e);
   }
-  return slot_enqueue(c, slot, a, r, op, n, untimed_schedule(c, s), dev, ep);
+  return slot_enqueue(c, slot, a, r, op, n, untimed_schedule(c, s), dev, ep, amp);
 }
 
 extern "C" {
@@ -1186,6 +1308,20 @@ int phc_host_step_submit_episode(PhcHostStep* c, int32_t slot, const PhcHostStep
                                  int64_t n) {
   if (!ep) return PHC_ERR_NULL;
   return submit(c, slot, a, r, r ? kStepReset : kStep, n, dev, env, true, ep);
+}
+
+int phc_host_step_submit_amp(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, const PhcHostResetArgs* r,
+                             const PhcHostDeviceOut* dev, const PhcHostEnvArgs* env, const PhcHostEpisodeOut* ep,
+                             const PhcHostAmp* amp, int64_t n) {
+  if (!amp) return PHC_ERR_NULL;
+  return submit(c, slot, a, r, r ? kStepReset : kStep, n, dev, env, true, ep, amp);
+}
+
+int phc_host_reset_submit_amp(PhcHostStep* c, int32_t slot, const PhcHostStepArgs* a, const PhcHostResetArgs* r,
+                              const PhcHostDeviceOut* dev, const PhcHostEnvArgs* env, const PhcHostAmp* amp,
+                              int64_t n) {
+  if (!amp) return PHC_ERR_NULL;
+  return submit(c, slot, a, r, kReset, n, dev, env, true, nullptr, amp);
 }
 
 int phc_host_step_set_initial_state(PhcHostStep* c, int32_t slot, const float* root_states, const float* dof_pos,

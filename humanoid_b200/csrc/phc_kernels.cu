@@ -4492,11 +4492,9 @@ int phc_episode_update(const PhcEpisodeArgs* a, int64_t n, phc_stream_t stream) 
   return launch_status();
 }
 
-static int amp_env_fill(const PhcAmpEnvArgs* a, int64_t n, AmpEnvParams& p) {
-  if (!a) return PHC_ERR_NULL;
-  if (n < 0) return PHC_ERR_SHAPE;
-  if (!a->amp_obs_buf || !a->body.pos.ptr || !a->body.rot.ptr || !a->body.vel.ptr || !a->body.ang_vel.ptr)
-    return PHC_ERR_NULL;
+// The shape rule of the AMP buffers: S, P against the flags / key bodies / dof subset, key body ids.  Also what
+// phc_host.cu checks before it enqueues anything.
+int amp_env_shape(const PhcAmpEnvArgs* a) {
   if (a->num_sel < 0 || a->num_sel % 3 != 0 || a->num_sel > 96 || a->num_key_bodies < 0 || a->num_key_bodies > 8 ||
       a->num_steps < 1 || a->num_steps > AMP_MAX_STEPS)
     return PHC_ERR_SHAPE;
@@ -4504,6 +4502,15 @@ static int amp_env_fill(const PhcAmpEnvArgs* a, int64_t n, AmpEnvParams& p) {
   if (a->obs_per_step != width) return PHC_ERR_SHAPE;
   for (int i = 0; i < a->num_key_bodies; ++i)
     if (a->key_body_ids[i] < 0 || a->key_body_ids[i] >= a->body.num_bodies) return PHC_ERR_SHAPE;
+  return PHC_OK;
+}
+
+static int amp_env_fill(const PhcAmpEnvArgs* a, int64_t n, AmpEnvParams& p) {
+  if (!a) return PHC_ERR_NULL;
+  if (n < 0) return PHC_ERR_SHAPE;
+  if (!a->amp_obs_buf || !a->body.pos.ptr || !a->body.rot.ptr || !a->body.vel.ptr || !a->body.ang_vel.ptr)
+    return PHC_ERR_NULL;
+  if (const int rc = amp_env_shape(a)) return rc;
   p.body = a->body;
   p.dof_pos = a->dof_pos;
   p.dof_vel = a->dof_vel;

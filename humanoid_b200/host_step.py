@@ -28,6 +28,11 @@ With ``episode=HostEpisodeBuffers`` a step also does the per-step bookkeeping of
 CUDA tensors, where the learner's experience buffer reads them, with no copy back to the device and no extra launch by
 the caller.  A loop over two batches on two slots logs both with ``HostEpisodeBuffers.log([ep0, ep1], log_interval)``.
 
+With ``amp=HostAmpBuffers`` (``HostStepBuffers.allocate(..., amp=True)`` for the physics' dof rows) a step also does
+``HumanoidPHC.step()``'s AMP work (``phc_host_step_submit_amp``): the history roll and the current AMP observation of
+every env, and with auto-reset ``_init_amp_obs`` of the envs it re-posed, into the discriminator's CUDA tensors; a host
+reset with ``amp`` initialises the masked envs' AMP rows, as ``HumanoidPHC.reset()`` does.
+
 Pinned buffers (``HostStepBuffers.allocate(..., pinned=True)``) take the fast paths; pageable ones work through
 staging.  The CUDA device of the motion library must be current when the context is created and stepped; after
 ``MotionLib.repack()`` synchronise the device before the next host step (the steps run on the context's own streams).
@@ -42,7 +47,8 @@ from typing import Any, List, Optional, Sequence, Union
 import torch
 
 from . import _cabi
-from .env import DEFAULT_REWARD
+from .common import dof_subset_smpl
+from .env import BODY_NAMES, DEFAULT_REWARD, KEY_BODIES
 from .puffer_env import episode_info
 
 _FIELDS = (  # name, dtype, trailing shape (T: the number of future steps of the task obs)
@@ -75,7 +81,9 @@ class HostStepBuffers:
     with the power reward, its term in column 4), ``reset_buf`` / ``terminate_buf`` uint8.
 
     Env options (attributes, not constructor arguments), None when off: ``dof_force`` / ``dof_vel`` [n, 69] f32 (inputs of the power reward: the physics'
-    dof force and the velocity half of its dof state), ``mpjpe`` [n] f32 (output, eval mode's ``extras["mpjpe"]``)."""
+    dof force and the velocity half of its dof state), ``mpjpe`` [n] f32 (output, eval mode's ``extras["mpjpe"]``),
+    ``dof_pos`` [n, 69] f32 (input of the AMP observations: the position half of the physics' dof state; with AMP
+    ``dof_vel`` is required too, shared with the power reward)."""
 
     state: torch.Tensor
     progress_buf: torch.Tensor
@@ -92,13 +100,15 @@ class HostStepBuffers:
     dof_force = None
     dof_vel = None
     mpjpe = None
+    dof_pos = None
 
     @classmethod
     def allocate(cls, n: int, time_steps: int = 1, pinned: bool = True, host_obs: bool = True, power: bool = False,
-                 mpjpe: bool = False) -> "HostStepBuffers":  # fmt: skip
+                 mpjpe: bool = False, amp: bool = False) -> "HostStepBuffers":  # fmt: skip
         """Zeroed buffers for ``n`` envs; ``pinned`` page-locks them (needs the CUDA driver).  ``host_obs=False``
         leaves ``obs_buf`` None, for steps whose rows go to a ``HostDeviceOutputs``.  ``power`` adds ``dof_force`` /
-        ``dof_vel`` and makes ``reward_raw`` [n, 5]; ``mpjpe`` adds ``mpjpe``."""
+        ``dof_vel`` and makes ``reward_raw`` [n, 5]; ``mpjpe`` adds ``mpjpe``; ``amp`` adds ``dof_pos`` (and ``dof_vel``
+        when ``power`` does not)."""
 
         def make(dtype, trailing):
             t = torch.zeros((n, *trailing), dtype=dtype)
@@ -111,25 +121,35 @@ class HostStepBuffers:
             b.dof_force, b.dof_vel = make(torch.float32, (_DOF,)), make(torch.float32, (_DOF,))
         if mpjpe:
             b.mpjpe = make(torch.float32, ())
+        if amp:
+            b.dof_pos = make(torch.float32, (_DOF,))
+            if b.dof_vel is None:
+                b.dof_vel = make(torch.float32, (_DOF,))
         return b
 
     @property
     def n(self) -> int:
         return int(self.state.shape[0])
 
-    def validate(self, time_steps: int = 1, device_out: bool = False, power: bool = False) -> int:
+    def validate(self, time_steps: int = 1, device_out: bool = False, power: bool = False, amp: bool = False) -> int:
         """Checks device (CPU), dtype, shape and contiguity of every tensor; returns ``n``.  ``obs_buf`` must be None
         when the rows go to device outputs (``device_out``), and a tensor otherwise.  ``power``: the step has the power
-        reward, so ``dof_force`` / ``dof_vel`` are required and ``reward_raw`` is [n, 5]; without it they must be None."""
+        reward, so ``dof_force`` / ``dof_vel`` are required and ``reward_raw`` is [n, 5]; without it they must be None
+        (but ``dof_vel`` of buffers with AMP's ``dof_pos``).  ``amp``: the step has AMP observations, so ``dof_pos`` /
+        ``dof_vel`` are required."""
         n = self.n
         if device_out and self.obs_buf is not None:
             raise _cabi.PhcError("obs_buf must be None when the rows go to device outputs")
-        if not power and (self.dof_force is not None or self.dof_vel is not None):
+        if not power and (self.dof_force is not None or (self.dof_vel is not None and self.dof_pos is None and not amp)):
             raise _cabi.PhcError("dof_force / dof_vel are given but the step has no power reward (use_power_reward)")
         checks = [(name, dtype, shape(time_steps)) for name, dtype, shape in _FIELDS]
         if power:
             checks[_NAMES.index("reward_raw")] = ("reward_raw", torch.float32, (5,))
-            checks += [("dof_force", torch.float32, (_DOF,)), ("dof_vel", torch.float32, (_DOF,))]
+            checks += [("dof_force", torch.float32, (_DOF,))]
+        if power or amp:
+            checks.append(("dof_vel", torch.float32, (_DOF,)))
+        if amp:
+            checks.append(("dof_pos", torch.float32, (_DOF,)))
         if self.mpjpe is not None:
             checks.append(("mpjpe", torch.float32, ()))
         for name, dtype, shape in checks:
@@ -138,6 +158,8 @@ class HostStepBuffers:
                 continue
             if power and t is None and name in ("dof_force", "dof_vel"):
                 raise _cabi.PhcError(f"the power reward needs {name} (HostStepBuffers.allocate(..., power=True))")
+            if amp and t is None and name in ("dof_pos", "dof_vel"):
+                raise _cabi.PhcError(f"the AMP observations need {name} (HostStepBuffers.allocate(..., amp=True))")
             if not isinstance(t, torch.Tensor) or t.device.type != "cpu":
                 raise _cabi.PhcError(f"{name} must be a CPU tensor (the host step takes host buffers)")
             if t.dtype != dtype:
@@ -444,6 +466,103 @@ class HostEpisodeBuffers:
         return [episode_info(stats, raw, log_interval)[0]]
 
 
+# what HumanoidPHC's AMP observation uses (humanoid_phc.py:186-194, 245, 1206-1211): the key bodies, the dof subset
+# without hands and toes, the config's flags; P = root height 1 + root 12 + 9 per selected joint + 3 per key body
+_AMP_KEY_IDS = [BODY_NAMES.index(name) for name in KEY_BODIES]
+_AMP_FLAGS = _cabi.OBS_LOCAL_ROOT | _cabi.OBS_ROOT_HEIGHT | _cabi.OBS_UPRIGHT
+_AMP_NUM_SEL = int(dof_subset_smpl("meta").shape[0])
+AMP_OBS_PER_STEP = 1 + 12 + 3 * _AMP_NUM_SEL + 3 * len(KEY_BODIES)
+AMP_MAX_STEPS = 16
+
+
+@dataclass(eq=False)
+class HostAmpBuffers:
+    """The CUDA tensors of ``HumanoidPHC``'s AMP observations for one batch of ``n`` envs (``amp`` of
+    ``HostStep.submit`` / ``step`` / ``reset_submit`` / ``reset``).  ``amp_obs`` f32 [n, S, P] in / out: slot 0 is the
+    current AMP observation, slots 1.. the history (``_amp_obs_buf``).  ``amp_obs_demo`` f32 [n, S, P] (optional): the
+    rows of the envs last re-posed (``_amp_obs_demo_buf``).  ``obs`` / ``demo`` are the [n, S P] views
+    ``HumanoidPHC.amp_obs`` / ``fetch_amp_obs_demo()`` return."""
+
+    amp_obs: torch.Tensor
+    amp_obs_demo: Optional[torch.Tensor] = None
+    dof_subset: Optional[torch.Tensor] = None  # int64 [57] on the tensors' device (dof_subset_smpl), set by allocate
+
+    @classmethod
+    def allocate(cls, n: int, num_steps: int = 10, device=None, demo: bool = True) -> "HostAmpBuffers":
+        """Zeroed tensors for ``n`` envs and ``num_steps`` (``num_amp_obs_steps``, config.py:141) on ``device``
+        (default: the current CUDA device), as ``HumanoidPHC(use_amp_obs=True)`` starts; ``demo`` adds
+        ``amp_obs_demo``."""
+        device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+        shape = (n, int(num_steps), AMP_OBS_PER_STEP)
+        return cls(
+            amp_obs=torch.zeros(shape, dtype=torch.float32, device=device),
+            amp_obs_demo=torch.zeros(shape, dtype=torch.float32, device=device) if demo else None,
+            dof_subset=dof_subset_smpl(device),
+        )  # fmt: skip
+
+    @property
+    def n(self) -> int:
+        return int(self.amp_obs.shape[0])
+
+    @property
+    def num_steps(self) -> int:
+        return int(self.amp_obs.shape[1])
+
+    @property
+    def obs(self) -> torch.Tensor:
+        return self.amp_obs.view(self.n, -1)
+
+    @property
+    def demo(self) -> Optional[torch.Tensor]:
+        return None if self.amp_obs_demo is None else self.amp_obs_demo.view(self.n, -1)
+
+    def validate(self, n: int) -> None:
+        """Checks dtype, shape ([n, S, P] with 1 <= S <= 16 and P the AMP observation's width), contiguity and that
+        every tensor lives on one CUDA device."""
+        a = self.amp_obs
+        S = int(a.shape[1]) if isinstance(a, torch.Tensor) and a.dim() == 3 else -1
+        if not 1 <= S <= AMP_MAX_STEPS:
+            raise ValueError(f"amp_obs must be [n, S, {AMP_OBS_PER_STEP}] with 1 <= S <= {AMP_MAX_STEPS}")
+        checks = [("amp_obs", a, torch.float32, (n, S, AMP_OBS_PER_STEP))]
+        if self.amp_obs_demo is not None:
+            checks.append(("amp_obs_demo", self.amp_obs_demo, torch.float32, (n, S, AMP_OBS_PER_STEP)))
+        if self.dof_subset is not None:
+            checks.append(("dof_subset", self.dof_subset, torch.int64, (_AMP_NUM_SEL,)))
+        dev = a.device
+        for name, t, dtype, shape in checks:
+            if not isinstance(t, torch.Tensor) or t.device.type != "cuda" or t.device != dev:
+                raise _cabi.PhcError(f"{name} must be a CUDA tensor on the device of amp_obs")
+            if t.dtype != dtype:
+                raise _cabi.PhcError(f"{name} must be {dtype}, got {t.dtype}")
+            if tuple(t.shape) != shape:
+                raise ValueError(f"{name} has shape {tuple(t.shape)}, expected {shape}")
+            if not t.is_contiguous():
+                raise _cabi.PhcError(f"{name} must be contiguous")
+
+    def _args(self, bufs: Optional["HostStepBuffers"]) -> _cabi.PhcHostAmp:
+        """``bufs``: the step's buffers, whose ``dof_pos`` / ``dof_vel`` are read (None for a host reset)."""
+        if self.dof_subset is None:
+            self.dof_subset = dof_subset_smpl(self.amp_obs.device)
+        a = _cabi.PhcHostAmp()
+        if bufs is not None:
+            a.dof_pos, a.dof_vel = _cabi.ptr(bufs.dof_pos), _cabi.ptr(bufs.dof_vel)
+        a.amp_obs, a.amp_obs_demo = self.amp_obs.data_ptr(), _cabi.ptr(self.amp_obs_demo)
+        a.num_steps, a.obs_per_step = self.num_steps, AMP_OBS_PER_STEP
+        for i, b in enumerate(_AMP_KEY_IDS):
+            a.key_body_ids[i] = b
+        a.num_key_bodies = len(_AMP_KEY_IDS)
+        a.num_sel, a.dof_subset = _AMP_NUM_SEL, self.dof_subset.data_ptr()
+        a.flags = _AMP_FLAGS
+        a.stream = _cabi.stream_ptr(self.amp_obs.device)
+        return a
+
+
+def _refuse_amp_state_init(amp, reset, state_init: str) -> None:
+    """The reference raises for StateInit.Default / Hybrid with AMP (humanoid_phc.py:795-797), as HumanoidPHC does."""
+    if amp is not None and reset is not None and state_init in ("default", "hybrid"):
+        raise NotImplementedError("Not tested yet")
+
+
 class HostStep:
     """A ``phc_host_step`` context on the current CUDA device for batches of up to ``max_envs`` envs.
 
@@ -477,6 +596,7 @@ class HostStep:
         self._inflight_reset: List[Optional[HostResetBuffers]] = [None] * _cabi.HOST_SLOTS
         self._inflight_dev: List[Optional[HostDeviceOutputs]] = [None] * _cabi.HOST_SLOTS
         self._inflight_ep: List[Optional[HostEpisodeBuffers]] = [None] * _cabi.HOST_SLOTS
+        self._inflight_amp: List[Optional[HostAmpBuffers]] = [None] * _cabi.HOST_SLOTS
         self.time_steps = int(time_steps)
         self._capi = _cabi.load()
         term = torch.as_tensor(termination_distances, dtype=torch.float32).cpu().expand(_cabi.NUM_BODIES)
@@ -500,13 +620,13 @@ class HostStep:
 
     def step(self, bufs: HostStepBuffers, reset: Optional[HostResetBuffers] = None, state_init: str = "random",
              flag_test: bool = False, device_out: Optional[HostDeviceOutputs] = None,
-             episode: Optional[HostEpisodeBuffers] = None) -> HostStepBuffers:  # fmt: skip
+             episode: Optional[HostEpisodeBuffers] = None, amp: Optional[HostAmpBuffers] = None) -> HostStepBuffers:  # fmt: skip
         """One step of ``bufs``; returns when every output is in ``bufs`` (``progress_buf`` advanced in place), in
-        ``device_out`` and in ``episode``.  With ``reset`` the envs the step flags are re-posed as well (see
-        ``submit``); with ``reset``, ``device_out`` or ``episode`` this runs on slot 0."""
-        if (reset is not None or device_out is not None or episode is not None or self.use_power_reward
-                or bufs.mpjpe is not None):  # fmt: skip
-            self.submit(0, bufs, reset, state_init, flag_test, device_out=device_out, episode=episode)
+        ``device_out``, in ``episode`` and in ``amp``.  With ``reset`` the envs the step flags are re-posed as well (see
+        ``submit``); with ``reset``, ``device_out``, ``episode`` or ``amp`` this runs on slot 0."""
+        if (reset is not None or device_out is not None or episode is not None or amp is not None
+                or self.use_power_reward or bufs.mpjpe is not None):  # fmt: skip
+            self.submit(0, bufs, reset, state_init, flag_test, device_out=device_out, episode=episode, amp=amp)
             return self.wait(0)
         n = bufs.validate(self.time_steps)
         args = bufs._args()
@@ -515,7 +635,7 @@ class HostStep:
 
     def submit(self, slot: int, bufs: HostStepBuffers, reset: Optional[HostResetBuffers] = None,
                state_init: str = "random", flag_test: bool = False, device_out: Optional[HostDeviceOutputs] = None,
-               episode: Optional[HostEpisodeBuffers] = None) -> None:  # fmt: skip
+               episode: Optional[HostEpisodeBuffers] = None, amp: Optional[HostAmpBuffers] = None) -> None:  # fmt: skip
         """Enqueue one step of ``bufs`` on ``slot`` (0 or 1) and return.  ``bufs`` (and ``reset``) belong to the library
         until ``wait(slot)`` returns: do not read or write them before then.
 
@@ -537,8 +657,16 @@ class HostStep:
         With ``episode`` the step also does ``PHCPufferEnv.step``'s bookkeeping into its CUDA tensors
         (``phc_host_step_submit_episode``), from the step's own flags (with ``reset``: those before the reset); the
         kernels writing them wait for the work enqueued so far on the current CUDA stream.  The tensors belong to the
-        library until ``wait(slot)`` returns; then they are complete."""
-        n = bufs.validate(self.time_steps, device_out=device_out is not None, power=self.use_power_reward)
+        library until ``wait(slot)`` returns; then they are complete.
+
+        With ``amp`` the step also does ``HumanoidPHC.step()``'s AMP work into ``amp``'s tensors
+        (``phc_host_step_submit_amp``): the history roll and slot 0 of every env from the post-physics state and
+        ``bufs.dof_pos`` / ``dof_vel``, and with ``reset`` ``_init_amp_obs`` of the envs the step re-posed (their
+        ``amp_obs_demo`` rows too).  The kernels writing them wait for the work enqueued so far on the current CUDA
+        stream.  State init "default" / "hybrid" raise ``NotImplementedError`` with AMP, as in ``HumanoidPHC``."""
+        _refuse_amp_state_init(amp, reset, state_init)
+        n = bufs.validate(self.time_steps, device_out=device_out is not None, power=self.use_power_reward,
+                          amp=amp is not None)  # fmt: skip
         env = self._env_args(slot, bufs, reset, state_init, n)
         rargs = None
         if reset is not None:
@@ -550,23 +678,33 @@ class HostStep:
             if device_out is not None and device_out.obs.device != episode.terminals.device:
                 raise _cabi.PhcError("episode and device_out must live on one CUDA device")
             name = "phc_host_step_submit_episode"
+        if amp is not None:
+            amp.validate(n)
+            name = "phc_host_step_submit_amp"
         # an auto-reset replaces counted rows and adds none
-        self._submit(name, slot, bufs, reset, rargs, device_out, env, n, lambda: n, episode)
+        self._submit(name, slot, bufs, reset, rargs, device_out, env, n, lambda: n, episode, amp)
 
-    def _submit(self, name, slot, bufs, reset, rargs, device_out, env, n, new_rows, episode=None):
+    def _submit(self, name, slot, bufs, reset, rargs, device_out, env, n, new_rows, episode=None, amp=None):
         """The C call of ``submit`` / ``reset_submit``; ``new_rows()``: the rows it adds to ``device_out``'s moments;
-        ``episode``: the bookkeeping tensors of ``phc_host_step_submit_episode``."""
+        ``episode``: the bookkeeping tensors of ``phc_host_step_submit_episode`` (and ``_amp``); ``amp``: the AMP
+        tensors of ``phc_host_step_submit_amp`` / ``phc_host_reset_submit_amp``."""
         dargs = None
         if device_out is not None:
             device_out.validate(n, self.time_steps)
             dargs = C.byref(device_out._args())
         fn = getattr(self._capi, name)
         eargs = None if env is None else C.byref(env)
-        args = (C.byref(bufs._args()), rargs, dargs, eargs) + (() if episode is None else (C.byref(episode._args()),))
+        args = (C.byref(bufs._args()), rargs, dargs, eargs)
+        if name == "phc_host_step_submit_amp":
+            args += (None if episode is None else C.byref(episode._args()),)
+        elif episode is not None:
+            args += (C.byref(episode._args()),)
+        if amp is not None:
+            args += (C.byref(amp._args(bufs if name == "phc_host_step_submit_amp" else None)),)
         _cabi.check(fn(self._live(), int(slot), *args, n), name)
         if device_out is not None and device_out.obs_moments is not None:
             device_out.rows += new_rows()
-        self._hold(slot, bufs, reset, device_out, episode)
+        self._hold(slot, bufs, reset, device_out, episode, amp)
 
     def _env_args(self, slot, bufs: HostStepBuffers, reset: Optional[HostResetBuffers], state_init: str,
                   n: int, step: bool = True) -> Optional[_cabi.PhcHostEnvArgs]:  # fmt: skip
@@ -614,34 +752,44 @@ class HostStep:
                     "phc_host_step_set_initial_state")  # fmt: skip
         self._initial_rows[slot] = n
 
-    def _hold(self, slot, bufs, reset, device_out, episode=None):
+    def _hold(self, slot, bufs, reset, device_out, episode=None, amp=None):
         """Keep a batch's tensors alive until its ``wait``."""
         self._inflight[slot] = bufs
         self._inflight_reset[slot] = reset
         self._inflight_dev[slot] = device_out
         self._inflight_ep[slot] = episode
+        self._inflight_amp[slot] = amp
 
     def reset_submit(self, slot: int, bufs: HostStepBuffers, reset: HostResetBuffers, state_init: str = "random",
-                     flag_test: bool = False, device_out: Optional[HostDeviceOutputs] = None) -> None:  # fmt: skip
+                     flag_test: bool = False, device_out: Optional[HostDeviceOutputs] = None,
+                     amp: Optional[HostAmpBuffers] = None) -> None:  # fmt: skip
         """Enqueue ``HumanoidPHC.reset(env_ids, phase)`` for the envs of ``reset.env_mask`` on ``slot`` and return:
         reads the clock and ids of ``bufs``; after ``wait``, for the masked envs only, ``obs_buf`` rows, ``state``,
         the clock, ``progress_buf`` = 0, ``reset_buf`` = ``terminate_buf`` = 0 and ``reset``'s root / dof rows hold
         the re-posed envs.  How a host loop gets its first observation.  With ``device_out`` the masked envs' rows go
         to ``device_out.obs`` / ``obs_norm`` and are added to ``obs_moments`` (rows no step has counted).  State init
-        "default" / "hybrid" as in ``submit`` (``phc_host_reset_submit_env``); the power inputs are not read."""
+        "default" / "hybrid" as in ``submit`` (``phc_host_reset_submit_env``); the power inputs are not read.  With
+        ``amp``, ``_init_amp_obs`` of the masked envs into ``amp``'s tensors (``phc_host_reset_submit_amp``): how an
+        AMP loop gets its first observation; the dof rows are not read."""
+        _refuse_amp_state_init(amp, reset, state_init)
         n = bufs.validate(self.time_steps, device_out=device_out is not None, power=self.use_power_reward)
         reset.validate(n)
         if reset.env_mask is None:
             raise ValueError("reset_submit needs reset.env_mask")
         rargs = C.byref(reset._args(bufs, state_init, flag_test))
         env = self._env_args(slot, bufs, reset, state_init, n, step=False)
-        self._submit("phc_host_reset_submit_env", slot, bufs, reset, rargs, device_out, env, n,
-                     lambda: int(reset.env_mask.count_nonzero()))  # fmt: skip
+        name = "phc_host_reset_submit_env"
+        if amp is not None:
+            amp.validate(n)
+            name = "phc_host_reset_submit_amp"
+        self._submit(name, slot, bufs, reset, rargs, device_out, env, n,
+                     lambda: int(reset.env_mask.count_nonzero()), amp=amp)  # fmt: skip
 
     def reset(self, bufs: HostStepBuffers, reset: HostResetBuffers, state_init: str = "random",
-              flag_test: bool = False, device_out: Optional[HostDeviceOutputs] = None) -> HostStepBuffers:  # fmt: skip
+              flag_test: bool = False, device_out: Optional[HostDeviceOutputs] = None,
+              amp: Optional[HostAmpBuffers] = None) -> HostStepBuffers:  # fmt: skip
         """``reset_submit`` on slot 0 + ``wait(0)``."""
-        self.reset_submit(0, bufs, reset, state_init, flag_test, device_out)
+        self.reset_submit(0, bufs, reset, state_init, flag_test, device_out, amp)
         return self.wait(0)
 
     def wait(self, slot: int) -> Optional[HostStepBuffers]:
@@ -672,6 +820,7 @@ class HostStep:
         self._inflight_reset = [None] * _cabi.HOST_SLOTS
         self._inflight_dev = [None] * _cabi.HOST_SLOTS
         self._inflight_ep = [None] * _cabi.HOST_SLOTS
+        self._inflight_amp = [None] * _cabi.HOST_SLOTS
 
     def __enter__(self) -> "HostStep":
         return self

@@ -694,6 +694,64 @@ PHC_API int phc_host_step_submit_episode(PhcHostStep* ctx, int32_t slot, const P
                                          const PhcHostEnvArgs* env /* may be NULL */, const PhcHostEpisodeOut* ep,
                                          int64_t n);
 
+/* AMP observations on the host-buffer path: HumanoidPHC.step()'s AMP work (humanoid_phc.py:153-157) and the reset's
+ * _init_amp_obs (:675-676, :791-819) done by the host step itself into the discriminator's device tensors, over the
+ * slot's device copies of the state, so a CPU-physics caller uploads nothing twice.  Added without a change to any
+ * existing struct or entry point, so PHC_ABI_VERSION stays 6; a caller finds these by their symbols.  The kernels are
+ * phc_amp_step's and phc_amp_init_ref's (their header block documents the rows), launched per chunk.
+ *
+ *   phc_host_step_submit_amp   phc_host_step_submit_episode (ep != NULL) or phc_host_step_submit_env (ep == NULL), plus:
+ *            the history roll and slot 0 from the post-physics state for every env (phc_amp_step with roll_history),
+ *            its dof rows from amp->dof_pos and amp->dof_vel (or env->dof_vel: the reference reads one _dof_vel).  With
+ *            auto-reset, then _init_amp_obs for the envs the step re-posed (its own reset flags): slot 0 from their new
+ *            state and dof rows, slots k >= 1 from the library at the new start time - k*dt, and their demo rows
+ *            (phc_amp_init_ref with init_slot0).  amp_obs_demo rows of other envs are not touched.
+ *   phc_host_reset_submit_amp  phc_host_reset_submit_env, plus _init_amp_obs(env_ids) for the masked envs only: how an
+ *            AMP host loop gets its first observation.  amp->dof_pos / dof_vel are not read (the reset writes the new
+ *            dof rows itself).
+ *   buffers  amp_obs [n, S, P] (slot 0 = _curr_amp_obs_buf, 1.. = _hist_amp_obs_buf) and amp_obs_demo [n, S, P], dense
+ *            fp32 device tensors on the context's device; dof_pos / dof_vel dense host [n, 69] (pin them for speed).  Each
+ *            chunk's dof rows are copied by the copy engine straight from these buffers into the slot's device scratch,
+ *            with its other inbound rows: 552 B per env inbound, 276 B when the power reward already carries the
+ *            velocities.  The AMP launches follow the chunk's host-bound outputs.  phc_host_step_h2d_bytes keeps describing the plain step.  Nothing AMP writes crosses the
+ *            link, so the direct and staged paths do the same AMP work.
+ *   ordering A submit records an event on amp->stream; each of the slot's streams waits for it before its first write
+ *            into these tensors (the roll reads and rewrites the whole history, so the discriminator may still be
+ *            reading the previous rows when the next submit is issued).  When phc_host_step_wait returns, they are
+ *            complete; work enqueued afterwards on any stream sees them.  The tensors and dof rows belong to the library
+ *            until then.
+ *   validation  Before anything is enqueued, on top of the checks of the matching submit: amp, amp_obs, dof_pos of a
+ *            step, or a step without velocity rows (neither amp->dof_vel nor env->dof_vel) -> PHC_ERR_NULL; num_steps
+ *            outside 1..16, obs_per_step that does not match flags / num_key_bodies / num_sel (phc_amp_step's rule), a
+ *            key body id outside 0..23, or amp->dof_vel and env->dof_vel both given but different -> PHC_ERR_SHAPE;
+ *            amp_obs, amp_obs_demo or dof_subset not device memory on the context's device, a dof row pointer that is
+ *            not host memory, or PHC_STATE_INIT_DEFAULT / HYBRID (the reference raises NotImplementedError there,
+ *            :795-797) -> PHC_ERR_UNSUPPORTED; a busy slot -> PHC_ERR_BUSY.  After any error the slot is idle and
+ *            nothing has been written.
+ *   schedule Not timed by the tuner; the settled schedule, as the other submits. */
+typedef struct PhcHostAmp {
+  const float* dof_pos;        /* host [n,69] dense: the physics' dof positions (step only)      humanoid_phc.py:535 */
+  const float* dof_vel;        /* host [n,69] dense, or NULL when env->dof_vel is given (step only)             :536 */
+  float* amp_obs;              /* device [n, S, P] in / out: _amp_obs_buf                                       :596 */
+  float* amp_obs_demo;         /* device [n, S, P] out, or NULL: _amp_obs_demo_buf                              :611 */
+  int32_t num_steps;           /* S, 1 .. 16                                                       config.py:141 */
+  int32_t obs_per_step;        /* P, as PhcAmpEnvArgs                                                            */
+  int32_t key_body_ids[8];     /* as PhcAmpEnvArgs                                                               */
+  int32_t num_key_bodies;
+  int32_t num_sel;             /* dofs used (69 when dof_subset is NULL), a multiple of 3                        */
+  const int64_t* dof_subset;   /* device [num_sel] or NULL                                                       */
+  uint32_t flags;              /* PHC_OBS_LOCAL_ROOT | PHC_OBS_ROOT_HEIGHT | PHC_OBS_UPRIGHT                     */
+  phc_stream_t stream;         /* the discriminator's stream that reads / writes these tensors                   */
+} PhcHostAmp;
+PHC_API int phc_host_step_submit_amp(PhcHostStep* ctx, int32_t slot, const PhcHostStepArgs* args,
+                                     const PhcHostResetArgs* reset /* may be NULL */,
+                                     const PhcHostDeviceOut* dev /* may be NULL */,
+                                     const PhcHostEnvArgs* env /* may be NULL */,
+                                     const PhcHostEpisodeOut* ep /* may be NULL */, const PhcHostAmp* amp, int64_t n);
+PHC_API int phc_host_reset_submit_amp(PhcHostStep* ctx, int32_t slot, const PhcHostStepArgs* args,
+                                      const PhcHostResetArgs* reset, const PhcHostDeviceOut* dev /* may be NULL */,
+                                      const PhcHostEnvArgs* env /* may be NULL */, const PhcHostAmp* amp, int64_t n);
+
 /* ------------------------------------------------------------------------------------
  * RunningNorm statistics                                   policies/running_norm.py:23-34
  * phc_obs_moments accumulates (+=) per-column fp64 sum and sum of squares of x[rows,cols]
