@@ -41,6 +41,8 @@ STATE_INIT_HYBRID = 3
 OBS_LOCAL_ROOT = 1
 OBS_ROOT_HEIGHT = 2
 OBS_UPRIGHT = 4
+OBS_TASK_V7 = 8  # PhcStepArgs / PhcResetArgs.obs_flags: imitation observation v7 rows (216 task floats per future step)
+TASK_OBS_DIM_V7 = 216
 STEP_OBS_FLAGS_SET = 0x80000000
 
 

@@ -28,6 +28,7 @@ namespace phc {
 constexpr int J24 = PHC_NUM_BODIES;
 constexpr int SELF_DIM = PHC_SELF_OBS_DIM;
 constexpr int TASK_DIM = PHC_TASK_OBS_DIM;
+constexpr int TASK_DIM_V7 = 9 * J24;  // 216: [d_pos | d_vel | l_pos] per future step (PHC_OBS_TASK_V7)
 
 static thread_local int g_last_cuda_error = 0;
 
@@ -752,7 +753,10 @@ struct ObsFlags {
   int hcol;        // 1: root height column present (root_height_obs)
   int local_root;  // local_root_obs
   int upright;     // upright (False: remove_base_rot before the heading)
+  int v7;          // PHC_OBS_TASK_V7: the task block of a future step is [d_pos | d_vel | l_pos]
 };
+// floats of one future step's task block
+__host__ __device__ __forceinline__ int task_width(const ObsFlags& f) { return f.v7 ? TASK_DIM_V7 : TASK_DIM; }
 
 // RunningNorm.forward of the rows a kernel writes (policies/running_norm.py:15-20)
 struct NormOut {
@@ -770,7 +774,7 @@ struct ResetParams {
   const int64_t* ids;
   const uint8_t* mask;
   int64_t n;
-  float* obs;  // [n, selfw + 576 T]: rows of the reset envs rewritten
+  float* obs;  // [n, selfw + task_width(of) T]: rows of the reset envs rewritten
   int64_t obs_stride;
   int T;
   float dt;
@@ -1024,6 +1028,25 @@ __device__ __forceinline__ void emit_task_obs(float* tk, int b, Heading hi, cons
   put6<DEF>(tk + 432 + b * 6, o.l_rot);
 }
 
+// one v7 block of 216 floats: the v6 block's [d_pos | d_vel | l_pos] (its columns 0:72, 216:288, 360:432) from the same
+// operations (task_obs_body without the rotation terms, as phc_imitation_obs mode 7)
+__device__ __forceinline__ void emit_task_obs_v7(float* tk, int b, Heading hi, const HeadingRot& hr, Vec3 root_pos, Vec3 pos,
+                                                 Quat rot, Vec3 vel, Vec3 ang, const RefBody& r) {
+  TaskObs o;
+  task_obs_body(hi, hr, root_pos, pos, rot, vel, ang, r, false, o);
+  st3(tk + b * 3, o.d_pos);
+  st3(tk + 72 + b * 3, o.d_vel);
+  st3(tk + 144 + b * 3, o.l_pos);
+}
+
+// the task block of the layout `v7` selects at run time (generic and reset kernels)
+template <bool DEF>
+__device__ __forceinline__ void emit_task(bool v7, float* tk, int b, Heading hi, const HeadingRot& hr, Vec3 root_pos,
+                                          Vec3 pos, Quat rot, Vec3 vel, Vec3 ang, const RefBody& r) {
+  if (v7) emit_task_obs_v7(tk, b, hi, hr, root_pos, pos, rot, vel, ang, r);
+  else emit_task_obs<DEF>(tk, b, hi, hr, root_pos, pos, rot, vel, ang, r);
+}
+
 // emit_self_obs(row) and emit_task_obs(row + SW) of one body, bit for bit, with the vector work paired into fp32x2
 // instructions (phc_math.cuh): the seven heading rotations as (p_b - p_root, v_b) | (d_pos, l_pos) | (d_vel, d_ang)
 // and w_b alone, the two heading products and tan-norms of q_b and the reference rotation together.
@@ -1064,6 +1087,35 @@ __device__ __forceinline__ void emit_obs_paired(float* row, int SW, const ObsFla
   const Quat dg = quat_mul(r.rot, quat_conj(rot));  // task_obs_body's d_rot
   quat_tan_norm(heading_mul_right(heading_mul_left(hi, dg), heading_conj(hi)), t6);
   put6<DEF>(tk + 72 + b * 6, t6);
+}
+
+// emit_self_obs(row) and emit_task_obs_v7(row + SW) of one body, bit for bit, paired as emit_obs_paired does:
+// (p_b - p_root, v_b) | (d_pos, l_pos) | (d_vel, w_b).  No reference rotation is read: the tan-norm of q_b stays scalar.
+template <bool DEF>
+__device__ __forceinline__ void emit_obs_paired_v7(float* row, int SW, const ObsFlags& of, int b, Vec3 root_pos, Heading hi,
+                                                   const HeadingRot& hr, Vec3 pos, Quat rot, Vec3 vel, Vec3 ang,
+                                                   const RefBody& r, float one) {
+  const int h = DEF ? 1 : of.hcol;
+  float* tk = row + SW;
+  const Vec3x2 pv = heading_rotate2(hr, pack3(pos - root_pos, vel));
+  const Vec3x2 dl = heading_rotate2(hr, sub3x2(pack3(r.pos, r.pos), pack3(pos, root_pos), one));
+  const Vec3x2 dw = heading_rotate2(hr, pack3(r.vel - vel, ang));
+  if (b == 0) {
+    if (h) row[0] = root_pos.z;
+  } else {
+    st3(row + h + (b - 1) * 3, lane0(pv));
+  }
+  st3(row + h + 213 + b * 3, lane1(pv));
+  st3(row + h + 285 + b * 3, lane1(dw));
+  st3(tk + b * 3, lane0(dl));
+  st3(tk + 72 + b * 3, lane0(dw));
+  st3(tk + 144 + b * 3, lane1(dl));
+  float t6[6];
+  if (!DEF && b == 0 && !of.local_root)
+    quat_tan_norm(heading_source(rot, of.upright), t6);
+  else
+    quat_tan_norm(heading_mul_left(hi, rot), t6);
+  put6<DEF>(row + h + 69 + b * 6, t6);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -1419,8 +1471,9 @@ __global__ void __launch_bounds__(EPB* J24) step_kernel(const StepParams p) {
   const Heading hi = {S.hz[e], S.hw[e]};
   const HeadingRot hr = heading_rot(hi);
   const int SW = p.selfw;           // 358 with the root height column, 357 without
-  const int RW = SW + TASK_DIM;     // floats of a staged row (self obs + one task block)
-  const int W = SW + TASK_DIM * T;
+  const int TW = task_width(p.of);  // 576 (v6) or 216 (v7)
+  const int RW = SW + TW;           // floats of a staged row (self obs + one task block)
+  const int W = SW + TW * T;
 
   for (int q = 1; q <= T; ++q) {
     cp_async_wait_all();
@@ -1432,16 +1485,16 @@ __global__ void __launch_bounds__(EPB* J24) step_kernel(const StepParams p) {
     float* row = S.buf + e * STAGE_FLOATS;  // staged rows keep the 934-float pitch whatever the flags
     if (valid) {
       if (q == 1) emit_self_obs<false>(row, p.of, b, root_pos, hi, hr, pos, rot, vel, ang);
-      emit_task_obs<false>(row + SW, b, hi, hr, root_pos, pos, rot, vel, ang, r);
+      emit_task<false>(p.of.v7, row + SW, b, hi, hr, root_pos, pos, rot, vel, ang, r);
     }
     __syncthreads();  // stage complete
 
-    // stream the staged columns out: q == 1 -> cols [0, RW), else [SW + 576(q-1), +576)
+    // stream the staged columns out: q == 1 -> cols [0, RW), else [SW + TW(q-1), +TW)
     const int s_off = q == 1 ? 0 : SW;
-    const int s_len = q == 1 ? RW : TASK_DIM;
-    const int64_t c_off = q == 1 ? 0 : SW + (int64_t)TASK_DIM * (q - 1);
+    const int s_len = q == 1 ? RW : TW;
+    const int64_t c_off = q == 1 ? 0 : SW + (int64_t)TW * (q - 1);
     if (p.obs_vec2 && (SW & 1) == 0) {
-      if (T == 1 && p.obs_stride == STAGE_FLOATS && !p.env_mask) {  // rows of the block are one contiguous span
+      if (T == 1 && RW == STAGE_FLOATS && p.obs_stride == STAGE_FLOATS && !p.env_mask) {  // rows of the block are one contiguous span
         float2* dst = reinterpret_cast<float2*>(p.obs + env0 * STAGE_FLOATS);
         const float2* src = reinterpret_cast<const float2*>(S.buf);
         for (int i = tid; i < nvalid * (STAGE_FLOATS / 2); i += NT) dst[i] = src[i];
@@ -1500,7 +1553,7 @@ __global__ void __launch_bounds__(EPB* J24) step_kernel(const StepParams p) {
 
 // the columns of an observation row that thread `b` of an env writes: f(first column, count)
 template <class F>
-__device__ __forceinline__ void for_owned_columns(int b, int hcol, int SW, int T, F f) {
+__device__ __forceinline__ void for_owned_columns(int b, int hcol, int SW, int T, bool v7, F f) {
   if (b == 0) {
     if (hcol) f(0, 1);
   } else {
@@ -1510,6 +1563,13 @@ __device__ __forceinline__ void for_owned_columns(int b, int hcol, int SW, int T
   f(hcol + 213 + b * 3, 3);
   f(hcol + 285 + b * 3, 3);
   for (int q = 1; q <= T; ++q) {
+    if (v7) {
+      const int base = SW + TASK_DIM_V7 * (q - 1);
+      f(base + b * 3, 3);
+      f(base + 72 + b * 3, 3);
+      f(base + 144 + b * 3, 3);
+      continue;
+    }
     const int base = SW + TASK_DIM * (q - 1);
     f(base + b * 3, 3);
     f(base + 72 + b * 6, 6);
@@ -1550,10 +1610,10 @@ __global__ void __launch_bounds__(K7_EPB* J24) reset_obs_kernel(const ResetParam
   const Heading hi = {s_root[e][3], s_root[e][4]};
   const HeadingRot hr = heading_rot(hi);
   float* row = p.obs + env * p.obs_stride;
-  const int SW = 357 + p.of.hcol, W = SW + TASK_DIM * p.T;
+  const int SW = 357 + p.of.hcol, TW = task_width(p.of), W = SW + TW * p.T;
   double* mom = p.moments ? p.moments + (int64_t)(blockIdx.x % p.moment_buckets) * 2 * W : nullptr;
   if (mom && p.moments_mode == 2) {  // the step that flagged this env counted the row it wrote: take it out again
-    for_owned_columns(b, p.of.hcol, SW, p.T, [&](int c0, int n) {
+    for_owned_columns(b, p.of.hcol, SW, p.T, p.of.v7, [&](int c0, int n) {
       for (int c = c0; c < c0 + n; ++c) {
         const double x = (double)__ldcg(row + c);
         atomicAdd(mom + c, -x);
@@ -1573,10 +1633,10 @@ __global__ void __launch_bounds__(K7_EPB* J24) reset_obs_kernel(const ResetParam
     // loading the t + dt frames together with the scatter's (before its stores) was measured: 10 more registers,
     // 3 instead of 4 blocks per SM — 0.6 us faster per loop step at 4 % flagged, 2.5 us slower at 31 %; not kept
     const RefBody r = reset_ref_body(p.L, q, p.dt, o.t, o.len, o.nf, o.mdt, o.st, b, o.soff, o.g0, o.g1, o.g2);
-    emit_task_obs<false>(row + SW + (int64_t)TASK_DIM * (q - 1), b, hi, hr, root_pos, o.pos, o.rot, o.vel, o.ang, r);
+    emit_task<false>(p.of.v7, row + SW + (int64_t)TW * (q - 1), b, hi, hr, root_pos, o.pos, o.rot, o.vel, o.ang, r);
   }
   if (mom || p.norm.out) {  // the thread's own stores above are visible to it
-    for_owned_columns(b, p.of.hcol, SW, p.T, [&](int c0, int n) {
+    for_owned_columns(b, p.of.hcol, SW, p.T, p.of.v7, [&](int c0, int n) {
       for (int c = c0; c < c0 + n; ++c) {
         const float v = row[c];
         if (mom) {
@@ -1722,7 +1782,7 @@ __device__ __forceinline__ void put13(float* d, Vec3 pos, Quat rot, Vec3 vel, Ve
   d[10] = ang.x, d[11] = ang.y, d[12] = ang.z;
 }
 
-template <int EPB, bool DEF>
+template <int EPB, bool DEF, bool V7>
 __device__ __forceinline__ void reset_in_step(const StepParams& p, FastSmem<EPB>& S, int f, int64_t env) {
   static_assert(EPB * J24 == 96, "three warps, one role each");
   const int w = threadIdx.x >> 5, b = threadIdx.x & 31;
@@ -1767,13 +1827,15 @@ __device__ __forceinline__ void reset_in_step(const StepParams& p, FastSmem<EPB>
   const Vec3 root_pos = {S.nroot[f][0], S.nroot[f][1], S.nroot[f][2]};
   const Heading hi = {S.nroot[f][3], S.nroot[f][4]};
   const HeadingRot hr = heading_rot(hi);
-  float* row = S.frames + f * (SW + TASK_DIM);
+  float* row = S.frames + f * (SW + (V7 ? TASK_DIM_V7 : TASK_DIM));
   if (w == 0) {
     emit_self_obs<DEF>(row, p.of, b, root_pos, hi, hr, own.pos, own.rot, own.vel, own.ang);
   } else {
     const float* d = S.sim + f * ROW13 + b * 13;
-    emit_task_obs<DEF>(row + SW, b, hi, hr, root_pos, Vec3{d[0], d[1], d[2]}, Quat{d[3], d[4], d[5], d[6]},
-                       Vec3{d[7], d[8], d[9]}, Vec3{d[10], d[11], d[12]}, own);
+    const Vec3 pos{d[0], d[1], d[2]}, vel{d[7], d[8], d[9]}, ang{d[10], d[11], d[12]};
+    const Quat rot{d[3], d[4], d[5], d[6]};
+    if constexpr (V7) emit_task_obs_v7(row + SW, b, hi, hr, root_pos, pos, rot, vel, ang, own);
+    else emit_task_obs<DEF>(row + SW, b, hi, hr, root_pos, pos, rot, vel, ang, own);
   }
 }
 
@@ -1784,7 +1846,9 @@ __device__ __forceinline__ void reset_in_step(const StepParams& p, FastSmem<EPB>
 // PLAIN: compiled without the per-step options — power reward, ref_dof_pos, mpjpe, eval mode (use_mean), RunningNorm
 // moments, rew_out, progress_mirror — and with goff set: the headline step issues their run-time branches in its
 // issue-bound phases, and the eval-mode selection arrays are most of its stack frame
-template <int EPB, int MINB, bool NORM = false, bool EP = false, bool RESET = false, bool DEF = true, bool PLAIN = false>
+// V7: the v7 task block (PHC_OBS_TASK_V7, 216 floats): rows of SW + 216 floats in the stage, the stores and the moments
+template <int EPB, int MINB, bool NORM = false, bool EP = false, bool RESET = false, bool DEF = true, bool PLAIN = false,
+          bool V7 = false>
 __global__ void __launch_bounds__(EPB* J24, MINB) step_fast_kernel(const __grid_constant__ StepParams p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   FastSmem<EPB>& S = *reinterpret_cast<FastSmem<EPB>*>(smem_raw);
@@ -1792,6 +1856,7 @@ __global__ void __launch_bounds__(EPB* J24, MINB) step_fast_kernel(const __grid_
   static_assert(4 * EPB <= 32, "reductions run on one warp");
   static_assert(!NORM || DEF, "the normaliser epilogue is laid out for the default 934-float rows");
   static_assert(!PLAIN || (!NORM && !EP && !RESET && DEF), "the plain step carries none of the epilogues");
+  static_assert(!NORM || !V7, "the normaliser epilogue is laid out for v6 rows");
   const bool use_mean = !PLAIN && p.use_mean;
   const bool dof_force = !PLAIN && p.dof_force;
   const bool ref_dof_pos = !PLAIN && p.ref_dof_pos;
@@ -2102,15 +2167,18 @@ __global__ void __launch_bounds__(EPB* J24, MINB) step_fast_kernel(const __grid_
 
   // ---- phase 2: observations into the stage ---------------------------------------------------
   const int SW = DEF ? SELF_DIM : p.selfw;  // 358 with the root height column, 357 without
-  const int RW = SW + TASK_DIM;             // floats of a staged row
+  const int RW = SW + (V7 ? TASK_DIM_V7 : TASK_DIM);  // floats of a staged row
   if (valid && !(RESET && my_rst)) {
     const Vec3 root_pos = {S.sim[e * ROW13 + 0], S.sim[e * ROW13 + 1], S.sim[e * ROW13 + 2]};
     const Heading hi = {S.hz[e], S.hw[e]};
     const HeadingRot hr = heading_rot(hi);
     float* row = S.frames + e * RW;
     if constexpr (RESET) {
-      emit_self_obs<DEF>(row, p.of, b, root_pos, hi, hr, pos, rot, vel, ang);     // common.py:23-103
-      emit_task_obs<DEF>(row + SW, b, hi, hr, root_pos, pos, rot, vel, ang, r1);  // common.py:106-176
+      emit_self_obs<DEF>(row, p.of, b, root_pos, hi, hr, pos, rot, vel, ang);  // common.py:23-103
+      if constexpr (V7) emit_task_obs_v7(row + SW, b, hi, hr, root_pos, pos, rot, vel, ang, r1);
+      else emit_task_obs<DEF>(row + SW, b, hi, hr, root_pos, pos, rot, vel, ang, r1);  // common.py:106-176
+    } else if constexpr (V7) {
+      emit_obs_paired_v7<DEF>(row, SW, p.of, b, root_pos, hi, hr, pos, rot, vel, ang, r1, p.one);
     } else {
       emit_obs_paired<DEF>(row, SW, p.of, b, root_pos, hi, hr, pos, rot, vel, ang, r1, p.one);  // common.py:23-176
     }
@@ -2119,7 +2187,7 @@ __global__ void __launch_bounds__(EPB* J24, MINB) step_fast_kernel(const __grid_
     if (rst_mask) {  // the rows of the flagged envs, from their new state (one env at a time, the whole block on it)
 #pragma unroll 1
       for (int i = 0; i < EPB; ++i)
-        if (rst_mask >> i & 1) reset_in_step<EPB, DEF>(p, S, i, env0 + i);
+        if (rst_mask >> i & 1) reset_in_step<EPB, DEF, V7>(p, S, i, env0 + i);
     }
   }
   fence_proxy_async();  // stage writes -> visible to the bulk-store engine
@@ -3894,6 +3962,7 @@ static int64_t g_trace_launch = 0;
 
 static ObsFlags obs_flags_from(uint32_t f) {
   ObsFlags of;
+  of.v7 = (f & PHC_OBS_TASK_V7) ? 1 : 0;  // whatever the self-obs bits say
   if (!(f & PHC_STEP_OBS_FLAGS_SET) && (f & 7u) == 0) f = PHC_OBS_LOCAL_ROOT | PHC_OBS_ROOT_HEIGHT | PHC_OBS_UPRIGHT;
   of.hcol = (f & PHC_OBS_ROOT_HEIGHT) ? 1 : 0;
   of.local_root = (f & PHC_OBS_LOCAL_ROOT) ? 1 : 0;
@@ -3924,7 +3993,7 @@ static int reset_fill(const PhcLib* lib, const PhcResetArgs* a, int64_t n, Reset
   if ((a->dof_pos && !lib->d.lrs) || (a->dof_vel && !lib->d.dvs) || (a->ref_dof_pos && !lib->d.lrs)) return PHC_ERR_NULL;
   if (a->time_steps < 1 || a->time_steps > PHC_MAX_TIME_STEPS) return PHC_ERR_SHAPE;
   const ObsFlags of = obs_flags_from(a->obs_flags);
-  const int64_t W = 357 + of.hcol + (int64_t)TASK_DIM * a->time_steps;
+  const int64_t W = 357 + of.hcol + (int64_t)task_width(of) * a->time_steps;
   if (a->obs_stride < W || ((a->dof_pos || a->dof_vel) && a->dof_elem_stride < 1)) return PHC_ERR_SHAPE;
   if (a->obs_norm && (!a->norm_mean || !a->norm_var)) return PHC_ERR_NULL;
   if (a->obs_norm && (a->obs_norm_stride < W || !(a->norm_clip > 0.0f))) return PHC_ERR_SHAPE;
@@ -3990,7 +4059,7 @@ static int step_fill_params(const PhcLib* lib, const PhcStepArgs* a, int64_t n, 
   if (a->time_steps < 1 || a->time_steps > PHC_MAX_TIME_STEPS) return PHC_ERR_SHAPE;
   p.of = obs_flags_from(a->obs_flags);
   p.selfw = 357 + p.of.hcol;
-  const int64_t W = p.selfw + (int64_t)TASK_DIM * a->time_steps;
+  const int64_t W = p.selfw + (int64_t)task_width(p.of) * a->time_steps;
   if (a->obs_stride < W || a->reward_raw_stride < 4) return PHC_ERR_SHAPE;
   p.rew_out = a->rew_out;
   p.reset_out = a->reset_out;
@@ -4013,7 +4082,8 @@ static int step_fill_params(const PhcLib* lib, const PhcStepArgs* a, int64_t n, 
         r->global_offset != a->global_offset || r->time_steps != a->time_steps || r->dt != a->dt)
       return PHC_ERR_SHAPE;
     const ObsFlags rf = obs_flags_from(r->obs_flags);
-    if (rf.hcol != p.of.hcol || rf.local_root != p.of.local_root || rf.upright != p.of.upright) return PHC_ERR_SHAPE;
+    if (rf.hcol != p.of.hcol || rf.local_root != p.of.local_root || rf.upright != p.of.upright || rf.v7 != p.of.v7)
+      return PHC_ERR_SHAPE;
     ResetParams rp;
     rc = reset_fill(lib, r, n, rp);
     if (rc) return rc;
@@ -4244,11 +4314,13 @@ int step_fused_mirrored(const PhcLib* lib, const PhcStepArgs* args, int64_t n, p
   init_options();
   // fast path: T == 1, AoS sim tensor (16-B aligned rows), dense 16-B aligned obs_buf.  Any self-obs flag combination
   // runs on it (rows of 933 floats without the height column: four of them are still a multiple of 16 B); the fused
-  // normaliser epilogue is laid out for the default 934-float rows only.
+  // normaliser epilogue is laid out for the default 934-float rows only.  v7 rows (574 floats) run on it with the default
+  // self-obs flags and without the normaliser; anything else with v7 runs on the generic kernel.
   const bool def = default_obs_flags(p.of);
-  const int RW = p.selfw + TASK_DIM;
+  const bool v7 = p.of.v7 != 0;
+  const int RW = p.selfw + task_width(p.of);
   const bool fast = !g_force_generic && p.T == 1 && p.aos && p.L.packed && p.obs_stride == RW &&
-                    ((uintptr_t)p.obs & 15) == 0 &&
+                    ((uintptr_t)p.obs & 15) == 0 && (!v7 || (def && !p.obs_norm)) &&
                     (!p.obs_norm || (def && p.obs_norm_stride == STAGE_FLOATS &&
                                      ((uintptr_t)p.obs_norm & (p.norm_bf16 ? 3 : 15)) == 0));
   static bool attr_gen[64] = {};
@@ -4257,7 +4329,7 @@ int step_fused_mirrored(const PhcLib* lib, const PhcStepArgs* args, int64_t n, p
   // (+ power reward, flag / reward copies); the optional epilogues stay with K6-fast.
   static bool attr_persist[3][64] = {};
   static int sm_count[64] = {};
-  const bool persist = fast && def && g_persist != 0 &&
+  const bool persist = fast && def && !v7 && g_persist != 0 &&
                        (g_persist >= 2 || p.n >= (p.moments ? g_persist_min_moments : g_persist_min)) && !p.obs_norm &&
                        !p.ep_returns && !p.reset_on && !p.ref_dof_pos && !p.trace && lib->tile_counters &&
                        !(args->flags & PHC_STEP_MAPPED_HOST_IO);
@@ -4311,12 +4383,13 @@ int step_fused_mirrored(const PhcLib* lib, const PhcStepArgs* args, int64_t n, p
     // previous step's blocks exit and speculate on a third candidate
     const int64_t grid = (p.n + 3) / 4;
     p.spec4_blocks = p.first_wave_blocks > grid ? (int)(p.first_wave_blocks - grid) : 0;
-    // instantiations <EPB, blocks/SM, NORM, EP, RESET, DEF, PLAIN>: <4, 8> carries none of the optional epilogues,
+    // instantiations <EPB, blocks/SM, NORM, EP, RESET, DEF, PLAIN, V7>: <4, 8> carries none of the optional epilogues,
     // the PLAIN one none of the per-step options either; the RESET ones are compiled with the bookkeeping too (both
-    // are switched at run time inside); one catch-all for non-default self-obs flags
+    // are switched at run time inside); one catch-all for non-default self-obs flags.  v7: a plain one and one with
+    // every option, the bookkeeping and the in-step reset switched at run time.
     const bool plain = !p.dof_force && !p.ref_dof_pos && !p.mpjpe && !p.use_mean && !p.moments && !p.rew_out &&
                        !p.progress_mirror && p.goff;
-    static bool attr[8][64] = {};
+    static bool attr[10][64] = {};
     const bool pdl = g_pdl != 0;
     constexpr size_t SM = sizeof(FastSmem<4>);
     // the moments epilogue leaves as TMA bulk reductions when the accumulators are 16-B aligned
@@ -4328,7 +4401,11 @@ int step_fused_mirrored(const PhcLib* lib, const PhcStepArgs* args, int64_t n, p
     StepParams pk = p;
     if (reset_after) pk.reset_on = 0;
     pk.ep_block0 = (int)(env0 / 4);
-    if (!def) rc = launch_step(step_fast_kernel<4, 8, false, true, true, false>, SM, 4, pk, stream, &attr[6][dev], pdl);
+    if (v7 && plain && !in_kernel && !p.ep_returns)
+      rc = launch_step(step_fast_kernel<4, 8, false, false, false, true, true, true>, SM, 4, pk, stream, &attr[8][dev], pdl);
+    else if (v7)
+      rc = launch_step(step_fast_kernel<4, 8, false, true, true, true, false, true>, SM, 4, pk, stream, &attr[9][dev], pdl);
+    else if (!def) rc = launch_step(step_fast_kernel<4, 8, false, true, true, false>, SM, 4, pk, stream, &attr[6][dev], pdl);
     else if (in_kernel) {
       if (p.obs_norm) rc = launch_step(step_fast_kernel<4, 8, true, true, true>, SM, 4, pk, stream, &attr[5][dev], pdl);
       else rc = launch_step(step_fast_kernel<4, 8, false, true, true>, SM, 4, pk, stream, &attr[4][dev], pdl);
@@ -4344,7 +4421,7 @@ int step_fused_mirrored(const PhcLib* lib, const PhcStepArgs* args, int64_t n, p
   float* raw_post = nullptr;  // the mapped reward_raw rows, posted by the bookkeeping (ep_raw)
   if (ep_raw) raw_post = p.raw, p.raw = ep_raw;
   // T > 1 on the AoS tensor + packed table: the pipelined TMA kernel
-  const bool multi = !g_force_generic && p.T > 1 && p.aos && p.L.packed && p.obs_vec2 && !p.obs_norm && def &&
+  const bool multi = !g_force_generic && p.T > 1 && p.aos && p.L.packed && p.obs_vec2 && !p.obs_norm && def && !v7 &&
                      !(args->flags & PHC_STEP_MAPPED_HOST_IO);
   static bool attr_multi[64] = {}, attr_multi2[64] = {};
   // two query groups per block (measured: 2048 envs 21.6 -> 18.3 us, 4096 envs 43.7 -> 37.2, 16384 envs 128.2 -> 127.5)

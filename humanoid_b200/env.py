@@ -28,6 +28,7 @@ from .common import (
     compute_humanoid_im_reset,
     compute_humanoid_observations_smpl_max,
     compute_imitation_observations_v6,
+    compute_imitation_observations_v7,
     compute_imitation_reward,
 )
 from .motion_lib import MotionLib
@@ -111,7 +112,10 @@ class HumanoidPHC:
         root_height_obs: bool = True,  # config.py:122
         has_upright_start: bool = True,  # config.py:61
         res_action: bool = False,  # config.py (False by default, humanoid_phc.py:1219)
+        obs_v: int = 6,  # imitation observation version (config obs_v): 6, or 7 = the [d_pos | d_vel | l_pos] columns of v6
     ):
+        if obs_v not in (6, 7):
+            raise ValueError(f"obs_v must be 6 or 7, got {obs_v!r}")
         dev = torch.device(device)
         if dev.type != "cuda":
             raise _cabi.PhcError("HumanoidPHC needs a CUDA device (there is no CPU path)")
@@ -134,7 +138,9 @@ class HumanoidPHC:
         self._obs_flags = (
             (_cabi.OBS_LOCAL_ROOT if self.local_root_obs else 0) | (_cabi.OBS_ROOT_HEIGHT if self.root_height_obs else 0)
             | (_cabi.OBS_UPRIGHT if self.has_upright_start else 0) | _cabi.STEP_OBS_FLAGS_SET
+            | (_cabi.OBS_TASK_V7 if obs_v == 7 else 0)
         )  # fmt: skip
+        self.obs_v = obs_v
         self.res_action = bool(res_action)
 
         N = num_envs
@@ -151,7 +157,8 @@ class HumanoidPHC:
         self._pd_action_scale = torch.ones(self.num_dof, dtype=torch.float32, device=dev)
 
         # env buffers (humanoid_phc.py:556-597)
-        self.num_obs = (_cabi.SELF_OBS_DIM - (0 if self.root_height_obs else 1)) + _cabi.TASK_OBS_DIM * self.time_steps  # :461-467
+        task_dim = _cabi.TASK_OBS_DIM_V7 if obs_v == 7 else _cabi.TASK_OBS_DIM
+        self.num_obs = (_cabi.SELF_OBS_DIM - (0 if self.root_height_obs else 1)) + task_dim * self.time_steps  # :461-467
         self.obs_buf = torch.zeros((N, self.num_obs), dtype=torch.float32, device=dev)
         self.rew_buf = torch.zeros(N, dtype=torch.float32, device=dev)  # (:560 calls the torch module; fixed)
         self.reward_raw = torch.zeros((N, 5), dtype=torch.float32, device=dev)  # 4 + power slot (:562-569)
@@ -906,7 +913,8 @@ class HumanoidPHC:
                 self.ref_dof_pos[:] = refs[0]["dof_pos"]
             else:
                 self.ref_dof_pos[env_ids] = refs[0]["dof_pos"]
-        return compute_imitation_observations_v6(
+        task_obs = compute_imitation_observations_v7 if self.obs_v == 7 else compute_imitation_observations_v6
+        return task_obs(
             pos[..., 0, :], rot[..., 0, :], pos, rot, vel, ang,
             stack("rg_pos"), stack("rb_rot"), stack("body_vel"), stack("body_ang_vel"), self.time_steps,
             self.has_upright_start,

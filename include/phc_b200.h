@@ -148,6 +148,12 @@ PHC_API int phc_motion_state(const PhcLib* lib, const int64_t* motion_ids, const
 #define PHC_OBS_LOCAL_ROOT 1u   /* local_root_obs   */
 #define PHC_OBS_ROOT_HEIGHT 2u  /* root_height_obs  */
 #define PHC_OBS_UPRIGHT 4u      /* upright          */
+/* PhcStepArgs / PhcResetArgs.obs_flags only (phc_self_obs_smpl_max and phc_amp_obs ignore it): the task block of each
+ * future step is the imitation observation v7 = [d_pos | d_vel | l_pos], 216 floats, bitwise the v6 columns 0:72,
+ * 216:288 and 360:432 of that step (compute_imitation_observations_v7, phc_imitation_obs mode 7).  A row is then
+ * selfw + 216 T floats (selfw = 358, or 357 without the height column); without the bit, selfw + 576 T (v6).  Applies
+ * whether or not PHC_STEP_OBS_FLAGS_SET is set: the three self-obs bits at 0 still mean the env's defaults. */
+#define PHC_OBS_TASK_V7 8u
 PHC_API int phc_self_obs_smpl_max(const PhcBodyState* body, int64_t n, uint32_t flags, float* out,
                           int64_t out_stride, phc_stream_t stream);
 
@@ -234,7 +240,7 @@ typedef struct PhcStepArgs {
   int32_t time_steps;                    /* future reference frames T (1 in the env)    */
   float dt;                              /* isaac_base.dt = 2*(1/60)    isaacgym_env.py:41 */
   PhcRewardSpec rwd;
-  float* obs_buf;                        /* [n, 358+576*T]              humanoid_phc.py:557 */
+  float* obs_buf;                        /* [n, row width W]: W = selfw + 576 T (v6) or selfw + 216 T (PHC_OBS_TASK_V7) */
   int64_t obs_stride;
   float* rew_buf;                        /* [n]                         humanoid_phc.py:560 */
   float* reward_raw;                     /* [n, >=4]                    humanoid_phc.py:562 */
@@ -252,23 +258,23 @@ typedef struct PhcStepArgs {
   int64_t dof_vel_elem_stride;           /* 2 for the reference's (pos, vel) interleaved state */
   float rew_power_coef;                  /* config.py rew_power_coef                          */
   int32_t power_col;                     /* column of reward_raw that receives r (4)          */
-  double* obs_moments;                   /* NULL, or [2*(358+576*T)] fp64: per-column sum
+  double* obs_moments;                   /* NULL, or [2*W] fp64 (row width W): per-column sum
                                             and sum of squares accumulated (+=) for
                                             RunningNorm.update           running_norm.py:23 */
   /* RunningNorm.forward fused into the obs epilogue (policies/running_norm.py:15-20), off when
    * obs_norm is NULL:  obs_norm = clamp((obs - mean) / sqrt(var + epsilon), -clip, clip), written
    * IN ADDITION to obs_buf (the experience buffer keeps the raw rows, RunningNorm.update needs them) */
-  float* obs_norm;                       /* NULL or [n, 358+576*T] fp32 (bf16 with PHC_STEP_OBS_NORM_BF16) */
+  float* obs_norm;                       /* NULL or [n, row width W] fp32 (bf16 with PHC_STEP_OBS_NORM_BF16) */
   int64_t obs_norm_stride;
-  const float* norm_mean;                /* [358+576*T] running_mean                         */
-  const float* norm_var;                 /* [358+576*T] running_var                          */
+  const float* norm_mean;                /* [W] running_mean (row width W)                   */
+  const float* norm_var;                 /* [W] running_var                                  */
   float norm_epsilon;                    /* 1e-5 in the reference                            */
   float norm_clip;                       /* 10.0 in the reference                            */
   float* mpjpe;                          /* NULL or [n]: extras["mpjpe"] of eval mode, the mean over all
                                             24 bodies of |rigid_body_pos - ref rg_pos| at the reward
                                             time                              humanoid_phc.py:159-167 */
-  int32_t obs_moments_buckets;           /* 0 / 1: obs_moments is one [2*(358+576*T)] accumulator.  B > 1: obs_moments is
-                                            [B][2*(358+576*T)] and block b adds into bucket b % B — fp64 atomics on ONE
+  int32_t obs_moments_buckets;           /* 0 / 1: obs_moments is one [2*W] accumulator (row width W).  B > 1: obs_moments is
+                                            [B][2*W] and block b adds into bucket b % B — fp64 atomics on ONE
                                             address serialise (~30 ns each), so 1024 blocks on a single accumulator cost
                                             35 us per 4096-env step; 32 buckets make the epilogue free.  The consumer
                                             sums the buckets (phc_obs_moments_fold).                                  */
@@ -310,7 +316,8 @@ typedef struct PhcStepArgs {
   /* self-observation flags of compute_humanoid_observations_smpl_max (humanoid_phc.py:963-998, config.py:61-69):
    * PHC_OBS_LOCAL_ROOT | PHC_OBS_ROOT_HEIGHT | PHC_OBS_UPRIGHT.  0 means the env's defaults (all three); any other
    * combination changes the self-obs columns (no height column: 357 + 576 T floats per row) and, for !upright, the
-   * heading both observations are expressed in.  PHC_STEP_OBS_FLAGS_SET marks the field as given.                   */
+   * heading both observations are expressed in.  PHC_STEP_OBS_FLAGS_SET marks the field as given.  PHC_OBS_TASK_V7
+   * selects the v7 task block (row width selfw + 216 T); auto_reset->obs_flags must agree with it (PHC_ERR_SHAPE).   */
   uint32_t obs_flags;
 } PhcStepArgs;
 #define PHC_STEP_OBS_FLAGS_SET 0x80000000u
@@ -320,7 +327,9 @@ typedef struct PhcStepArgs {
  * warp-specialised kernel, whose blocks draw env tiles from a device-side counter owned by `lib` (256 counter slots used
  * round robin, each left zero by the launch that used it: launches of one PhcLib may overlap on different streams as
  * long as fewer than 256 of them are in flight or captured in concurrently replayed graphs); T > 1 runs the pipelined
- * multi-query kernel; anything else (strided views, non-default flags with T > 1) the generic kernel. */
+ * multi-query kernel; anything else (strided views, non-default flags with T > 1) the generic kernel.  v7 rows
+ * (PHC_OBS_TASK_V7) run on the single-wave kernel at T == 1 with the default self flags and no obs_norm, at any n;
+ * otherwise on the generic kernel. */
 PHC_API int phc_step_fused(const PhcLib* lib, const PhcStepArgs* args, int64_t n, phc_stream_t stream);
 
 /* ------------------------------------------------------------------------------------
@@ -368,22 +377,22 @@ typedef struct PhcResetArgs {
   int32_t flag_test;                      /* motion_times[:] = 0         humanoid_phc.py:856  */
   int32_t time_steps;                     /* T of the observation                             */
   float dt;
-  float* obs_buf;                         /* [n, 358+576*T]: rows of the selected envs rewritten */
+  float* obs_buf;                         /* [n, row width W]: rows of the selected envs rewritten */
   int64_t obs_stride;
   /* ---- ABI 3: keep the step's fused epilogues consistent with the rows a reset rewrites ------------------------- */
   float* obs_norm;                        /* NULL, or the normalised copy of obs_buf (PhcStepArgs.obs_norm): the rows of
                                              the selected envs are rewritten too          policies/running_norm.py:15-20 */
   int64_t obs_norm_stride;
-  const float* norm_mean;                 /* [358+576*T] */
-  const float* norm_var;                  /* [358+576*T] */
+  const float* norm_mean;                 /* [W] */
+  const float* norm_var;                  /* [W] */
   float norm_epsilon, norm_clip;
   int32_t obs_norm_bf16;                  /* obs_norm holds bfloat16 rows */
   int32_t obs_moments_mode;               /* 0: moments untouched; 1: the new rows are ADDED (an initial reset: the rows
                                              were never counted); 2: the old rows are REPLACED (subtract old, add new:
                                              the step that flagged the envs had counted the rows it wrote)             */
-  double* obs_moments;                    /* NULL, or [buckets][2*(358+576*T)] fp64 accumulators as in PhcStepArgs      */
+  double* obs_moments;                    /* NULL, or [buckets][2*W] fp64 accumulators as in PhcStepArgs                */
   int32_t obs_moments_buckets;
-  uint32_t obs_flags;                     /* as PhcStepArgs.obs_flags (0 = the env's defaults)                          */
+  uint32_t obs_flags;                     /* as PhcStepArgs.obs_flags (0 = the env's defaults; PHC_OBS_TASK_V7: v7 rows) */
   float* ref_dof_pos;                     /* NULL or [n, 69]: _compute_task_obs(env_ids) of the reset keeps the dof_pos of
                                              the query at t + dt for res_action            humanoid_phc.py:1115-1120 */
   int64_t ref_dof_pos_stride;
